@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""bench.py - LS operator applies/s on B200 (driver contract, see the task statement).
+"""bench.py - LS operator applies/s on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 2048]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 2048] [--dump-outputs DIR]
 
 Workload at every N: BASELINE.json configs[1] at its headline size - the 2-D Greengard-Vico
 Lippmann-Schwinger operator apply on a 2048 x 2048 grid (padded 8192 x 8192), 10 points per
@@ -27,6 +27,9 @@ single-GPU time measured in the same run and the strong-scaling efficiency), `gm
 `krylov_kernels`, `device_peaks` (FP64 and copy microbenchmarks run live).
 `--impl reference` times the CPU path alone (the reference is Julia; Julia/FFTW are not in
             this image, so the oracle port is the reference arm - see DESIGN.md).
+`--dump-outputs DIR`: after the timed steps, writes the apply's output y = M * b of the last timed step as
+            DIR/y.npy (rank 0's replica; see dump_outputs for the format), so that two builds - or the two
+            arms - can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -51,6 +54,19 @@ os.environ.setdefault("DUCC0_NUM_THREADS", str(os.cpu_count() or 1))
 
 METRIC = "ls_operator_applies_per_s_2d"
 UNIT = "applies/s"
+DUMP_MAX_POINTS = 1 << 21           # 2^21 complex values = 32 MiB of float64 (re, im) pairs
+
+
+def dump_outputs(outdir, outputs):
+    """Writes each complex output vector as outdir/<name>.npy: float64 of shape (points, 2), columns (re, im).  A vector
+    longer than DUMP_MAX_POINTS is reduced to the entries at a fixed sample of indices (seeded, sorted), the same in
+    every run of the same size."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, y in outputs.items():
+        y = np.ascontiguousarray(y, dtype=np.complex128)
+        if y.size > DUMP_MAX_POINTS:
+            y = y[np.sort(np.random.default_rng(0).choice(y.size, DUMP_MAX_POINTS, replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), y.view(np.float64).reshape(-1, 2))
 
 
 def measured_peaks():
@@ -152,8 +168,10 @@ def run_reference(args, rank, world):
         O.fastconvolution(M, b)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.fastconvolution(M, b)
+        y = O.fastconvolution(M, b)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": y})
     val = args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
@@ -621,15 +639,16 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip everything but the headline apply")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step to DIR/y.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 20      # bounded sample: ~1-2 s of host CPU work per apply at 2048^2
         run_reference(args, rank, world)
         return
 
@@ -690,6 +709,8 @@ def main():
     phase_ms, phase_cnt = M.profile_read(3)
     M.profile_enable(False)
     launches = M.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"y": dy.to_host()})
     # the timed region lasts milliseconds, an nvidia-smi query ~0.1 s: keep the GPU under the same load (untimed applies)
     # for ~1.5 s so that the sampler sees the clocks / throttle reasons this workload runs at
     if rank == 0:
