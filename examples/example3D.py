@@ -5,12 +5,13 @@ The shipped 3-D example: h = 1/48, k = 1/h, smooth Gaussian bump, Greengard_Vico
 general-size path (Bluestein lines); powers of two in {64, 128, 256, 512} take the pruned fast path with
 the spectrum generated on the device.
 
-    python examples/example3D.py [--n 48] [--precond]
+    python examples/example3D.py [--n 48] [--precond [--msp {host,gpu}]]
 
 --precond builds the sparsifying preconditioner of example3D.jl:56-67 (27-point As and
 Mapproxsp = As + k^2 AG diag(nu)) from 343 unit-vector applies on the GPU operator
-(fast_solver_lippmann_schwinger_b200.sparsifier), keeps As on the GPU and factorises Mapproxsp on the host
-(SuperLU here, MKL PARDISO upstream: the LU of a 3-D stencil matrix is what limits n).
+(fast_solver_lippmann_schwinger_b200.sparsifier) and keeps As on the GPU.  --msp host (default) factorises
+Mapproxsp on the host (SuperLU here, MKL PARDISO upstream: the LU of a 3-D stencil matrix is what limits n);
+--msp gpu factorises it on the device (ls_msp_factor3d), so the whole GMRES loop stays there.
 """
 import argparse
 import os
@@ -29,6 +30,7 @@ def main():
     ap.add_argument("--n", type=int, default=48)
     ap.add_argument("--ppw", type=float, default=None, help="points per wavelength (default: k = 1/h as in example3D.jl)")
     ap.add_argument("--precond", action="store_true", help="sparsifying preconditioner (example3D.jl:56-67)")
+    ap.add_argument("--msp", choices=("host", "gpu"), default="host", help="where lu(Mapproxsp) is factorised and solved")
     args = ap.parse_args()
     n = args.n
     h = 1.0 / n
@@ -48,9 +50,14 @@ def main():
         As, Mapproxsp = sparsifier.sparsifying_matrices_3d(k, X, Y, Z, fastconv, n, n, n, nu)
         print("As, Mapproxsp from 343 GPU applies in %.2f s (nnz %d)" % (time.time() - t0, As.nnz))
         t0 = time.time()
-        precond = ls.SparsifyingPreconditioner(Mapproxsp, As, solverType="MKLPARDISO")
-        print("lu(Mapproxsp) on the host in %.2f s; As on the GPU as %s (%d classes)" % (
-            time.time() - t0, precond.As.format, precond.As.nclasses))
+        if args.msp == "gpu":
+            precond = ls.SparsifyingPreconditioner(Mapproxsp, As, solverType="GPU", grid=(n, n, n))
+            where = "on the GPU (%.2f GB of factors)" % (precond.MspGPU.factor_bytes / 1e9)
+        else:
+            precond = ls.SparsifyingPreconditioner(Mapproxsp, As, solverType="MKLPARDISO")
+            where = "on the host"
+        print("lu(Mapproxsp) %s in %.2f s; As on the GPU as %s (%d classes)" % (
+            where, time.time() - t0, precond.As.format, precond.As.nclasses))
     u_inc = np.exp(1j * k * X)
     rhs = -(fastconv * u_inc - u_inc)
     u = np.zeros(n ** 3, dtype=np.complex128)

@@ -103,6 +103,7 @@ def lib():
         "ls_gmres": (ci, [vp, vp, vp, SOLVE_CB, vp, vp, vp, ci, i64, dbl, dbl, ci, vp, i64,
                           C.POINTER(i64), C.POINTER(ci), C.POINTER(i64), ci]),
         "ls_msp_factor": (ci, [C.POINTER(vp), i64, i64, vp, vp, vp]),
+        "ls_msp_factor3d": (ci, [C.POINTER(vp), i64, i64, i64, vp, vp, vp]),
         "ls_msp_solve": (ci, [vp, vp, vp, ci]),
         "ls_msp_info": (ci, [vp, C.POINTER(i64), C.POINTER(ci), C.POINTER(dbl)]),
         "ls_msp_plan": (ci, [vp, C.c_char_p, i64]),

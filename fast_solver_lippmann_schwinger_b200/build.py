@@ -85,6 +85,11 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = Non
         link += ["-L" + cublas_dir, "-l:libcublas.so.12", "-Xlinker", "-rpath", "-Xlinker", cublas_dir]
     else:
         link += ["-lcublas"]
+    cusolver_dir = _pip_libdir("nvidia.cusolver", "libcusolver.so.11")
+    if cusolver_dir:
+        link += ["-L" + cusolver_dir, "-l:libcusolver.so.11", "-Xlinker", "-rpath", "-Xlinker", cusolver_dir]
+    else:
+        link += ["-lcusolver"]
     p = subprocess.run(link, capture_output=True, text=True)
     if p.returncode != 0:
         raise RuntimeError("link failed:\n%s\n%s" % (p.stdout, p.stderr))

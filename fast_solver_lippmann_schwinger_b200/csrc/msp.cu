@@ -1,4 +1,4 @@
-// Device-resident direct solve with the sparsified system matrix  Msp = As + k^2 AG diag(nu)  (2-D).
+// Device-resident direct solve with the sparsified system matrix  Msp = As + k^2 AG diag(nu)  (2-D and 3-D).
 //
 // Stands behind `MspInv = lu(Msp)` (preconditioner.jl:35, UMFPACK; :41-55 MKL PARDISO) and the solve that runs in
 // every GMRES iteration, `MspInv \ (As*b)` (preconditioner.jl:138,142,159,163).  Upstream that solve is a CPU
@@ -6,14 +6,16 @@
 // host triangular solve per iteration (SURVEY.md hard part H1), so the factorisation lives on the device here.
 //
 // Msp is a 9-point stencil matrix on the n x m grid (unknown i + n*j couples to (i+-1, j+-1); buildSparseA /
-// buildSparseAG, SparsifyingMatrix2D.jl:806-884, :351-438).  Geometric nested dissection: the grid is bisected
-// recursively by one-node-wide separators into a complete binary tree of depth D; the leaves are boxes of at most
-// LEAF x LEAF unknowns.  Node t eliminates its own unknowns S (separator, or the whole leaf box) against the ring B of
-// ancestor-separator unknowns around its region (multifrontal method):
+// buildSparseAG, SparsifyingMatrix2D.jl:806-884, :351-438) or a 27-point one on the n x m x l grid (example3D.jl:56-61).
+// Geometric nested dissection (msp_symbolic.h): the grid is bisected recursively by separators one cell thick into a
+// complete binary tree of depth D; the leaves are boxes of at most LEAF unknowns per side.  Node t eliminates its own
+// unknowns S (separator, or the whole leaf box) against the ring B of ancestor-separator unknowns around its region
+// (multifrontal method):
 //      F = [F_SS F_SB; F_BS F_BB] = (entries of Msp) + (update matrices of the two children)
 //      Sinv = F_SS^-1 (partial pivoting),   Y = Sinv F_SB,   update U = F_BB - F_BS Y  -> parent.
 // All nodes of one depth have sizes within +-1 of each other, so a depth is one uniform batch (padded with identity
-// rows): the factorisation is cuBLAS batched LU / inverse / GEMM calls (one-time set-up, like `lu(Msp)`), the
+// rows): the factorisation is cuBLAS batched LU / inverse / GEMM calls (one-time set-up, like `lu(Msp)`; on a 3-D grid
+// the depths with large, few fronts take cuSOLVER's LU one node at a time instead), the
 // per-iteration SOLVE is hand-written: per depth three batched matrix-vector kernels on the way up
 //      g = [f_S; 0] + extend(t_child0) + extend(t_child1);   z = Sinv g_S;   t = g_B - F_BS z
 // and one on the way down,  u_S = z - Y u_B,  all memory-bound sweeps over the stored blocks (about 200 N complex
@@ -21,7 +23,10 @@
 #include "ls_common.cuh"
 #include "spmv.cuh"
 #include "msp_gemv.cuh"
+#include "msp_symbolic.h"
+#include "line_kernels.cuh"
 #include <cublas_v2.h>
+#include <cusolverDn.h>
 #include <algorithm>
 #include <chrono>
 #include <cstdlib>
@@ -31,12 +36,12 @@ using namespace ls;
 
 namespace {
 
-struct Box { int i0, i1, j0, j1; };      // region [i0, i1) x [j0, j1)
-
 struct Level {                            // all 2^d nodes of one depth
     int count = 0, Sp = 0, Bp = 0;        // padded sizes of S and B
     bool leaf = false;
-    int axis = 0;                         // split axis of this depth (0: x, 1: y), internal levels
+    int axis = 0;                         // split axis of this depth (0: x, 1: y, 2: z), internal levels
+    bool lu_cusolver = false;             // F_SS factorised by cuSOLVER one node at a time (else cuBLAS batched)
+    bool gather_s = false, gather_y = false;   // X of sweep 0 / 2 longer than the shared memory: assembled by k_msp_gather
     int* d_Sidx = nullptr;                // [count][Sp]  global unknown, -1 = padding
     int* d_Bidx = nullptr;                // [count][Bp]
     int* d_pmap = nullptr;                // [count][2][Sp+Bp]  position in child's B list, -1 = none (internal levels)
@@ -54,12 +59,14 @@ struct Level {                            // all 2^d nodes of one depth
 };
 
 struct Msp : MspBase {
-    long gn = 0, gm = 0;
+    long gn = 0, gm = 0, gl = 1;
     std::vector<Level> lev;
     cd* d_in = nullptr; cd* d_out = nullptr;      // staging for host-pointer solves
     size_t factor_bytes = 0;
     double factor_seconds = 0.0;
     cublasHandle_t cublas = nullptr;
+    cusolverDnHandle_t cusolver = nullptr;
+    size_t smem_max = 48 * 1024;                  // the device's opt-in shared memory per block
     // solver 1: uniform (identity-padded) batches, k_msp_gather + k_msp_gemv (round-2 first version, kept selectable);
     // solver 2 (default): tightly packed blocks, gather fused into the sweeps, per-launch geometry (msp_gemv.cuh).
     // LS_MSP_SOLVER / LS_MSP_FUSE / LS_MSP_TUNE are read when the handle is created.
@@ -71,6 +78,7 @@ struct Msp : MspBase {
     int solve_launch2(const cd* rhs, cd* out, cudaStream_t s);
     int sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) const;
     int tune_sweeps();
+    size_t xs_limit(int cols_p) const;
     // the 4 x (depth + 1) dependent launches of one solve, captured once per (rhs, out) pair and replayed as a CUDA graph
     // (GMRES calls the solve with at most restart + 2 different pairs): removes the launch gaps between the small kernels
     struct Captured { const cd* rhs; cd* out; cudaGraphExec_t exec; };
@@ -79,6 +87,7 @@ struct Msp : MspBase {
     ~Msp() override {
         for (auto& g : graphs) cudaGraphExecDestroy(g.exec);
         if (cublas) cublasDestroy(cublas);
+        if (cusolver) cusolverDnDestroy(cusolver);
     }
 };
 
@@ -206,16 +215,26 @@ typedef void (*gemv2_fn)(const lsmsp::Gemv2, const lsmsp::Geo);
 const gemv2_fn gemv2_table[6][4][2] = { LS_G2_L(1), LS_G2_L(2), LS_G2_L(4), LS_G2_L(8), LS_G2_L(16), LS_G2_L(32) };
 constexpr size_t GEMV2_SMEM_MAX = 48 * 1024;      // the default dynamic shared-memory limit: no per-device opt-in needed
 
-inline bool gemv2_valid(const lsmsp::Gemv2& a, const lsmsp::Choice& ch) {
+// `limit`: the staging bytes a launch may use (Msp::xs_limit)
+inline bool gemv2_valid(const lsmsp::Gemv2& a, const lsmsp::Choice& ch, size_t limit) {
     if (ch.lanes_log2 < 0 || ch.lanes_log2 > 5 || ch.unr_log2 < 0 || ch.unr_log2 > 3) return false;
-    return lsmsp::launch_geo(a.rows_p, a.cols_p, a.nodes, ch).smem <= GEMV2_SMEM_MAX;
+    return lsmsp::launch_geo(a.rows_p, a.cols_p, a.nodes, ch).smem <= limit;
 }
 
-int launch_gemv2(const lsmsp::Gemv2& a, lsmsp::Choice ch, cudaStream_t s) {
+int launch_gemv2(const lsmsp::Gemv2& a, lsmsp::Choice ch, size_t limit, cudaStream_t s) {
     if (a.nodes <= 0 || a.rows_p <= 0) return LS_OK;
-    if (!gemv2_valid(a, ch)) ch.xs = 0;                // X too long for the staging buffer: every group fetches it itself
+    if (!gemv2_valid(a, ch, limit)) ch.xs = 0;         // X too long for the staging buffer: every group fetches it itself
     const lsmsp::LaunchGeo L = lsmsp::launch_geo(a.rows_p, a.cols_p, a.nodes, ch);
     gemv2_table[ch.lanes_log2][ch.unr_log2][ch.xs ? 1 : 0]<<<L.grid, 256, L.smem, s>>>(a, L.g);
+    return LS_OK;
+}
+
+// lets every staging kernel use `smem` bytes of dynamic shared memory on the current device (done once, at
+// factorisation: the solve launches are captured into a graph)
+int optin_staging(size_t smem) {
+    static unsigned long long done[6][4] = {};
+    for (int ll = 0; ll < 6; ++ll)
+        for (int ul = 0; ul < 4; ++ul) LS_CUDA_TRY(lsk::smem_optin(gemv2_table[ll][ul][1], (int)smem, done[ll][ul]));
     return LS_OK;
 }
 
@@ -319,198 +338,54 @@ __global__ void k_msp_pack(const cd* __restrict__ Cinv, const cd* __restrict__ Y
 
 inline unsigned grid_for(long total) { return (unsigned)std::min<long>((total + 255) / 256, 148L * 32); }
 
-// ---- host-side symbolic analysis --------------------------------------------------------------------------------
-struct Symbolic {
-    int n, m;
-    std::vector<std::vector<Box>> boxes;           // per depth
-    std::vector<int> axis;                         // per depth (internal)
-    int D = 0;
-    // position of (i, j) in the ring around `b` (enumeration order: row j0-1, then the side columns of rows
-    // j0..j1-1, then row j1; everything clipped to the grid); -1 if (i, j) is not on the ring
-    int ring_index(const Box& b, int i, int j) const {
-        const int ia = std::max(b.i0 - 1, 0), ib = std::min(b.i1, n - 1);
-        const int wrow = ib - ia + 1;
-        int pos = 0;
-        if (b.j0 - 1 >= 0) {
-            if (j == b.j0 - 1) return (i >= ia && i <= ib) ? pos + (i - ia) : -1;
-            pos += wrow;
-        }
-        const bool hasL = b.i0 - 1 >= 0, hasR = b.i1 < n;
-        const int per = (hasL ? 1 : 0) + (hasR ? 1 : 0);
-        if (j >= b.j0 && j < b.j1) {
-            const int base = pos + (j - b.j0) * per;
-            if (hasL && i == b.i0 - 1) return base;
-            if (hasR && i == b.i1) return base + (hasL ? 1 : 0);
-            return -1;
-        }
-        pos += (b.j1 - b.j0) * per;
-        if (b.j1 < m) {
-            if (j == b.j1) return (i >= ia && i <= ib) ? pos + (i - ia) : -1;
-            pos += wrow;
-        }
-        return -1;
-    }
-    void ring_list(const Box& b, std::vector<int>& out) const {
-        out.clear();
-        const int ia = std::max(b.i0 - 1, 0), ib = std::min(b.i1, n - 1);
-        if (b.j0 - 1 >= 0) for (int i = ia; i <= ib; ++i) out.push_back(i + n * (b.j0 - 1));
-        for (int j = b.j0; j < b.j1; ++j) {
-            if (b.i0 - 1 >= 0) out.push_back(b.i0 - 1 + n * j);
-            if (b.i1 < n) out.push_back(b.i1 + n * j);
-        }
-        if (b.j1 < m) for (int i = ia; i <= ib; ++i) out.push_back(i + n * b.j1);
-    }
-    // own unknowns of a node: the separator line (internal) or the whole box (leaf)
-    void own_list(const Box& b, bool leaf, int ax, std::vector<int>& out) const {
-        out.clear();
-        if (leaf) {
-            for (int j = b.j0; j < b.j1; ++j)
-                for (int i = b.i0; i < b.i1; ++i) out.push_back(i + n * j);
-        } else if (ax == 0) {
-            const int mid = b.i0 + (b.i1 - b.i0) / 2;
-            for (int j = b.j0; j < b.j1; ++j) out.push_back(mid + n * j);
-        } else {
-            const int mid = b.j0 + (b.j1 - b.j0) / 2;
-            for (int i = b.i0; i < b.i1; ++i) out.push_back(i + n * mid);
-        }
-    }
-    void build(int n_, int m_, int leafmax) {
-        n = n_; m = m_;
-        boxes.clear(); axis.clear();
-        boxes.push_back({Box{0, n, 0, m}});
-        for (;;) {
-            const auto& cur = boxes.back();
-            int maxw = 0, maxh = 0;
-            for (const Box& b : cur) { maxw = std::max(maxw, b.i1 - b.i0); maxh = std::max(maxh, b.j1 - b.j0); }
-            if (std::max(maxw, maxh) <= leafmax) break;
-            const int ax = (maxw >= maxh) ? 0 : 1;
-            axis.push_back(ax);
-            std::vector<Box> next;
-            next.reserve(cur.size() * 2);
-            for (const Box& b : cur) {
-                if (ax == 0) {
-                    const int mid = b.i0 + (b.i1 - b.i0) / 2;
-                    next.push_back(Box{b.i0, mid, b.j0, b.j1});
-                    next.push_back(Box{mid + 1, b.i1, b.j0, b.j1});
-                } else {
-                    const int mid = b.j0 + (b.j1 - b.j0) / 2;
-                    next.push_back(Box{b.i0, b.i1, b.j0, mid});
-                    next.push_back(Box{b.i0, b.i1, mid + 1, b.j1});
-                }
-            }
-            boxes.push_back(std::move(next));
-        }
-        D = (int)boxes.size() - 1;
-    }
-};
+#define LS_CUSOLVER_TRY(expr)                                                                        \
+    do {                                                                                             \
+        cusolverStatus_t _s = (expr);                                                                \
+        if (_s != CUSOLVER_STATUS_SUCCESS) {                                                         \
+            set_error("%s failed at %s:%d: cuSOLVER status %d", #expr, __FILE__, __LINE__, (int)_s); \
+            return LS_ERR_CUDA;                                                                      \
+        }                                                                                            \
+    } while (0)
 
-int msp_factor(Msp* M, int n, int m, const int64_t* colptr, const int64_t* rowval, const cd* nzval, int leafmax) {
+__global__ void k_msp_eye(cd* C, int Sp, long total) {
+    for (long e = (long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long)gridDim.x * blockDim.x) {
+        const long t = e / Sp;
+        const int i = (int)(e % Sp);
+        C[t * (long)Sp * Sp + i + (long)i * Sp] = make_double2(1.0, 0.0);
+    }
+}
+
+// Pivot blocks of at least this many unknowns on a 3-D grid go through cuSOLVER's blocked LU one node at a time:
+// the batched cuBLAS LU / inverse are built for small matrices, and in 3-D the upper depths hold a few fronts of
+// thousands of unknowns.  Depths with more nodes than LU_CUSOLVER_MAX_NODES keep the batched route (per-node calls
+// would be launch-bound).  2-D handles keep the batched route at every depth.
+constexpr int LU_CUSOLVER_MIN_SP = 128;
+constexpr int LU_CUSOLVER_MAX_NODES = 1024;
+
+// `sym` has been analysed and its memory need checked; builds the lists, routes the entries and factorises
+int msp_factor(Msp* M, lsmsp::Symbolic& sym, const int64_t* colptr, const int64_t* rowval, const cd* nzval) {
     const auto t_start = std::chrono::steady_clock::now();
-    const long N = (long)n * m;
-    const int64_t nnz = colptr[N] - 1;
-    Symbolic sym;
-    sym.build(n, m, leafmax);
+    const int64_t nnz = colptr[sym.N()] - 1;
     const int D = sym.D;
     M->lev.assign((size_t)D + 1, Level());
     cudaStream_t s = M->stream;
     int rc;
-
-    // ---- owners, per-node lists ----
-    std::vector<unsigned char> own_depth((size_t)N, 255);
-    std::vector<int> own_node((size_t)N, -1), own_loc((size_t)N, -1);
-    std::vector<std::vector<int>> hSidx((size_t)D + 1), hBidx((size_t)D + 1);
-    std::vector<int> tmp;
+    if ((rc = sym.lists()) || (rc = sym.route(colptr, rowval)) || (rc = sym.maps())) {
+        set_error("%s", sym.err.c_str());
+        return rc;
+    }
     for (int d = 0; d <= D; ++d) {
         Level& L = M->lev[d];
-        const auto& bx = sym.boxes[d];
-        L.count = (int)bx.size();
-        L.leaf = (d == D);
-        L.axis = L.leaf ? 0 : sym.axis[d];
-        int Sp = 0, Bp = 0;
-        for (const Box& b : bx) {
-            LS_REQUIRE(b.i1 > b.i0 && b.j1 > b.j0, LS_ERR_UNSUPPORTED, "ls_msp_factor: empty region in the dissection of a %d x %d grid", n, m);
-            sym.own_list(b, L.leaf, L.axis, tmp);
-            Sp = std::max(Sp, (int)tmp.size());
-            sym.ring_list(b, tmp);
-            Bp = std::max(Bp, (int)tmp.size());
-        }
-        L.Sp = Sp; L.Bp = Bp;
-        hSidx[d].assign((size_t)L.count * Sp, -1);
-        hBidx[d].assign((size_t)L.count * std::max(Bp, 1), -1);
-        for (int t = 0; t < L.count; ++t) {
-            sym.own_list(bx[t], L.leaf, L.axis, tmp);
-            for (size_t q = 0; q < tmp.size(); ++q) {
-                const int g = tmp[q];
-                hSidx[d][(size_t)t * Sp + q] = g;
-                own_depth[g] = (unsigned char)d; own_node[g] = t; own_loc[g] = (int)q;
-            }
-            sym.ring_list(bx[t], tmp);
-            for (size_t q = 0; q < tmp.size(); ++q) hBidx[d][(size_t)t * Bp + q] = tmp[q];
-        }
+        const lsmsp::LevelShape& S = sym.lev[d];
+        L.count = S.count; L.Sp = S.Sp; L.Bp = S.Bp; L.leaf = S.leaf; L.axis = S.axis;
+        L.lu_cusolver = M->gl > 1 && L.Sp >= LU_CUSOLVER_MIN_SP && L.count <= LU_CUSOLVER_MAX_NODES;
     }
-    for (long g = 0; g < N; ++g)
-        LS_REQUIRE(own_node[g] >= 0, LS_ERR_CUDA, "ls_msp_factor: internal error, unknown %ld has no owner", g);
-
-    // ---- route every matrix entry to the front that assembles it ----
-    std::vector<std::vector<long>> edest((size_t)D + 1);
-    std::vector<std::vector<int>> esrc((size_t)D + 1);
-    for (long c = 0; c < N; ++c) {
-        for (int64_t p = colptr[c] - 1; p < colptr[c + 1] - 1; ++p) {
-            const long r = rowval[p] - 1;
-            LS_REQUIRE(r >= 0 && r < N, LS_ERR_INVALID, "ls_msp_factor: row index out of range");
-            const int dr = own_depth[r], dc = own_depth[c];
-            int d, t, lr, lc;
-            if (dr == dc) {
-                LS_REQUIRE(own_node[r] == own_node[c], LS_ERR_UNSUPPORTED,
-                           "ls_msp_factor: entry (%ld, %ld) couples unknowns further apart than the 9-point stencil", r + 1, c + 1);
-                d = dr; t = own_node[r]; lr = own_loc[r]; lc = own_loc[c];
-            } else if (dr > dc) {
-                d = dr; t = own_node[r]; lr = own_loc[r];
-                const int q = sym.ring_index(sym.boxes[d][t], (int)(c % n), (int)(c / n));
-                LS_REQUIRE(q >= 0, LS_ERR_UNSUPPORTED,
-                           "ls_msp_factor: entry (%ld, %ld) couples unknowns further apart than the 9-point stencil", r + 1, c + 1);
-                lc = M->lev[d].Sp + q;
-            } else {
-                d = dc; t = own_node[c]; lc = own_loc[c];
-                const int q = sym.ring_index(sym.boxes[d][t], (int)(r % n), (int)(r / n));
-                LS_REQUIRE(q >= 0, LS_ERR_UNSUPPORTED,
-                           "ls_msp_factor: entry (%ld, %ld) couples unknowns further apart than the 9-point stencil", r + 1, c + 1);
-                lr = M->lev[d].Sp + q;
-            }
-            const long Fp = M->lev[d].Sp + M->lev[d].Bp;
-            edest[d].push_back((long)t * Fp * Fp + lr + (long)lc * Fp);
-            esrc[d].push_back((int)p);
-        }
-    }
-
-    // ---- child -> parent maps ----
-    // cmap[d+1][child][k]   = position of the child's k-th ring unknown in the parent's [S; B] numbering
-    // pmap[d][parent][side][p] = k with cmap == p, or -1
-    std::vector<std::vector<int>> hcmap((size_t)D + 1), hpmap((size_t)D + 1);
-    for (int d = 0; d < D; ++d) {
-        const Level& L = M->lev[d];
-        const Level& Lc = M->lev[d + 1];
-        const int Fp = L.Sp + L.Bp;
-        hpmap[d].assign((size_t)L.count * 2 * Fp, -1);
-        hcmap[d + 1].assign((size_t)Lc.count * std::max(Lc.Bp, 1), -1);
-        for (int t = 0; t < L.count; ++t)
-            for (int side = 0; side < 2; ++side) {
-                const int c = 2 * t + side;
-                for (int k = 0; k < Lc.Bp; ++k) {
-                    const int g = hBidx[d + 1][(size_t)c * Lc.Bp + k];
-                    if (g < 0) continue;
-                    int p;
-                    if (own_depth[g] == d && own_node[g] == t) p = own_loc[g];
-                    else {
-                        const int q = sym.ring_index(sym.boxes[d][t], g % n, g / n);
-                        LS_REQUIRE(q >= 0, LS_ERR_CUDA, "ls_msp_factor: internal error, child ring unknown outside the parent front");
-                        p = L.Sp + q;
-                    }
-                    hcmap[d + 1][(size_t)c * Lc.Bp + k] = p;
-                    hpmap[d][((size_t)t * 2 + side) * Fp + p] = k;
-                }
-            }
-    }
+    const auto& hSidx = sym.Sidx;
+    const auto& hBidx = sym.Bidx;
+    const auto& hpmap = sym.pmap;
+    const auto& hcmap = sym.cmap;
+    const auto& edest = sym.edest;
+    const auto& esrc = sym.esrc;
 
     // ---- device: index maps, solve storage ----
     size_t fbytes = 0;
@@ -592,11 +467,34 @@ int msp_factor(Msp* M, int n, int m, const int64_t* colptr, const int64_t* rowva
         if ((rc = M->dmalloc((void**)&pC, (size_t)cnt * sizeof(cd*)))) return rc;
         if ((rc = M->dmalloc((void**)&piv, (size_t)cnt * Sp * sizeof(int)))) return rc;
         if ((rc = M->dmalloc((void**)&info, (size_t)cnt * 2 * sizeof(int)))) return rc;
-        k_msp_ptrs<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(pA, F, Fp * Fp, (int)cnt);
-        k_msp_ptrs<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(pC, Cinv, Sp * Sp, (int)cnt);
-        LS_CUBLAS_TRY(cublasZgetrfBatched(M->cublas, (int)Sp, reinterpret_cast<cuDoubleComplex**>(pA), (int)Fp, piv, info, (int)cnt));
-        LS_CUBLAS_TRY(cublasZgetriBatched(M->cublas, (int)Sp, reinterpret_cast<cuDoubleComplex**>(pA), (int)Fp, piv,
-                                          reinterpret_cast<cuDoubleComplex**>(pC), (int)Sp, info + cnt, (int)cnt));
+        if (L.lu_cusolver) {
+            // F_SS = P L U in place (as the batched route), then Sinv = getrs(F_SS, I)
+            if (!M->cusolver) {
+                LS_CUSOLVER_TRY(cusolverDnCreate(&M->cusolver));
+                LS_CUSOLVER_TRY(cusolverDnSetStream(M->cusolver, s));
+            }
+            int lwork = 0;
+            LS_CUSOLVER_TRY(cusolverDnZgetrf_bufferSize(M->cusolver, (int)Sp, (int)Sp, reinterpret_cast<cuDoubleComplex*>(F), (int)Fp, &lwork));
+            cd* work = nullptr;
+            if ((rc = M->dmalloc((void**)&work, (size_t)std::max(lwork, 1) * sizeof(cd)))) return rc;
+            LS_CUDA_TRY(cudaMemsetAsync(Cinv, 0, (size_t)cnt * Sp * Sp * sizeof(cd), s));
+            k_msp_eye<<<grid_for(cnt * Sp), 256, 0, s>>>(Cinv, (int)Sp, cnt * Sp);
+            for (long t = 0; t < cnt; ++t) {
+                cuDoubleComplex* A = reinterpret_cast<cuDoubleComplex*>(F + t * Fp * Fp);
+                LS_CUSOLVER_TRY(cusolverDnZgetrf(M->cusolver, (int)Sp, (int)Sp, A, (int)Fp, reinterpret_cast<cuDoubleComplex*>(work),
+                                                 piv + t * Sp, info + t));
+                LS_CUSOLVER_TRY(cusolverDnZgetrs(M->cusolver, CUBLAS_OP_N, (int)Sp, (int)Sp, A, (int)Fp, piv + t * Sp,
+                                                 reinterpret_cast<cuDoubleComplex*>(Cinv + t * Sp * Sp), (int)Sp, info + cnt + t));
+            }
+            LS_CUDA_TRY(cudaStreamSynchronize(s));
+            M->dfree(work);
+        } else {
+            k_msp_ptrs<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(pA, F, Fp * Fp, (int)cnt);
+            k_msp_ptrs<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(pC, Cinv, Sp * Sp, (int)cnt);
+            LS_CUBLAS_TRY(cublasZgetrfBatched(M->cublas, (int)Sp, reinterpret_cast<cuDoubleComplex**>(pA), (int)Fp, piv, info, (int)cnt));
+            LS_CUBLAS_TRY(cublasZgetriBatched(M->cublas, (int)Sp, reinterpret_cast<cuDoubleComplex**>(pA), (int)Fp, piv,
+                                              reinterpret_cast<cuDoubleComplex**>(pC), (int)Sp, info + cnt, (int)cnt));
+        }
         {
             std::vector<int> hinfo((size_t)cnt * 2);
             LS_CUDA_TRY(cudaMemcpyAsync(hinfo.data(), info, hinfo.size() * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -709,6 +607,13 @@ int Msp::solve_launch(const cd* rhs, cd* out, cudaStream_t s) {
 }
 
 // ---- solver 2 ----------------------------------------------------------------------------------------------------
+// Staging bytes a sweep with cols_p columns may use: the default 48 KB, or the device's opt-in limit (227 KB on B200)
+// when one node's X alone is longer than 48 KB (separators and rings of more than 3072 unknowns, 3-D grids).  Beyond
+// that, sweeps 0 and 2 read X assembled once by k_msp_gather (Level::gather_s / gather_y).
+size_t Msp::xs_limit(int cols_p) const {
+    return (size_t)cols_p * sizeof(cd) > GEMV2_SMEM_MAX ? smem_max : GEMV2_SMEM_MAX;
+}
+
 // arguments of sweep `which` of depth d:  0  z = Sinv g_S   1  t = g_B - F_BS z   2  u_S = z - Y u_B
 int Msp::sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) const {
     const int D = (int)lev.size() - 1;
@@ -720,7 +625,7 @@ int Msp::sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) c
     a.pmap = Lc ? L.d_pmap : nullptr; a.tchild = Lc ? Lc->d_t : nullptr; a.Fp = Fp; a.Bpc = Lc ? Lc->Bp : 0;
     if (which == 0) {
         a.M = L.d_Sinv; a.moff = L.d_offS; a.nrows = L.d_ns; a.ncols = L.d_ns; a.rows_p = L.Sp; a.cols_p = L.Sp;
-        if (fuse) { a.xmode = 2; a.f = rhs; a.sidx = L.d_Sidx; }
+        if (fuse && !L.gather_s) { a.xmode = 2; a.f = rhs; a.sidx = L.d_Sidx; }
         else { a.xmode = 0; a.x = L.d_g; a.xstride = Fp; }
         a.ymode = 0; a.sign = 1.0;
         a.out = L.d_z; a.ostride = L.Sp;
@@ -733,7 +638,8 @@ int Msp::sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) c
         a.out = L.d_t; a.ostride = L.Bp;
     } else {
         a.M = L.d_Y; a.moff = L.d_offB; a.nrows = L.d_ns; a.ncols = L.d_nb; a.rows_p = L.Sp; a.cols_p = L.Bp;
-        a.xmode = 1; a.xidx = L.d_Bidx; a.xg = out;
+        if (L.gather_y) { a.xmode = 0; a.x = L.d_g; a.xstride = L.Bp; }
+        else { a.xmode = 1; a.xidx = L.d_Bidx; a.xg = out; }
         a.ymode = 1; a.y0 = L.d_z; a.y0stride = L.Sp; a.sign = -1.0;
         a.oidx = L.d_Sidx; a.og = out;
     }
@@ -745,7 +651,7 @@ int Msp::solve_launch2(const cd* rhs, cd* out, cudaStream_t s) {
     lsmsp::Gemv2 a;
     for (int d = D; d >= 0; --d) {                      // upward: leaves -> root
         Level& L = lev[d];
-        if (!fuse) {
+        if (!fuse || L.gather_s) {
             const int Fp = L.Sp + L.Bp;
             const long total = (long)L.count * Fp;
             const Level* Lc = d < D ? &lev[d + 1] : nullptr;
@@ -753,15 +659,20 @@ int Msp::solve_launch2(const cd* rhs, cd* out, cudaStream_t s) {
                                                          Lc ? Lc->Bp : 0, total, L.d_g);
         }
         sweep_args(d, 0, rhs, out, a);
-        launch_gemv2(a, L.ch_sinv, s);
+        launch_gemv2(a, L.ch_sinv, xs_limit(a.cols_p), s);
         if (L.Bp > 0) {
             sweep_args(d, 1, rhs, out, a);
-            launch_gemv2(a, L.ch_fbs, s);
+            launch_gemv2(a, L.ch_fbs, xs_limit(a.cols_p), s);
         }
     }
     for (int d = 0; d <= D; ++d) {                      // downward: root -> leaves, u_S written straight into `out`
+        const Level& L = lev[d];
+        if (L.gather_y) {                               // u_B = out[Bidx] into d_g (free once the upward pass is done)
+            const long total = (long)L.count * L.Bp;
+            k_msp_gather<<<grid_for(total), 256, 0, s>>>(out, L.d_Bidx, nullptr, nullptr, L.Bp, L.Bp, 0, total, L.d_g);
+        }
         sweep_args(d, 2, rhs, out, a);
-        launch_gemv2(a, lev[d].ch_y, s);
+        launch_gemv2(a, L.ch_y, xs_limit(a.cols_p), s);
     }
     launches += launches_per_solve;
     LS_CUDA_TRY(cudaGetLastError());
@@ -802,21 +713,22 @@ int Msp::tune_sweeps() {
         sweep_args(d, which, f, u, a);
         if (a.nodes <= 0 || a.rows_p <= 0) return LS_OK;
         const lsmsp::Choice def = lsmsp::default_choice(a.cols_p, a.xmode);
+        const size_t limit = xs_limit(a.cols_p);
         float best_ms = 1e30f;
         lsmsp::Choice pick = def;
-        if (!gemv2_valid(a, pick)) pick.xs = 0;
+        if (!gemv2_valid(a, pick, limit)) pick.xs = 0;
         for (int ll = std::max(0, def.lanes_log2 - 2); ll <= std::min(5, def.lanes_log2 + 1); ++ll)
             for (int ul = 0; ul <= 3; ++ul)
                 for (int xs = 0; xs <= 1; ++xs) {
                     const lsmsp::Choice ch{ll, ul, xs};
-                    if (!gemv2_valid(a, ch)) continue;
+                    if (!gemv2_valid(a, ch, limit)) continue;
                     if ((1 << ul) > std::max(a.rows_p, 1) * 2) continue;          // more rows per group than the block has
-                    launch_gemv2(a, ch, s);                                        // warm-up: instruction cache, first touch
+                    launch_gemv2(a, ch, limit, s);                                 // warm-up: instruction cache, first touch
                     float ms = 1e30f;
                     for (int rep = 0; rep < 2; ++rep) {
                         if (flush) LS_CUDA_TRY(cudaMemsetAsync(flush, 0, flush_bytes, s));
                         LS_CUDA_TRY(cudaEventRecord(e0, s));
-                        launch_gemv2(a, ch, s);
+                        launch_gemv2(a, ch, limit, s);
                         LS_CUDA_TRY(cudaEventRecord(e1, s));
                         LS_CUDA_TRY(cudaEventSynchronize(e1));
                         float t = 0.f;
@@ -843,37 +755,88 @@ int Msp::tune_sweeps() {
     return rc;
 }
 
-extern "C" {
-
-int ls_msp_factor(ls_handle* out, int64_t n, int64_t m, const int64_t* colptr, const int64_t* rowval, const ls_cdouble* nzval) {
-    LS_REQUIRE(out && colptr && rowval && nzval, LS_ERR_INVALID, "ls_msp_factor: null pointer");
-    LS_REQUIRE(n > 0 && m > 0 && n * m < (int64_t)2147483647, LS_ERR_INVALID, "ls_msp_factor: bad grid %ld x %ld", (long)n, (long)m);
-    LS_REQUIRE(colptr[0] == 1, LS_ERR_INVALID, "ls_msp_factor: colptr must be 1-based (Julia SparseMatrixCSC)");
-    LS_REQUIRE(colptr[n * m] - 1 < (int64_t)2147483647, LS_ERR_UNSUPPORTED, "ls_msp_factor: nnz exceeds the 32-bit index range");
+// ls_msp_factor (l = 1) and ls_msp_factor3d.  Refusals come as early and as cheaply as possible: arguments (no device
+// needed), then the memory the dissection needs against the free device memory (before anything is allocated), then
+// the entries as they are routed (pattern, duplicates).
+static int msp_factor_entry(const char* fn, ls_handle* out, int64_t n, int64_t m, int64_t l, const int64_t* colptr,
+                            const int64_t* rowval, const ls_cdouble* nzval) {
+    char grid[96];
+    if (l == 1) snprintf(grid, sizeof grid, "%ld x %ld", (long)n, (long)m);
+    else snprintf(grid, sizeof grid, "%ld x %ld x %ld", (long)n, (long)m, (long)l);
+    LS_REQUIRE(out && colptr && rowval && nzval, LS_ERR_INVALID, "%s: null pointer", fn);
+    const int64_t I32 = 2147483647;
+    LS_REQUIRE(n > 0 && m > 0 && l > 0 && n < I32 && m < I32 && l < I32 && n * m < I32 && n * m * l < I32, LS_ERR_INVALID,
+               "%s: bad grid %s", fn, grid);
+    const int64_t N = n * m * l;
+    LS_REQUIRE(colptr[0] == 1, LS_ERR_INVALID, "%s: colptr must be 1-based (Julia SparseMatrixCSC)", fn);
+    LS_REQUIRE(colptr[N] >= 1, LS_ERR_INVALID, "%s: colptr[end] = %ld is not a 1-based column pointer", fn, (long)colptr[N]);
+    LS_REQUIRE(colptr[N] - 1 < I32, LS_ERR_UNSUPPORTED, "%s: nnz exceeds the 32-bit index range", fn);
     int leaf = 4;
     if (const char* e = getenv("LS_MSP_LEAF")) { const int v = atoi(e); if (v >= 3 && v <= 16) leaf = v; }
+    int solver = 2;
+    bool fuse = true, tune = true;
+    if (const char* e = getenv("LS_MSP_SOLVER")) solver = atoi(e) == 1 ? 1 : 2;
+    if (const char* e = getenv("LS_MSP_FUSE")) fuse = atoi(e) != 0;
+    if (const char* e = getenv("LS_MSP_TUNE")) tune = atoi(e) != 0;
+
+    lsmsp::Symbolic sym;
+    sym.fn = fn;
+    int rc = sym.analyse((int)n, (int)m, (int)l, leaf);
+    if (rc) { set_error("%s", sym.err.c_str()); return rc; }
+    {
+        // cuBLAS / cuSOLVER handles and work space, allocation granularity
+        const size_t reserve = (size_t)256 << 20;
+        const size_t need = sym.need_bytes(colptr[N] - 1, solver == 2);
+        size_t free_b = 0, total_b = 0;
+        LS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        LS_REQUIRE(need + reserve <= free_b, LS_ERR_NOMEM,
+                   "%s: factorising the %s grid needs %zu bytes of device memory (plus %zu reserved for library work space); "
+                   "%zu of %zu bytes are free", fn, grid, need, reserve, free_b, total_b);
+    }
+
     Msp* M = new Msp();
-    int rc = M->init_base(KIND_MSP);
+    rc = M->init_base(KIND_MSP);
     if (rc) { delete M; return rc; }
-    M->n = n * m; M->gn = n; M->gm = m;
-    if (const char* e = getenv("LS_MSP_SOLVER")) M->solver = atoi(e) == 1 ? 1 : 2;
-    if (const char* e = getenv("LS_MSP_FUSE")) M->fuse = atoi(e) != 0;
-    if (const char* e = getenv("LS_MSP_TUNE")) M->tune = atoi(e) != 0;
-    rc = msp_factor(M, (int)n, (int)m, colptr, rowval, reinterpret_cast<const cd*>(nzval), leaf);
+    M->n = N; M->gn = n; M->gm = m; M->gl = l;
+    M->solver = solver; M->fuse = fuse; M->tune = tune;
+    {
+        int v = 0;
+        if (cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, M->device) == cudaSuccess && (size_t)v > M->smem_max)
+            M->smem_max = (size_t)v;
+        cudaGetLastError();
+    }
+    rc = msp_factor(M, sym, colptr, rowval, reinterpret_cast<const cd*>(nzval));
     if (rc) { delete M; return rc; }
     if (M->solver == 2) {
+        bool wide = false;
         for (Level& L : M->lev) {
-            L.ch_sinv = lsmsp::default_choice(L.Sp, M->fuse ? 2 : 0);
+            L.gather_s = M->fuse && (size_t)L.Sp * sizeof(cd) > M->smem_max;
+            L.gather_y = (size_t)L.Bp * sizeof(cd) > M->smem_max;
+            wide = wide || M->xs_limit(L.Sp) > GEMV2_SMEM_MAX || M->xs_limit(L.Bp) > GEMV2_SMEM_MAX;
+            L.ch_sinv = lsmsp::default_choice(L.Sp, (M->fuse && !L.gather_s) ? 2 : 0);
             L.ch_fbs = lsmsp::default_choice(L.Sp, 0);
-            L.ch_y = lsmsp::default_choice(L.Bp, 1);
+            L.ch_y = lsmsp::default_choice(L.Bp, L.gather_y ? 0 : 1);
         }
+        if (wide && (rc = optin_staging(M->smem_max))) { delete M; return rc; }
         M->launches_per_solve = 0;
-        for (const Level& L : M->lev) M->launches_per_solve += (M->fuse ? 0 : 1) + 2 + (L.Bp > 0 ? 1 : 0);
+        for (const Level& L : M->lev)
+            M->launches_per_solve += ((M->fuse && !L.gather_s) ? 0 : 1) + 2 + (L.Bp > 0 ? 1 : 0) + (L.gather_y ? 1 : 0);
         if (M->tune) rc = M->tune_sweeps();
         if (rc) { delete M; return rc; }
     }
     *out = reinterpret_cast<ls_handle>(M);
     return LS_OK;
+}
+
+extern "C" {
+
+int ls_msp_factor(ls_handle* out, int64_t n, int64_t m, const int64_t* colptr, const int64_t* rowval, const ls_cdouble* nzval) {
+    return msp_factor_entry("ls_msp_factor", out, n, m, 1, colptr, rowval, nzval);
+}
+
+int ls_msp_factor3d(ls_handle* out, int64_t n, int64_t m, int64_t l, const int64_t* colptr, const int64_t* rowval,
+                    const ls_cdouble* nzval) {
+    return msp_factor_entry("ls_msp_factor3d", out, n, m, l, colptr, rowval, nzval);
 }
 
 int ls_msp_solve(ls_handle h, const ls_cdouble* rhs, ls_cdouble* x, int memloc) {
@@ -929,6 +892,7 @@ int ls_msp_plan(ls_handle h, char* buf, int64_t cap) {
                 out += line;
             }
         }
+        if (M->gl > 1) out += L.lu_cusolver ? " lu cusolver" : " lu batched";
         out += "\n";
     }
     const size_t ncopy = std::min<size_t>(out.size(), (size_t)cap - 1);

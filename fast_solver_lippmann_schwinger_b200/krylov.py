@@ -11,10 +11,11 @@
     gmres!(x, A, b; Pl, log, restart, maxiter, reltol, ...)    gmres_(x, A, b, Pl=, log=, ...)
       IterativeSolvers.jl (un-vendored), examples/example.jl:85
 
-    lu(Msp)  (MspInv, preconditioner.jl:35)                    GPUMspFactorization(Msp, n, m)  [solverType="GPU"]
+    lu(Msp)  (MspInv, preconditioner.jl:35)                    GPUMspFactorization(Msp, n, m[, l])  [solverType="GPU"]
 
 The sparse direct solve `MspInv \\ .` (UMFPACK / MKL PARDISO upstream) has two routes here (SURVEY.md H1):
-solverType="GPU" factorises Msp on the device (ls_msp_factor: nested dissection, 2-D 9-point matrices) so the
+solverType="GPU" factorises Msp on the device (ls_msp_factor / ls_msp_factor3d: nested dissection, 2-D 9-point and
+3-D 27-point matrices) so the
 whole preconditioned GMRES loop runs without PCIe traffic; solverType="UMFPACK" keeps it on the host with the
 caller - scipy's SuperLU plays UMFPACK's part and is reached through the ls_solve_cb callback.
 """
@@ -97,16 +98,27 @@ def cscmv_(transa, alpha, matdescra, A: GPUSparseMatrixCSC, x, beta, y):
 
 class GPUMspFactorization(_Handle):
     """``lu(Msp)`` (preconditioner.jl:35) on the GPU: nested-dissection factorisation of the 9-point matrix Msp of
-    the n x m grid (ls_msp_factor).  ``solve(b)`` = ``MspInv \\ b`` on host arrays or DeviceBuffers."""
+    the n x m grid (ls_msp_factor), or with ``l`` of the 27-point matrix of the n x m x l grid (ls_msp_factor3d,
+    examples/example3D.jl:56-61).  ``solve(b)`` = ``MspInv \\ b`` on host arrays or DeviceBuffers.  A scipy matrix is
+    canonicalised first (duplicates summed, indices sorted; the caller's matrix is not modified)."""
 
-    def __init__(self, Msp, n, m):
+    def __init__(self, Msp, n, m, l=None):
         super().__init__()
+        if not isinstance(Msp, tuple):
+            Msp = Msp.tocsc(copy=True)
+            Msp.sum_duplicates()
+            Msp.sort_indices()
         nrows, ncols, colptr, rowval, nzval = _julia_csc(Msp)
         self.n, self.m = int(n), int(m)
-        if nrows != ncols or nrows != self.n * self.m:
-            raise ValueError("DimensionMismatch: Msp is %d x %d, the grid has %d unknowns" % (nrows, ncols, self.n * self.m))
+        self.l = 1 if l is None else int(l)
+        N = self.n * self.m * self.l
+        if nrows != ncols or nrows != N:
+            raise ValueError("DimensionMismatch: Msp is %d x %d, the grid has %d unknowns" % (nrows, ncols, N))
         self.N = nrows
-        check(lib().ls_msp_factor(C.byref(self._h), self.n, self.m, ptr(colptr), ptr(rowval), ptr(nzval)))
+        if l is None:
+            check(lib().ls_msp_factor(C.byref(self._h), self.n, self.m, ptr(colptr), ptr(rowval), ptr(nzval)))
+        else:
+            check(lib().ls_msp_factor3d(C.byref(self._h), self.n, self.m, self.l, ptr(colptr), ptr(rowval), ptr(nzval)))
         fb, dep, sec = C.c_int64(), C.c_int(), C.c_double()
         check(lib().ls_msp_info(self.handle, C.byref(fb), C.byref(dep), C.byref(sec)))
         self.factor_bytes, self.depth, self.factor_seconds = int(fb.value), int(dep.value), float(sec.value)
@@ -133,7 +145,8 @@ class SparsifyingPreconditioner:
     """``struct SparsifyingPreconditioner`` (preconditioner.jl:27-58).
 
     As lives on the GPU.  MspInv is the host sparse LU (solverType "UMFPACK" / "MKLPARDISO" as upstream; SuperLU
-    here) or, with solverType="GPU" and the grid size, the device factorisation (no host work inside gmres!).
+    here) or, with solverType="GPU" and the grid size (n, m) or (n, m, l), the device factorisation (no host work
+    inside gmres!).
     """
 
     def __init__(self, Msp, As, solverType="UMFPACK", grid=None):
@@ -148,8 +161,8 @@ class SparsifyingPreconditioner:
         self.MspGPU = None
         if solverType == "GPU":
             if grid is None:
-                raise ValueError("solverType='GPU' needs grid=(n, m)")
-            self.MspGPU = GPUMspFactorization(self.Msp, grid[0], grid[1])
+                raise ValueError("solverType='GPU' needs grid=(n, m) or (n, m, l)")
+            self.MspGPU = GPUMspFactorization(self.Msp, *grid)
             self.MspInv = self.MspGPU
             self._cb = C.cast(None, SOLVE_CB)
             return

@@ -185,9 +185,16 @@ int ls_gmres(ls_handle krylov, ls_handle op, ls_handle As, ls_solve_cb msp_solve
  * is a 9-point stencil matrix on the n x m grid (unknown i + n*j, x fastest), given as Julia holds it (1-based CSC).
  * Factorised on the GPU by geometric nested dissection (multifrontal, partial pivoting inside the pivot blocks);
  * every solve is a fixed sequence of batched matrix-vector kernels - no PCIe traffic, no host work per iteration.
- * 2-D only (a 27-point 3-D matrix keeps the ls_solve_cb route): entries outside the 9-point pattern -> LS_ERR_UNSUPPORTED. */
+ * 2-D grids; ls_msp_factor3d serves the 27-point matrices of 3-D grids.  Entries outside the 9-point pattern ->
+ * LS_ERR_UNSUPPORTED, a duplicate (row, col) entry -> LS_ERR_INVALID, a singular pivot block -> LS_ERR_INVALID (depth
+ * and node named), more device memory needed than is free -> LS_ERR_NOMEM before anything is allocated.           */
 int ls_msp_factor(ls_handle* out, int64_t n, int64_t m, const int64_t* colptr, const int64_t* rowval,
                   const ls_cdouble* nzval);
+/* the same for Msp = As + k^2 AG diag(nu) of examples/example3D.jl:56-61: a 27-point stencil matrix on the n x m x l grid
+ * (unknown i + n*(j + m*p), x fastest), 1-based CSC.  Nested dissection by separator planes; the handle works with
+ * ls_msp_solve / ls_msp_info / ls_msp_plan / ls_gmres_msp unchanged.  l = 1 is exactly ls_msp_factor.              */
+int ls_msp_factor3d(ls_handle* out, int64_t n, int64_t m, int64_t l, const int64_t* colptr, const int64_t* rowval,
+                    const ls_cdouble* nzval);
 /* x <- Msp^-1 rhs (x may alias rhs); host or device pointers per memloc */
 int ls_msp_solve(ls_handle msp, const ls_cdouble* rhs, ls_cdouble* x, int memloc);
 int ls_msp_info(ls_handle msp, int64_t* factor_bytes, int* depth, double* factor_seconds);
@@ -195,7 +202,8 @@ int ls_msp_info(ls_handle msp, int64_t* factor_bytes, int* depth, double* factor
  * group, X staged in shared memory) chosen for its three sweeps; first line: solver version, fusion, tuning time.
  * Writes at most `cap` bytes including the terminator into `buf` (diagnostics for bench / profiles).               */
 int ls_msp_plan(ls_handle msp, char* buf, int64_t cap);
-/* ls_gmres with ldiv!(Pl, v) = Msp^-1 (As v) entirely on the device (`msp` from ls_msp_factor, `As` nullable) */
+/* ls_gmres with ldiv!(Pl, v) = Msp^-1 (As v) entirely on the device (`msp` from ls_msp_factor / ls_msp_factor3d, `As`
+ * nullable); single-GPU: a sharded operator -> LS_ERR_UNSUPPORTED                                                  */
 int ls_gmres_msp(ls_handle krylov, ls_handle op, ls_handle As, ls_handle msp,
                  const ls_cdouble* b, ls_cdouble* x, int restart, int64_t maxiter, double reltol,
                  double abstol, int initially_zero, double* resnorm_hist, int64_t hist_cap,

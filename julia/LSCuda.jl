@@ -190,7 +190,7 @@ end
 
 """
 `lu(Msp)` (preconditioner.jl:35) on the GPU: nested-dissection factorisation of the 9-point matrix Msp of the
-n x m grid.  `F \\ b` solves on host vectors; inside `gmres_gpu!` the solve never leaves the device.
+n x m grid, or (with `l`) of the 27-point matrix of the n x m x l grid (examples/example3D.jl:56-61).  `F \\ b` solves on host vectors; inside `gmres_gpu!` the solve never leaves the device.
 """
 struct GPUMspFactorization
     h::Handle
@@ -202,6 +202,13 @@ function GPUMspFactorization(Msp::SparseMatrixCSC{ComplexF64,Int64}, n::Integer,
     check(ccall((:ls_msp_factor, libls), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{ComplexF64}),
                 out, n, m, Msp.colptr, Msp.rowval, Msp.nzval))
     return GPUMspFactorization(Handle(out[]), n * m)
+end
+function GPUMspFactorization(Msp::SparseMatrixCSC{ComplexF64,Int64}, n::Integer, m::Integer, l::Integer)
+    size(Msp, 1) == size(Msp, 2) == n * m * l || throw(DimensionMismatch("Msp is $(size(Msp)), the grid has $(n*m*l) unknowns"))
+    out = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:ls_msp_factor3d, libls), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{ComplexF64}),
+                out, n, m, l, Msp.colptr, Msp.rowval, Msp.nzval))
+    return GPUMspFactorization(Handle(out[]), n * m * l)
 end
 function \(F::GPUMspFactorization, b::Vector{ComplexF64})
     x = similar(b)
@@ -225,10 +232,10 @@ struct GPUSparsifyingPreconditioner      # preconditioner.jl:27-58
     MspInv                                 # lu(Msp): UMFPACK on the host, or GPUMspFactorization (solverType = "GPU")
     solverType::String
 end
-"solverType = \"UMFPACK\" / \"MKLPARDISO\" as upstream (host LU, reached through the ls_solve_cb callback), or \"GPU\" with grid = (n, m)."
+"solverType = \"UMFPACK\" / \"MKLPARDISO\" as upstream (host LU, reached through the ls_solve_cb callback), or \"GPU\" with grid = (n, m) or (n, m, l)."
 GPUSparsifyingPreconditioner(Msp, As; solverType::String="UMFPACK", grid=nothing) =
     GPUSparsifyingPreconditioner(Msp, GPUSparseMatrixCSC(As),
-                                 solverType == "GPU" ? GPUMspFactorization(Msp, grid[1], grid[2]) : lu(Msp), solverType)
+                                 solverType == "GPU" ? GPUMspFactorization(Msp, grid...) : lu(Msp), solverType)
 \(M::GPUSparsifyingPreconditioner, b::Array{ComplexF64,1}) = M.MspInv \ (M.As * b)                     # :132-145
 function ldiv!(M::GPUSparsifyingPreconditioner, b::AbstractArray{ComplexF64,1})                        # :147-166
     b[:] = M.MspInv \ (M.As * Vector(b))
