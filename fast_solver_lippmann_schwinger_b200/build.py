@@ -47,23 +47,18 @@ def _digest():
     return h.hexdigest()
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), out: str = None) -> str:
-    """defines / out: build a variant of the library (tuning experiments, e.g. defines=("-DLS_LINESB512=8",)) to `out`."""
+def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(LIBDIR, exist_ok=True)
     os.makedirs(OBJDIR, exist_ok=True)
-    variant = bool(defines) or out is not None
-    LIB = out if out is not None else globals()["LIB"]
-    objdir = OBJDIR if not variant else os.path.join(OBJDIR, "variant_" + hashlib.sha1(" ".join(defines).encode()).hexdigest()[:8])
-    os.makedirs(objdir, exist_ok=True)
-    stamp = os.path.join(LIBDIR, "libls_cuda.sha256") if not variant else LIB + ".sha256"
-    digest = _digest() + " ".join(defines)
+    stamp = os.path.join(LIBDIR, "libls_cuda.sha256")
+    digest = _digest()
     if not force and os.path.exists(LIB) and os.path.exists(stamp) and open(stamp).read().strip() == digest:
         return LIB
     nvcc = _nvcc()
-    extra = (["-Xptxas", "-v"] if verbose else []) + list(defines)
+    extra = ["-Xptxas", "-v"] if verbose else []
 
     def compile_one(src):
-        obj = os.path.join(objdir, os.path.basename(src)[:-3] + ".o")
+        obj = os.path.join(OBJDIR, os.path.basename(src)[:-3] + ".o")
         cmd = [nvcc] + NVCC_FLAGS + extra + ["-I", os.path.join(ROOT, "include"), "-c", src, "-o", obj]
         p = subprocess.run(cmd, capture_output=True, text=True)
         if p.returncode != 0:

@@ -204,10 +204,9 @@ template <int N> struct LayA {
 // threads per CTA, so two CTAs fit an SM): a quarter warp spans two points t, t+1 (t even) of four lines, i.e. two
 // 64-byte pieces that must fall into different halves of the 32 banks - true when the two logical addresses differ in
 // parity, which the XOR with bit log2(RLAST) arranges for the last stage (addresses 8t + a and 8(t+1) + a there).
-#ifndef LS_LINESB512
-#define LS_LINESB512 4
-#endif
-template <int N> struct LinesB { static constexpr int value = (N == 512) ? LS_LINESB512 : 8; };
+// Measured on B200 (profiles/r2_l_512_variants.log): 512^3 apply 18.9 ms with LB = 4 against 21.2 ms with LB = 8.
+constexpr int lines_b512 = 4;
+template <int N> struct LinesB { static constexpr int value = (N == 512) ? lines_b512 : 8; };
 template <int N> struct LayB {
     static constexpr int LB = LinesB<N>::value;
     static constexpr int XOR_LANE = LB;          // lane = t * LB + line

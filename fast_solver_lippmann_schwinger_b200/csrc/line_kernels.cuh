@@ -14,7 +14,6 @@
 //                   strided lines (es large, ls == 1) are read/written as 128-byte segments.
 #pragma once
 #include "fft_engine.cuh"
-#include <cooperative_groups.h>
 
 namespace lsk {
 using namespace lsfft;
@@ -35,17 +34,15 @@ template <int N> struct GeoB {
 };
 // resident CTAs per SM asked of ptxas: 128-thread CTAs 3 (168 registers); the 256-thread CTAs of the 4-line mode-B
 // geometry 2 (128 registers: E = 8 points per thread there); everything else 1
-#ifndef LS_INV512_MINB
-#define LS_INV512_MINB 2        // measured (profiles/r2_l_512_variants.log): 512^3 P4 3.67 -> 3.19 ms, 2-D 512^2 apply 0.0353 -> 0.0332 ms
-#endif
 template <int N, bool MODE_B> struct MinB {
     static constexpr int TH = MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static constexpr int value = (TH <= 128) ? 3 : ((MODE_B && GeoB<N>::LB == 4 && TH == 256) ? 2 : 1);
 };
 // the inverse pass keeps E accumulators next to the E working values: at 512 points (E = 16 since r2) the 168-register
-// cap of three CTAs per SM spills inside the loop
+// cap of three CTAs per SM spills inside the loop, so it asks for two.  Measured on B200
+// (profiles/r2_l_512_variants.log): 512^3 P4 3.67 -> 3.19 ms, 2-D 512^2 apply 0.0353 -> 0.0332 ms.
 template <int N, bool MODE_B> struct MinBInv {
-    static constexpr int value = (N == 512 && MinB<N, MODE_B>::value == 3) ? LS_INV512_MINB : MinB<N, MODE_B>::value;
+    static constexpr int value = (N == 512 && MinB<N, MODE_B>::value == 3) ? 2 : MinB<N, MODE_B>::value;
 };
 
 // thread -> (line within CTA, thread within line, smem layout)
@@ -111,13 +108,12 @@ __device__ __forceinline__ long slot_off(const LineAddr& a, long s, long es) {
 __device__ __forceinline__ long line_in(const LineAddr& a, long L) { return (L % a.ldim0) * a.in_ls0 + (L / a.ldim0) * a.in_ls1; }
 __device__ __forceinline__ long line_out(const LineAddr& a, long L) { return (L % a.ldim0) * a.out_ls0 + (L / a.ldim0) * a.out_ls1; }
 
-// per-CTA shared memory: [exchange: LPC*N][(mid only) x copy: LPC*N][(mid only) spectrum: LPC*N][tw1][mbarrier]
+// per-CTA shared memory: [exchange: LPC*N][(mid only) x copy: LPC*N][(mid, mode B only) spectrum: LPC*N][tw1][mbarrier]
 template <int N, bool MODE_B> struct Smem {
     static constexpr int LPC = MODE_B ? GeoB<N>::LPC : GeoA<N>::LPC;
     static constexpr int TW1N = EngTab<N>::TW1N;
     static constexpr int fwd_bytes = (LPC * N + TW1N) * (int)sizeof(cd);
-    static constexpr int mid_bytes = (3 * LPC * N + TW1N) * (int)sizeof(cd) + 16;
-    static constexpr int mid_bytes_direct = (2 * LPC * N + TW1N) * (int)sizeof(cd) + 16;
+    static constexpr int mid_bytes = ((MODE_B ? 3 : 2) * LPC * N + TW1N) * (int)sizeof(cd) + 16;
 };
 
 // ---- forward, pruned: N inputs -> 4N slots -------------------------------------------
@@ -180,18 +176,16 @@ k_fwd_pruned(const cd* __restrict__ in, const double* __restrict__ nu, cd* __res
 // in  : line L point j at in[L*in_ls + j*in_es]
 // G   : spectrum of line L, block r, slot s at G[(L*4 + r)*N + s]                 (mode A)
 //       or at G[((L/8)*4 + r)*8N + s*8 + L%8]                                     (mode B)
-//       -> per (unit, r) one contiguous chunk, fetched by TMA bulk copy into shared memory
-//          while the previous block's inverse transform runs.
+//       mode A: the values go straight from memory into registers, requested before the last butterfly stage
+//       mode B: per (unit, r) one contiguous chunk, fetched by TMA bulk copy into shared memory
+//               while the previous block's inverse transform runs.
 // out : line L point j at out[L*out_ls + j*out_es]  (may alias in when strides agree)
-// ASM: how many of the E per-thread accumulators live in (thread-private) shared memory instead of
-//      registers - the register diet that lets a third CTA fit on the SM (see DESIGN.md section 5).
-template <int N, bool MODE_B, bool GSM = true, int MINB = 1, int ASM = 0>
+template <int N, bool MODE_B, int MINB = 1>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MINB)
 k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict__ TAB,
             const LineAddr la, long line0) {
     typedef Map<N, MODE_B> M;
     constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
-    constexpr int AR = E - ASM, TH = MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     constexpr int LBK = MODE_B ? GeoB<N>::LB : 1;     // lines interleaved in a spectrum chunk
     constexpr int UNIT = LBK * N;                     // points per spectrum chunk
     constexpr int UPC = LPC * N / UNIT;               // chunks per CTA and r
@@ -199,9 +193,8 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
     M mp;
     cd* ex = sm + sm_group_off(mp);
     cd* xs = sm + LPC * N + sm_group_off(mp);   // thread-private copy of the input line
-    cd* gb = sm + 2 * LPC * N;                  // spectrum chunk(s) of the current r (GSM only)
-    cd* accs = sm + (GSM ? 3 : 2) * LPC * N + threadIdx.x;   // accumulator tail, element k at accs[k*TH]
-    cd* tw1 = sm + (GSM ? 3 : 2) * LPC * N + ASM * TH;
+    cd* gb = sm + 2 * LPC * N;                  // spectrum chunk(s) of the current r (mode B only)
+    cd* tw1 = sm + (MODE_B ? 3 : 2) * LPC * N;
     unsigned long long* bar = reinterpret_cast<unsigned long long*>(tw1 + Smem<N, MODE_B>::TW1N);
     const long Lcta = line0 + (long)blockIdx.x * LPC;
     const long L = Lcta + mp.line;
@@ -215,7 +208,7 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
         for (int u = 0; u < UPC; ++u)
             bulk_g2s(gb + u * UNIT, gsrc + ((long)u * nr + rr) * UNIT, (unsigned)(UNIT * sizeof(cd)), bar);
     };
-    if (GSM && threadIdx.x == 0) {
+    if (MODE_B && threadIdx.x == 0) {
         mbar_init(bar, 1);
         fence_proxy_async();
         issue_g(0);
@@ -227,22 +220,19 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
 #pragma unroll
         for (int a = 0; a < E; ++a) xs[mp.lay.phys(a * T + t)] = p[(long)(a * T) * la.in_es];
     }
-    // direct-load variant: pull spectrum chunk r into L2 one r ahead (one request per 128-byte line)
+    // mode A: pull spectrum chunk r into L2 one r ahead (one request per 128-byte line)
     auto prefetch_g = [&](int rr) {
-        if (!GSM && rr < nr) {
-            const cd* g = MODE_B ? gsrc + ((long)(mp.line / LBK) * nr + rr) * UNIT + mp.lay_lam()
-                                 : gsrc + ((long)mp.line * nr + rr) * UNIT;
-            constexpr int gs = LBK;
-            if (MODE_B ? (mp.lay_lam() == 0) : ((t & 7) == 0)) {
+        if (!MODE_B && rr < nr) {
+            const cd* g = gsrc + ((long)mp.line * nr + rr) * UNIT;
+            if ((t & 7) == 0) {
 #pragma unroll
-                for (int e = 0; e < E; ++e) prefetch_l2(&g[(t + T * e) * gs]);
+                for (int e = 0; e < E; ++e) prefetch_l2(&g[t + T * e]);
             }
         }
     };
     prefetch_g(0);
     __syncthreads();   // tw1 + mbarrier init visible
-    cd acc[AR];
-    const int goff = MODE_B ? 0 : mp.line * N;     // mode B: lay.phys already interleaves the 8 lines
+    cd acc[E];
 #pragma unroll 1
     for (int rr = 0; rr < nr; ++rr) {
         const int r = rr * rstep;
@@ -250,79 +240,44 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
 #pragma unroll
         for (int a = 0; a < E; ++a) v[a] = xs[mp.lay.phys(a * T + t)];
         prefetch_g(rr + 1);
-        if (!GSM && MINB >= 3) {
-            // three CTAs per SM: registers are the scarce resource, the other CTAs hide the load latency
-            fft_fwd<N>(v, t, r, ex, mp.lay, tw);
-            const cd* g = MODE_B ? gsrc + ((long)(mp.line / LBK) * nr + rr) * UNIT + mp.lay_lam()
-                                 : gsrc + ((long)mp.line * nr + rr) * UNIT;
-            constexpr int gs = LBK;
-#pragma unroll
-            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], __ldg(&g[(t + T * e) * gs]));
-        } else if (!GSM) {
-            // spectrum values are requested before the last butterfly stage and consumed after it
-            cd gv[E];
-            fft_fwd<N>(v, t, r, ex, mp.lay, tw, [&]() {
-                const cd* g = MODE_B ? gsrc + ((long)(mp.line / LBK) * nr + rr) * UNIT + mp.lay_lam()
-                                     : gsrc + ((long)mp.line * nr + rr) * UNIT;
-                constexpr int gs = LBK;
-#pragma unroll
-                for (int e = 0; e < E; ++e) gv[e] = __ldg(&g[(t + T * e) * gs]);
-            });
-#pragma unroll
-            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], gv[e]);
-        } else {
-        fft_fwd<N>(v, t, r, ex, mp.lay, tw);
-        mbar_wait(bar, (unsigned)(rr & 1));
         if (MODE_B) {
+            fft_fwd<N>(v, t, r, ex, mp.lay, tw);
+            mbar_wait(bar, (unsigned)(rr & 1));
             const cd* g = gb + sm_group_off(mp);
 #pragma unroll
             for (int e = 0; e < E; ++e) v[e] = cmul(v[e], g[(t + T * e) * LBK + mp.lay_lam()]);
         } else {
-            const cd* g = gb + goff;
+            // spectrum values are requested before the last butterfly stage and consumed after it
+            cd gv[E];
+            fft_fwd<N>(v, t, r, ex, mp.lay, tw, [&]() {
+                const cd* g = gsrc + ((long)mp.line * nr + rr) * UNIT;
 #pragma unroll
-            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], g[t + T * e]);
-        }
+                for (int e = 0; e < E; ++e) gv[e] = __ldg(&g[t + T * e]);
+            });
+#pragma unroll
+            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], gv[e]);
         }
         fft_inv<N>(v, t, r, ex, mp.lay, tw, [&]() {
             // every thread has consumed gb (the multiply precedes this barrier): refill it
-            if (GSM && rr + 1 < nr && threadIdx.x == 0) {
+            if (MODE_B && rr + 1 < nr && threadIdx.x == 0) {
                 fence_proxy_async();
                 issue_g(rr + 1);
             }
         });
-        if (ASM == 0) {
-            demod_accumulate<N>(acc, v, r);
-        } else if (r == 0) {
-#pragma unroll
-            for (int a = 0; a < AR; ++a) acc[a] = v[a];
-#pragma unroll
-            for (int a = AR; a < E; ++a) accs[(a - AR) * TH] = v[a];
-        } else {
-            acc[0] = cadd(acc[0], v[0]);
-#pragma unroll
-            for (int a = 1; a < AR; ++a) acc[a] = cfmac(v[a], c64(r * a * (16 / E)), acc[a]);
-#pragma unroll
-            for (int a = AR; a < E; ++a) accs[(a - AR) * TH] = cfmac(v[a], c64(r * a * (16 / E)), accs[(a - AR) * TH]);
-        }
+        demod_accumulate<N>(acc, v, r);
     }
     cd* o = out + line_out(la, L) + (long)t * la.out_es;
 #pragma unroll
-    for (int a = 0; a < AR; ++a) o[(long)(a * T) * la.out_es] = acc[a];
-#pragma unroll
-    for (int a = AR; a < E; ++a) o[(long)(a * T) * la.out_es] = accs[(a - AR) * TH];
+    for (int a = 0; a < E; ++a) o[(long)(a * T) * la.out_es] = acc[a];
 }
 
 // ---- middle, fused, 2x padding, no accumulator registers ("swap" variant, mode A) ----------------------------
-// Same arithmetic and the same bits as k_mid_fused with nr = 2 and direct spectrum loads.  k_mid_fused keeps the
-// input line in shared memory AND 16 accumulators in registers (248 registers: two 128-thread CTAs per SM, and the
-// pass is latency-bound at 8 warps per SM).  With two sub-transforms only one thread-private buffer is needed: it
+// Same arithmetic and the same bits as k_mid_fused with nr = 2 in mode A.  k_mid_fused keeps the input line in shared
+// memory AND 16 accumulators in registers.  With two sub-transforms only one thread-private buffer is needed: it
 // holds the input line x while r = 0 is transformed, then x and the r = 0 result trade places (each thread swaps
-// its own 16 elements, no barrier), and the r = 2 result is combined with the held one on the way out.  Without
-// the accumulators the kernel fits 168 registers and 66 KB of shared memory: three CTAs per SM.
-// GL: how the spectrum chunk reaches the multiply.  0: all E values requested before the last butterfly stage and
-// held in registers across it (64 more live registers); 1: the chunk is pulled into L2 by prefetches issued before
-// the last butterfly stage and loaded right at the multiply (the other CTAs of the SM cover the L2 latency).
-template <int N, int MINB, int GL>
+// its own 16 elements, no barrier), and the r = 2 result is combined with the held one on the way out.  The spectrum
+// values are requested before the last butterfly stage and held in registers across it.
+template <int N, int MINB>
 __global__ void __launch_bounds__(GeoA<N>::THREADS, MINB)
 k_mid_swap(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict__ TAB, const LineAddr la, long line0) {
     typedef Map<N, false> M;
@@ -350,24 +305,13 @@ k_mid_swap(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict
     for (int rr = 0; rr < 2; ++rr) {
         const int r = 2 * rr;
         const cd* g = gline + (long)rr * N;
-        if constexpr (GL == 0) {
-            cd gv[E];
-            fft_fwd<N>(v, t, r, ex, mp.lay, tw, [&]() {
+        cd gv[E];
+        fft_fwd<N>(v, t, r, ex, mp.lay, tw, [&]() {
 #pragma unroll
-                for (int e = 0; e < E; ++e) gv[e] = __ldg(&g[t + T * e]);
-            });
+            for (int e = 0; e < E; ++e) gv[e] = __ldg(&g[t + T * e]);
+        });
 #pragma unroll
-            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], gv[e]);
-        } else {
-            fft_fwd<N>(v, t, r, ex, mp.lay, tw, [&]() {
-                if ((t & 7) == 0) {       // one request per 128-byte line
-#pragma unroll
-                    for (int e = 0; e < E; ++e) prefetch_l2(&g[t + T * e]);
-                }
-            });
-#pragma unroll
-            for (int e = 0; e < E; ++e) v[e] = cmul(v[e], __ldg(&g[t + T * e]));
-        }
+        for (int e = 0; e < E; ++e) v[e] = cmul(v[e], gv[e]);
         fft_inv<N>(v, t, r, ex, mp.lay, tw);
         if (rr == 0) {
             // x and the r = 0 result trade places
@@ -385,7 +329,7 @@ k_mid_swap(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict
     for (int a = 1; a < E; ++a) o[(long)(a * T) * la.out_es] = cfmac(v[a], c64(2 * a * (16 / E)), hold[a * TH]);
 }
 
-// cp.async helpers (inverse pass staging; experiment kernels)
+// cp.async helpers (inverse pass staging)
 __device__ __forceinline__ void cp_async16(void* dst_smem, const void* src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src) : "memory");
 }
@@ -395,11 +339,11 @@ template <int K> __device__ __forceinline__ void cp_async_wait() { asm volatile(
 // ---- inverse, pruned: 4N slots -> N outputs, optional identity-plus-contrast combine --
 // in  : line L slot s at in[L*in_ls + s*in_es]
 // out : line L point j at out[L*out_ls + j*out_es];  if bsrc: out = bsrc + scale*result
-// PF: contiguous lines only - pull the next slot block (and the b values) into L2 one block ahead
-// PF = 1: next block / b values prefetched into L2.  PF = 2: next block / b values staged in shared memory by
-// cp.async while the current block is transformed (each thread stages exactly the elements it consumes: no
-// extra barrier), which takes two of the kernel's three exposed DRAM latencies off the critical path.
-template <int N, bool MODE_B, int PF = 0>
+// STAGED: the next slot block (at the end, the b values) is staged in shared memory by cp.async while the current
+// block is transformed (each thread stages exactly the elements it consumes: no extra barrier), which takes two of
+// the kernel's three exposed DRAM latencies off the critical path.  The applies run staged; the set-up passes of the
+// compact spectrum do not.
+template <int N, bool MODE_B, bool STAGED = false>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MinBInv<N, MODE_B>::value)
 k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __restrict__ TAB, double scale,
              const LineAddr la, long line0) {
@@ -418,13 +362,13 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
     cd acc[E];
     const int nr = la.nr, rstep = 4 / la.nr;
     constexpr int TH = MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
-    cd* stg = sm + LPC * N + EngTab<N>::TW1N + threadIdx.x;      // PF == 2: element e of this thread at stg[TH*e]
+    cd* stg = sm + LPC * N + EngTab<N>::TW1N + threadIdx.x;      // STAGED: element e of this thread at stg[TH*e]
 #pragma unroll 1
     for (int rr = 0; rr < nr; ++rr) {
         const int r = rr * rstep;
         cd v[E];
         const cd* p = in + in_base;
-        if (PF == 2 && rr > 0) {
+        if (STAGED && rr > 0) {
             cp_async_wait<0>();
 #pragma unroll
             for (int e = 0; e < E; ++e) v[e] = stg[TH * e];
@@ -432,10 +376,7 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
 #pragma unroll
             for (int e = 0; e < E; ++e) v[e] = p[slot_off(la, (long)(rr * N + t + T * e), la.in_es)];
         }
-        // pull the next block (or, at the end, the b values of the combine) into L2 while this one is transformed
-        // (contiguous lines only: measured on B200, prefetching scattered 16-byte pieces costs more L2
-        //  requests than the latency it hides - 2-D P3 0.177 -> 0.223 ms, 3-D P5 0.54 -> 0.44 ms)
-        if (PF == 2) {
+        if (STAGED) {
             if (rr + 1 < nr) {
 #pragma unroll
                 for (int e = 0; e < E; ++e) cp_async16(&stg[TH * e], &p[slot_off(la, (long)((rr + 1) * N + t + T * e), la.in_es)]);
@@ -445,15 +386,6 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
                 for (int a = 0; a < E; ++a) cp_async16(&stg[TH * a], &bsrc[out_base + (long)(a * T + t) * la.out_es]);
                 cp_async_commit();
             }
-        } else if (!PF) {
-        } else if (rr + 1 < nr) {
-            if (!MODE_B && la.in_es == 1 && (t & 7) == 0) {
-#pragma unroll
-                for (int e = 0; e < E; ++e) prefetch_l2(&p[slot_off(la, (long)((rr + 1) * N + t + T * e), 1)]);
-            }
-        } else if (bsrc != nullptr && !MODE_B && la.in_es == 1 && (t & 7) == 0) {
-#pragma unroll
-            for (int a = 0; a < E; ++a) prefetch_l2(&bsrc[out_base + (long)(a * T + t) * la.out_es]);
         }
         fft_inv<N>(v, t, r, ex, mp.lay, tw);
         if (la.cblock == 0) demod_accumulate<N>(acc, v, r);
@@ -465,9 +397,9 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
         long off = out_base + (long)(a * T + t) * la.out_es;
         cd res = cscale(acc[a], scale);
         if (bsrc != nullptr) {
-            if (PF == 2 && a == 0) cp_async_wait<0>();
-            const cd bv = (PF == 2) ? stg[TH * a] : bsrc[off];
-            res = make_double2(__fma_rn(acc[a].x, scale, bv.x), __fma_rn(acc[a].y, scale, bv.y));   // one rounding, same bits in every variant
+            if (STAGED && a == 0) cp_async_wait<0>();
+            const cd bv = STAGED ? stg[TH * a] : bsrc[off];
+            res = make_double2(__fma_rn(acc[a].x, scale, bv.x), __fma_rn(acc[a].y, scale, bv.y));   // one rounding, same bits staged or not
         }
         out[off] = res;
     }
@@ -502,36 +434,41 @@ inline cudaError_t launch_fwd(cudaStream_t s, long nlines, const cd* in, const d
     return cudaPeekAtLastError();
 }
 
-template <int N, bool B, bool GSM>
+template <int N, bool B>
 inline cudaError_t launch_mid(cudaStream_t s, long nlines, const cd* in, cd* out, const cd* G, const cd* TAB,
                               const LineAddr& la) {
-    constexpr int smem = GSM ? Smem<N, B>::mid_bytes : Smem<N, B>::mid_bytes_direct;
+    constexpr int smem = Smem<N, B>::mid_bytes;
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
     constexpr int MB = (B && GeoB<N>::LB == 4) ? 2 : 1;      // 4-line geometry: two CTAs per SM (128 registers)
-    { cudaError_t e = smem_optin(k_mid_fused<N, B, GSM, MB>, smem, optin); if (e != cudaSuccess) return e; }
-    k_mid_fused<N, B, GSM, MB><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, out, G, TAB, la, 0);
+    { cudaError_t e = smem_optin(k_mid_fused<N, B, MB>, smem, optin); if (e != cudaSuccess) return e; }
+    k_mid_fused<N, B, MB><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, out, G, TAB, la, 0);
     return cudaPeekAtLastError();
 }
 
-template <int N, int MINB, int GL>
+// CTAs per SM asked of ptxas: 3 up to N = 256, 2 from 512 to 2048, 1 at 4096 (256-thread CTAs).  Measured on B200
+// (profiles/r2_e_notes.md): at N >= 1024 three CTAs are slower than two (168-register cap -> spills, and 3 x 66 KB of
+// shared memory leaves 30 KB of L1 for the strided line loads: 2048^2 0.297 vs 0.211 ms); at small N several lines
+// share a CTA and three CTAs win.
+template <int N>
 inline cudaError_t launch_mid_swap(cudaStream_t s, long nlines, const cd* in, cd* out, const cd* G, const cd* TAB,
                                    const LineAddr& la) {
+    constexpr int MINB = GeoA<N>::THREADS > 128 ? 1 : (N <= 256 ? 3 : 2);
     constexpr int smem = (2 * GeoA<N>::LPC * N + EngTab<N>::TW1N) * (int)sizeof(cd);
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_mid_swap<N, MINB, GL>, smem, optin); if (e != cudaSuccess) return e; }
-    k_mid_swap<N, MINB, GL><<<(unsigned)(nlines / GeoA<N>::LPC), GeoA<N>::THREADS, smem, s>>>(in, out, G, TAB, la, 0);
+    { cudaError_t e = smem_optin(k_mid_swap<N, MINB>, smem, optin); if (e != cudaSuccess) return e; }
+    k_mid_swap<N, MINB><<<(unsigned)(nlines / GeoA<N>::LPC), GeoA<N>::THREADS, smem, s>>>(in, out, G, TAB, la, 0);
     return cudaPeekAtLastError();
 }
 
-template <int N, bool B, int PF = 0>
+template <int N, bool B, bool STAGED = false>
 inline cudaError_t launch_inv(cudaStream_t s, long nlines, const cd* in, const cd* bsrc, cd* out, const cd* TAB,
                               double scale, const LineAddr& la) {
-    constexpr int smem = Smem<N, B>::fwd_bytes + (PF == 2 ? Smem<N, B>::LPC * N * (int)sizeof(cd) : 0);
+    constexpr int smem = Smem<N, B>::fwd_bytes + (STAGED ? Smem<N, B>::LPC * N * (int)sizeof(cd) : 0);
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_inv_pruned<N, B, PF>, smem, optin); if (e != cudaSuccess) return e; }
-    k_inv_pruned<N, B, PF><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, bsrc, out, TAB, scale, la, 0);
+    { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED>, smem, optin); if (e != cudaSuccess) return e; }
+    k_inv_pruned<N, B, STAGED><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, bsrc, out, TAB, scale, la, 0);
     return cudaPeekAtLastError();
 }
 

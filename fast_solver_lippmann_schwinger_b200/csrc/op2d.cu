@@ -2,7 +2,7 @@
 // Stands behind struct FastM and its `*` / mul! / fastconvolution / FFTconvolution methods
 // (reference FastConvolution.jl:11-154).  Three launches per apply:
 //   P1  k_fwd_pruned  columns (x, contiguous):  b, nu      -> A  [ne x m]   (slot order in x)
-//   P2  k_mid_fused   rows (y): A, Green spectrum          -> C  [m x ne]   (line contiguous)
+//   P2  k_mid_swap    rows (y): A, Green spectrum          -> C  [m x ne]   (k_mid_fused with LS_FLAG_PAD4)
 //   P3  k_inv_pruned  columns (x): C, b                    -> y
 // Padding.  The reference pads 4x per dimension (Greengard_Vico) because the truncated-kernel spectrum has
 // to be *built* on the 4n grid; the apply itself only ever touches the spatial kernel g = ifft2(GFFT) at the
@@ -18,14 +18,16 @@
 #include "op2d_base.cuh"
 #include "line_kernels.cuh"
 #include "gv_spectrum2d.cuh"
-#ifdef LS_EXPERIMENTS
-#include "line_kernels_experiments.cuh"   // measured-and-rejected variants: only with -DLS_EXPERIMENTS (profiles/r1_b_notes.md)
-#endif
 
 using namespace ls;
 using namespace lsk;
 
 namespace {
+
+// x-slot interleave of the P2 -> P3 intermediate C: P3's strided reads then cover 64-byte runs.  Measured at 2048^2 on
+// B200: P2 + P3 = 0.326 / 0.313 / 0.304 / 0.31 ms for 1 / 2 / 4 / 8 interleaved slots.
+constexpr int CW_SHIFT = 2;
+constexpr long CW = 1L << CW_SHIFT;
 
 struct Op2D : Op2DBase {
     int nr = 4;               // padding factor actually used by the applies (4: literal, 2: compact)
@@ -34,8 +36,7 @@ struct Op2D : Op2DBase {
     cd* d_G = nullptr;        // [sx][ry][slot_y] on the pn x pm grid, normalisation folded in
     cd* d_TABn = nullptr; cd* d_TABm = nullptr;   // engine tables (fft_engine.cuh EngTab)
     cd* d_A = nullptr;        // pn x m
-    cd* d_C = nullptr;        // P2 output: slot sx of column j at C[(sx/cw)*(cw*m) + cw*j + sx%cw]
-    int cw = 1;               // x-slot interleave of C: P3's strided reads then cover whole sectors (default 4: 64-byte runs)
+    cd* d_C = nullptr;        // P2 output: slot sx of column j at C[(sx/CW)*(CW*m) + CW*j + sx%CW]
     int apply_dev(const cd* b, cd* y, int mode) override;
 };
 
@@ -85,185 +86,6 @@ __global__ void k_fill_g2d_centred(cd* __restrict__ gout, long ne, long me, Gv2d
     gout[idx] = gtrunc2d_eval(p, idx % ne, idx / ne, ne, me);
 }
 
-template <int N> int launch_fwd(Op2D* op, const cd* b, const double* nu) {
-    constexpr int smem = Smem<N, false>::fwd_bytes;
-    static unsigned long long optin = 0;
-    LS_CUDA_TRY(smem_optin(k_fwd_pruned<N, false>, smem, optin));
-    dim3 grid((unsigned)(op->m / GeoA<N>::LPC));
-    LineAddr la{1L << 40, op->n, 0, 1, op->pn, 0, 1};
-    la.nr = op->nr;
-    op->phase_begin(0);
-    k_fwd_pruned<N, false><<<grid, GeoA<N>::THREADS, smem, op->stream>>>(b, nu, op->d_A, op->d_TABn, la, 0);
-    op->phase_end();
-    op->launches++;
-    return LS_OK;
-}
-template <int N, bool GSM, int MINB, int ASM = 0> int launch_mid_v(Op2D* op) {
-    static int extra = -1;      // diagnostic: LS_P2_EXTRA_SMEM pads the request to lower the CTAs/SM
-    if (extra < 0) { const char* e = getenv("LS_P2_EXTRA_SMEM"); extra = e ? atoi(e) : 0; }
-    const int smem = (GSM ? Smem<N, false>::mid_bytes : Smem<N, false>::mid_bytes_direct) + extra
-                     + ASM * GeoA<N>::THREADS * (int)sizeof(cd);
-    static unsigned long long optin = 0;
-    LS_CUDA_TRY(smem_optin(k_mid_fused<N, false, GSM, MINB, ASM>, smem, optin));
-    dim3 grid((unsigned)(op->pn / GeoA<N>::LPC));
-    // line = x slot sx; point j at A[sx + pn*j]; output: cw adjacent x-slots interleaved, C[(sx/cw)*(cw*m) + cw*j + sx%cw]
-    const long cw = op->cw;
-    LineAddr la{cw, 1, cw, op->pn, 1, cw * op->m, cw};
-    la.nr = op->nr;
-    op->phase_begin(1);
-    k_mid_fused<N, false, GSM, MINB, ASM><<<grid, GeoA<N>::THREADS, smem, op->stream>>>(
-        op->d_A, op->d_C, op->d_G, op->d_TABm, la, 0);
-    op->phase_end();
-    op->launches++;
-    return LS_OK;
-}
-#ifdef LS_EXPERIMENTS
-template <int N, int ASM> int launch_mid_dual(Op2D* op) {
-    const int smem = (3 * GeoA<N>::LPC * N + EngTab<N>::TW1N + ASM * GeoA<N>::THREADS) * (int)sizeof(cd);
-    static unsigned long long optin = 0;
-    LS_CUDA_TRY(smem_optin(k_mid_fused_dual<N, ASM>, smem, optin));
-    dim3 grid((unsigned)(op->ne / GeoA<N>::LPC));
-    op->phase_begin(1);
-    k_mid_fused_dual<N, ASM><<<grid, GeoA<N>::THREADS, smem, op->stream>>>(
-        op->d_A, op->d_C, op->d_G, op->d_TABm, LineAddr{1L << 40, 1, 0, op->ne, op->m, 0, 1}, 0);
-    op->phase_end();
-    op->launches++;
-    return LS_OK;
-}
-#endif
-// 2x padding: the swap kernel (no accumulator registers, three CTAs per SM; see line_kernels.cuh)
-template <int N> int launch_mid_swap_op(Op2D* op) {
-    const long cw = op->cw;
-    LineAddr la{cw, 1, cw, op->pn, 1, cw * op->m, cw};
-    la.nr = 2;
-    static int gl = -1, minb = -1;   // LS_P2_GLOAD: 0 spectrum held in registers across the last stage, 1 L2 prefetch + load at the multiply
-    if (gl < 0) { const char* e = getenv("LS_P2_GLOAD"); gl = e ? atoi(e) : 0; }
-    // CTAs per SM (128-thread CTAs).  Measured on B200 (profiles/r2_e_notes.md): at N >= 1024 three CTAs are slower than two
-    // (168-register cap -> spills, and 3 x 66 KB of shared memory leaves 30 KB of L1 for the strided line loads:
-    // 2048^2 0.297 vs 0.211 ms); at N <= 512 several lines share a CTA and three CTAs win (512^2 0.0189 vs 0.0194 ms).
-    if (minb < 0) { const char* e = getenv("LS_P2_MINB"); minb = e ? atoi(e) : 0; }
-    const int use_minb = minb ? minb : (N <= 256 ? 3 : 2);      // 16 points per thread from N = 512 up
-    constexpr int MB = (GeoA<N>::THREADS <= 128 ? 3 : 1);
-    op->phase_begin(1);
-    cudaError_t e;
-    constexpr int MB2 = (MB == 3 ? 2 : 1);      // 128-thread CTAs: two per SM by default (255 registers, no spills)
-    if (use_minb == 2 || MB == 1) e = gl ? lsk::launch_mid_swap<N, MB2, 1>(op->stream, op->pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
-                                     : lsk::launch_mid_swap<N, MB2, 0>(op->stream, op->pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la);
-    else e = gl ? lsk::launch_mid_swap<N, MB, 1>(op->stream, op->pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
-                : lsk::launch_mid_swap<N, MB, 0>(op->stream, op->pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la);
-    op->phase_end();
-    op->launches++;
-    LS_CUDA_TRY(e);
-    return LS_OK;
-}
-template <int N> int launch_mid(Op2D* op) {
-    static int kernel = -1;          // LS_P2_KERNEL: 1 (default) swap kernel, 0 k_mid_fused (accumulators in registers)
-    if (kernel < 0) { const char* e = getenv("LS_P2_KERNEL"); kernel = e ? atoi(e) : 1; }
-    if (op->nr == 2 && kernel == 1) return launch_mid_swap_op<N>(op);
-#ifndef LS_EXPERIMENTS
-    return launch_mid_v<N, false, 1>(op);       // spectrum straight from HBM into registers, requested before the last butterfly stage
-#else
-    static int variant = -1;
-    if (op->nr != 4) return launch_mid_v<N, false, 1>(op);      // the experiment kernels below are 4x-padding only
-    // variants measured on B200 at 2048^2 (profiles/r1_b_notes.md): 1 = spectrum straight from HBM into
-    // registers (0.706 ms), 0 = spectrum staged in shared memory by TMA bulk copies (0.761 ms)
-    if (variant < 0) { const char* e = getenv("LS_P2_VARIANT"); variant = e ? atoi(e) : 1; }
-    if (variant == 0) return launch_mid_v<N, true, 1>(op);
-    // experiment kept for the record: persistent CTAs, next input line prefetched by cp.async (0.714-0.720 ms)
-    if constexpr (N == 2048) if (variant == 8) {
-        static int ctas = -1;
-        if (ctas < 0) { const char* e = getenv("LS_P2_CTAS"); ctas = e ? atoi(e) : 2 * 148; }
-        op->phase_begin(1);
-        cudaError_t e = launch_mid_persist<N>(op->stream, op->ne, op->d_A, op->d_C, op->d_G, op->d_TABm,
-                                              LineAddr{1L << 40, 1, 0, op->ne, op->m, 0, 1}, ctas);
-        op->phase_end();
-        op->launches++;
-        LS_CUDA_TRY(e);
-        return LS_OK;
-    }
-    // experiment kept for the record: one sub-transform per CTA, thread-block cluster of 4, DSMEM reduction
-    // (3-4 CTAs/SM, no spills, bit-identical result - but 1.05-1.08 ms at 2048^2: two cluster.sync() per CTA and
-    // four times the per-CTA fixed costs outweigh the better pipe overlap)
-    if constexpr (N == 2048) if (variant == 6 || variant == 7) {
-        op->phase_begin(1);
-        const LineAddr la{1L << 40, 1, 0, op->ne, op->m, 0, 1};
-        cudaError_t e = (variant == 6) ? launch_mid_cluster<N, false, 3>(op->stream, op->ne, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
-                                       : launch_mid_cluster<N, false, 4>(op->stream, op->ne, op->d_A, op->d_C, op->d_G, op->d_TABm, la);
-        op->phase_end();
-        op->launches++;
-        LS_CUDA_TRY(e);
-        return LS_OK;
-    }
-    // experiment kept for the record (profiles/r1_b_notes.md): two sub-transforms in flight per thread;
-    // correct, but 255 registers + 590 B of spills make it slower (0.92 ms) - instantiated for 2048 only
-    if constexpr (N == 2048) { if (variant == 5) return launch_mid_dual<N, 4>(op); }
-    if (variant == 2) return launch_mid_v<N, false, 3, 4>(op);
-    if (variant == 3) return launch_mid_v<N, false, 3, 2>(op);
-    return launch_mid_v<N, false, 1>(op);
-#endif
-}
-template <int N, int PF> int launch_inv_v(Op2D* op, const cd* bsrc, cd* y, double scale) {
-    constexpr int smem = Smem<N, false>::fwd_bytes + (PF == 2 ? Smem<N, false>::LPC * N * (int)sizeof(cd) : 0);
-    static unsigned long long optin = 0;
-    LS_CUDA_TRY(smem_optin(k_inv_pruned<N, false, PF>, smem, optin));
-    dim3 grid((unsigned)(op->m / GeoA<N>::LPC));
-    // line = column j; slot sx at C[(sx/cw)*(cw*m) + cw*j + sx%cw]: adjacent lanes read adjacent slots
-    const long cw = op->cw;
-    int cshift = 0;
-    while ((1L << cshift) < cw) ++cshift;
-    LineAddr la{1L << 40, cw, 0, 1, op->n, 0, 1};
-    la.split_shift = cshift; la.split_stride = cw * op->m;
-    la.nr = op->nr;
-    op->phase_begin(2);
-    k_inv_pruned<N, false, PF><<<grid, GeoA<N>::THREADS, smem, op->stream>>>(op->d_C, bsrc, y, op->d_TABn, scale, la, 0);
-    op->phase_end();
-    op->launches++;
-    return LS_OK;
-}
-template <int N> int launch_inv(Op2D* op, const cd* bsrc, cd* y, double scale) {
-    // LS_P3_STAGE: 1 (default) = next slot block and b staged in shared memory by cp.async while the current block is
-    // transformed, 0 = plain loads (2048^2 on B200: 0.131 -> 0.077 ms together with the 4-slot interleave of C)
-    static int stage = -1;
-    if (stage < 0) { const char* e = getenv("LS_P3_STAGE"); stage = e ? atoi(e) : 1; }
-    return stage ? launch_inv_v<N, 2>(op, bsrc, y, scale) : launch_inv_v<N, 0>(op, bsrc, y, scale);
-}
-
-#define LS_DISPATCH_N(N_, CALL)                                       \
-    switch (N_) {                                                     \
-        case 64:   rc = CALL(64); break;                              \
-        case 128:  rc = CALL(128); break;                             \
-        case 256:  rc = CALL(256); break;                             \
-        case 512:  rc = CALL(512); break;                             \
-        case 1024: rc = CALL(1024); break;                            \
-        case 2048: rc = CALL(2048); break;                            \
-        case 4096: rc = CALL(4096); break;                            \
-        default: rc = LS_ERR_UNSUPPORTED;                             \
-    }
-
-int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
-    int rc = LS_OK;
-    const double* nu = (mode == LS_APPLY_FASTCONVOLUTION) ? op->d_nu : nullptr;   // Q2: GV FFTconvolution has no nu
-#define CALL_FWD(N) launch_fwd<N>(op, b, nu)
-    LS_DISPATCH_N(op->n, CALL_FWD);
-    if (rc) return rc;
-#define CALL_MID(N) launch_mid<N>(op)
-    LS_DISPATCH_N(op->m, CALL_MID);
-    if (rc) return rc;
-    const cd* bsrc = (mode == LS_APPLY_FASTCONVOLUTION) ? b : nullptr;
-    double scale = (mode == LS_APPLY_FASTCONVOLUTION) ? op->omega * op->omega : 1.0;
-#define CALL_INV(N) launch_inv<N>(op, bsrc, y, scale)
-    LS_DISPATCH_N(op->n, CALL_INV);
-    if (rc) return rc;
-    LS_CUDA_TRY(cudaGetLastError());
-    return LS_OK;
-}
-
-}  // namespace
-
-int Op2D::apply_dev(const cd* b, cd* y, int mode) { return apply_device(this, b, y, mode); }
-
-namespace {
-
 #define LS_DISPATCH_E(N_, CALL)                                                    \
     switch (N_) {                                                                  \
         case 64:   e = CALL(64); break;                                            \
@@ -275,6 +97,56 @@ namespace {
         case 4096: e = CALL(4096); break;                                          \
         default: e = cudaErrorInvalidValue;                                        \
     }
+
+int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
+    cudaError_t e = cudaSuccess;
+    cudaStream_t s = op->stream;
+    const long n = op->n, m = op->m, pn = op->pn;
+    const bool full = (mode == LS_APPLY_FASTCONVOLUTION);
+    const double* nu = full ? op->d_nu : nullptr;   // Q2: GV FFTconvolution has no nu
+    // P1: columns (x, contiguous): point i of column j at b[i + n*j] -> slot sx at A[sx + pn*j]
+    {
+        LineAddr la{1L << 40, n, 0, 1, pn, 0, 1};
+        la.nr = op->nr;
+        op->phase_begin(0);
+#define P1(N) launch_fwd<N, false>(s, m, b, nu, op->d_A, op->d_TABn, la)
+        LS_DISPATCH_E(n, P1);
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    // P2: rows (y): line = x slot sx, point j at A[sx + pn*j]; output: CW adjacent x-slots interleaved,
+    //     C[(sx/CW)*(CW*m) + CW*j + sx%CW].  2x padding: the swap kernel (no accumulator registers, see line_kernels.cuh)
+    {
+        LineAddr la{CW, 1, CW, pn, 1, CW * m, CW};
+        la.nr = op->nr;
+        op->phase_begin(1);
+#define P2S(N) launch_mid_swap<N>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
+#define P2F(N) launch_mid<N, false>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
+        if (op->nr == 2) { LS_DISPATCH_E(m, P2S); } else { LS_DISPATCH_E(m, P2F); }
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    // P3: columns (x) + combine: line = column j; slot sx at C[(sx/CW)*(CW*m) + CW*j + sx%CW]: adjacent lanes read
+    //     adjacent slots.  The next slot block and b are staged in shared memory while the current block is transformed
+    //     (2048^2 on B200: 0.131 -> 0.077 ms together with the 4-slot interleave of C)
+    {
+        LineAddr la{1L << 40, CW, 0, 1, n, 0, 1};
+        la.split_shift = CW_SHIFT; la.split_stride = CW * m;
+        la.nr = op->nr;
+        op->phase_begin(2);
+#define P3(N) launch_inv<N, false, true>(s, m, op->d_C, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
+        LS_DISPATCH_E(n, P3);
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    return LS_OK;
+}
+
+}  // namespace
+
+int Op2D::apply_dev(const cd* b, cd* y, int mode) { return apply_device(this, b, y, mode); }
+
+namespace {
 
 // Compact (2x) spectrum from the reference's 4x one.  g4s: [sx4][ry][sy] slot order on the 4n x 4m grid,
 // already scaled by 1/(ne me).  On return op->d_G holds G2 = fft2(g wrapped onto 2n x 2m) in the slot order
@@ -425,14 +297,6 @@ static int op2d_create_impl(ls_handle* out, int64_t n, int64_t m, int64_t ne, in
         TRY(compact_spectrum(op, g4s));
     }
     op->pn = op->nr * n; op->pm = op->nr * m;
-    {   // x-slot interleave of the P2 -> P3 intermediate (LS_C_INTERLEAVE = 1 / 2 / 4 / 8, diagnostic)
-        const char* ev = getenv("LS_C_INTERLEAVE");
-        int cw = ev ? atoi(ev) : 4;        // measured at 2048^2: P2 + P3 = 0.326 / 0.313 / 0.304 / 0.31 ms for 1 / 2 / 4 / 8
-        if (cw != 1 && cw != 2 && cw != 4 && cw != 8) cw = 4;
-        const char* pv = getenv("LS_P2_VARIANT");
-        if (op->nr == 4 && pv && atoi(pv) >= 5) cw = 1;      // the 4x-only experiment kernels write plain rows
-        op->cw = cw;
-    }
     TRY(op->dmalloc((void**)&op->d_A, (size_t)op->pn * m * sizeof(cd)));
     TRY(op->dmalloc((void**)&op->d_C, (size_t)op->pn * m * sizeof(cd)));
     TRY(op->dmalloc((void**)&op->d_b, N * sizeof(cd)));

@@ -19,9 +19,6 @@
 // All-to-all volume per rank and direction: 16*nr*N*(P-1)/P^2 bytes.
 #include "ls_common.cuh"
 #include "line_kernels.cuh"
-#ifdef LS_EXPERIMENTS
-#include "line_kernels_experiments.cuh"   // measured-and-rejected variants: only with -DLS_EXPERIMENTS
-#endif
 #include "dist.cuh"
 #include "gv_spectrum.cuh"
 
@@ -90,7 +87,7 @@ struct Op3D : HandleBase {
     }
 };
 
-inline int lines_b(long N) { return N == 512 ? LS_LINESB512 : 8; }      // LinesB<N> of the mode-B kernels (fft_engine.cuh)
+inline int lines_b(long N) { return N == 512 ? lines_b512 : 8; }      // LinesB<N> of the mode-B kernels (fft_engine.cuh)
 
 struct GenParams {
     int lb = 8;         // x-adjacent z lines interleaved per spectrum unit
@@ -286,9 +283,6 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             LS_CUDA_TRY(cudaEventRecord(op->evIn[c], sc));
         }
     }
-    static int variant = -1, stage45 = -1;
-    if (variant < 0) { const char* ev = getenv("LS_P3_VARIANT"); variant = ev ? atoi(ev) : 1; }   // 1: spectrum chunks staged by TMA bulk copies, 0: direct loads
-    if (stage45 < 0) { const char* ev = getenv("LS_P45_STAGE"); stage45 = ev ? atoi(ev) : 3; }    // bit 0: P5, bit 1: P4 stage their next slot block (and b) in shared memory by cp.async (256^3: 1.94 -> 1.80 ms)
     for (int c = 0; c < Cx; ++c) {
         const cd* a1t = (P > 1 ? op->d_A1T : op->d_A1) + c * cstride;     // chunk c re-slabbed: nelc x m x l
         cd* c1t = (P > 1 ? op->d_A1T : op->d_A1) + c * cstride;
@@ -309,27 +303,19 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             LineAddr la{1L << 40, 1, 0, nelc * me, 1, 0, nelc * me};
             la.nr = nr;
             op->phase_begin(2);
-#define C3(N) launch_mid<N, true, false>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
-#define C3T(N) launch_mid<N, true, true>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
-#define C3L2(N) launch_mid_lean<N, 2>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
-#define C3L3(N) launch_mid_lean<N, (GeoB<N>::THREADS <= 128 ? 3 : 1)>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
-#ifdef LS_EXPERIMENTS
-            if (variant == 1 || nr != 4) { LS3_DISPATCH(l, C3T); } else if (variant == 2) { LS3_DISPATCH(l, C3L2); }
-            else if (variant == 3) { LS3_DISPATCH(l, C3L3); } else { LS3_DISPATCH(l, C3); }
-#else
-            if (variant != 0) { LS3_DISPATCH(l, C3T); } else { LS3_DISPATCH(l, C3); }
-#endif
+#define C3(N) launch_mid<N, true>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
+            LS3_DISPATCH(l, C3);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
         }
-        // P4: inverse y lines (sxc, p): slots at A2[sxc + nelc*me*p + nelc*sy]; out C1T[sxc + nelc*m*p + nelc*j]
+        // P4: inverse y lines (sxc, p): slots at A2[sxc + nelc*me*p + nelc*sy]; out C1T[sxc + nelc*m*p + nelc*j].
+        //     P4 and P5 stage their next slot block (and b) in shared memory by cp.async (256^3: 1.94 -> 1.80 ms)
         {
             LineAddr la{nelc, 1, nelc * me, nelc, 1, nelc * m, nelc};
             la.nr = nr;
             op->phase_begin(3);
-#define C4(N) launch_inv<N, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la)
-#define C4S(N) launch_inv<N, true, 2>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la)
-            if (stage45 & 2) { LS3_DISPATCH(m, C4S); } else { LS3_DISPATCH(m, C4); }
+#define C4(N) launch_inv<N, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la)
+            LS3_DISPATCH(m, C4);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
         }
@@ -347,14 +333,13 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
         LS_CUDA_TRY(cudaEventRecord(op->evDone, sc));
         LS_CUDA_TRY(cudaStreamWaitEvent(s, op->evDone, 0));
     }
-    // P5: inverse x lines + combine; slot sx of line (j, p_loc) addressed as in P1
+    // P5: inverse x lines + combine (staged like P4); slot sx of line (j, p_loc) addressed as in P1
     {
         LineAddr la{1L << 40, nelc, 0, 1, n, 0, 1};
         la.split_shift = shc; la.split_stride = cstride; la.split2_shift = shr; la.split2_stride = blk; la.nr = nr;
         op->phase_begin(4);
-#define C5(N) launch_inv<N, false, 1>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
-#define C5S(N) launch_inv<N, false, 2>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
-        if (stage45 & 1) { LS3_DISPATCH(n, C5S); } else { LS3_DISPATCH(n, C5); }
+#define C5(N) launch_inv<N, false, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
+        LS3_DISPATCH(n, C5);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
     }
