@@ -5,7 +5,10 @@ k = 1/h, Greengard_Vico quadrature; example.jl:30-54) with GMRES, the operator a
 Arnoldi kernels and the Krylov basis living on the B200.  `--n 2048` runs the power-of-two
 high-frequency configuration (10 points per wavelength) instead.
 
-    python examples/example.py [--n 201] [--reltol 1.49e-8]
+    python examples/example.py [--n 201] [--reltol 1.49e-8] [--embed]
+
+`--embed` runs the operator on the power-of-two kernels with the grid zero-embedded, which serves any n <= 4096
+(`--n 1001 --embed --precond conv`: h = 1/1000).
 
 The sparsifying preconditioner of example.jl:64-71: `--precond conv` builds As and Mapproxsp with the
 convolution-sampled variants of the reference's setup code (buildSparseAConv / buildSparseAGConv,
@@ -32,6 +35,9 @@ def main():
     ap.add_argument("--precond", default=None)
     ap.add_argument("--msp", default="gpu", choices=["gpu", "host"],
                     help="MspInv = lu(Msp) on the device (ls_msp_factor) or on the host (SuperLU through the solve callback)")
+    ap.add_argument("--embed", action="store_true",
+                    help="run the operator on the power-of-two kernels with the grid zero-embedded (LS_FLAG_EMBED): "
+                         "any n <= 4096, e.g. h = 1/1000 (--n 1001), which the Bluestein general path refuses")
     args = ap.parse_args()
     n = args.n
     if n % 2 == 1:                       # example.jl: x = -a/2:h:a/2, k = 1/h
@@ -46,8 +52,10 @@ def main():
     Y = np.repeat(x[None, :], n, axis=0).reshape(-1, order="F")
     nu = nu_gaussian_2d(X, Y)
     t0 = time.time()
-    fastconv = ls.FastM(gv_spectrum_2d(n, n, h, k), nu, 4 * n, 4 * n, n, n, k, quadRule="Greengard_Vico")
-    print("operator on the GPU in %.2f s (n = %d, padded %d)" % (time.time() - t0, n, 4 * n))
+    fastconv = ls.FastM(gv_spectrum_2d(n, n, h, k), nu, 4 * n, 4 * n, n, n, k, quadRule="Greengard_Vico", embed=args.embed)
+    info = fastconv.info()
+    print("operator on the GPU in %.2f s (n = %d, padded %d, route %s, lines %d)"
+          % (time.time() - t0, n, 4 * n, ("pow2", "bluestein", "embedded")[info["route"]], info["n_line"]))
     precond = None
     if args.precond == "conv":
         from fast_solver_lippmann_schwinger_b200 import sparsifier

@@ -20,6 +20,8 @@ LS_ERR_INVALID, LS_ERR_UNSUPPORTED, LS_ERR_CUDA, LS_ERR_NOMEM, LS_ERR_NCCL, LS_E
 MEM_HOST, MEM_DEVICE = 0, 1
 QUAD_TRAPEZOIDAL, QUAD_GREENGARD_VICO = 0, 1
 APPLY_FASTCONVOLUTION, APPLY_FFTCONVOLUTION = 0, 1
+FLAG_FORCE_GENERIC, FLAG_PAD4, FLAG_EMBED = 1, 2, 4
+ROUTE_POW2, ROUTE_BLUESTEIN, ROUTE_EMBEDDED = 0, 1, 2
 
 QUADRULES = {"trapezoidal": QUAD_TRAPEZOIDAL, "Greengard_Vico": QUAD_GREENGARD_VICO}
 
@@ -83,6 +85,7 @@ def lib():
         "ls_op2d_create": (ci, [C.POINTER(vp), i64, i64, i64, i64, vp, vp, dbl, ci, ci]),
         "ls_op2d_create_gv": (ci, [C.POINTER(vp), i64, i64, vp, dbl, dbl, dbl, ci]),
         "ls_op2d_apply": (ci, [vp, vp, vp, ci, ci]),
+        "ls_op2d_info": (ci, [vp, C.POINTER(ci), C.POINTER(i64), C.POINTER(i64), C.POINTER(ci)]),
         "ls_op3d_create": (ci, [C.POINTER(vp), i64, i64, i64, i64, i64, i64, vp, vp, dbl, dbl, dbl, ci]),
         "ls_op3d_apply": (ci, [vp, vp, vp, ci, ci]),
         "ls_op3d_info": (ci, [vp, C.POINTER(ci), C.POINTER(ci), C.POINTER(ci)]),

@@ -99,7 +99,12 @@ struct LineAddr {
     int nr = 4;
     int cblock = 0;     // inverse: which N-block [cblock*N, (cblock+1)*N) of the padded output line is kept
     int full2 = 0;      // forward: the input line has 2N points (no zero padding), nr must be 2
+    // MASK instantiations only (zero-embedded sizes, op2d.cu): points >= mask_pts of a line and lines >= mask_lines
+    // read as zero (forward) / are not written (inverse).  16 bits suffice (<= 4096) and fill the tail padding: the
+    // struct stays 104 bytes, so the parameter layout of every unmasked kernel is unchanged.
+    int16_t mask_pts = 0, mask_lines = 0;
 };
+static_assert(sizeof(LineAddr) == 104, "LineAddr: kernel parameter layout");
 __device__ __forceinline__ long slot_off(const LineAddr& a, long s, long es) {
     return (s & ((1L << a.split_shift) - 1)) * es
          + ((s & ((1L << a.split2_shift) - 1)) >> a.split_shift) * a.split_stride
@@ -119,7 +124,8 @@ template <int N, bool MODE_B> struct Smem {
 // ---- forward, pruned: N inputs -> 4N slots -------------------------------------------
 // in  : line L point j at in[L*in_ls + j*in_es], optionally scaled by the real nu (same addressing)
 // out : line L slot  s at out[L*out_ls + s*out_es], s = r*N + slot
-template <int N, bool MODE_B>
+// MASK: points >= la.mask_pts and lines >= la.mask_lines are zeros (not read); their slots are written
+template <int N, bool MODE_B, bool MASK = false>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MinB<N, MODE_B>::value)
 k_fwd_pruned(const cd* __restrict__ in, const double* __restrict__ nu, cd* __restrict__ out,
              const cd* __restrict__ TAB, const LineAddr la, long line0) {
@@ -135,9 +141,14 @@ k_fwd_pruned(const cd* __restrict__ in, const double* __restrict__ nu, cd* __res
     const TwState<N> tw = make_tw<N>(t, TAB, tw1);
     const long in_base = line_in(la, L), out_base = line_out(la, L);
     const long in_es = la.in_es, out_es = la.out_es;
+    const int npts = (!MASK || L < la.mask_lines) ? la.mask_pts : 0;   // MASK: valid points of this line
     cd x[E];
 #pragma unroll
     for (int a = 0; a < E; ++a) {
+        if (MASK && a * T + t >= npts) {
+            x[a] = make_double2(0.0, 0.0);
+            continue;
+        }
         long off = in_base + (long)(a * T + t) * in_es;
         cd val = in[off];
         if (nu != nullptr) {
@@ -343,7 +354,8 @@ template <int K> __device__ __forceinline__ void cp_async_wait() { asm volatile(
 // block is transformed (each thread stages exactly the elements it consumes: no extra barrier), which takes two of
 // the kernel's three exposed DRAM latencies off the critical path.  The applies run staged; the set-up passes of the
 // compact spectrum do not.
-template <int N, bool MODE_B, bool STAGED = false>
+// MASK: only points < la.mask_pts of lines < la.mask_lines are written (and only their b values staged)
+template <int N, bool MODE_B, bool STAGED = false, bool MASK = false>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MinBInv<N, MODE_B>::value)
 k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __restrict__ TAB, double scale,
              const LineAddr la, long line0) {
@@ -363,6 +375,7 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
     const int nr = la.nr, rstep = 4 / la.nr;
     constexpr int TH = MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     cd* stg = sm + LPC * N + EngTab<N>::TW1N + threadIdx.x;      // STAGED: element e of this thread at stg[TH*e]
+    const int npts = (!MASK || L < la.mask_lines) ? la.mask_pts : 0;   // MASK: kept points of this line
 #pragma unroll 1
     for (int rr = 0; rr < nr; ++rr) {
         const int r = rr * rstep;
@@ -383,7 +396,8 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
                 cp_async_commit();
             } else if (bsrc != nullptr) {
 #pragma unroll
-                for (int a = 0; a < E; ++a) cp_async16(&stg[TH * a], &bsrc[out_base + (long)(a * T + t) * la.out_es]);
+                for (int a = 0; a < E; ++a)
+                    if (!MASK || a * T + t < npts) cp_async16(&stg[TH * a], &bsrc[out_base + (long)(a * T + t) * la.out_es]);
                 cp_async_commit();
             }
         }
@@ -392,8 +406,10 @@ k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __res
         else demod_accumulate_block<N>(acc, v, r, 16 * r * la.cblock);     // kept block c: extra factor w_4^(-r c)
         __syncthreads();
     }
+    if (MASK && STAGED && bsrc != nullptr) cp_async_wait<0>();
 #pragma unroll
     for (int a = 0; a < E; ++a) {
+        if (MASK && a * T + t >= npts) continue;
         long off = out_base + (long)(a * T + t) * la.out_es;
         cd res = cscale(acc[a], scale);
         if (bsrc != nullptr) {
@@ -423,14 +439,17 @@ template <class K> inline cudaError_t smem_optin(K kernel, int smem, unsigned lo
     return e;
 }
 
-template <int N, bool B>
+// MASK launchers cover ceil(nlines / LPC) CTAs: nlines need not be a multiple of the lines per CTA (the lines past
+// nlines in the last CTA are masked by la.mask_lines and must still be addressable for the unmasked side)
+template <int N, bool B, bool MASK = false>
 inline cudaError_t launch_fwd(cudaStream_t s, long nlines, const cd* in, const double* nu, cd* out, const cd* TAB,
                               const LineAddr& la) {
     constexpr int smem = Smem<N, B>::fwd_bytes;
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_fwd_pruned<N, B>, smem, optin); if (e != cudaSuccess) return e; }
-    k_fwd_pruned<N, B><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, nu, out, TAB, la, 0);
+    { cudaError_t e = smem_optin(k_fwd_pruned<N, B, MASK>, smem, optin); if (e != cudaSuccess) return e; }
+    const long grid = MASK ? (nlines + LPC - 1) / LPC : nlines / LPC;
+    k_fwd_pruned<N, B, MASK><<<(unsigned)grid, TH, smem, s>>>(in, nu, out, TAB, la, 0);
     return cudaPeekAtLastError();
 }
 
@@ -461,14 +480,15 @@ inline cudaError_t launch_mid_swap(cudaStream_t s, long nlines, const cd* in, cd
     return cudaPeekAtLastError();
 }
 
-template <int N, bool B, bool STAGED = false>
+template <int N, bool B, bool STAGED = false, bool MASK = false>
 inline cudaError_t launch_inv(cudaStream_t s, long nlines, const cd* in, const cd* bsrc, cd* out, const cd* TAB,
                               double scale, const LineAddr& la) {
     constexpr int smem = Smem<N, B>::fwd_bytes + (STAGED ? Smem<N, B>::LPC * N * (int)sizeof(cd) : 0);
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED>, smem, optin); if (e != cudaSuccess) return e; }
-    k_inv_pruned<N, B, STAGED><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, bsrc, out, TAB, scale, la, 0);
+    { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED, MASK>, smem, optin); if (e != cudaSuccess) return e; }
+    const long grid = MASK ? (nlines + LPC - 1) / LPC : nlines / LPC;
+    k_inv_pruned<N, B, STAGED, MASK><<<(unsigned)grid, TH, smem, s>>>(in, bsrc, out, TAB, scale, la, 0);
     return cudaPeekAtLastError();
 }
 

@@ -14,6 +14,11 @@
 // 4x evaluation (tests compare the two).
 // Algorithmic HBM bytes per apply: 2x padding 24N + 64N + 64N + 64N + 32N = 248*N;
 //                                  4x padding (SURVEY.md section 8(d)) 568*N.
+// Zero embedding (LS_FLAG_EMBED, any n, m <= 4096, both quadratures).  The same restriction argument: an n x m apply
+// only touches the lags (-n, n) x (-m, m), and those are a subset of the lags (-n', n') x (-m', m') of the power-of-two
+// grid n' = max(64, nextpow2(n)).  The handle extracts exactly those lags from the reference's spectrum (op2d_embed.cu),
+// wraps them onto 2n' x 2m' and runs the n' x m' compact apply with masked P1 / P3 kernels: inputs past (n, m) read as
+// zero, outputs past (n, m) are not written.
 #include "ls_common.cuh"
 #include "op2d_base.cuh"
 #include "line_kernels.cuh"
@@ -37,7 +42,12 @@ struct Op2D : Op2DBase {
     cd* d_TABn = nullptr; cd* d_TABm = nullptr;   // engine tables (fft_engine.cuh EngTab)
     cd* d_A = nullptr;        // pn x m
     cd* d_C = nullptr;        // P2 output: slot sx of column j at C[(sx/CW)*(CW*m) + CW*j + sx%CW]
+    bool embed = false;       // LS_FLAG_EMBED: lines of ln x lm points carry the n x m grid (ln = n, lm = m otherwise)
+    long ln = 0, lm = 0;
     int apply_dev(const cd* b, cd* y, int mode) override;
+    void info(int* route, int64_t* n_line, int64_t* m_line, int* padding) const override {
+        *route = embed ? 2 : 0; *n_line = ln; *m_line = lm; *padding = nr;
+    }
 };
 
 __global__ void k_scale(cd* a, long n, double s) {
@@ -142,11 +152,89 @@ int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
     return LS_OK;
 }
 
+// Zero-embedded apply: the three launches of apply_device at 2x padding on the ln x lm grid.  P1 reads the n x m input
+// (column stride n) with points >= n and lines >= m as zeros and covers ceil(m / LPC) CTAs; columns [m, lm) of A that
+// P2 reads stay zero from create time.  P3 writes points < n of lines < m only.  Greengard_Vico FFTconvolution has no
+// nu (Q2); the trapezoidal rule applies it in both modes (FastConvolution.jl:122 vs :141).
+int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
+    cudaError_t e = cudaSuccess;
+    cudaStream_t s = op->stream;
+    const long n = op->n, m = op->m, ln = op->ln, lm = op->lm, pn = op->pn;
+    const bool full = (mode == LS_APPLY_FASTCONVOLUTION);
+    const double* nu = (full || op->quadrule == LS_QUAD_TRAPEZOIDAL) ? op->d_nu : nullptr;
+    {
+        LineAddr la{1L << 40, n, 0, 1, pn, 0, 1};
+        la.nr = 2;
+        la.mask_pts = (int16_t)n; la.mask_lines = (int16_t)m;
+        op->phase_begin(0);
+#define E1(N) launch_fwd<N, false, true>(s, m, b, nu, op->d_A, op->d_TABn, la)
+        LS_DISPATCH_E(ln, E1);
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    {
+        LineAddr la{CW, 1, CW, pn, 1, CW * lm, CW};
+        la.nr = 2;
+        op->phase_begin(1);
+#define E2(N) launch_mid_swap<N>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
+        LS_DISPATCH_E(lm, E2);
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    {
+        LineAddr la{1L << 40, CW, 0, 1, n, 0, 1};
+        la.split_shift = CW_SHIFT; la.split_stride = CW * lm;
+        la.nr = 2;
+        la.mask_pts = (int16_t)n; la.mask_lines = (int16_t)m;
+        op->phase_begin(2);
+#define E3(N) launch_inv<N, false, true, true>(s, m, op->d_C, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
+        LS_DISPATCH_E(ln, E3);
+        op->phase_end(); op->launches++;
+        LS_CUDA_TRY(e);
+    }
+    return LS_OK;
+}
+
 }  // namespace
 
-int Op2D::apply_dev(const cd* b, cd* y, int mode) { return apply_device(this, b, y, mode); }
+int Op2D::apply_dev(const cd* b, cd* y, int mode) {
+    return embed ? apply_embedded(this, b, y, mode) : apply_device(this, b, y, mode);
+}
 
 namespace {
+
+// G2 = fft2(g2) / (2n 2m) in the slot order of the nr = 2 kernels (n, m: the line lengths, powers of two).
+// g2[jx2 + 2n*jy2]: the spatial kernel with its lags wrapped onto the 2n x 2m grid (negative lags at the end).
+// Takes ownership of g2 (freed here); on return op->d_G = G2 and op->nr = 2.
+int lag_spectrum(Op2D* op, cd* g2, long n, long m) {
+    cudaStream_t s = op->stream;
+    cudaError_t e = cudaSuccess;
+    cd *t2 = nullptr, *G2 = nullptr;
+    int rc;
+    if ((rc = op->dmalloc((void**)&t2, (size_t)(2 * n) * (2 * m) * sizeof(cd)))) return rc;
+    if ((rc = op->dmalloc((void**)&G2, (size_t)(2 * n) * (2 * m) * sizeof(cd)))) return rc;
+    {   // (3) forward along x on the full 2n-point lines: T2[sx2 + 2n*jy2]
+        LineAddr la{1L << 40, 2 * n, 0, 1, 2 * n, 0, 1};
+        la.nr = 2; la.full2 = 1;
+#define S3(N) launch_fwd<N, false>(s, 2 * m, g2, nullptr, t2, op->d_TABn, la)
+        LS_DISPATCH_E(n, S3);
+        LS_CUDA_TRY(e);
+    }
+    {   // (4) forward along y: G2[sx2*2m + (ry*m + sy)]
+        LineAddr la{1L << 40, 1, 0, 2 * n, 2 * m, 0, 1};
+        la.nr = 2; la.full2 = 1;
+#define S4(N) launch_fwd<N, false>(s, 2 * n, t2, nullptr, G2, op->d_TABm, la)
+        LS_DISPATCH_E(m, S4);
+        LS_CUDA_TRY(e);
+    }
+    k_scale<<<148 * 8, 256, 0, s>>>(G2, (2 * n) * (2 * m), 1.0 / ((double)(2 * n) * (double)(2 * m)));
+    LS_CUDA_TRY(cudaStreamSynchronize(s));
+    op->dfree(g2);
+    op->dfree(t2);
+    op->d_G = G2;
+    op->nr = 2;
+    return LS_OK;
+}
 
 // Compact (2x) spectrum from the reference's 4x one.  g4s: [sx4][ry][sy] slot order on the 4n x 4m grid,
 // already scaled by 1/(ne me).  On return op->d_G holds G2 = fft2(g wrapped onto 2n x 2m) in the slot order
@@ -155,7 +243,7 @@ int compact_spectrum(Op2D* op, cd* g4s) {
     const long n = op->n, m = op->m;
     cudaStream_t s = op->stream;
     cudaError_t e = cudaSuccess;
-    cd *t1 = nullptr, *g2 = nullptr, *t2 = nullptr, *G2 = nullptr;
+    cd *t1 = nullptr, *g2 = nullptr;
     int rc;
     if ((rc = op->dmalloc((void**)&t1, (size_t)(4 * n) * (2 * m) * sizeof(cd)))) return rc;
     // (1) inverse along y, keep lags [0, m) and [-m, 0): T1[sx4*2m + jy2]
@@ -181,28 +269,64 @@ int compact_spectrum(Op2D* op, cd* g4s) {
     }
     LS_CUDA_TRY(cudaStreamSynchronize(s));
     op->dfree(t1);
-    if ((rc = op->dmalloc((void**)&t2, (size_t)(2 * n) * (2 * m) * sizeof(cd)))) return rc;
-    if ((rc = op->dmalloc((void**)&G2, (size_t)(2 * n) * (2 * m) * sizeof(cd)))) return rc;
-    {   // (3) forward along x on the full 2n-point lines: T2[sx2 + 2n*jy2]
-        LineAddr la{1L << 40, 2 * n, 0, 1, 2 * n, 0, 1};
-        la.nr = 2; la.full2 = 1;
-#define S3(N) launch_fwd<N, false>(s, 2 * m, g2, nullptr, t2, op->d_TABn, la)
-        LS_DISPATCH_E(n, S3);
-        LS_CUDA_TRY(e);
+    return lag_spectrum(op, g2, n, m);    // (3), (4) and the 1/(2n 2m) scale
+}
+
+// nextpow2, at least 64 (the smallest engine size)
+long embed_len(long n) {
+    long p = 64;
+    while (p < n) p *= 2;
+    return p;
+}
+
+// LS_FLAG_EMBED: any n, m <= 4096, both quadratures.  gfft: host spectrum, or nullptr for the Greengard_Vico
+// spectrum generated on the device from (L, Lp).
+int create_embedded(ls_handle* out, long n, long m, long ne, long me, const double* nu, const ls_cdouble* gfft,
+                    double omega, int quadrule, double L, double Lp) {
+    Op2D* op = new Op2D();
+    int rc = op->init_base(KIND_OP2D);
+    if (rc) { delete op; return rc; }
+    op->n = n; op->m = m; op->ne = ne; op->me = me; op->omega = omega; op->quadrule = quadrule;
+    op->embed = true;
+    op->ln = embed_len(n); op->lm = embed_len(m);
+    const long ln = op->ln, lm = op->lm;
+    const size_t N = (size_t)n * m, NE = (size_t)ne * me;
+#define TRY(x) do { rc = (x); if (rc) { delete op; return rc; } } while (0)
+    TRY(op->dupload((void**)&op->d_nu, nu, N * sizeof(double)));
+    {
+        auto Tn = engine_table((int)ln), Tm = engine_table((int)lm);
+        TRY(op->dupload((void**)&op->d_TABn, Tn.data(), Tn.size() * sizeof(cd)));
+        TRY(op->dupload((void**)&op->d_TABm, Tm.data(), Tm.size() * sizeof(cd)));
     }
-    {   // (4) forward along y: G2[sx2*2m + (ry*m + sy)]
-        LineAddr la{1L << 40, 1, 0, 2 * n, 2 * m, 0, 1};
-        la.nr = 2; la.full2 = 1;
-#define S4(N) launch_fwd<N, false>(s, 2 * n, t2, nullptr, G2, op->d_TABm, la)
-        LS_DISPATCH_E(m, S4);
-        LS_CUDA_TRY(e);
+    {
+        // the centred spectrum as the reference holds it, then its lags (-n, n) x (-m, m) wrapped onto 2ln x 2lm
+        cd* d_gin = nullptr;
+        cd* g2 = nullptr;
+        if (gfft) {
+            TRY(op->dupload((void**)&d_gin, gfft, NE * sizeof(cd)));
+        } else {
+            TRY(op->dmalloc((void**)&d_gin, NE * sizeof(cd)));
+            k_fill_g2d_centred<<<(unsigned)((NE + 255) / 256), 256, 0, op->stream>>>(d_gin, ne, me, gv2d_params(L, Lp, omega));
+            cudaError_t e = cudaGetLastError();
+            if (e != cudaSuccess) { set_error("spectrum generation failed: %s", cudaGetErrorString(e)); delete op; return LS_ERR_CUDA; }
+        }
+        TRY(op->dmalloc((void**)&g2, (size_t)(2 * ln) * (2 * lm) * sizeof(cd)));
+        TRY(embed_lag_grid(op, d_gin, n, m, ne, me, quadrule == LS_QUAD_TRAPEZOIDAL, g2, 2 * ln, 2 * lm));
+        op->dfree(d_gin);
+        TRY(lag_spectrum(op, g2, ln, lm));
     }
-    k_scale<<<148 * 8, 256, 0, s>>>(G2, (2 * n) * (2 * m), 1.0 / ((double)(2 * n) * (double)(2 * m)));
-    LS_CUDA_TRY(cudaStreamSynchronize(s));
-    op->dfree(g2);
-    op->dfree(t2);
-    op->d_G = G2;
-    op->nr = 2;
+    op->pn = 2 * ln; op->pm = 2 * lm;
+    TRY(op->dmalloc((void**)&op->d_A, (size_t)op->pn * lm * sizeof(cd)));
+    TRY(op->dmalloc((void**)&op->d_C, (size_t)op->pn * lm * sizeof(cd)));
+    {   // columns [m, lm) of A are read by P2 and never written by P1
+        cudaError_t e = cudaMemsetAsync(op->d_A, 0, (size_t)op->pn * lm * sizeof(cd), op->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(op->stream);
+        if (e != cudaSuccess) { set_error("embedded set-up failed: %s", cudaGetErrorString(e)); delete op; return LS_ERR_CUDA; }
+    }
+    TRY(op->dmalloc((void**)&op->d_b, N * sizeof(cd)));
+    TRY(op->dmalloc((void**)&op->d_y, N * sizeof(cd)));
+#undef TRY
+    *out = reinterpret_cast<ls_handle>(op);
     return LS_OK;
 }
 
@@ -232,6 +356,22 @@ static int op2d_create_impl(ls_handle* out, int64_t n, int64_t m, int64_t ne, in
     LS_REQUIRE(n > 0 && m > 0 && ne > 0 && me > 0, LS_ERR_INVALID, "ls_op2d_create: non-positive size");
     LS_REQUIRE(quadrule == LS_QUAD_TRAPEZOIDAL || quadrule == LS_QUAD_GREENGARD_VICO, LS_ERR_INVALID,
                "ls_op2d_create: unknown quadRule %d", quadrule);
+    if (flags & LS_FLAG_EMBED) {
+        // every refusal before any CUDA call
+        LS_REQUIRE(!(flags & LS_FLAG_FORCE_GENERIC), LS_ERR_INVALID,
+                   "ls_op2d_create: LS_FLAG_EMBED and LS_FLAG_FORCE_GENERIC select different routes");
+        LS_REQUIRE(!(flags & LS_FLAG_PAD4), LS_ERR_UNSUPPORTED,
+                   "ls_op2d_create: the zero-embedded route runs with 2x padding only (no literal 4x evaluation)");
+        if (quadrule == LS_QUAD_TRAPEZOIDAL)
+            LS_REQUIRE(ne == 2 * n - 1 && me == 2 * m - 1, LS_ERR_INVALID,
+                       "ls_op2d_create: trapezoidal needs ne = 2n-1, me = 2m-1 (FastConvolution.jl:183)");
+        else
+            LS_REQUIRE(ne == 4 * n && me == 4 * m, LS_ERR_INVALID,
+                       "ls_op2d_create: Greengard_Vico needs ne = 4n, me = 4m (FastConvolution.jl:201)");
+        LS_REQUIRE(n <= 4096 && m <= 4096, LS_ERR_UNSUPPORTED,
+                   "ls_op2d_create: n=%ld, m=%ld: the zero-embedded route serves n, m <= 4096", (long)n, (long)m);
+        return create_embedded(out, n, m, ne, me, nu, gfft, omega, quadrule, L, Lp);
+    }
     if (quadrule == LS_QUAD_TRAPEZOIDAL) {
         LS_REQUIRE(ne == 2 * n - 1 && me == 2 * m - 1, LS_ERR_INVALID,
                    "ls_op2d_create: trapezoidal needs ne = 2n-1, me = 2m-1 (FastConvolution.jl:183)");
@@ -259,6 +399,7 @@ static int op2d_create_impl(ls_handle* out, int64_t n, int64_t m, int64_t ne, in
     int rc = op->init_base(KIND_OP2D);
     if (rc) { delete op; return rc; }
     op->n = n; op->m = m; op->ne = ne; op->me = me; op->omega = omega; op->quadrule = quadrule;
+    op->ln = n; op->lm = m;
     const size_t N = (size_t)n * m, NE = (size_t)ne * me;
 #define TRY(x) do { rc = (x); if (rc) { delete op; return rc; } } while (0)
     TRY(op->dupload((void**)&op->d_nu, nu, N * sizeof(double)));
@@ -326,6 +467,20 @@ int ls_op2d_apply(ls_handle h, const ls_cdouble* b, ls_cdouble* y, int mode, int
     if (rc) return rc;
     LS_CUDA_TRY(cudaMemcpyAsync(y, op->d_y, bytes, cudaMemcpyDeviceToHost, op->stream));
     LS_CUDA_TRY(cudaStreamSynchronize(op->stream));
+    return LS_OK;
+}
+
+int ls_op2d_info(ls_handle h, int* route, int64_t* n_line, int64_t* m_line, int* padding_factor) {
+    LS_REQUIRE(h, LS_ERR_INVALID, "ls_op2d_info: null handle");
+    Op2DBase* op = reinterpret_cast<Op2DBase*>(h);
+    LS_REQUIRE(op->kind == KIND_OP2D, LS_ERR_INVALID, "ls_op2d_info: not a 2-D operator handle");
+    int r = 0, pf = 0;
+    int64_t nl = 0, ml = 0;
+    op->info(&r, &nl, &ml, &pf);
+    if (route) *route = r;
+    if (n_line) *n_line = nl;
+    if (m_line) *m_line = ml;
+    if (padding_factor) *padding_factor = pf;
     return LS_OK;
 }
 

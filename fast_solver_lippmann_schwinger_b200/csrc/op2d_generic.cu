@@ -31,6 +31,10 @@ struct Op2DGeneric : Op2DBase {
     cd* d_A = nullptr;     // ne x m
     cd* d_C = nullptr;     // m x ne
     int apply_dev(const cd* b, cd* y, int mode) override;
+    // the spectrum is the reference's: padded 4n (Greengard_Vico) or 2n - 1 (trapezoidal)
+    void info(int* route, int64_t* n_line, int64_t* m_line, int* padding) const override {
+        *route = 1; *n_line = X.Nb; *m_line = Y.Nb; *padding = quadrule == LS_QUAD_TRAPEZOIDAL ? 2 : 4;
+    }
 };
 
 // Gd[kx*me + ky] = GFFT[(kx + sx) % ne, (ky + sy) % me] * scale   (sx = ne/2 for Greengard_Vico, 0 otherwise)

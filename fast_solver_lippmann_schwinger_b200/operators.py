@@ -92,15 +92,22 @@ class FastM(_Handle):
     GFFT is given exactly as the reference holds it: (ne, me) complex128, for
     Greengard_Vico in centred wave-number order (the fftshift/ifftshift of :94/:98 is folded
     into a one-time device permutation).
+
+    ``embed=True`` (LS_FLAG_EMBED) serves any grid with n, m <= 4096 in both quadratures on the
+    power-of-two kernels of n' = max(64, nextpow2(n)), the grid zero-embedded; ``info()`` tells
+    which route a handle runs.
     """
 
-    def __init__(self, GFFT, nu, ne, me, n, m, k, quadRule="trapezoidal", force_generic=False, pad4=False, L=None, Lp=None):
+    def __init__(self, GFFT, nu, ne, me, n, m, k, quadRule="trapezoidal", force_generic=False, pad4=False, L=None, Lp=None,
+                 embed=False):
         super().__init__()
         self.ne, self.me, self.n, self.m = int(ne), int(me), int(n), int(m)
         self.omega = float(k)
         self.quadRule = quadRule
         if quadRule not in _lib.QUADRULES:
             raise ValueError("unknown quadRule %r" % (quadRule,))
+        flags = ((_lib.FLAG_FORCE_GENERIC if force_generic else 0) | (_lib.FLAG_PAD4 if pad4 else 0)
+                 | (_lib.FLAG_EMBED if embed else 0))
         if GFFT is None:
             # Greengard_Vico spectrum Gtruncated2D(L, k, S) evaluated on the device (FastConvolution.jl:185-231)
             if quadRule != "Greengard_Vico" or L is None or Lp is None:
@@ -111,8 +118,7 @@ class FastM(_Handle):
             if nu.shape[0] != self.n * self.m:
                 raise ValueError("DimensionMismatch: nu has %d entries, expected %d" % (nu.shape[0], self.n * self.m))
             self.N = self.n * self.m
-            check(lib().ls_op2d_create_gv(C.byref(self._h), self.n, self.m, ptr(nu), self.omega, float(L), float(Lp),
-                                          (1 if force_generic else 0) | (2 if pad4 else 0)))
+            check(lib().ls_op2d_create_gv(C.byref(self._h), self.n, self.m, ptr(nu), self.omega, float(L), float(Lp), flags))
             return
         GFFT = np.asarray(GFFT)
         if GFFT.shape != (self.ne, self.me):
@@ -123,8 +129,15 @@ class FastM(_Handle):
         self.N = self.n * self.m
         g = np.asfortranarray(GFFT.astype(np.complex128, copy=False))   # column-major, as Julia stores it
         check(lib().ls_op2d_create(C.byref(self._h), self.n, self.m, self.ne, self.me, ptr(nu),
-                                   C.c_void_p(g.ctypes.data), self.omega, _lib.QUADRULES[quadRule],
-                                   (1 if force_generic else 0) | (2 if pad4 else 0)))
+                                   C.c_void_p(g.ctypes.data), self.omega, _lib.QUADRULES[quadRule], flags))
+
+    def info(self):
+        """ls_op2d_info: route (_lib.ROUTE_POW2 / ROUTE_BLUESTEIN / ROUTE_EMBEDDED), the line lengths the kernels run
+        and the padding factor of the spectrum the applies use."""
+        route, pf = C.c_int(), C.c_int()
+        nl, ml = C.c_int64(), C.c_int64()
+        check(lib().ls_op2d_info(self.handle, C.byref(route), C.byref(nl), C.byref(ml), C.byref(pf)))
+        return {"route": int(route.value), "n_line": int(nl.value), "m_line": int(ml.value), "padding_factor": int(pf.value)}
 
     # size / eltype, FastConvolution.jl:31-41 (Q1: size(M) is a tuple of tuples upstream)
     def size(self, dim=None):

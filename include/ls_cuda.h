@@ -42,6 +42,10 @@ typedef struct ls_handle_s* ls_handle;
 #define LS_FLAG_PAD4          2   /* evaluate with the reference's literal 4x zero padding; default: the handle restricts
                                      the kernel to the lags the cropped apply touches and runs with 2x padding (same
                                      operator to rounding, see csrc/op2d.cu) */
+#define LS_FLAG_EMBED         4   /* 2-D, any n, m <= 4096, both quadratures: the lags the apply touches are extracted once
+                                     and the apply runs on the power-of-two kernels of n' = max(64, nextpow2(n)) (and m')
+                                     with the grid zero-embedded (csrc/op2d_embed.cu).  With LS_FLAG_PAD4 ->
+                                     LS_ERR_UNSUPPORTED, with LS_FLAG_FORCE_GENERIC -> LS_ERR_INVALID */
 
 #define LS_MEM_HOST   0
 #define LS_MEM_DEVICE 1
@@ -76,7 +80,10 @@ int ls_host_free_pinned(void* hptr);
  * two (pruned radix-8/16 transforms).  Every other case the reference accepts - any n, m
  * (examples/example.jl ships n = 201, ne = 804) and the trapezoidal rule (ne = 2n-1, crop
  * [n:2n-1], FastConvolution.jl:64-83) - runs on the general path: arbitrary-length line DFTs
- * by Bluestein's algorithm on the same engine, as long as ne + n - 1 <= 4096.             */
+ * by Bluestein's algorithm on the same engine, as long as ne + n - 1 <= 4096 (Greengard_Vico
+ * n <= 819, trapezoidal n <= 1366); larger sizes are refused (LS_ERR_UNSUPPORTED).  With
+ * LS_FLAG_EMBED every such grid up to n, m <= 4096 (h = 1/1000: n = 1001) runs instead on the
+ * power-of-two kernels of n' = max(64, nextpow2(n)), zero-embedded.                        */
 int ls_op2d_create(ls_handle* out, int64_t n, int64_t m, int64_t ne, int64_t me,
                    const double* nu, const ls_cdouble* gfft, double omega,
                    int quadrule, int flags);
@@ -88,6 +95,11 @@ int ls_op2d_create_gv(ls_handle* out, int64_t n, int64_t m, const double* nu, do
 /* y = M*b (mode 0; `*` FastConvolution.jl:43-48, mul! :50-54) or FFTconvolution(M,b) (mode 1).
  * b and y hold n*m complex values and may alias.                                          */
 int ls_op2d_apply(ls_handle h, const ls_cdouble* b, ls_cdouble* y, int mode, int memloc);
+/* how the handle evaluates: route (0 power-of-two fast path, 1 Bluestein general path, 2 zero-embedded), the line
+ * lengths its kernels run (n, m; the Bluestein convolution lengths Nb; n', m') and the padding factor of the spectrum
+ * the applies use (2 compact, 4 literal; Bluestein: the reference's, 4 Greengard_Vico / 2 trapezoidal).  Any pointer
+ * may be NULL.                                                                             */
+int ls_op2d_info(ls_handle h, int* route, int64_t* n_line, int64_t* m_line, int* padding_factor);
 /* size(M,dim) / eltype, FastConvolution.jl:31-41: writes N = n*m */
 int ls_op_size(ls_handle h, int64_t* N);
 

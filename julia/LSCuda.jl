@@ -18,7 +18,7 @@ import LinearAlgebra: mul!, ldiv!
 const libls = get(ENV, "LS_CUDA_LIB", "libls_cuda.so")
 
 const LS_MEM_HOST, LS_MEM_DEVICE = Cint(0), Cint(1)
-const LS_FLAG_FORCE_GENERIC, LS_FLAG_PAD4 = Cint(1), Cint(2)
+const LS_FLAG_FORCE_GENERIC, LS_FLAG_PAD4, LS_FLAG_EMBED = Cint(1), Cint(2), Cint(4)
 const LS_ORTH = Dict("ModifiedGramSchmidt" => Cint(0), "ClassicalGramSchmidt" => Cint(1), "DGKS" => Cint(2))
 const LS_QUAD = Dict("trapezoidal" => Cint(0), "Greengard_Vico" => Cint(1))
 
@@ -52,14 +52,20 @@ struct GPUFastM
     quadRule::String
 end
 
-"GPUFastM(GFFT, nu, ne, me, n, m, k; quadRule) - same constructor as FastM (FastConvolution.jl:24)."
-function GPUFastM(GFFT::Array{ComplexF64,2}, nu::Vector{Float64}, ne, me, n, m, k; quadRule::String="trapezoidal")
+"""
+    GPUFastM(GFFT, nu, ne, me, n, m, k; quadRule, embed=false)
+
+Same constructor as FastM (FastConvolution.jl:24).  `embed=true` (LS_FLAG_EMBED) runs any grid with n, m <= 4096 on the
+power-of-two kernels with the grid zero-embedded (h = 1/1000: n = 1001, beyond the Bluestein general path).
+"""
+function GPUFastM(GFFT::Array{ComplexF64,2}, nu::Vector{Float64}, ne, me, n, m, k; quadRule::String="trapezoidal",
+                  embed::Bool=false)
     size(GFFT) == (ne, me) || throw(DimensionMismatch("GFFT is $(size(GFFT)), expected ($ne, $me)"))
     length(nu) == n * m || throw(DimensionMismatch("nu has $(length(nu)) entries, expected $(n*m)"))
     out = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:ls_op2d_create, libls), Cint,
                 (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Ptr{Float64}, Ptr{ComplexF64}, Float64, Cint, Cint),
-                out, n, m, ne, me, nu, GFFT, Float64(k), LS_QUAD[quadRule], 0))
+                out, n, m, ne, me, nu, GFFT, Float64(k), LS_QUAD[quadRule], embed ? LS_FLAG_EMBED : Cint(0)))
     return GPUFastM(Handle(out[]), nu, ne, me, n, m, Float64(k), quadRule)
 end
 "Move an existing reference operator to the GPU."
@@ -70,15 +76,22 @@ GPUFastM(M) = GPUFastM(M.GFFT, M.nu, M.ne, M.me, M.n, M.m, M.omega; quadRule=M.q
 GPU twin of `buildFastConvolution(x, y, h, k, nu, quadRule = "Greengard_Vico")` (FastConvolution.jl:185-231) that never
 builds GFFT on the host: the spectrum Gtruncated2D(L, k, S) is evaluated on the device (ls_op2d_create_gv).
 """
-function GPUFastM(x::AbstractVector, y::AbstractVector, h::Real, k::Real, nu::Function)
+function GPUFastM(x::AbstractVector, y::AbstractVector, h::Real, k::Real, nu::Function; embed::Bool=false)
     (n, m) = length(x), length(y)
     Lp = 4 * (abs(x[end] - x[1]) + h); L = 1.5 * (abs(x[end] - x[1]) + h)
     X = repeat(x, 1, m)[:]; Y = repeat(y', n, 1)[:]
     nuv = Vector{Float64}(nu(X, Y))
     out = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:ls_op2d_create_gv, libls), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Ptr{Float64}, Float64, Float64, Float64, Cint),
-                out, n, m, nuv, Float64(k), Float64(L), Float64(Lp), 0))
+                out, n, m, nuv, Float64(k), Float64(L), Float64(Lp), embed ? LS_FLAG_EMBED : Cint(0)))
     return GPUFastM(Handle(out[]), nuv, 4n, 4m, n, m, Float64(k), "Greengard_Vico")
+end
+
+"(route: 0 power of two / 1 Bluestein / 2 zero-embedded, line lengths the kernels run, padding factor in use)"
+function op2d_info(M::GPUFastM)
+    r = Ref{Cint}(0); nl = Ref{Int64}(0); ml = Ref{Int64}(0); p = Ref{Cint}(0)
+    check(ccall((:ls_op2d_info, libls), Cint, (Ptr{Cvoid}, Ref{Cint}, Ref{Int64}, Ref{Int64}, Ref{Cint}), M.h.ptr, r, nl, ml, p))
+    return (route=r[], n_line=nl[], m_line=ml[], padding=p[])
 end
 
 size(M::GPUFastM, dim) = length(M.nu)                       # FastConvolution.jl:31-33
@@ -284,7 +297,7 @@ function gmres_gpu!(x::Vector{ComplexF64}, A, b::Vector{ComplexF64}; Pl=nothing,
     return log ? (x, (resnorm=hist[1:niter[]], iters=niter[], isconverged=conv[] != 0, mvps=mv[])) : x
 end
 
-export GPUFastM, GPUFastM3D, GPUFastM3DSharded, nccl_unique_id, GPUSparsifyingPreconditioner, GPUSparseMatrixCSC, GPUMspFactorization, msp_info, fastconvolution, FFTconvolution,
+export GPUFastM, op2d_info, GPUFastM3D, GPUFastM3DSharded, nccl_unique_id, GPUSparsifyingPreconditioner, GPUSparseMatrixCSC, GPUMspFactorization, msp_info, fastconvolution, FFTconvolution,
        gmres_gpu!, cscmv!, set_device
 
 end # module
