@@ -385,8 +385,16 @@ int compact_spectrum3d(Op3D* op, const cd* d_gin, const int* d_fx, const int* d_
     const long lz2 = 2 * l / P;             // 2x z planes of this rank (intermediate slab)
     LS_REQUIRE(nel2 % 8 == 0 && lz2 >= 1 && (2 * l) % P == 0, LS_ERR_UNSUPPORTED,
                "compact padding needs 2n/P to be a multiple of 8 and 2l divisible by P");
+    // set-up chunks: the 4x slab is generated and pruned C x-slot chunks at a time, so that no more than ~20 GB of it
+    // is resident at once.  LS_OP3D_SETUP_CHUNKS forces C (a power of two that leaves each chunk >= 16 x-slots).
     int C = 1;
-    while ((double)(64.0 * n * m * l * 16.0) / P / C > 20e9 && nel4 / (2 * C) >= 8) C *= 2;
+    if (const char* cv = getenv("LS_OP3D_SETUP_CHUNKS")) {
+        C = atoi(cv);
+        LS_REQUIRE(C >= 1 && (C & (C - 1)) == 0 && nel4 / (2 * C) >= 8, LS_ERR_INVALID,
+                   "LS_OP3D_SETUP_CHUNKS=%s: needs a power of two C with 4n/P/C >= 16 x-slots per chunk (4n/P = %ld)", cv, nel4);
+    } else {
+        while ((double)(64.0 * n * m * l * 16.0) / P / C > 20e9 && nel4 / (2 * C) >= 8) C *= 2;
+    }
     const long nelc = nel4 / C;
     cd *g4c = nullptr, *t1c = nullptr, *T2 = nullptr, *R = nullptr, *g2 = nullptr, *X = nullptr, *Y = nullptr, *Z = nullptr, *G2 = nullptr;
     const size_t slab4 = (size_t)nel4 * (2 * m) * (2 * l);          // elements of T2 (this rank)
