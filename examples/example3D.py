@@ -5,7 +5,10 @@ The shipped 3-D example: h = 1/48, k = 1/h, smooth Gaussian bump, Greengard_Vico
 general-size path (Bluestein lines); powers of two in {64, 128, 256, 512} take the pruned fast path with
 the spectrum generated on the device.
 
-    python examples/example3D.py [--n 48] [--precond [--msp {host,gpu}]]
+    python examples/example3D.py [--n 48] [--embed] [--precond [--msp {host,gpu}]]
+
+--embed runs the operator on the power-of-two kernels with the grid zero-embedded (n' = max(64, nextpow2(n))), which
+serves any n <= 512 (`--n 400 --embed`: h = 1/400, beyond what the Bluestein path's memory allows).
 
 --precond builds the sparsifying preconditioner of example3D.jl:56-67 (27-point As and
 Mapproxsp = As + k^2 AG diag(nu)) from 343 unit-vector applies on the GPU operator
@@ -31,6 +34,9 @@ def main():
     ap.add_argument("--ppw", type=float, default=None, help="points per wavelength (default: k = 1/h as in example3D.jl)")
     ap.add_argument("--precond", action="store_true", help="sparsifying preconditioner (example3D.jl:56-67)")
     ap.add_argument("--msp", choices=("host", "gpu"), default="host", help="where lu(Mapproxsp) is factorised and solved")
+    ap.add_argument("--embed", action="store_true",
+                    help="run the operator on the power-of-two kernels with the grid zero-embedded (LS_FLAG_EMBED): "
+                         "any n <= 512")
     args = ap.parse_args()
     n = args.n
     h = 1.0 / n
@@ -38,8 +44,10 @@ def main():
     x = -0.5 + h * np.arange(n)
     nu = nu_gaussian_3d_grid(n)
     t0 = time.time()
-    fastconv = ls.FastM3D(None, nu, 4 * n, 4 * n, 4 * n, n, n, n, k, L=1.8 * n * h, Lp=4.0 * n * h)
-    print("operator on the GPU in %.2f s (n = %d, padded %d^3, spectrum generated on the device)" % (time.time() - t0, n, 4 * n))
+    fastconv = ls.FastM3D(None, nu, 4 * n, 4 * n, 4 * n, n, n, n, k, L=1.8 * n * h, Lp=4.0 * n * h, embed=args.embed)
+    lines = fastconv.lines()
+    print("operator on the GPU in %.2f s (n = %d, padded %d^3, spectrum generated on the device, route %s, lines %d x %d)"
+          % (time.time() - t0, n, 4 * n, ("pow2", "bluestein", "embedded")[lines["route"]], lines["n_line"], lines["l_line"]))
     X = np.broadcast_to(x[:, None, None], (n, n, n)).reshape(-1, order="F")
     precond = None
     if args.precond:

@@ -89,6 +89,7 @@ def lib():
         "ls_op3d_create": (ci, [C.POINTER(vp), i64, i64, i64, i64, i64, i64, vp, vp, dbl, dbl, dbl, ci]),
         "ls_op3d_apply": (ci, [vp, vp, vp, ci, ci]),
         "ls_op3d_info": (ci, [vp, C.POINTER(ci), C.POINTER(ci), C.POINTER(ci)]),
+        "ls_op3d_lines": (ci, [vp, C.POINTER(ci), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
         "ls_nccl_unique_id": (ci, [vp]),
         "ls_op3d_create_dist": (ci, [C.POINTER(vp), i64, i64, i64, vp, dbl, dbl, dbl, ci, ci, vp, ci]),
         "ls_op_size": (ci, [vp, C.POINTER(i64)]),

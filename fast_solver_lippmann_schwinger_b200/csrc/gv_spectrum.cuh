@@ -3,7 +3,7 @@
 // Julia's sinc(x) = sin(pi x)/(pi x)).  The sinc argument goes through pi*(Ls/pi) exactly like the
 // oracle's numpy.sinc so that both round the same way at arguments ~1e3.
 #pragma once
-#include "fft_engine.cuh"
+#include "ls_common.cuh"
 
 namespace ls {
 
@@ -37,5 +37,15 @@ __device__ __forceinline__ double gv_radius(double dk, long ix, long iy, long iz
 
 int create_op3d_generic(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_t me, int64_t le,
                         const double* nu, const ls_cdouble* gfft, double omega, double L, double Lp);
+// ls_op3d_lines of a general-size handle: its Bluestein convolution lengths
+void op3d_generic_lines(const HandleBase* h, int64_t* n_line, int64_t* m_line, int64_t* l_line);
+
+// Zero-embedded 3-D route, create time (op3d_embed.cu): the lags (-n, n)^2 x (-l, l) of the spatial kernel
+// g = ifftn(GFFT) wrapped onto the zeroed n2 x n2 x l2 grid (negative lags at the end), this rank's z slab of it:
+// g2[jx + n2*(jy + n2*jz_loc)], planes [rank*l2/P, (rank+1)*l2/P).  gin: the 4n x 4n x 4l centred spectrum on the
+// device, or nullptr to evaluate Gtruncated3D(L, omega) on the grid of period Lp.  Rank r contracts the x-slots
+// [r*4n/P, (r+1)*4n/P) of the spectrum; P > 1 sums the partial grids with one ncclReduceScatter over `comm`.
+int embed_lag_grid3d(HandleBase* op, const lsfft::cd* gin, long n, long l, double omega, double L, double Lp,
+                     int rank, int P, ncclComm_t comm, lsfft::cd* g2, long n2, long l2);
 
 }  // namespace ls

@@ -88,6 +88,9 @@ struct LineAddr {
     // slab split of the 4N-slot axis (multi-GPU transposes): slot s lives at
     // (s & (2^shift - 1))*es + (s >> shift)*split_stride.  shift = 62 disables it.
     int split_shift = 62;
+    // MASK instantiations only: lines >= mask_lines read as zero (forward) / are not written (inverse).  32 bits (3-D
+    // line counts reach 2^19) in the alignment gap after split_shift: no other member moves.
+    int mask_lines = 0;
     long split_stride = 0;
     // optional second level (x-slot chunks inside a rank's slab, pipelined transposes): bits
     // [split_shift, split2_shift) select the chunk (stride split_stride), bits >= split2_shift the
@@ -99,12 +102,13 @@ struct LineAddr {
     int nr = 4;
     int cblock = 0;     // inverse: which N-block [cblock*N, (cblock+1)*N) of the padded output line is kept
     int full2 = 0;      // forward: the input line has 2N points (no zero padding), nr must be 2
-    // MASK instantiations only (zero-embedded sizes, op2d.cu): points >= mask_pts of a line and lines >= mask_lines
-    // read as zero (forward) / are not written (inverse).  16 bits suffice (<= 4096) and fill the tail padding: the
-    // struct stays 104 bytes, so the parameter layout of every unmasked kernel is unchanged.
-    int16_t mask_pts = 0, mask_lines = 0;
+    // MASK instantiations only (zero-embedded sizes, op2d.cu, op3d.cu): points >= mask_pts of a line read as zero
+    // (forward) / are not written (inverse).  16 bits suffice (<= 4096) and fill the tail padding: the struct stays
+    // 104 bytes, so the parameter layout of every unmasked kernel is unchanged.
+    int16_t mask_pts = 0;
 };
 static_assert(sizeof(LineAddr) == 104, "LineAddr: kernel parameter layout");
+static_assert(offsetof(LineAddr, split_stride) == 64 && offsetof(LineAddr, nr) == 88, "LineAddr: member offsets");
 __device__ __forceinline__ long slot_off(const LineAddr& a, long s, long es) {
     return (s & ((1L << a.split_shift) - 1)) * es
          + ((s & ((1L << a.split2_shift) - 1)) >> a.split_shift) * a.split_stride

@@ -124,6 +124,13 @@ inline bool fft_size_supported(long n) {
     return n == 64 || n == 128 || n == 256 || n == 512 || n == 1024 || n == 2048 || n == 4096;
 }
 
+// line length of the zero-embedded routes (LS_FLAG_EMBED): nextpow2(n), at least 64 (the smallest engine size)
+inline long embed_len(long n) {
+    long p = 64;
+    while (p < n) p *= 2;
+    return p;
+}
+
 // slot -> frequency map of the forward engine for size N (mirrors Stage<>::addr logic)
 std::vector<int> slot_freq(int N);
 // exp(-2 pi i k / N), k < count, evaluated in long double

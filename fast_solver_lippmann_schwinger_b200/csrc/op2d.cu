@@ -165,7 +165,7 @@ int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
     {
         LineAddr la{1L << 40, n, 0, 1, pn, 0, 1};
         la.nr = 2;
-        la.mask_pts = (int16_t)n; la.mask_lines = (int16_t)m;
+        la.mask_pts = (int16_t)n; la.mask_lines = (int)m;
         op->phase_begin(0);
 #define E1(N) launch_fwd<N, false, true>(s, m, b, nu, op->d_A, op->d_TABn, la)
         LS_DISPATCH_E(ln, E1);
@@ -185,7 +185,7 @@ int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
         LineAddr la{1L << 40, CW, 0, 1, n, 0, 1};
         la.split_shift = CW_SHIFT; la.split_stride = CW * lm;
         la.nr = 2;
-        la.mask_pts = (int16_t)n; la.mask_lines = (int16_t)m;
+        la.mask_pts = (int16_t)n; la.mask_lines = (int)m;
         op->phase_begin(2);
 #define E3(N) launch_inv<N, false, true, true>(s, m, op->d_C, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
         LS_DISPATCH_E(ln, E3);
@@ -270,13 +270,6 @@ int compact_spectrum(Op2D* op, cd* g4s) {
     LS_CUDA_TRY(cudaStreamSynchronize(s));
     op->dfree(t1);
     return lag_spectrum(op, g2, n, m);    // (3), (4) and the 1/(2n 2m) scale
-}
-
-// nextpow2, at least 64 (the smallest engine size)
-long embed_len(long n) {
-    long p = 64;
-    while (p < n) p *= 2;
-    return p;
 }
 
 // LS_FLAG_EMBED: any n, m <= 4096, both quadratures.  gfft: host spectrum, or nullptr for the Greengard_Vico

@@ -15,34 +15,11 @@
 // 2n' x 2m' grid of the power-of-two apply and transforms it (lag_spectrum).
 #include "ls_common.cuh"
 #include "op2d_base.cuh"
-#include <cublas_v2.h>
+#include "lag_dft.cuh"
 
 using namespace ls;
 
 namespace {
-
-#define LS_CUBLAS_TRY(expr)                                                                        \
-    do {                                                                                           \
-        cublasStatus_t _s = (expr);                                                                \
-        if (_s != CUBLAS_STATUS_SUCCESS) {                                                         \
-            set_error("%s failed at %s:%d: cuBLAS status %d", #expr, __FILE__, __LINE__, (int)_s); \
-            return LS_ERR_CUDA;                                                                    \
-        }                                                                                          \
-    } while (0)
-
-// F[k + K*dd], k < K, dd < 2nv - 1 (lag d = dd - (nv - 1))
-__global__ void k_dft_lags(cd* __restrict__ F, long K, long nv, long shift, int trapezoidal) {
-    const long nl = 2 * nv - 1, total = K * nl;
-    for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
-        const long k = idx % K, dd = idx / K;
-        const long col = trapezoidal ? dd : ((dd - (nv - 1)) % K + K) % K;
-        const long row = ((k - shift) % K + K) % K;
-        const long r = (row * col) % K;
-        double s, c;
-        sincospi(2.0 * (double)r / (double)K, &s, &c);
-        F[idx] = make_double2(c, s);
-    }
-}
 
 // g2[(dx mod n2) + n2 * (dy mod m2)] = g[ddx + (2n-1) ddy],  d = dd - (n - 1)
 __global__ void k_place_lags(const cd* __restrict__ g, cd* __restrict__ g2, long n, long m, long n2, long m2) {
@@ -52,11 +29,6 @@ __global__ void k_place_lags(const cd* __restrict__ g, cd* __restrict__ g2, long
         g2[(dx < 0 ? dx + n2 : dx) + n2 * (dy < 0 ? dy + m2 : dy)] = g[idx];
     }
 }
-
-struct CublasGuard {
-    cublasHandle_t h = nullptr;
-    ~CublasGuard() { if (h) cublasDestroy(h); }
-};
 
 }  // namespace
 

@@ -17,10 +17,20 @@
 // spectrum; a second all-to-all brings the result back to z slabs for P5.  Neither exchange needs
 // a pack or unpack pass: both sides read/write the exchange buffers in place (slot_off()).
 // All-to-all volume per rank and direction: 16*nr*N*(P-1)/P^2 bytes.
+//
+// Zero embedding (LS_FLAG_EMBED, any n = m, l <= 512, one GPU or sharded): the same five launches on the lines of the
+// power-of-two grid n' = max(64, nextpow2(n)), l' likewise, with the kernel's lags (-n, n)^2 x (-l, l) extracted at
+// create time (op3d_embed.cu).  The arrays keep the real extents wherever a pass does not transform along them
+// (A1: 2n' x m x l, A2: 2n' x 2m' x l'), so the exchanges move 2n' x m x l.  Masked passes:
+//   P1 reads n of n' points; P2 reads m of m' points and writes zero lines for the planes l..l'-1, which P3 (in
+//   place, all l' points) would otherwise take from the previous apply; P4 writes m points of planes < l; P5 writes
+//   n points and stages b with stride n.
 #include "ls_common.cuh"
 #include "line_kernels.cuh"
 #include "dist.cuh"
 #include "gv_spectrum.cuh"
+#include <chrono>
+#include <climits>
 
 using namespace ls;
 using namespace lsk;
@@ -29,8 +39,11 @@ namespace {
 
 struct Op3D : HandleBase {
     long n = 0, m = 0, l = 0, ne = 0, me = 0, le = 0;
+    // LS_FLAG_EMBED: lines of ln x lm x ll points carry the n x m x l grid (ln = n, lm = m, ll = l otherwise)
+    bool embed = false;
+    long ln = 0, lm = 0, ll = 0;
     int nr = 4;                        // padding factor used by the applies (4: literal, 2: compact - see op2d.cu)
-    long pn = 0, pm = 0, pl = 0;       // padded sizes nr*n, nr*m, nr*l
+    long pn = 0, pm = 0, pl = 0;       // padded sizes nr*ln, nr*lm, nr*ll
     int P = 1, rank = 0;
     long nel = 0, lloc = 0;            // x-slots (pn/P) / z-planes (l/P) owned by this rank
     ncclComm_t comm = nullptr;
@@ -253,6 +266,8 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
     cudaError_t e = cudaSuccess;
     cudaStream_t s = op->stream, sc = op->cstream;
     const long n = op->n, m = op->m, l = op->l, me = op->pm, nel = op->nel, lloc = op->lloc, nelc = op->nelc;
+    const long ln = op->ln, lm = op->lm, ll = op->ll;
+    const bool embed = op->embed;
     const int nr = op->nr, Cx = op->Cx, P = op->P;
     const bool full = (mode == LS_APPLY_FASTCONVOLUTION);
     const long blk = nelc * m * lloc;                // elements exchanged with each peer per chunk
@@ -262,12 +277,16 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
     while ((1L << shr) < nel) ++shr;
     // P1: x lines (j, p_loc): in b[n*line + i]; slot sx -> rank q = sx/nel, chunk c = (sx%nel)/nelc:
     //     A1[c*cstride + q*blk + nelc*line + sx%nelc]
+    //     embed: m*lloc need not fill the last CTA; its surplus lines wrap (ldim0) onto lines 0.. and write the same bits
+    //     there (zeros would race with the real lines, and past the block they would land in the next one)
     {
         LineAddr la{1L << 40, n, 0, 1, nelc, 0, 1};
         la.split_shift = shc; la.split_stride = cstride; la.split2_shift = shr; la.split2_stride = blk; la.nr = nr;
+        if (embed) { la.ldim0 = m * lloc; la.mask_pts = (int16_t)n; la.mask_lines = INT_MAX; }
         op->phase_begin(0);
-#define C1(N) launch_fwd<N, false>(s, m * lloc, b, full ? op->d_nu : nullptr, op->d_A1, op->d_TABn, la)
-        LS3_DISPATCH(n, C1);
+#define C1(N) (embed ? launch_fwd<N, false, true>(s, m * lloc, b, full ? op->d_nu : nullptr, op->d_A1, op->d_TABn, la) \
+                     : launch_fwd<N, false>(s, m * lloc, b, full ? op->d_nu : nullptr, op->d_A1, op->d_TABn, la))
+        LS3_DISPATCH(ln, C1);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
     }
@@ -289,12 +308,16 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
         const cd* Gc = op->d_G + (long)c * nelc * me * op->pl;
         if (P > 1) LS_CUDA_TRY(cudaStreamWaitEvent(s, op->evIn[c], 0));
         // P2: y lines (sxc, p): in A1T[sxc + nelc*m*p + nelc*j]; out A2[sxc + nelc*me*p + nelc*sy]
+        //     embed: the plane index p is the slowest part of the line index, so the lines of planes l..l'-1 are the
+        //     lines >= nelc*l: they are written as zeros
         {
             LineAddr la{nelc, 1, nelc * m, nelc, 1, nelc * me, nelc};
             la.nr = nr;
+            if (embed) { la.mask_pts = (int16_t)m; la.mask_lines = (int)(nelc * l); }
+#define C2(N) (embed ? launch_fwd<N, true, true>(s, nelc * ll, a1t, nullptr, op->d_A2, op->d_TABm, la) \
+                     : launch_fwd<N, true>(s, nelc * l, a1t, nullptr, op->d_A2, op->d_TABm, la))
             op->phase_begin(1);
-#define C2(N) launch_fwd<N, true>(s, nelc * l, a1t, nullptr, op->d_A2, op->d_TABm, la)
-            LS3_DISPATCH(m, C2);
+            LS3_DISPATCH(lm, C2);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
         }
@@ -304,18 +327,21 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             la.nr = nr;
             op->phase_begin(2);
 #define C3(N) launch_mid<N, true>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
-            LS3_DISPATCH(l, C3);
+            LS3_DISPATCH(ll, C3);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
         }
         // P4: inverse y lines (sxc, p): slots at A2[sxc + nelc*me*p + nelc*sy]; out C1T[sxc + nelc*m*p + nelc*j].
         //     P4 and P5 stage their next slot block (and b) in shared memory by cp.async (256^3: 1.94 -> 1.80 ms)
+        //     embed: planes < l only (the surplus lines of the last CTA read planes >= l and are not written)
         {
             LineAddr la{nelc, 1, nelc * me, nelc, 1, nelc * m, nelc};
             la.nr = nr;
+            if (embed) { la.mask_pts = (int16_t)m; la.mask_lines = (int)(nelc * l); }
             op->phase_begin(3);
-#define C4(N) launch_inv<N, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la)
-            LS3_DISPATCH(m, C4);
+#define C4(N) (embed ? launch_inv<N, true, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la) \
+                     : launch_inv<N, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la))
+            LS3_DISPATCH(lm, C4);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
         }
@@ -334,12 +360,15 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
         LS_CUDA_TRY(cudaStreamWaitEvent(s, op->evDone, 0));
     }
     // P5: inverse x lines + combine (staged like P4); slot sx of line (j, p_loc) addressed as in P1
+    //     embed: the surplus lines of the last CTA wrap like P1's (their reads stay inside A1) and are not written
     {
         LineAddr la{1L << 40, nelc, 0, 1, n, 0, 1};
         la.split_shift = shc; la.split_stride = cstride; la.split2_shift = shr; la.split2_stride = blk; la.nr = nr;
+        if (embed) { la.ldim0 = m * lloc; la.mask_pts = (int16_t)n; la.mask_lines = (int)(m * lloc); }
         op->phase_begin(4);
-#define C5(N) launch_inv<N, false, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
-        LS3_DISPATCH(n, C5);
+#define C5(N) (embed ? launch_inv<N, false, true, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la) \
+                     : launch_inv<N, false, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la))
+        LS3_DISPATCH(ln, C5);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
     }
@@ -366,6 +395,8 @@ __global__ void k_scale3(cd* a, long n, double s) {
         a[i] = make_double2(v.x * s, v.y * s);
     }
 }
+
+int lag_spectrum3d(Op3D* op, cd* g2, long n, long m, long l);
 
 // Compact (2x) spectrum, 3-D version of compact_spectrum() in op2d.cu: the kernel g = ifftn(GFFT) is only
 // needed at the lags (-n,n) x (-m,m) x (-l,l).  Rank r owns the x-slot slab [r*4n/P, (r+1)*4n/P) of the 4x
@@ -396,13 +427,12 @@ int compact_spectrum3d(Op3D* op, const cd* d_gin, const int* d_fx, const int* d_
         while ((double)(64.0 * n * m * l * 16.0) / P / C > 20e9 && nel4 / (2 * C) >= 8) C *= 2;
     }
     const long nelc = nel4 / C;
-    cd *g4c = nullptr, *t1c = nullptr, *T2 = nullptr, *R = nullptr, *g2 = nullptr, *X = nullptr, *Y = nullptr, *Z = nullptr, *G2 = nullptr;
+    cd *g4c = nullptr, *t1c = nullptr, *T2 = nullptr, *R = nullptr, *g2 = nullptr;
     const size_t slab4 = (size_t)nel4 * (2 * m) * (2 * l);          // elements of T2 (this rank)
     const size_t slab2 = (size_t)(2 * n) * (2 * m) * lz2;           // elements of g2 / X (this rank) == nel2*2m*2l
     if ((rc = op->dmalloc((void**)&T2, slab4 * sizeof(cd)))) return rc;
     if ((rc = op->dmalloc((void**)&g4c, (size_t)nelc * (4 * m) * (4 * l) * sizeof(cd)))) return rc;
     if ((rc = op->dmalloc((void**)&t1c, (size_t)nelc * (4 * m) * (2 * l) * sizeof(cd)))) return rc;
-    const long LBl = lines_b(l);             // lines per unit of the final (2x) spectrum = what the fused z pass reads
     for (int c = 0; c < C; ++c) {
         p.nel = nelc; p.sx0 = (long)rank * nel4 + c * nelc;
         p.lb = 8;                            // set-up buffer: units of 8 lines, read below through explicit strides
@@ -450,6 +480,22 @@ int compact_spectrum3d(Op3D* op, const cd* d_gin, const int* d_fx, const int* d_
     }
     LS_CUDA_TRY(cudaStreamSynchronize(s));
     op->dfree(R);
+    return lag_spectrum3d(op, g2, n, m, l);     // (4) - (6), the 1/(8 n m l) scale and the chunk-major order
+}
+
+// G2 = fftn(g2) / (2n 2m 2l) in the z-pass chunk layout of the nr = 2 kernels (n, m, l: the line lengths, powers of
+// two).  g2: this rank's z slab (planes [rank*2l/P, (rank+1)*2l/P)) of the spatial kernel with its lags wrapped onto
+// the 2n x 2m x 2l grid, g2[jx2 + 2n*(jy2 + 2m*jz2_loc)].  Takes ownership of g2; on return op->d_G = G2, op->nr = 2.
+int lag_spectrum3d(Op3D* op, cd* g2, long n, long m, long l) {
+    const int P = op->P;
+    cudaStream_t s = op->stream;
+    cudaError_t e = cudaSuccess;
+    int rc;
+    const long nel2 = 2 * n / P;            // 2x x-slots of this rank (final slab)
+    const long lz2 = 2 * l / P;             // 2x z planes of this rank (intermediate slab)
+    const size_t slab2 = (size_t)(2 * n) * (2 * m) * lz2;           // elements of g2 / X (this rank) == nel2*2m*2l
+    const long LBl = lines_b(l);             // lines per unit of the final (2x) spectrum = what the fused z pass reads
+    cd *Y = nullptr, *X = nullptr, *Z = nullptr, *G2 = nullptr;
     if ((rc = op->dmalloc((void**)&X, slab2 * sizeof(cd)))) return rc;
     {   // (4) forward x on the unpadded 2n-point lines: X[sx2 + 2n*line]
         LineAddr la{1L << 40, 2 * n, 0, 1, 2 * n, 0, 1};
@@ -508,8 +554,18 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
                "ls_op3d_create: Greengard_Vico needs ne = 4n, me = 4m, le = 4l (FastConvolution3D.jl:100)");
     LS_REQUIRE(n == m, LS_ERR_INVALID,
                "ls_op3d_create: FFTconvolution pads (ne, ne, le): n must equal m (FastConvolution3D.jl:48)");
+    const bool embed = (flags & LS_FLAG_EMBED) != 0;
+    if (embed) {
+        // every refusal before any CUDA or NCCL call
+        LS_REQUIRE(!(flags & LS_FLAG_FORCE_GENERIC), LS_ERR_INVALID,
+                   "ls_op3d_create: LS_FLAG_EMBED and LS_FLAG_FORCE_GENERIC select different routes");
+        LS_REQUIRE(!(flags & LS_FLAG_PAD4), LS_ERR_UNSUPPORTED,
+                   "ls_op3d_create: the zero-embedded route runs with 2x padding only (no literal 4x evaluation)");
+        LS_REQUIRE(n <= 512 && l <= 512, LS_ERR_UNSUPPORTED,
+                   "ls_op3d_create: n=%ld, l=%ld: the zero-embedded route serves n, l <= 512", (long)n, (long)l);
+    }
     auto ok3 = [](long v) { return v == 64 || v == 128 || v == 256 || v == 512; };
-    if (!(ok3(n) && ok3(m) && ok3(l))) {
+    if (!embed && !(ok3(n) && ok3(m) && ok3(l))) {
         LS_REQUIRE(nranks == 1, LS_ERR_UNSUPPORTED,
                    "ls_op3d_create_dist: n=%ld m=%ld l=%ld - the sharded path serves powers of two in [64, 512]", (long)n, (long)m, (long)l);
         LS_REQUIRE(gfft != nullptr || (L > 0 && Lp > 0), LS_ERR_INVALID,
@@ -524,12 +580,17 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
     LS_REQUIRE(nranks == 1 || nccl_id != nullptr, LS_ERR_INVALID, "ls_op3d_create_dist: null NCCL id");
     LS_REQUIRE(nranks == 1 || gfft == nullptr, LS_ERR_UNSUPPORTED,
                "ls_op3d_create_dist: the sharded operator generates its spectrum slab on the device (pass NULL, L, Lp)");
+    LS_REQUIRE(!embed || l % nranks == 0, LS_ERR_UNSUPPORTED,
+               "ls_op3d_create_dist: l=%ld over %d ranks: the z planes must divide evenly between the ranks", (long)l, nranks);
 
     Op3D* op = new Op3D();
     int rc = op->init_base(KIND_OP3D);
     if (rc) { delete op; return rc; }
     op->n = n; op->m = m; op->l = l; op->ne = ne; op->me = me; op->le = le; op->omega = omega;
     op->P = nranks; op->rank = rank; op->nel = ne / nranks; op->lloc = l / nranks;
+    op->embed = embed;
+    op->ln = embed ? embed_len(n) : n; op->lm = embed ? embed_len(m) : m; op->ll = embed ? embed_len(l) : l;
+    const long ln = op->ln, lm = op->lm, ll = op->ll;
     if (nranks > 1) {
         ncclUniqueId id;
         memcpy(&id, nccl_id, sizeof(id));
@@ -545,7 +606,7 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
     {   // x-slot chunks (pipelined transposes).  Default: chunks of >= 16 MB per peer, at most 4 (measured on 8 GPUs:
         // 512^3 4.70 -> 4.05 ms with 4 chunks of 17 MB; 256^3 with 8 MB per peer is fastest unchunked).
         // LS_OP3D_CHUNKS overrides; chunks keep >= 8 x-slots.
-        const long nelf = (compact ? 2 : 4) * n / nranks;
+        const long nelf = (compact ? 2 : 4) * ln / nranks;
         const char* ev = getenv("LS_OP3D_CHUNKS");
         int cx = 1;
         if (ev) cx = atoi(ev);
@@ -564,12 +625,30 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
 #define TRY(x) do { rc = (x); if (rc) { delete op; return rc; } } while (0)
     TRY(op->dupload((void**)&op->d_nu, nu, Nloc * sizeof(double)));
     {
-        auto Tn = engine_table((int)n), Tm = engine_table((int)m), Tl = engine_table((int)l);
+        auto Tn = engine_table((int)ln), Tm = engine_table((int)lm), Tl = engine_table((int)ll);
         TRY(op->dupload((void**)&op->d_TABn, Tn.data(), Tn.size() * sizeof(cd)));
         TRY(op->dupload((void**)&op->d_TABm, Tm.data(), Tm.size() * sizeof(cd)));
         TRY(op->dupload((void**)&op->d_TABl, Tl.data(), Tl.size() * sizeof(cd)));
     }
-    {
+    if (embed) {
+        // the kernel's lags on this rank's z slab of the 2n' x 2m' x 2l' grid, then the compact path's final passes
+        cd *d_gin = nullptr, *g2 = nullptr;
+        if (gfft) TRY(op->dupload((void**)&d_gin, gfft, (size_t)ne * me * le * sizeof(cd)));
+        TRY(op->dmalloc((void**)&g2, (size_t)(2 * ln) * (2 * lm) * (2 * ll / nranks) * sizeof(cd)));
+        const auto t0 = std::chrono::steady_clock::now();
+        TRY(embed_lag_grid3d(op, d_gin, n, l, omega, L, Lp, rank, nranks, op->comm, g2, 2 * ln, 2 * ll));
+        const auto t1 = std::chrono::steady_clock::now();
+        if (d_gin) op->dfree(d_gin);
+        TRY(lag_spectrum3d(op, g2, ln, lm, ll));
+        if (getenv("LS_DEBUG")) {    // scripts/probe3d_embed.py reads this line
+            const double tl = std::chrono::duration<double>(t1 - t0).count();
+            const double ts = std::chrono::duration<double>(std::chrono::steady_clock::now() - t1).count();
+            const double lx = 2.0 * n - 1, lz = 2.0 * l - 1;     // the three contractions of this rank's x-slots
+            const double flop = 8.0 * ((double)ne / nranks) * ((double)me * le * lz + (double)me * lx * lz + lx * lx * lz);
+            fprintf(stderr, "[ls_cuda] rank %d: embedded create: lag extraction %.3f s (%.3e flop), spectrum %.3f s\n",
+                    rank, tl, flop, ts);
+        }
+    } else {
         auto fx = slot_freq((int)n), fy = slot_freq((int)m), fz = slot_freq((int)l);
         int *d_fx = nullptr, *d_fy = nullptr, *d_fz = nullptr;
         cd* d_gin = nullptr;
@@ -599,12 +678,12 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
         if (d_gin) op->dfree(d_gin);
         op->dfree(d_fx); op->dfree(d_fy); op->dfree(d_fz);
     }
-    op->pn = op->nr * n; op->pm = op->nr * m; op->pl = op->nr * l;
+    op->pn = op->nr * ln; op->pm = op->nr * lm; op->pl = op->nr * ll;
     op->nel = nel = op->pn / nranks;
     op->nelc = nel / op->Cx;
     TRY(op->dmalloc((void**)&op->d_A1, (size_t)op->pn * m * lloc * sizeof(cd)));
     if (nranks > 1) TRY(op->dmalloc((void**)&op->d_A1T, (size_t)nel * m * l * sizeof(cd)));
-    TRY(op->dmalloc((void**)&op->d_A2, (size_t)op->nelc * op->pm * l * sizeof(cd)));
+    TRY(op->dmalloc((void**)&op->d_A2, (size_t)op->nelc * op->pm * ll * sizeof(cd)));
     if (nranks > 1) {
         int lo = 0, hi = 0;
         cudaError_t ce = cudaDeviceGetStreamPriorityRange(&lo, &hi);
@@ -683,6 +762,24 @@ int ls_op3d_info(ls_handle h, int* padding_factor, int* x_slot_chunks, int* exch
     if (padding_factor) *padding_factor = op ? op->nr : 4;
     if (x_slot_chunks) *x_slot_chunks = op ? op->Cx : 1;
     if (exchange) *exchange = (op && op->P > 1) ? (op->ce_exchange ? 2 : 1) : 0;
+    return LS_OK;
+}
+
+int ls_op3d_lines(ls_handle h, int* route, int64_t* n_line, int64_t* m_line, int64_t* l_line) {
+    LS_REQUIRE(h, LS_ERR_INVALID, "ls_op3d_lines: null handle");
+    HandleBase* base = reinterpret_cast<HandleBase*>(h);
+    LS_REQUIRE(base->kind == KIND_OP3D, LS_ERR_INVALID, "ls_op3d_lines: not a 3-D operator handle");
+    int r = 1;
+    int64_t a = 0, b = 0, c = 0;
+    if (const Op3D* op = dynamic_cast<const Op3D*>(base)) {
+        r = op->embed ? 2 : 0; a = op->ln; b = op->lm; c = op->ll;
+    } else {
+        op3d_generic_lines(base, &a, &b, &c);
+    }
+    if (route) *route = r;
+    if (n_line) *n_line = a;
+    if (m_line) *m_line = b;
+    if (l_line) *l_line = c;
     return LS_OK;
 }
 

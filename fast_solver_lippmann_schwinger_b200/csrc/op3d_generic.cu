@@ -97,6 +97,11 @@ int Op3DGeneric::apply_dev(const cd* b, cd* y, int mode) {
 
 namespace ls {
 
+void op3d_generic_lines(const HandleBase* h, int64_t* n_line, int64_t* m_line, int64_t* l_line) {
+    const Op3DGeneric* op = static_cast<const Op3DGeneric*>(h);
+    *n_line = op->X.Nb; *m_line = op->Y.Nb; *l_line = op->Z.Nb;
+}
+
 int create_op3d_generic(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_t me, int64_t le,
                         const double* nu, const ls_cdouble* gfft, double omega, double L, double Lp) {
     LS_REQUIRE(ne + n - 1 <= 4096 && me + m - 1 <= 4096 && le + l - 1 <= 4096, LS_ERR_UNSUPPORTED,

@@ -67,9 +67,10 @@ def broadcast_unique_id(rank, group=None):
 
 class FastM3DSharded(_Handle):
     """The FastM3D operator slab-decomposed over `nranks` GPUs (collective object: every rank
-    constructs it and calls each apply).  Vectors are this rank's z slab."""
+    constructs it and calls each apply).  Vectors are this rank's z slab.  ``embed=True``: any n = m, l <= 512
+    with l divisible by nranks, zero-embedded on the power-of-two kernels (see FastM3D)."""
 
-    def __init__(self, nu_slab, n, m, l, k, L, Lp, rank, nranks, unique_id, pad4=False):
+    def __init__(self, nu_slab, n, m, l, k, L, Lp, rank, nranks, unique_id, pad4=False, embed=False):
         super().__init__()
         self.n, self.m, self.l = int(n), int(m), int(l)
         self.ne, self.me, self.le = 4 * self.n, 4 * self.m, 4 * self.l
@@ -83,7 +84,8 @@ class FastM3DSharded(_Handle):
             raise ValueError("DimensionMismatch: nu slab has %d entries, expected %d" % (nu_slab.shape[0], self.N))
         idbuf = C.create_string_buffer(unique_id, 128) if self.nranks > 1 else None
         check(lib().ls_op3d_create_dist(C.byref(self._h), self.n, self.m, self.l, ptr(nu_slab), self.omega,
-                                        float(L), float(Lp), self.rank, self.nranks, idbuf, 2 if pad4 else 0))
+                                        float(L), float(Lp), self.rank, self.nranks, idbuf,
+                                        (_lib.FLAG_PAD4 if pad4 else 0) | (_lib.FLAG_EMBED if embed else 0)))
 
     def size(self, dim=None):
         if dim is not None:
@@ -99,6 +101,7 @@ class FastM3DSharded(_Handle):
         check(lib().ls_op3d_info(self.handle, C.byref(p), C.byref(c), C.byref(x)))
         return int(p.value), int(c.value), ("single", "nccl", "copy-engine")[x.value]
 
+    lines = FastM3D.lines
     _apply = FastM3D._apply
     __mul__ = FastM3D.__mul__
     __matmul__ = FastM3D.__mul__

@@ -186,9 +186,14 @@ class FastM3D(_Handle):
     Gtruncated3D evaluated on the device (the only practical way at 256^3 and above).
     The reference defines only ``*`` for this type (Q4); ``mul_``, ``size`` and ``eltype`` are
     added so that gmres! (which needs them) takes the operator.
+
+    ``embed=True`` (LS_FLAG_EMBED) serves any n = m, l <= 512 on the power-of-two kernels of
+    n' = max(64, nextpow2(n)) and l' likewise, the grid zero-embedded; ``lines()`` tells which
+    route a handle runs.
     """
 
-    def __init__(self, GFFT, nu, ne, me, le, n, m, l, k, quadRule="Greengard_Vico", L=None, Lp=None, pad4=False):
+    def __init__(self, GFFT, nu, ne, me, le, n, m, l, k, quadRule="Greengard_Vico", L=None, Lp=None, pad4=False,
+                 embed=False):
         super().__init__()
         self.ne, self.me, self.le, self.n, self.m, self.l = (int(v) for v in (ne, me, le, n, m, l))
         self.omega = float(k)
@@ -210,7 +215,16 @@ class FastM3D(_Handle):
             g = np.asfortranarray(GFFT.astype(np.complex128, copy=False))
             gp = C.c_void_p(g.ctypes.data)
         check(lib().ls_op3d_create(C.byref(self._h), self.n, self.m, self.l, self.ne, self.me, self.le, ptr(nu), gp,
-                                   self.omega, float(L or 0.0), float(Lp or 0.0), 2 if pad4 else 0))
+                                   self.omega, float(L or 0.0), float(Lp or 0.0),
+                                   (_lib.FLAG_PAD4 if pad4 else 0) | (_lib.FLAG_EMBED if embed else 0)))
+
+    def lines(self):
+        """ls_op3d_lines: route (_lib.ROUTE_POW2 / ROUTE_BLUESTEIN / ROUTE_EMBEDDED) and the line lengths the
+        kernels run along x, y and z."""
+        route = C.c_int()
+        nl, ml, ll = C.c_int64(), C.c_int64(), C.c_int64()
+        check(lib().ls_op3d_lines(self.handle, C.byref(route), C.byref(nl), C.byref(ml), C.byref(ll)))
+        return {"route": int(route.value), "n_line": int(nl.value), "m_line": int(ml.value), "l_line": int(ll.value)}
 
     def size(self, dim=None):
         if dim is not None:

@@ -45,7 +45,11 @@ typedef struct ls_handle_s* ls_handle;
 #define LS_FLAG_EMBED         4   /* 2-D, any n, m <= 4096, both quadratures: the lags the apply touches are extracted once
                                      and the apply runs on the power-of-two kernels of n' = max(64, nextpow2(n)) (and m')
                                      with the grid zero-embedded (csrc/op2d_embed.cu).  With LS_FLAG_PAD4 ->
-                                     LS_ERR_UNSUPPORTED, with LS_FLAG_FORCE_GENERIC -> LS_ERR_INVALID */
+                                     LS_ERR_UNSUPPORTED, with LS_FLAG_FORCE_GENERIC -> LS_ERR_INVALID.
+                                     3-D (ls_op3d_create, ls_op3d_create_dist), any n = m, l <= 512: the apply runs on
+                                     the kernels of n' = m' = max(64, nextpow2(n)), l' = max(64, nextpow2(l))
+                                     (csrc/op3d_embed.cu), sharded too when l is divisible by the rank count.  The same
+                                     two refusals; n or l > 512 -> LS_ERR_UNSUPPORTED */
 
 #define LS_MEM_HOST   0
 #define LS_MEM_DEVICE 1
@@ -110,7 +114,8 @@ int ls_op_size(ls_handle h, int64_t* N);
  * (at 256^3 the array is 17 GB, at 512^3 137 GB - too big to ship from the host).
  * Served: n == m (the reference pads (ne, ne, le), :48).  Fast path: n, m, l in {64,128,256,512};
  * any other size with 5n - 1 <= 4096 (examples/example3D.jl ships n = 48) runs on the general path
- * (Bluestein lines, single GPU).                                                              */
+ * (Bluestein lines, single GPU).  With LS_FLAG_EMBED every n = m, l <= 512 runs instead on the
+ * power-of-two kernels of n' = max(64, nextpow2(n)) and l', zero-embedded, on one GPU or sharded. */
 int ls_op3d_create(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_t me, int64_t le,
                    const double* nu, const ls_cdouble* gfft_or_null, double omega, double L, double Lp,
                    int flags);
@@ -128,6 +133,10 @@ int ls_op3d_create_dist(ls_handle* out, int64_t n, int64_t m, int64_t l, const d
 /* how the handle evaluates: padding factor in use (2 compact / 4 literal), x-slot chunks of the pipelined transposes,
  * transpose route (0: single GPU, 1: NCCL grouped send/recv, 2: copy-engine pushes into IPC-mapped peer buffers)      */
 int ls_op3d_info(ls_handle h, int* padding_factor, int* x_slot_chunks, int* exchange);
+/* which route the handle runs (0 power-of-two fast path, 1 Bluestein general path, 2 zero-embedded; numbered as in
+ * ls_op2d_info) and the line lengths its kernels run along x, y and z (n, m, l; the Bluestein convolution lengths;
+ * n', m', l').  Any 3-D handle, sharded or not.  Any pointer may be NULL.                   */
+int ls_op3d_lines(ls_handle h, int* route, int64_t* n_line, int64_t* m_line, int64_t* l_line);
 /* mode 0: `*(M::FastM3D, b)` = b + omega^2 FFTconvolution(M, nu.*b)  (FastConvolution3D.jl:31-37)
  * mode 1: FFTconvolution(M, b)                                      (FastConvolution3D.jl:39-63) */
 int ls_op3d_apply(ls_handle h, const ls_cdouble* b, ls_cdouble* y, int mode, int memloc);

@@ -119,13 +119,15 @@ struct GPUFastM3D
     quadRule::String
 end
 
-"GFFT === nothing: the Greengard-Vico spectrum is generated on the device from (L, Lp) (FastConvolution3D.jl:72-99)."
-function GPUFastM3D(GFFT, nu::Vector{Float64}, ne, me, le, n, m, l, k; L=0.0, Lp=0.0, quadRule="Greengard_Vico")
+"""GFFT === nothing: the Greengard-Vico spectrum is generated on the device from (L, Lp) (FastConvolution3D.jl:72-99).
+`embed=true` (LS_FLAG_EMBED) runs any n = m, l <= 512 on the power-of-two kernels with the grid zero-embedded."""
+function GPUFastM3D(GFFT, nu::Vector{Float64}, ne, me, le, n, m, l, k; L=0.0, Lp=0.0, quadRule="Greengard_Vico",
+                    embed::Bool=false)
     out = Ref{Ptr{Cvoid}}(C_NULL)
     g = GFFT === nothing ? Ptr{ComplexF64}(C_NULL) : pointer(GFFT)
     GC.@preserve GFFT check(ccall((:ls_op3d_create, libls), Cint,
                 (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Int64, Int64, Ptr{Float64}, Ptr{ComplexF64}, Float64, Float64, Float64, Cint),
-                out, n, m, l, ne, me, le, nu, g, Float64(k), Float64(L), Float64(Lp), 0))
+                out, n, m, l, ne, me, le, nu, g, Float64(k), Float64(L), Float64(Lp), embed ? LS_FLAG_EMBED : Cint(0)))
     return GPUFastM3D(Handle(out[]), nu, ne, me, le, n, m, l, Float64(k), quadRule)
 end
 "GPUFastM3D(M) - GPU twin of a reference `FastM3D`."
@@ -152,11 +154,12 @@ function nccl_unique_id()
     return id
 end
 function GPUFastM3DSharded(nu_slab::Vector{Float64}, n, m, l, k, L, Lp, rank::Integer, nranks::Integer,
-                           id::Vector{UInt8}; pad4::Bool=false)
+                           id::Vector{UInt8}; pad4::Bool=false, embed::Bool=false)
     out = Ref{Ptr{Cvoid}}(C_NULL)
+    flags = (pad4 ? LS_FLAG_PAD4 : Cint(0)) | (embed ? LS_FLAG_EMBED : Cint(0))
     check(ccall((:ls_op3d_create_dist, libls), Cint,
                 (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Ptr{Float64}, Float64, Float64, Float64, Cint, Cint, Ptr{UInt8}, Cint),
-                out, n, m, l, nu_slab, Float64(k), Float64(L), Float64(Lp), rank, nranks, id, pad4 ? LS_FLAG_PAD4 : 0))
+                out, n, m, l, nu_slab, Float64(k), Float64(L), Float64(Lp), rank, nranks, id, flags))
     return GPUFastM3D(Handle(out[]), nu_slab, 4n, 4m, 4l, n, m, l, Float64(k), "Greengard_Vico")
 end
 
@@ -165,6 +168,13 @@ function op3d_info(M::GPUFastM3D)
     p = Ref{Cint}(0); c = Ref{Cint}(0); x = Ref{Cint}(0)
     check(ccall((:ls_op3d_info, libls), Cint, (Ptr{Cvoid}, Ref{Cint}, Ref{Cint}, Ref{Cint}), M.h.ptr, p, c, x))
     return (padding=p[], chunks=c[], exchange=x[])
+end
+
+"(route: 0 power of two / 1 Bluestein / 2 zero-embedded, line lengths the kernels run along x, y, z)"
+function op3d_lines(M::GPUFastM3D)
+    r = Ref{Cint}(0); nl = Ref{Int64}(0); ml = Ref{Int64}(0); ll = Ref{Int64}(0)
+    check(ccall((:ls_op3d_lines, libls), Cint, (Ptr{Cvoid}, Ref{Cint}, Ref{Int64}, Ref{Int64}, Ref{Int64}), M.h.ptr, r, nl, ml, ll))
+    return (route=r[], n_line=nl[], m_line=ml[], l_line=ll[])
 end
 
 """
@@ -297,7 +307,7 @@ function gmres_gpu!(x::Vector{ComplexF64}, A, b::Vector{ComplexF64}; Pl=nothing,
     return log ? (x, (resnorm=hist[1:niter[]], iters=niter[], isconverged=conv[] != 0, mvps=mv[])) : x
 end
 
-export GPUFastM, op2d_info, GPUFastM3D, GPUFastM3DSharded, nccl_unique_id, GPUSparsifyingPreconditioner, GPUSparseMatrixCSC, GPUMspFactorization, msp_info, fastconvolution, FFTconvolution,
+export GPUFastM, op2d_info, GPUFastM3D, GPUFastM3DSharded, op3d_lines, nccl_unique_id, GPUSparsifyingPreconditioner, GPUSparseMatrixCSC, GPUMspFactorization, msp_info, fastconvolution, FFTconvolution,
        gmres_gpu!, cscmv!, set_device
 
 end # module
