@@ -45,7 +45,8 @@ void op3d_generic_lines(const HandleBase* h, int64_t* n_line, int64_t* m_line, i
 // g2[jx + n2*(jy + n2*jz_loc)], planes [rank*l2/P, (rank+1)*l2/P).  gin: the 4n x 4n x 4l centred spectrum on the
 // device, or nullptr to evaluate Gtruncated3D(L, omega) on the grid of period Lp.  Rank r contracts the x-slots
 // [r*4n/P, (r+1)*4n/P) of the spectrum; P > 1 sums the partial grids with one ncclReduceScatter over `comm`.
+// chunk_slots > 0 sets the x-slots per chunk of the contraction (0: as many as 8 GB of spectrum hold).
 int embed_lag_grid3d(HandleBase* op, const lsfft::cd* gin, long n, long l, double omega, double L, double Lp,
-                     int rank, int P, ncclComm_t comm, lsfft::cd* g2, long n2, long l2);
+                     int rank, int P, ncclComm_t comm, lsfft::cd* g2, long n2, long l2, long chunk_slots);
 
 }  // namespace ls

@@ -29,6 +29,7 @@
 #include "line_kernels.cuh"
 #include "dist.cuh"
 #include "gv_spectrum.cuh"
+#include <cerrno>
 #include <chrono>
 #include <climits>
 
@@ -555,6 +556,7 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
     LS_REQUIRE(n == m, LS_ERR_INVALID,
                "ls_op3d_create: FFTconvolution pads (ne, ne, le): n must equal m (FastConvolution3D.jl:48)");
     const bool embed = (flags & LS_FLAG_EMBED) != 0;
+    long embed_slots = 0;              // x-slots per chunk of the lag extraction; 0: by size (embed_lag_grid3d)
     if (embed) {
         // every refusal before any CUDA or NCCL call
         LS_REQUIRE(!(flags & LS_FLAG_FORCE_GENERIC), LS_ERR_INVALID,
@@ -563,6 +565,14 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
                    "ls_op3d_create: the zero-embedded route runs with 2x padding only (no literal 4x evaluation)");
         LS_REQUIRE(n <= 512 && l <= 512, LS_ERR_UNSUPPORTED,
                    "ls_op3d_create: n=%ld, l=%ld: the zero-embedded route serves n, l <= 512", (long)n, (long)l);
+        // LS_OP3D_EMBED_CHUNK_SLOTS forces the chunk width (a value at or above the rank's 4n/P x-slots: one chunk)
+        if (const char* cv = getenv("LS_OP3D_EMBED_CHUNK_SLOTS")) {
+            char* end = nullptr;
+            errno = 0;
+            embed_slots = strtol(cv, &end, 10);
+            LS_REQUIRE(end != cv && *end == '\0' && errno == 0 && embed_slots > 0, LS_ERR_INVALID,
+                       "LS_OP3D_EMBED_CHUNK_SLOTS=%s: needs a positive integer (x-slots per lag-extraction chunk)", cv);
+        }
     }
     auto ok3 = [](long v) { return v == 64 || v == 128 || v == 256 || v == 512; };
     if (!embed && !(ok3(n) && ok3(m) && ok3(l))) {
@@ -636,7 +646,7 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
         if (gfft) TRY(op->dupload((void**)&d_gin, gfft, (size_t)ne * me * le * sizeof(cd)));
         TRY(op->dmalloc((void**)&g2, (size_t)(2 * ln) * (2 * lm) * (2 * ll / nranks) * sizeof(cd)));
         const auto t0 = std::chrono::steady_clock::now();
-        TRY(embed_lag_grid3d(op, d_gin, n, l, omega, L, Lp, rank, nranks, op->comm, g2, 2 * ln, 2 * ll));
+        TRY(embed_lag_grid3d(op, d_gin, n, l, omega, L, Lp, rank, nranks, op->comm, g2, 2 * ln, 2 * ll, embed_slots));
         const auto t1 = std::chrono::steady_clock::now();
         if (d_gin) op->dfree(d_gin);
         TRY(lag_spectrum3d(op, g2, ln, lm, ll));

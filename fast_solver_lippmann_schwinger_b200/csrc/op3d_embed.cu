@@ -7,7 +7,7 @@
 //     T1 = S  *_z Fz   (one ZGEMM),   T2 = T1 *_y Fy   (strided-batched over the z lags),   g += Fx^T *_x T2 / (ne me le)
 // Native FP64 ZGEMM in cuBLAS's default math mode.  The 4n x 4n x 4l spectrum S (136 GB at n = l = 511) is never
 // resident: it is generated (Gtruncated3D, as k_fill_g3d does) or gathered from the uploaded GFFT in x-slot chunks of
-// at most CHUNK_BYTES, and the x contraction accumulates over the chunks.  About 1.2e14 flop at n = l = 511, 5e13 at
+// at most CHUNK_BYTES (LS_OP3D_EMBED_CHUNK_SLOTS forces the width), and the x contraction accumulates over the chunks.  About 1.2e14 flop at n = l = 511, 5e13 at
 // 400 (estimates).  Sharded, rank r contracts only its x-slots [r*4n/P, (r+1)*4n/P): its partial lags are placed on
 // the whole 2n' x 2n' x 2l' grid and one ncclReduceScatter over z-plane blocks leaves every rank its 2l'/P summed
 // planes, the slab op3d.cu's lag_spectrum3d transforms.
@@ -48,12 +48,13 @@ __global__ void k_place_lags3(const cd* __restrict__ g, cd* __restrict__ g2, lon
 namespace ls {
 
 int embed_lag_grid3d(HandleBase* op, const cd* gin, long n, long l, double omega, double L, double Lp,
-                     int rank, int P, ncclComm_t comm, cd* g2, long n2, long l2) {
+                     int rank, int P, ncclComm_t comm, cd* g2, long n2, long l2, long chunk_slots) {
     cudaStream_t s = op->stream;
     const long ne = 4 * n, me = 4 * n, le = 4 * l;
     const long lx = 2 * n - 1, lz = 2 * l - 1;
     const long x0 = ne * rank / P, x1 = ne * (rank + 1) / P;          // this rank's x-slots of the spectrum
-    const long cw = std::max(1L, std::min(x1 - x0, (long)(CHUNK_BYTES / ((double)me * le * sizeof(cd)))));
+    const long by_size = (long)(CHUNK_BYTES / ((double)me * le * sizeof(cd)));
+    const long cw = std::max(1L, std::min(x1 - x0, chunk_slots > 0 ? chunk_slots : by_size));
     const double dk = gin ? 0.0 : 2.0 * 3.141592653589793 / Lp;
     CublasGuard cb;
     LS_CUBLAS_TRY(cublasCreate(&cb.h));

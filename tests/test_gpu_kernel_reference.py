@@ -1,5 +1,11 @@
 """Every line-kernel instantiation of the 2-D and 3-D applies, at full line length, against an exact reference.
 
+Each route is covered at every line length its kernels run: the power-of-two routes (compact 2x spectrum and pad4),
+the Bluestein route of the sizes that are not powers of two and of every trapezoidal operator (every convolution
+length Nb = 64 ... 4096 on each side and, in 2-D, in both quadratures), and the zero-embedded route (LS_FLAG_EMBED: the
+masked kernels at every n' and l' = 64 ... 512, on one GPU and, where the GPUs are present, sharded over 2, 4 and 8;
+the 3-D lag extraction also in forced x-slot chunks).
+
 The reference needs no padded FFT: for a separable spectrum G = Gx (x) Gy (x) Gz the operator factorises exactly.
 Each factor gives a spatial kernel along its axis,
 
@@ -16,8 +22,15 @@ not; it shares no code with the product or the oracle.  The CPU tests check it a
 bound its own rounding at the largest case in long double.  The GPU tests hold the convolution part of each apply to
 relative L2 <= 2e-14 and worst entry <= 2e-13 x RMS, far below the 1e-12 parity bar on y = b + omega^2 G(nu b), which
 b dominates.  Run with -s for the table of measured errors.
+
+Every GPU case ends with an apply of a b full of NaN followed by the case's b again, which must give the first result
+bit for bit: a buffer region that an apply reads without rewriting it (the padding planes l..l'-1, surplus lines, the
+Bluestein work arrays) would carry the NaN into every later apply, and into every later GMRES iteration.
 """
 import ctypes as C
+import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -29,27 +42,65 @@ L2_BAR = 2e-14
 WORST_BAR = 2e-13
 LINES = [64, 128, 256, 512, 1024, 2048, 4096]
 
-# (route, quadRule, n, m); the route picks the flags: compact (default), pad4 (LS_FLAG_PAD4), embed (LS_FLAG_EMBED)
+# (route, quadRule, n, m); the route picks the flags: compact (default), pad4 (LS_FLAG_PAD4), embed (LS_FLAG_EMBED),
+# bluestein (default: the sizes that are not powers of two, and every trapezoidal operator), forced
+# (LS_FLAG_FORCE_GENERIC: the Bluestein route on a power-of-two grid).  The Bluestein cases put Lf + n - 1 at or just
+# under the convolution length Nb (Lf = 4n Greengard_Vico, 2n - 1 trapezoidal), where an off-by-one in the wrap aliases.
 _THIN = [(4096, 64), (64, 4096), (2048, 256), (256, 2048), (1024, 128), (128, 1024), (512, 512), (2048, 2048)]
 CASES_2D = ([("compact", "Greengard_Vico", n, m) for n, m in _THIN + [(4096, 4096)]]
             + [("pad4", "Greengard_Vico", n, m) for n, m in _THIN]
             + [("embed", "Greengard_Vico", n, m) for n, m in [(4001, 65), (65, 4001), (33, 257), (257, 33), (200, 130),
                                                               (4001, 4001)]]
-            + [("embed", "trapezoidal", n, m) for n, m in [(2047, 601), (601, 2047), (1025, 1025)]])
-# (pad4, n, l); n = m (FFTconvolution pads (ne, ne, le), FastConvolution3D.jl:48)
-CASES_3D = [(pad4, n, l) for pad4 in (False, True) for n, l in [(256, 64), (64, 256), (128, 128), (64, 512)]]
+            + [("embed", "trapezoidal", n, m) for n, m in [(2047, 601), (601, 2047), (1025, 1025)]]
+            # (201, 201): examples/example.jl as shipped
+            + [("bluestein", "Greengard_Vico", n, m) for n, m in [(819, 13), (13, 819), (409, 25), (25, 409), (205, 51),
+                                                                  (51, 205), (102, 102), (201, 201)]]
+            + [("forced", "Greengard_Vico", 128, 64)]
+            + [("bluestein", "trapezoidal", n, m) for n, m in [(1366, 22), (22, 1366), (683, 43), (43, 683), (342, 86),
+                                                               (86, 342), (171, 171)]])
+# (route, n, l); n = m (FFTconvolution pads (ne, ne, le), FastConvolution3D.jl:48).  Bluestein: every Nb on the x/y
+# side and on the z side.  Embedded: every n' and l', (5, 9) with 45 x lines (the surplus lines of P1/P5's last CTA),
+# n = n' at both ends, P2's zero planes l..l'-1 from 1 (7, 511) to 255 (65, 257).
+CASES_3D = ([(route, n, l) for route in ("compact", "pad4") for n, l in [(256, 64), (64, 256), (128, 128), (64, 512)]]
+            + [("bluestein", n, l) for n, l in [(13, 819), (25, 409), (51, 205), (102, 102), (205, 51), (409, 20),
+                                                (819, 5)]]
+            + [("embed", n, l) for n, l in [(5, 9), (64, 64), (33, 200), (7, 511), (100, 37), (65, 257), (129, 65),
+                                            (255, 33), (257, 5), (512, 3)]])
 LARGEST_2D = ("compact", "Greengard_Vico", 4096, 4096)
+ROUTE = {"compact": 0, "pad4": 0, "bluestein": 1, "forced": 1, "embed": 2}    # _lib.ROUTE_POW2 / BLUESTEIN / EMBEDDED
 
 
 def _embed_len(n):
     return max(64, 1 << (n - 1).bit_length())
 
 
-def _expected_info(route, n, m):
-    """FastM.info() of a 2-D case: the route and the line lengths its P1/P3 (n_line) and P2 (m_line) kernels run."""
+def _bluestein_len(n, ne):
+    """Nb = nextpow2(max(64, ne + n - 1)): the circular convolution that holds a length-ne DFT of n inputs."""
+    return max(64, 1 << (ne + n - 2).bit_length())
+
+
+def _expected_info(route, n, m, quad="Greengard_Vico"):
+    """FastM.info() of a 2-D case: the route and the line lengths its P1/P3 (n_line) and P2 (m_line) kernels run
+    (Bluestein: the convolution lengths Nb; padding_factor: the reference's own 4 or 2)."""
     if route == "embed":
         return {"route": 2, "n_line": _embed_len(n), "m_line": _embed_len(m), "padding_factor": 2}
+    if route in ("bluestein", "forced"):
+        gv = quad == "Greengard_Vico"
+        ne, me = (4 * n, 4 * m) if gv else (2 * n - 1, 2 * m - 1)
+        return {"route": 1, "n_line": _bluestein_len(n, ne), "m_line": _bluestein_len(m, me),
+                "padding_factor": 4 if gv else 2}
     return {"route": 0, "n_line": n, "m_line": m, "padding_factor": 4 if route == "pad4" else 2}
+
+
+def _expected_lines(route, n, l):
+    """FastM3D.lines() of a 3-D case."""
+    if route == "embed":
+        ln, ll = _embed_len(n), _embed_len(l)
+    elif route == "bluestein":
+        ln, ll = _bluestein_len(n, 4 * n), _bluestein_len(l, 4 * l)
+    else:
+        ln, ll = n, l
+    return {"route": ROUTE[route], "n_line": ln, "m_line": ln, "l_line": ll}
 
 
 def _id2(case):
@@ -58,8 +109,8 @@ def _id2(case):
 
 
 def _id3(case):
-    pad4, n, l = case
-    return "%s-%dx%dx%d" % ("pad4" if pad4 else "compact", n, n, l)
+    route, n, l = case
+    return "%s-%dx%dx%d" % (route, n, n, l)
 
 
 def _toeplitz(g, n, off):
@@ -161,10 +212,21 @@ def measured():
             print("  %-28s %-18s L2 %.2e  worst/RMS %.2e" % r)
 
 
-def _check(measured, case, what, d, ref, y=None, at_b=()):
-    l2, worst = _errors(d, ref, y, at_b)
+def _record(measured, case, what, l2, worst):
     measured.append((case, what, l2, worst))
     assert l2 <= L2_BAR and worst <= WORST_BAR, "%s %s: relative L2 %.2e, worst/RMS %.2e" % (case, what, l2, worst)
+
+
+def _check(measured, case, what, d, ref, y=None, at_b=()):
+    _record(measured, case, what, *_errors(d, ref, y, at_b))
+
+
+def _check_recovers(M, b, y):
+    """An apply of a b full of NaN, then b again: y bit for bit, no NaN left (a NaN is data, not a fault)."""
+    M * np.full(b.shape, complex(np.nan, np.nan))
+    y2 = M * b
+    assert not np.isnan(y2).any()
+    assert np.array_equal(y2, y)
 
 
 def _omega(b, conv):
@@ -195,8 +257,18 @@ def test_separable_reference_matches_oracle_2d(quad, n, m):
 
 
 def test_separable_reference_matches_oracle_3d():
+    _reference_against_oracle_3d(8, 16)
+
+
+def test_separable_reference_matches_oracle_3d_odd():
+    """An odd, non-cubic grid like the embedded route's smallest case: the oracle's FastM3D built directly, as
+    tests/test_gpu_apply3d_embed.py does (its builder refuses odd n)."""
+    _reference_against_oracle_3d(5, 9)
+
+
+def _reference_against_oracle_3d(n, l):
     from oracle import ls_oracle as O
-    f = Sep3D(8, 16)
+    f = Sep3D(n, l)
     Mo = O.FastM3D(f.spectrum(), f.nu, f.ne, f.me, f.le, f.n, f.m, f.l, 0.9)
     yo = Mo * f.b
     assert np.linalg.norm(0.9 ** 2 * f.conv(f.nu * f.b) - (yo - f.b)) <= 1e-14 * np.linalg.norm(yo - f.b)
@@ -254,18 +326,36 @@ def test_reference_rows_against_longdouble():
 
 def test_cases_cover_every_line_length():
     """Every line kernel at every line length is launched by one of the cases below: the n side (P1/P3) and the m side
-    (P2) of each 2-D route, and the x/y and z lines of both 3-D paddings."""
-    for route in ("compact", "pad4", "embed"):
-        info = [_expected_info(r, n, m) for r, q, n, m in CASES_2D if r == route]
-        assert {i["n_line"] for i in info} == set(LINES), route
-        assert {i["m_line"] for i in info} == set(LINES), route
+    (P2) of each 2-D route, the Bluestein route in each quadrature, and the x/y and z lines of each 3-D route."""
+    for route, quad in [("compact", None), ("pad4", None), ("embed", None), ("bluestein", "Greengard_Vico"),
+                        ("bluestein", "trapezoidal")]:
+        info = [_expected_info(r, n, m, q) for r, q, n, m in CASES_2D if r == route and quad in (None, q)]
+        assert {i["n_line"] for i in info} == set(LINES), (route, quad)
+        assert {i["m_line"] for i in info} == set(LINES), (route, quad)
     assert _expected_info("embed", 4001, 65) == {"route": 2, "n_line": 4096, "m_line": 128, "padding_factor": 2}
     assert _expected_info("embed", 1025, 1025)["n_line"] == 2048          # the worst embedding, ln = 2n - 2
     assert _expected_info("pad4", 64, 4096) == {"route": 0, "n_line": 64, "m_line": 4096, "padding_factor": 4}
-    for pad4 in (False, True):
-        assert {n for p, n, l in CASES_3D if p == pad4} == {64, 128, 256}
-        assert {l for p, n, l in CASES_3D if p == pad4} == {64, 128, 256, 512}
-    assert all(16 * (4 * n) ** 2 * 4 * l <= 4.3e9 for p, n, l in CASES_3D)    # host spectra at most 4.3 GB
+    # Nb = nextpow2(max(64, 5n - 1)) for Greengard_Vico, nextpow2(max(64, 3n - 2)) trapezoidal
+    assert _expected_info("bluestein", 819, 13) == {"route": 1, "n_line": 4096, "m_line": 64, "padding_factor": 4}
+    assert _expected_info("bluestein", 1366, 22, "trapezoidal") == {"route": 1, "n_line": 4096, "m_line": 64,
+                                                                    "padding_factor": 2}
+    assert _expected_info("forced", 128, 64)["n_line"] == 1024
+    for r, q, n, m in CASES_2D:          # the Bluestein lengths at their edge: Lf + n - 1 at most 4 under Nb
+        if r == "bluestein" and (n, m) != (201, 201):
+            for k in (n, m):
+                lf = 4 * k if q == "Greengard_Vico" else 2 * k - 1
+                assert 0 <= _bluestein_len(k, lf) - (lf + k - 1) <= 4, (q, n, m)
+    assert any(r == "forced" and n & (n - 1) == 0 and m & (m - 1) == 0 for r, q, n, m in CASES_2D)
+    # 3-D, x/y and z lines; the power-of-two routes stop at 256 on the x/y side (a 512^2 x l host spectrum is 17 l GB)
+    for route, xy, z in [("compact", [64, 128, 256], [64, 128, 256, 512]), ("pad4", [64, 128, 256], [64, 128, 256, 512]),
+                         ("bluestein", LINES, LINES), ("embed", [64, 128, 256, 512], [64, 128, 256, 512])]:
+        expected = [_expected_lines(r, n, l) for r, n, l in CASES_3D if r == route]
+        assert {e["n_line"] for e in expected} == set(xy), route
+        assert {e["l_line"] for e in expected} == set(z), route
+    assert _expected_lines("bluestein", 409, 20) == {"route": 1, "n_line": 2048, "m_line": 2048, "l_line": 128}
+    assert _expected_lines("embed", 5, 9) == {"route": 2, "n_line": 64, "m_line": 64, "l_line": 64}
+    assert any(r == "embed" and (n * l) % 2 for r, n, l in CASES_3D)          # an odd count of P1/P5 lines
+    assert all(16 * (4 * n) ** 2 * 4 * l <= 4.3e9 for r, n, l in CASES_3D)    # host spectra at most 4.3 GB
 
 
 # --------------------------------------------------------------------------------------------------------------------
@@ -282,10 +372,11 @@ def test_2d_apply_against_separable_reference(case, measured):
     conv = f.conv(f.nu * f.b)
     omega = _omega(f.b, conv)
     G = f.spectrum()
-    M = ls.FastM(G, f.nu, f.ne, f.me, n, m, omega, quadRule=quad, pad4=route == "pad4", embed=route == "embed")
+    M = ls.FastM(G, f.nu, f.ne, f.me, n, m, omega, quadRule=quad, pad4=route == "pad4", embed=route == "embed",
+                 force_generic=route == "forced")
     del G
     try:
-        assert M.info() == _expected_info(route, n, m)
+        assert M.info() == _expected_info(route, n, m, quad)
         y = M * f.b
         _check(measured, name, "random b", y - f.b, omega ** 2 * conv)
         del conv
@@ -296,7 +387,6 @@ def test_2d_apply_against_separable_reference(case, measured):
             M.sync()
             assert np.array_equal(db.to_host(), y)
             db.free()
-        del y
         for idx in (0, N - 1):                                   # the extreme lags +-(n-1), +-(m-1) in isolation
             e = np.zeros(N, complex)
             e[idx] = 1.0
@@ -305,6 +395,7 @@ def test_2d_apply_against_separable_reference(case, measured):
         if n == m:
             ref = f.conv(f.b if quad == "Greengard_Vico" else f.nu * f.b)   # Q2: no nu for Greengard_Vico
             _check(measured, name, "FFTconvolution", ls.FFTconvolution(M, f.b), ref)
+        _check_recovers(M, f.b, y)
     finally:
         M.destroy()
 
@@ -312,11 +403,16 @@ def test_2d_apply_against_separable_reference(case, measured):
 # --------------------------------------------------------------------------------------------------------------------
 # GPU: 3-D
 # --------------------------------------------------------------------------------------------------------------------
-def _padding_3d(M):
+def _info_3d(M):
+    """ls_op3d_info: (padding factor, x-slot chunks of the apply)."""
     from fast_solver_lippmann_schwinger_b200 import _lib
     pf, cx, ex = C.c_int(), C.c_int(), C.c_int()
     _lib.check(_lib.lib().ls_op3d_info(M.handle, C.byref(pf), C.byref(cx), C.byref(ex)))
-    return pf.value
+    return pf.value, cx.value
+
+
+def _padding_3d(M):
+    return _info_3d(M)[0]
 
 
 def _check_3d(measured, name, M, f, omega):
@@ -331,24 +427,160 @@ def _check_3d(measured, name, M, f, omega):
         _check(measured, name, "impulse %d" % idx, ye - e, omega ** 2 * f.nu[idx] * f.column(idx), ye, (idx,))
     from fast_solver_lippmann_schwinger_b200 import FFTconvolution
     _check(measured, name, "FFTconvolution", FFTconvolution(M, f.b), f.conv(f.b))
+    _check_recovers(M, f.b, y)
     return y
+
+
+def _gv_device(ls, f, **kw):
+    """Handle on the device-generated Greengard_Vico spectrum of f's grid (h = 1/n, L = 1.8, Lp = 4, 8.3 points per
+    wavelength) with f's nu."""
+    n, l = f.n, f.l
+    return ls.FastM3D(None, f.nu, f.ne, f.me, f.le, n, n, l, 2 * np.pi * n / 8.3, L=1.8, Lp=4.0, **kw)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", CASES_3D, ids=_id3)
 def test_3d_apply_against_separable_reference(case, measured):
     import fast_solver_lippmann_schwinger_b200 as ls
-    pad4, n, l = case
+    route, n, l = case
     f = Sep3D(n, l)
     omega = _omega(f.b, f.conv(f.nu * f.b))
     G = f.spectrum()
-    M = ls.FastM3D(G, f.nu, f.ne, f.me, f.le, n, n, l, omega, pad4=pad4)
+    M = ls.FastM3D(G, f.nu, f.ne, f.me, f.le, n, n, l, omega, pad4=route == "pad4", embed=route == "embed")
     del G
     try:
-        assert _padding_3d(M) == (4 if pad4 else 2)
+        assert M.lines() == _expected_lines(route, n, l)
+        if route != "bluestein":
+            assert _padding_3d(M) == (4 if route == "pad4" else 2)
         _check_3d(measured, _id3(case), M, f, omega)
     finally:
         M.destroy()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n,l,slots", [(5, 9, 1), (5, 9, 3), (5, 9, 7), (129, 65, 100)])
+def test_3d_embed_lag_extraction_in_chunks(n, l, slots, monkeypatch, measured):
+    """LS_OP3D_EMBED_CHUNK_SLOTS splits the embedded route's lag extraction into x-slot chunks whose x contractions
+    accumulate (by itself only from n = l = 199 up, where no exact reference is cheap).  20 x-slots in chunks of 1, 3
+    (a last chunk of 2) and 7 (of 6); 516 in chunks of 100 (of 16)."""
+    import fast_solver_lippmann_schwinger_b200 as ls
+    monkeypatch.setenv("LS_OP3D_EMBED_CHUNK_SLOTS", str(slots))
+    f = Sep3D(n, l)
+    omega = _omega(f.b, f.conv(f.nu * f.b))
+    G = f.spectrum()
+    M = ls.FastM3D(G, f.nu, f.ne, f.me, f.le, n, n, l, omega, embed=True)
+    del G
+    try:
+        assert M.lines() == _expected_lines("embed", n, l)
+        _check_3d(measured, "embed-%dx%dx%d-S%d" % (n, n, l, slots), M, f, omega)
+    finally:
+        M.destroy()
+
+
+@pytest.mark.gpu
+def test_3d_embed_lag_chunks_device_spectrum(monkeypatch, measured):
+    """The device-generated spectrum through the chunked lag extraction against the unchunked one: the same
+    gtrunc3d_eval values summed in another order, so agreement at the bars, not bit for bit.  A chunk width at the
+    x-slot count (4n = 516) is one chunk: the same bits as without the variable."""
+    import fast_solver_lippmann_schwinger_b200 as ls
+    n, l = 129, 65
+    f = Sep3D(n, l)
+    name = "embed-dev-%dx%dx%d-S100" % (n, n, l)
+    out = {}
+    for slots in (None, "100", "516"):
+        if slots is None:
+            monkeypatch.delenv("LS_OP3D_EMBED_CHUNK_SLOTS", raising=False)
+        else:
+            monkeypatch.setenv("LS_OP3D_EMBED_CHUNK_SLOTS", slots)
+        M = _gv_device(ls, f, embed=True)
+        try:
+            y = M * f.b
+            out[slots] = (y, ls.FFTconvolution(M, f.b))
+            if slots == "100":
+                _check_recovers(M, f.b, y)
+        finally:
+            M.destroy()
+    _check(measured, name, "y - b", out["100"][0] - f.b, out[None][0] - f.b)
+    _check(measured, name, "FFTconvolution", out["100"][1], out[None][1])
+    assert all(np.array_equal(a, b) for a, b in zip(out["516"], out[None]))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n,l", [(5, 9), (100, 37)])
+def test_3d_embed_apply_chunks(n, l, monkeypatch, measured):
+    """LS_OP3D_CHUNKS splits the embedded apply's P2-P4 into x-slot chunks (the spectrum chunk-major): the same
+    arithmetic per line, so the same bits as one chunk."""
+    import fast_solver_lippmann_schwinger_b200 as ls
+    f = Sep3D(n, l)
+    omega = _omega(f.b, f.conv(f.nu * f.b))
+    G = f.spectrum()
+    out = {}
+    for cx in (1, 2, 8):
+        monkeypatch.setenv("LS_OP3D_CHUNKS", str(cx))
+        M = ls.FastM3D(G, f.nu, f.ne, f.me, f.le, n, n, l, omega, embed=True)
+        try:
+            assert _info_3d(M) == (2, cx)
+            y = M * f.b if cx == 1 else _check_3d(measured, "embed-%dx%dx%d-Cx%d" % (n, n, l, cx), M, f, omega)
+            out[cx] = (y, ls.FFTconvolution(M, f.b))
+        finally:
+            M.destroy()
+    for cx in (2, 8):
+        assert all(np.array_equal(a, b) for a, b in zip(out[cx], out[1])), cx
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n,l", [(64, 64), (128, 64)])
+def test_3d_embed_device_spectrum_against_power_of_two_route(n, l, measured):
+    """On a power-of-two grid the embedded route and the default one take their lags from the same gtrunc3d_eval
+    values by two independent extractions (ZGEMM lag DFTs against the pruned inverse FFTs of compact_spectrum3d)."""
+    import fast_solver_lippmann_schwinger_b200 as ls
+    f = Sep3D(n, l)
+    name = "embed-dev-%dx%dx%d" % (n, n, l)
+    out = {}
+    for embed in (False, True):
+        M = _gv_device(ls, f, embed=embed)
+        try:
+            assert M.lines()["route"] == (2 if embed else 0)
+            y = M * f.b
+            out[embed] = (y, ls.FFTconvolution(M, f.b))
+            if embed:
+                _check_recovers(M, f.b, y)
+        finally:
+            M.destroy()
+    _check(measured, name, "y - b", out[True][0] - f.b, out[False][0] - f.b)
+    _check(measured, name, "FFTconvolution", out[True][1], out[False][1])
+
+
+def _gpu_count():
+    try:
+        out = subprocess.run(["nvidia-smi", "-L"], capture_output=True, text=True, timeout=20).stdout
+        return sum(1 for line in out.splitlines() if line.startswith("GPU "))
+    except Exception:
+        return 0
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("world,chunks", [(1, 1), (2, 1), (4, 1), (8, 1), (2, 2)], ids=["P1", "P2", "P4", "P8", "P2-Cx2"])
+def test_sharded_embedded_against_single_gpu(world, chunks, measured):
+    """n = 97, l = 40 sharded (tests/dist_reference_worker.py): n' = 128, an odd count of P1/P5 lines per rank, 5 planes
+    per rank on 8.  The gathered apply, FFTconvolution and impulses at the first and last index of every rank's slab
+    against a single-GPU embedded handle on the same device spectrum (tied to the exact reference above).  P = 1 runs
+    the worker through ls_op3d_create_dist on one GPU, where the sharded tests skip."""
+    if _gpu_count() < world:
+        pytest.skip("needs %d GPUs" % world)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world),
+           "--master-addr", "127.0.0.1", "--master-port", str(29680 + 10 * (chunks - 1) + world),
+           os.path.join(root, "tests", "dist_reference_worker.py"), "97", "40"]
+    env = dict(os.environ)
+    env.setdefault("OMP_NUM_THREADS", "4")
+    env["LS_OP3D_CHUNKS"] = str(chunks)
+    p = subprocess.run(cmd, capture_output=True, text=True, timeout=1200, env=env, cwd=root)
+    assert p.returncode == 0 and "DIST_REFERENCE_OK" in p.stdout, p.stdout[-3000:] + p.stderr[-4000:]
+    rows = [line.split("|") for line in p.stdout.splitlines() if line.startswith("ROW|")]
+    assert len(rows) == 2 * world + 2
+    for _, what, l2, worst in rows:
+        _record(measured, "sharded-P%d-Cx%d-97x97x40" % (world, chunks), what, float(l2), float(worst))
 
 
 @pytest.mark.gpu

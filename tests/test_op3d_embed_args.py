@@ -68,6 +68,19 @@ def test_default_sharded_non_power_of_two_still_refused(built_lib):
     assert _create(L, 900, 900, 2, 0) == -2 and b"5n - 1" in L.ls_last_error()
 
 
+@pytest.mark.parametrize("bad", ["0", "-4", "", "abc", "12x", "3.5", "99999999999999999999999"])
+def test_embed_chunk_slots_refused(built_lib, monkeypatch, bad):
+    """LS_OP3D_EMBED_CHUNK_SLOTS (x-slots per chunk of the lag extraction) takes a positive integer; anything else is
+    refused before any CUDA or NCCL call, on one GPU and sharded."""
+    from fast_solver_lippmann_schwinger_b200._lib import lib
+    L = lib()
+    monkeypatch.setenv("LS_OP3D_EMBED_CHUNK_SLOTS", bad)
+    assert _create(L, 48, 48, 48, EMBED) == -1
+    assert b"LS_OP3D_EMBED_CHUNK_SLOTS" in L.ls_last_error()
+    assert _create(L, 48, 48, 48, EMBED, gfft=False) == -1
+    assert _create_dist(L, 48, 48, 0, 2, EMBED) == -1 and b"LS_OP3D_EMBED_CHUNK_SLOTS" in L.ls_last_error()
+
+
 def test_python_mirror(built_lib):
     import fast_solver_lippmann_schwinger_b200 as ls
     from fast_solver_lippmann_schwinger_b200 import dist as lsd
