@@ -38,7 +38,14 @@ def main():
     ap.add_argument("--embed", action="store_true",
                     help="run the operator on the power-of-two kernels with the grid zero-embedded (LS_FLAG_EMBED): "
                          "any n <= 4096, e.g. h = 1/1000 (--n 1001), which the Bluestein general path refuses")
+    ap.add_argument("--nrhs", type=int, default=1,
+                    help="solve for K incident plane waves exp(ik(x cos t + y sin t)), t = 0, pi/K, ..., (K-1) pi/K, in one "
+                         "lockstep GMRES (ls_gmres_msp_batch); needs the device Msp (--msp gpu), implies --precond conv")
     args = ap.parse_args()
+    if args.nrhs > 1:
+        if args.msp != "gpu":
+            ap.error("--nrhs > 1 needs --msp gpu")
+        args.precond = args.precond or "conv"
     n = args.n
     if n % 2 == 1:                       # example.jl: x = -a/2:h:a/2, k = 1/h
         h = 1.0 / (n - 1)
@@ -76,6 +83,19 @@ def main():
         Msp = sp.csc_matrix((d["Msp_nzval"], d["Msp_rowval"] - 1, d["Msp_colptr"] - 1), shape=(N, N))
         precond = (ls.SparsifyingPreconditioner(Msp, As, solverType="GPU", grid=(n, n)) if args.msp == "gpu"
                    else ls.SparsifyingPreconditioner(Msp, As))
+    if args.nrhs > 1:
+        thetas = np.pi * np.arange(args.nrhs) / args.nrhs
+        rhs = np.stack([-k ** 2 * ls.FFTconvolution(fastconv, nu * np.exp(1j * k * (X * np.cos(t) + Y * np.sin(t))))
+                        for t in thetas], axis=1)
+        u = np.zeros(rhs.shape, dtype=np.complex128, order="F")
+        t0 = time.time()
+        u, hists = ls.gmres_(u, fastconv, rhs, Pl=precond, reltol=args.reltol, log=True)
+        print("gmres! for %d directions in lockstep: %.3f s" % (args.nrhs, time.time() - t0))
+        for t, hq, q in zip(thetas, hists, range(args.nrhs)):
+            res = np.linalg.norm(fastconv * np.ascontiguousarray(u[:, q]) - rhs[:, q]) / np.linalg.norm(rhs[:, q])
+            print("direction %d theta %.4f: %d iterations, converged %s, true relative residual %.3e"
+                  % (q, t, hq.iters, hq.isconverged, res))
+        return
     u_inc = np.exp(1j * k * X)
     rhs = -k ** 2 * ls.FFTconvolution(fastconv, nu * u_inc)          # example.jl:77
     u = np.zeros(n * n, dtype=np.complex128)

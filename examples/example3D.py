@@ -37,7 +37,12 @@ def main():
     ap.add_argument("--embed", action="store_true",
                     help="run the operator on the power-of-two kernels with the grid zero-embedded (LS_FLAG_EMBED): "
                          "any n <= 512")
+    ap.add_argument("--nrhs", type=int, default=1,
+                    help="solve for K incident plane waves exp(ik(x cos t + y sin t)), t = 0, pi/K, ..., (K-1) pi/K, in one "
+                         "lockstep GMRES (ls_gmres_msp_batch); implies --precond --msp gpu")
     args = ap.parse_args()
+    if args.nrhs > 1:
+        args.precond, args.msp = True, "gpu"
     n = args.n
     h = 1.0 / n
     k = 1.0 / h if args.ppw is None else 2 * np.pi / (args.ppw * h)
@@ -49,10 +54,10 @@ def main():
     print("operator on the GPU in %.2f s (n = %d, padded %d^3, spectrum generated on the device, route %s, lines %d x %d)"
           % (time.time() - t0, n, 4 * n, ("pow2", "bluestein", "embedded")[lines["route"]], lines["n_line"], lines["l_line"]))
     X = np.broadcast_to(x[:, None, None], (n, n, n)).reshape(-1, order="F")
+    Y = np.broadcast_to(x[None, :, None], (n, n, n)).reshape(-1, order="F")
     precond = None
     if args.precond:
         from fast_solver_lippmann_schwinger_b200 import sparsifier
-        Y = np.broadcast_to(x[None, :, None], (n, n, n)).reshape(-1, order="F")
         Z = np.broadcast_to(x[None, None, :], (n, n, n)).reshape(-1, order="F")
         t0 = time.time()
         As, Mapproxsp = sparsifier.sparsifying_matrices_3d(k, X, Y, Z, fastconv, n, n, n, nu)
@@ -66,6 +71,19 @@ def main():
             where = "on the host"
         print("lu(Mapproxsp) %s in %.2f s; As on the GPU as %s (%d classes)" % (
             where, time.time() - t0, precond.As.format, precond.As.nclasses))
+    if args.nrhs > 1:
+        thetas = np.pi * np.arange(args.nrhs) / args.nrhs
+        incs = [np.exp(1j * k * (X * np.cos(t) + Y * np.sin(t))) for t in thetas]
+        rhs = np.stack([-(fastconv * ui - ui) for ui in incs], axis=1)
+        u = np.zeros(rhs.shape, dtype=np.complex128, order="F")
+        t0 = time.time()
+        u, hists = ls.gmres_(u, fastconv, rhs, Pl=precond, log=True)
+        print("gmres! for %d directions in lockstep: %.3f s" % (args.nrhs, time.time() - t0))
+        for q, (t, hq) in enumerate(zip(thetas, hists)):
+            res = np.linalg.norm(fastconv * np.ascontiguousarray(u[:, q]) - rhs[:, q]) / np.linalg.norm(rhs[:, q])
+            print("direction %d theta %.4f: %d iterations, converged %s, true relative residual %.3e"
+                  % (q, t, hq.iters, hq.isconverged, res))
+        return
     u_inc = np.exp(1j * k * X)
     rhs = -(fastconv * u_inc - u_inc)
     u = np.zeros(n ** 3, dtype=np.complex128)

@@ -109,10 +109,13 @@ def lib():
         "ls_msp_factor": (ci, [C.POINTER(vp), i64, i64, vp, vp, vp]),
         "ls_msp_factor3d": (ci, [C.POINTER(vp), i64, i64, i64, vp, vp, vp]),
         "ls_msp_solve": (ci, [vp, vp, vp, ci]),
+        "ls_msp_solve_batch": (ci, [vp, vp, i64, vp, i64, ci, ci]),
         "ls_msp_info": (ci, [vp, C.POINTER(i64), C.POINTER(ci), C.POINTER(dbl)]),
         "ls_msp_plan": (ci, [vp, C.c_char_p, i64]),
         "ls_gmres_msp": (ci, [vp, vp, vp, vp, vp, vp, ci, i64, dbl, dbl, ci, vp, i64,
                               C.POINTER(i64), C.POINTER(ci), C.POINTER(i64), ci]),
+        "ls_gmres_msp_batch": (ci, [vp, vp, vp, vp, ci, vp, i64, vp, i64, ci, i64, dbl, dbl, ci, vp, i64,
+                                    vp, vp, vp, ci]),
         "ls_krylov_last_precond_host_seconds": (ci, [vp, C.POINTER(dbl)]),
         "ls_sample_rows": (ci, [vp, vp, vp, ci, vp, i64]),
         "ls_gram": (ci, [vp, vp, i64, ci, vp]),

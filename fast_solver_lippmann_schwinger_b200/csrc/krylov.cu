@@ -324,6 +324,20 @@ struct Krylov : HandleBase {
     cd* d_V = nullptr; long v_cols = 0;
     cd* d_ax = nullptr; cd* d_b = nullptr; cd* d_x = nullptr;
     cd* h_stage = nullptr;        // pinned staging for the preconditioner callback
+    // ls_gmres_msp_batch: the systems' Krylov bases, the columns of the batched Msp solve, host-pointer b / x staging
+    cd* d_Vb = nullptr; size_t Vb_bytes = 0;
+    cd* d_Pb = nullptr; size_t Pb_bytes = 0;
+    cd* d_bxb = nullptr; size_t bxb_bytes = 0;
+    // (re)allocates *p when it holds fewer than `bytes`
+    int ensure(cd** p, size_t& have, size_t bytes) {
+        if (have >= bytes) return LS_OK;
+        if (*p) dfree(*p);
+        *p = nullptr; have = 0;
+        int rc = dmalloc((void**)p, bytes);
+        if (rc) return rc;
+        have = bytes;
+        return LS_OK;
+    }
     double t_precond_host_s = 0.0; // last ls_gmres: wall time inside D2H + callback + H2D of the Msp solve
 
     int grid_stream(long nn) const { long b = (nn + 255) / 256; return (int)(b < 148 * 16 ? (b > 0 ? b : 1) : 148 * 16); }
@@ -774,6 +788,206 @@ static int gmres_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, ls_sol
     return LS_OK;
 }
 
+// ls_gmres_msp_batch: nrhs independent GMRES(restart) runs of gmres_driver side by side with one operator, As and Msp.
+// Every system keeps its own basis, Hessenberg matrix, restarts, tolerance and history, and goes through exactly the
+// steps gmres_driver takes for it (same kernels, same inputs), so its history, counts and x have the bits of a run on its
+// own.  In each lockstep iteration the applies, SpMVs and Gram-Schmidt steps run system by system; the Msp^-1 of all
+// active systems is one batched solve (ls_msp_solve_batch: each factor block is read once per chunk of columns).  All
+// active systems share the iteration count and the position k in the restart cycle; a system that converges or
+// reaches maxiter drops out of the later solves.
+static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, int nrhs, const ls_cdouble* b, int64_t ldb,
+                              ls_cdouble* x, int64_t ldx, int restart, int64_t maxiter, double reltol, double abstol,
+                              int initially_zero, double* resnorm_hist, int64_t hist_cap, int64_t* niter, int* converged,
+                              int64_t* mv_products, int memloc) {
+    const char* fn = "ls_gmres_msp_batch";
+    LS_REQUIRE(op->op_size() == K->n, LS_ERR_INVALID, "%s: operator size %ld != workspace size %ld", fn, (long)op->op_size(), (long)K->n);
+    LS_REQUIRE(op->nccl_comm() == nullptr, LS_ERR_UNSUPPORTED, "%s: the device Msp factorisation is single-GPU", fn);
+    if (As) LS_REQUIRE(As->kind == KIND_SPM && As->nrows == K->n && As->x_len() == K->n && As->halo == 0, LS_ERR_INVALID,
+                       "%s: As must be an N x N sparse-matrix handle", fn);
+    LS_REQUIRE(msp->kind == KIND_MSP && msp->n == K->n, LS_ERR_INVALID, "%s: the Msp factorisation has %ld unknowns, the operator %ld",
+               fn, (long)msp->n, (long)K->n);
+    const long n = K->n;
+    if (restart <= 0) restart = 20;
+    LS_REQUIRE(restart <= 64, LS_ERR_UNSUPPORTED, "%s: restart > 64 is not supported", fn);
+    if (maxiter < 0) maxiter = n;
+    cudaStream_t s = op->stream;
+    const size_t vb = (size_t)n * sizeof(cd);
+    const bool host = memloc == LS_MEM_HOST;
+
+    // memory: nrhs bases of restart + 1 columns, nrhs columns for the batched solve, host staging of b and x, the
+    // batched solve's work arrays - checked against the free device memory before anything is allocated
+    const size_t needV = vb * (size_t)(restart + 1) * nrhs, needP = vb * nrhs, needBX = host ? 2 * vb * nrhs : 0;
+    size_t need = (K->Vb_bytes < needV ? needV : 0) + (K->Pb_bytes < needP ? needP : 0) + (K->bxb_bytes < needBX ? needBX : 0) +
+                  (K->d_ax ? 0 : 3 * vb) + msp->batch_bytes(nrhs, false, true);
+    if (need > 0) {
+        size_t free_b = 0, total_b = 0;
+        LS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        LS_REQUIRE(need <= free_b, LS_ERR_NOMEM,
+                   "%s: %d systems of %ld unknowns with restart %d need %zu more bytes of device memory; %zu of %zu bytes are free",
+                   fn, nrhs, n, restart, need, free_b, total_b);
+    }
+    int rc;
+    if ((rc = K->ensure(&K->d_Vb, K->Vb_bytes, needV))) return rc;
+    if ((rc = K->ensure(&K->d_Pb, K->Pb_bytes, needP))) return rc;
+    if (host && (rc = K->ensure(&K->d_bxb, K->bxb_bytes, needBX))) return rc;
+    if (!K->d_ax) {
+        if ((rc = K->dmalloc((void**)&K->d_ax, vb))) return rc;
+        if ((rc = K->dmalloc((void**)&K->d_b, vb))) return rc;
+        if ((rc = K->dmalloc((void**)&K->d_x, vb))) return rc;
+    }
+    if ((rc = msp->batch_reserve(nrhs, false, true))) return rc;
+
+    struct Sys {
+        cd* V; const cd* db; cd* dx;
+        std::vector<cplx> H, nullvec;
+        double beta = 0.0, current = 0.0, accumulator = 1.0, rbeta = 0.0, tol = 0.0;
+        int k = 1;
+        int64_t iteration = 0, nh = 0, mv = 0;
+        bool active = true;
+    };
+    const int ldh = restart + 1;
+    std::vector<Sys> sys((size_t)nrhs);
+    for (int q = 0; q < nrhs; ++q) {
+        Sys& S = sys[q];
+        S.V = K->d_Vb + (size_t)q * (restart + 1) * n;
+        if (host) {
+            cd* db = K->d_bxb + (size_t)q * n;
+            S.dx = K->d_bxb + (size_t)(nrhs + q) * n;
+            LS_CUDA_TRY(cudaMemcpyAsync(db, b + (size_t)q * ldb, vb, cudaMemcpyHostToDevice, s));
+            LS_CUDA_TRY(cudaMemcpyAsync(S.dx, x + (size_t)q * ldx, vb, cudaMemcpyHostToDevice, s));
+            S.db = db;
+        } else {
+            S.db = reinterpret_cast<const cd*>(b) + (size_t)q * ldb;
+            S.dx = reinterpret_cast<cd*>(x) + (size_t)q * ldx;
+        }
+        S.H.assign((size_t)ldh * restart, cplx{0.0, 0.0});
+        S.nullvec.assign((size_t)restart + 1, cplx{1.0, 0.0});
+        S.mv = initially_zero ? 1 : 0;
+    }
+    const int gs = K->grid_stream(n);
+
+    // ldiv!(Pl, v) for the listed vectors: As v into the solve's columns, one batched Msp^-1 in place, back into v
+    auto precond = [&](const std::vector<cd*>& vs) -> int {
+        const int na = (int)vs.size();
+        if (na == 0) return LS_OK;
+        for (int i = 0; i < na; ++i) {
+            cd* col = K->d_Pb + (size_t)i * n;
+            if (As) {
+                int r = As->mv_dev(make_double2(1.0, 0.0), vs[i], make_double2(0.0, 0.0), col, s);
+                if (r) return r;
+                K->launches++;
+            } else {
+                LS_CUDA_TRY(cudaMemcpyAsync(col, vs[i], vb, cudaMemcpyDeviceToDevice, s));
+            }
+        }
+        int r = msp->solve_batch_dev(K->d_Pb, n, K->d_Pb, n, na, s);
+        if (r) return r;
+        K->launches += (int64_t)msp->launches_per_solve * na;
+        for (int i = 0; i < na; ++i) LS_CUDA_TRY(cudaMemcpyAsync(vs[i], K->d_Pb + (size_t)i * n, vb, cudaMemcpyDeviceToDevice, s));
+        return LS_OK;
+    };
+    // init! of the listed systems: V1 = Pl^-1 (b - A x); beta = ||V1||; V1 /= beta
+    auto init = [&](const std::vector<int>& which, bool first) -> int {
+        std::vector<cd*> vs;
+        for (int q : which) {
+            Sys& S = sys[q];
+            if (first && initially_zero) {
+                LS_CUDA_TRY(cudaMemcpyAsync(S.V, S.db, vb, cudaMemcpyDeviceToDevice, s));
+            } else {
+                int r = op->apply_dev(S.dx, K->d_ax, LS_APPLY_FASTCONVOLUTION);
+                if (r) return r;
+                k_sub<<<gs, 256, 0, s>>>(S.db, K->d_ax, S.V, n);
+                K->launches++;
+            }
+            vs.push_back(S.V);
+        }
+        int r = precond(vs);
+        if (r) return r;
+        for (int q : which) {
+            Sys& S = sys[q];
+            if ((r = K->nrm2(S.V, K->d_scal, s))) return r;
+            k_scal_inv_dev<<<gs, 256, 0, s>>>(K->d_scal, S.V, n);
+            K->launches++;
+            LS_CUDA_TRY(cudaMemcpyAsync(K->h_scal, K->d_scal, sizeof(double), cudaMemcpyDeviceToHost, s));
+            LS_CUDA_TRY(cudaStreamSynchronize(s));
+            S.beta = K->h_scal[0];
+        }
+        return LS_OK;
+    };
+
+    std::vector<int> all((size_t)nrhs);
+    for (int q = 0; q < nrhs; ++q) all[q] = q;
+    if ((rc = init(all, true))) return rc;
+    for (Sys& S : sys) {
+        S.current = S.beta; S.accumulator = 1.0; S.rbeta = S.beta;
+        S.tol = fmax(reltol * S.current, abstol);
+        S.active = !(S.iteration >= maxiter || S.current <= S.tol);
+    }
+    std::vector<cplx> y;
+    for (;;) {
+        std::vector<int> act;
+        for (int q = 0; q < nrhs; ++q) if (sys[q].active) act.push_back(q);
+        if (act.empty()) break;
+        // expand!: V_{k+1} = Pl^-1 (A V_k) for every active system
+        std::vector<cd*> ws;
+        for (int q : act) {
+            Sys& S = sys[q];
+            cd* w = S.V + (long)S.k * n;
+            if ((rc = op->apply_dev(S.V + (long)(S.k - 1) * n, w, LS_APPLY_FASTCONVOLUTION))) return rc;
+            ws.push_back(w);
+        }
+        if ((rc = precond(ws))) return rc;
+        std::vector<int> restarting;
+        for (size_t i = 0; i < act.size(); ++i) {
+            Sys& S = sys[act[i]];
+            const int k = S.k;
+            S.mv++;
+            if ((rc = K->orthogonalize(S.V, n, k, ws[i], s))) return rc;
+            LS_CUDA_TRY(cudaMemcpyAsync(K->h_scal, K->d_scal, 2 * (size_t)(k + 1) * sizeof(double), cudaMemcpyDeviceToHost, s));
+            LS_CUDA_TRY(cudaStreamSynchronize(s));
+            for (int r = 0; r <= k; ++r) S.H[r + (size_t)(k - 1) * ldh] = {K->h_scal[2 * r], K->h_scal[2 * r + 1]};
+            cplx acc = {0.0, 0.0};
+            for (int r = 0; r < k; ++r) acc = caddh(acc, cmulh(conjh(S.nullvec[r]), S.H[r + (size_t)(k - 1) * ldh]));
+            const cplx qv = cdivh(acc, S.H[k + (size_t)(k - 1) * ldh]);
+            S.nullvec[k] = {-qv.re, qv.im};
+            S.accumulator += S.nullvec[k].re * S.nullvec[k].re + S.nullvec[k].im * S.nullvec[k].im;
+            S.current = S.rbeta / sqrt(S.accumulator);
+            S.k++;
+            const bool conv = S.current <= S.tol;
+            if (S.k == restart + 1 || conv) {
+                std::vector<cplx> Hc(S.H);
+                solve_least_squares(Hc, ldh, S.beta, S.k - 1, y);
+                LS_CUDA_TRY(cudaMemcpyAsync(K->d_y, y.data(), (size_t)(S.k - 1) * sizeof(cd), cudaMemcpyHostToDevice, s));
+                k_update_solution<<<gs, 256, 0, s>>>(S.V, n, S.k - 1, K->d_y, S.dx, n);
+                K->launches++;
+                LS_CUDA_TRY(cudaStreamSynchronize(s));
+                S.k = 1;
+                if (!conv) restarting.push_back(act[i]);
+            }
+            S.iteration++;
+            if (resnorm_hist && S.nh < hist_cap) resnorm_hist[(size_t)act[i] * hist_cap + S.nh++] = S.current;
+        }
+        // restart of the unconverged systems at the end of a cycle (init does not change `current`: the history entry
+        // above is the one gmres_driver logs after its init)
+        if (!restarting.empty()) {
+            if ((rc = init(restarting, false))) return rc;
+            for (int q : restarting) { Sys& S = sys[q]; S.accumulator = 1.0; S.rbeta = S.beta; S.mv++; }
+        }
+        for (int q : act) { Sys& S = sys[q]; S.active = !(S.iteration >= maxiter || S.current <= S.tol); }
+    }
+    LS_CUDA_TRY(cudaGetLastError());
+    if (host)
+        for (int q = 0; q < nrhs; ++q)
+            LS_CUDA_TRY(cudaMemcpyAsync(x + (size_t)q * ldx, sys[q].dx, vb, cudaMemcpyDeviceToHost, s));
+    LS_CUDA_TRY(cudaStreamSynchronize(s));
+    for (int q = 0; q < nrhs; ++q) {
+        if (niter) niter[q] = sys[q].iteration;
+        if (converged) converged[q] = sys[q].current <= sys[q].tol ? 1 : 0;
+        if (mv_products) mv_products[q] = sys[q].mv;
+    }
+    return LS_OK;
+}
+
 int ls_gmres(ls_handle kh, ls_handle op_h, ls_handle as_h, ls_solve_cb msp_solve, void* user,
              const ls_cdouble* b, ls_cdouble* x, int restart, int64_t maxiter, double reltol, double abstol,
              int initially_zero, double* resnorm_hist, int64_t hist_cap, int64_t* niter, int* converged,
@@ -794,6 +1008,24 @@ int ls_gmres_msp(ls_handle kh, ls_handle op_h, ls_handle as_h, ls_handle msp_h,
     return gmres_driver(K, reinterpret_cast<HandleBase*>(op_h), reinterpret_cast<SpM*>(as_h), reinterpret_cast<MspBase*>(msp_h),
                         nullptr, nullptr, b, x, restart, maxiter, reltol, abstol, initially_zero, resnorm_hist, hist_cap,
                         niter, converged, mv_products, memloc);
+}
+
+// Argument refusals come before any CUDA call.
+int ls_gmres_msp_batch(ls_handle kh, ls_handle op_h, ls_handle as_h, ls_handle msp_h, int nrhs, const ls_cdouble* b, int64_t ldb,
+                       ls_cdouble* x, int64_t ldx, int restart, int64_t maxiter, double reltol, double abstol, int initially_zero,
+                       double* resnorm_hist, int64_t hist_cap, int64_t* niter, int* converged, int64_t* mv_products, int memloc) {
+    LS_REQUIRE(nrhs >= 1, LS_ERR_INVALID, "ls_gmres_msp_batch: nrhs = %d, at least one system needed", nrhs);
+    LS_REQUIRE(kh && op_h && msp_h && b && x, LS_ERR_INVALID, "ls_gmres_msp_batch: null argument");
+    LS_REQUIRE(!resnorm_hist || hist_cap >= 0, LS_ERR_INVALID, "ls_gmres_msp_batch: hist_cap = %ld", (long)hist_cap);
+    Krylov* K = reinterpret_cast<Krylov*>(kh);
+    LS_REQUIRE(K->kind == KIND_VEC, LS_ERR_INVALID, "ls_gmres_msp_batch: not a Krylov workspace handle");
+    LS_REQUIRE(ldb >= K->n && ldx >= K->n, LS_ERR_INVALID, "ls_gmres_msp_batch: leading dimensions ldb = %ld, ldx = %ld must be >= N = %ld",
+               (long)ldb, (long)ldx, (long)K->n);
+    LS_REQUIRE(memloc == LS_MEM_HOST || memloc == LS_MEM_DEVICE, LS_ERR_INVALID, "ls_gmres_msp_batch: unknown memloc %d", memloc);
+    LS_CUDA_TRY(cudaSetDevice(K->device));
+    return gmres_batch_driver(K, reinterpret_cast<HandleBase*>(op_h), reinterpret_cast<SpM*>(as_h), reinterpret_cast<MspBase*>(msp_h),
+                              nrhs, b, ldb, x, ldx, restart, maxiter, reltol, abstol, initially_zero, resnorm_hist, hist_cap, niter,
+                              converged, mv_products, memloc);
 }
 
 // ---- sparsifier sampling on the device (SURVEY.md 8(f) row 2) --------------------------------------------------------

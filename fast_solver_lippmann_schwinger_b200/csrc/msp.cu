@@ -76,7 +76,6 @@ struct Msp : MspBase {
     int solve_dev(const cd* rhs, cd* out, cudaStream_t s) override;
     int solve_launch(const cd* rhs, cd* out, cudaStream_t s);
     int solve_launch2(const cd* rhs, cd* out, cudaStream_t s);
-    int sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) const;
     int tune_sweeps();
     size_t xs_limit(int cols_p) const;
     // the 4 x (depth + 1) dependent launches of one solve, captured once per (rhs, out) pair and replayed as a CUDA graph
@@ -84,8 +83,47 @@ struct Msp : MspBase {
     struct Captured { const cd* rhs; cd* out; cudaGraphExec_t exec; };
     std::vector<Captured> graphs;
     int use_graph = -1;
+
+    // ---- several right-hand sides (ls_msp_solve_batch) ----
+    // Columns go in chunks of cols_max (4), ..., 2 and 1; a chunk of w >= 2 runs the multi-column sweeps (one factor read for w
+    // columns) on work arrays of its own (per depth: w columns of g, z, t), allocated on first use and kept; a chunk of 1
+    // is the single-vector solve.  Each chunk is captured and replayed as a CUDA graph per (pointers, strides, width).
+    struct BatchWork { std::vector<cd*> g, z, t; };
+    BatchWork bwork[4];                           // index log2(w): 1, 2, 3
+    cd* d_bstage = nullptr;                       // host-pointer calls: cols_max columns of staging
+    bool cols_optin = false;
+    struct CapturedB { const cd* rhs; long ldr; cd* out; long ldx; int w; cudaGraphExec_t exec; };
+    std::vector<CapturedB> bgraphs;
+    int use_graph_cols = -1;                      // own flag: a failed batched capture leaves ls_msp_solve's graphs alone
+    // widest chunk (LS_MSP_BATCH_COLS = 2, 4 or 8, read when the handle is created).  Default 4: measured on B200, one
+    // chunk of 8 columns takes longer than two chunks of 4 at 2048^2, 48^3 and 64^3 (DESIGN.md 3.5)
+    int cols_max = 4;
+    int chunk_width(int left) const { for (int w = cols_max; w > 1; w >>= 1) if (left >= w) return w; return 1; }
+    // chunk widths (bit log2 w) a batch of nrhs columns uses; with `subsets` also those of every smaller count (the
+    // lockstep GMRES solves fewer columns as its systems converge)
+    unsigned width_mask(int nrhs, bool subsets) const {
+        unsigned m = 0;
+        if (subsets) { for (int w = 2; w <= cols_max && w <= nrhs; w <<= 1) m |= 1u << log2w(w); return m; }
+        for (int left = nrhs; left > 0;) { const int w = chunk_width(left); left -= w; if (w > 1) m |= 1u << log2w(w); }
+        return m;
+    }
+    static int log2w(int w) { return w >= 8 ? 3 : w >= 4 ? 2 : 1; }
+    // bw: the work arrays of a multi-column chunk (null: the level's own); their column strides, and ldr / ldx for the
+    // caller's vectors, go to *cs
+    int sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a, const BatchWork* bw = nullptr,
+                   lsmsp::Cols* cs = nullptr, long ldr = 0, long ldx = 0) const;
+    size_t work_bytes(int w) const;
+    size_t batch_bytes(int nrhs, bool host, bool subsets) const override;
+    int batch_reserve(int nrhs, bool host, bool subsets) override;
+    int solve_batch_dev(const cd* rhs, long ldr, cd* out, long ldx, int nrhs, cudaStream_t s) override;
+    int solve_launch_cols(int w, const cd* rhs, long ldr, cd* out, long ldx, cudaStream_t s);
+    lsmsp::Choice cols_choice(int d, int which, int w) const;
+    // staging bytes a multi-column launch may use: half the opt-in limit, so that two CTAs still share an SM
+    size_t cols_limit() const { return std::max<size_t>(48 * 1024, smem_max / 2); }
+
     ~Msp() override {
         for (auto& g : graphs) cudaGraphExecDestroy(g.exec);
+        for (auto& g : bgraphs) cudaGraphExecDestroy(g.exec);
         if (cublas) cublasDestroy(cublas);
         if (cusolver) cusolverDnDestroy(cusolver);
     }
@@ -235,6 +273,34 @@ int optin_staging(size_t smem) {
     static unsigned long long done[6][4] = {};
     for (int ll = 0; ll < 6; ++ll)
         for (int ul = 0; ul < 4; ++ul) LS_CUDA_TRY(lsk::smem_optin(gemv2_table[ll][ul][1], (int)smem, done[ll][ul]));
+    return LS_OK;
+}
+
+// multi-column sweeps, NRHS = 2, 4, 8: [log2(NRHS) - 1][lanes_log2][unr_log2][xs]; UNR past lsmsp::cols_unr_cap_log2 maps
+// onto the capped instantiation (cols_choice never asks for it)
+typedef void (*gemv2c_fn)(const lsmsp::Gemv2, const lsmsp::Cols, const lsmsp::Geo);
+#define LS_G2C_UR(L, U, R) lsmsp::k_msp_gemv2_cols<L, ((U) * (R) <= 8 ? (U) : 8 / (R)), false, R>, \
+                           lsmsp::k_msp_gemv2_cols<L, ((U) * (R) <= 8 ? (U) : 8 / (R)), true, R>
+#define LS_G2C_U(L, U, R) { LS_G2C_UR(L, U, R) }
+#define LS_G2C_L(L, R) { LS_G2C_U(L, 1, R), LS_G2C_U(L, 2, R), LS_G2C_U(L, 4, R), LS_G2C_U(L, 8, R) }
+#define LS_G2C_R(R) { LS_G2C_L(1, R), LS_G2C_L(2, R), LS_G2C_L(4, R), LS_G2C_L(8, R), LS_G2C_L(16, R), LS_G2C_L(32, R) }
+const gemv2c_fn gemv2c_table[3][6][4][2] = { LS_G2C_R(2), LS_G2C_R(4), LS_G2C_R(8) };
+
+inline int log2_width(int w) { return w >= 8 ? 3 : w >= 4 ? 2 : 1; }
+
+int launch_gemv2_cols(const lsmsp::Gemv2& a, const lsmsp::Cols& cs, const lsmsp::Choice& ch, int w, cudaStream_t s) {
+    if (a.nodes <= 0 || a.rows_p <= 0) return LS_OK;
+    lsmsp::LaunchGeo L = lsmsp::launch_geo(a.rows_p, a.cols_p, a.nodes, ch);
+    L.smem *= (size_t)w;
+    gemv2c_table[log2_width(w) - 1][ch.lanes_log2][ch.unr_log2][ch.xs ? 1 : 0]<<<L.grid, 256, L.smem, s>>>(a, cs, L.g);
+    return LS_OK;
+}
+
+int optin_staging_cols(size_t smem) {
+    static unsigned long long done[3][6][4] = {};
+    for (int wl = 0; wl < 3; ++wl)
+        for (int ll = 0; ll < 6; ++ll)
+            for (int ul = 0; ul < 4; ++ul) LS_CUDA_TRY(lsk::smem_optin(gemv2c_table[wl][ll][ul][1], (int)smem, done[wl][ll][ul]));
     return LS_OK;
 }
 
@@ -615,34 +681,45 @@ size_t Msp::xs_limit(int cols_p) const {
 }
 
 // arguments of sweep `which` of depth d:  0  z = Sinv g_S   1  t = g_B - F_BS z   2  u_S = z - Y u_B
-int Msp::sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a) const {
+int Msp::sweep_args(int d, int which, const cd* rhs, cd* out, lsmsp::Gemv2& a, const BatchWork* bw, lsmsp::Cols* cs,
+                    long ldr, long ldx) const {
     const int D = (int)lev.size() - 1;
     const Level& L = lev[d];
     const Level* Lc = d < D ? &lev[d + 1] : nullptr;
     const int Fp = L.Sp + L.Bp;
+    cd* g = bw ? bw->g[d] : L.d_g;
+    cd* z = bw ? bw->z[d] : L.d_z;
+    cd* t = bw ? bw->t[d] : L.d_t;
+    cd* tc = Lc ? (bw ? bw->t[d + 1] : Lc->d_t) : nullptr;
+    // column strides of the work arrays: their per-column sizes (work_bytes)
+    const long gcs = (long)L.count * Fp, zcs = (long)L.count * L.Sp, tcs = std::max<long>((long)L.count * L.Bp, 1);
+    const long tccs = Lc ? std::max<long>((long)Lc->count * Lc->Bp, 1) : 0;
     a = lsmsp::Gemv2{};
+    lsmsp::Cols c{};
+    c.f = ldr; c.xg = ldx; c.tchild = tccs;
     a.nodes = L.count;
-    a.pmap = Lc ? L.d_pmap : nullptr; a.tchild = Lc ? Lc->d_t : nullptr; a.Fp = Fp; a.Bpc = Lc ? Lc->Bp : 0;
+    a.pmap = Lc ? L.d_pmap : nullptr; a.tchild = tc; a.Fp = Fp; a.Bpc = Lc ? Lc->Bp : 0;
     if (which == 0) {
         a.M = L.d_Sinv; a.moff = L.d_offS; a.nrows = L.d_ns; a.ncols = L.d_ns; a.rows_p = L.Sp; a.cols_p = L.Sp;
         if (fuse && !L.gather_s) { a.xmode = 2; a.f = rhs; a.sidx = L.d_Sidx; }
-        else { a.xmode = 0; a.x = L.d_g; a.xstride = Fp; }
+        else { a.xmode = 0; a.x = g; a.xstride = Fp; c.x = gcs; }
         a.ymode = 0; a.sign = 1.0;
-        a.out = L.d_z; a.ostride = L.Sp;
+        a.out = z; a.ostride = L.Sp; c.out = zcs;
     } else if (which == 1) {
         a.M = L.d_FBS; a.moff = L.d_offB; a.nrows = L.d_nb; a.ncols = L.d_ns; a.rows_p = L.Bp; a.cols_p = L.Sp;
-        a.xmode = 0; a.x = L.d_z; a.xstride = L.Sp;
+        a.xmode = 0; a.x = z; a.xstride = L.Sp; c.x = zcs;
         if (fuse) a.ymode = 2;
-        else { a.ymode = 1; a.y0 = L.d_g + L.Sp; a.y0stride = Fp; }
+        else { a.ymode = 1; a.y0 = g + L.Sp; a.y0stride = Fp; c.y0 = gcs; }
         a.sign = -1.0;
-        a.out = L.d_t; a.ostride = L.Bp;
+        a.out = t; a.ostride = L.Bp; c.out = tcs;
     } else {
         a.M = L.d_Y; a.moff = L.d_offB; a.nrows = L.d_ns; a.ncols = L.d_nb; a.rows_p = L.Sp; a.cols_p = L.Bp;
-        if (L.gather_y) { a.xmode = 0; a.x = L.d_g; a.xstride = L.Bp; }
+        if (L.gather_y) { a.xmode = 0; a.x = g; a.xstride = L.Bp; c.x = gcs; }
         else { a.xmode = 1; a.xidx = L.d_Bidx; a.xg = out; }
-        a.ymode = 1; a.y0 = L.d_z; a.y0stride = L.Sp; a.sign = -1.0;
-        a.oidx = L.d_Sidx; a.og = out;
+        a.ymode = 1; a.y0 = z; a.y0stride = L.Sp; a.sign = -1.0; c.y0 = zcs;
+        a.oidx = L.d_Sidx; a.og = out; c.out = ldx;
     }
+    if (cs) *cs = c;
     return LS_OK;
 }
 
@@ -755,6 +832,160 @@ int Msp::tune_sweeps() {
     return rc;
 }
 
+// ---- several right-hand sides ----------------------------------------------------------------------------------------
+// geometry of sweep `which` of depth d for chunks of w columns: the LANES of the single-vector plan, so that every column
+// has the single solve's bits (msp_gemv.cuh), UNR / XS by lsmsp::cols_choice
+lsmsp::Choice Msp::cols_choice(int d, int which, int w) const {
+    lsmsp::Gemv2 a;
+    sweep_args(d, which, nullptr, nullptr, a);
+    const Level& L = lev[d];
+    const lsmsp::Choice& single = which == 0 ? L.ch_sinv : which == 1 ? L.ch_fbs : L.ch_y;
+    return lsmsp::cols_choice(single, w, a.rows_p, a.cols_p, a.nodes, a.xmode, cols_limit());
+}
+
+size_t Msp::work_bytes(int w) const {
+    size_t b = 0;
+    for (const Level& L : lev)
+        b += (size_t)w * ((size_t)L.count * (L.Sp + L.Bp) + (size_t)L.count * L.Sp + std::max<size_t>((size_t)L.count * L.Bp, 1));
+    return b * sizeof(cd);
+}
+
+size_t Msp::batch_bytes(int nrhs, bool host, bool subsets) const {
+    size_t b = 0;
+    if (solver == 2) {
+        const unsigned m = width_mask(nrhs, subsets);
+        for (int wl = 1; wl <= 3; ++wl)
+            if ((m >> wl & 1u) && bwork[wl].g.empty()) b += work_bytes(1 << wl);
+    }
+    if (host && !d_bstage) b += (size_t)n * cols_max * sizeof(cd);
+    return b;
+}
+
+int Msp::batch_reserve(int nrhs, bool host, bool subsets) {
+    int rc;
+    if (host && !d_bstage && (rc = dmalloc((void**)&d_bstage, (size_t)n * cols_max * sizeof(cd)))) return rc;
+    if (solver != 2) return LS_OK;
+    if (!cols_optin && smem_max > 48 * 1024) {
+        if ((rc = optin_staging_cols(cols_limit()))) return rc;
+        cols_optin = true;
+    }
+    const unsigned m = width_mask(nrhs, subsets);
+    for (int wl = 1; wl <= 3; ++wl) {
+        BatchWork& W = bwork[wl];
+        if (!(m >> wl & 1u) || !W.g.empty()) continue;
+        const int w = 1 << wl;
+        for (const Level& L : lev) {
+            const size_t nb[3] = {(size_t)w * L.count * (L.Sp + L.Bp), (size_t)w * L.count * L.Sp,
+                                  (size_t)w * std::max<size_t>((size_t)L.count * L.Bp, 1)};
+            cd* p[3];
+            for (int q = 0; q < 3; ++q) {
+                if ((rc = dmalloc((void**)&p[q], std::max<size_t>(nb[q], 1) * sizeof(cd)))) return rc;
+                LS_CUDA_TRY(cudaMemsetAsync(p[q], 0, std::max<size_t>(nb[q], 1) * sizeof(cd), stream));
+            }
+            W.g.push_back(p[0]); W.z.push_back(p[1]); W.t.push_back(p[2]);
+        }
+        LS_CUDA_TRY(cudaStreamSynchronize(stream));
+    }
+    return LS_OK;
+}
+
+// the solve_launch2 sequence for w columns: the same sweeps, gathers and order, on the chunk's work arrays
+int Msp::solve_launch_cols(int w, const cd* rhs, long ldr, cd* out, long ldx, cudaStream_t s) {
+    const int D = (int)lev.size() - 1;
+    const BatchWork& W = bwork[log2_width(w)];
+    lsmsp::Gemv2 a;
+    lsmsp::Cols cs;
+    for (int d = D; d >= 0; --d) {                      // upward: leaves -> root
+        const Level& L = lev[d];
+        // the separate gathers (unfused solves, separators too long to stage) run once per column: they read N-sized
+        // vectors, not factor blocks, and take no part in the sweeps' sharing of the factor reads
+        if (!fuse || L.gather_s) {
+            const int Fp = L.Sp + L.Bp;
+            const long total = (long)L.count * Fp;
+            const Level* Lc = d < D ? &lev[d + 1] : nullptr;
+            const long tccs = Lc ? std::max<long>((long)Lc->count * Lc->Bp, 1) : 0;
+            for (int j = 0; j < w; ++j)
+                k_msp_gather<<<grid_for(total), 256, 0, s>>>(rhs + j * ldr, L.d_Sidx, Lc ? L.d_pmap : nullptr,
+                                                             Lc ? W.t[d + 1] + j * tccs : nullptr, L.Sp, Fp, Lc ? Lc->Bp : 0,
+                                                             total, W.g[d] + j * total);
+        }
+        sweep_args(d, 0, rhs, out, a, &W, &cs, ldr, ldx);
+        launch_gemv2_cols(a, cs, cols_choice(d, 0, w), w, s);
+        if (L.Bp > 0) {
+            sweep_args(d, 1, rhs, out, a, &W, &cs, ldr, ldx);
+            launch_gemv2_cols(a, cs, cols_choice(d, 1, w), w, s);
+        }
+    }
+    for (int d = 0; d <= D; ++d) {                      // downward: root -> leaves, u_S written straight into `out`
+        const Level& L = lev[d];
+        if (L.gather_y) {
+            const long total = (long)L.count * L.Bp;
+            const long gcs = (long)L.count * (L.Sp + L.Bp);
+            for (int j = 0; j < w; ++j)
+                k_msp_gather<<<grid_for(total), 256, 0, s>>>(out + j * ldx, L.d_Bidx, nullptr, nullptr, L.Bp, L.Bp, 0, total,
+                                                             W.g[d] + j * gcs);
+        }
+        sweep_args(d, 2, rhs, out, a, &W, &cs, ldr, ldx);
+        launch_gemv2_cols(a, cs, cols_choice(d, 2, w), w, s);
+    }
+    LS_CUDA_TRY(cudaGetLastError());
+    return LS_OK;
+}
+
+int Msp::solve_batch_dev(const cd* rhs, long ldr, cd* out, long ldx, int nrhs, cudaStream_t s) {
+    // solver 1 (the first version, uniform batches) has no multi-column sweeps: its columns are solved one by one
+    if (solver != 2) {
+        for (int j = 0; j < nrhs; ++j) {
+            int rc = solve_dev(rhs + j * ldr, out + j * ldx, s);
+            if (rc) return rc;
+        }
+        return LS_OK;
+    }
+    if (use_graph_cols < 0) { const char* e = getenv("LS_MSP_GRAPH"); use_graph_cols = e ? atoi(e) : 1; }
+    for (int j0 = 0; j0 < nrhs;) {
+        const int w = chunk_width(nrhs - j0);
+        const cd* r = rhs + j0 * ldr;
+        cd* o = out + j0 * ldx;
+        j0 += w;
+        int rc;
+        if (w == 1) {
+            if ((rc = solve_dev(r, o, s))) return rc;
+            continue;
+        }
+        LS_REQUIRE(!bwork[log2_width(w)].g.empty(), LS_ERR_INVALID,
+                   "Msp batched solve: no work arrays for chunks of %d columns (batch_reserve first)", w);
+        const int per = launches_per_solve + (w - 1) * (int)std::count_if(lev.begin(), lev.end(), [this](const Level& L) {
+            return !fuse || L.gather_s; }) + (w - 1) * (int)std::count_if(lev.begin(), lev.end(), [](const Level& L) { return L.gather_y; });
+        bool done = false;
+        if (use_graph_cols) {
+            for (auto& g : bgraphs)
+                if (g.rhs == r && g.ldr == ldr && g.out == o && g.ldx == ldx && g.w == w) {
+                    LS_CUDA_TRY(cudaGraphLaunch(g.exec, s));
+                    done = true;
+                    break;
+                }
+            if (!done && bgraphs.size() < 64) {
+                cudaGraph_t graph = nullptr;
+                cudaGraphExec_t exec = nullptr;
+                if (cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+                    rc = solve_launch_cols(w, r, ldr, o, ldx, s);
+                    const cudaError_t ce = cudaStreamEndCapture(s, &graph);
+                    if (rc == LS_OK && ce == cudaSuccess && graph && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
+                        bgraphs.push_back(CapturedB{r, ldr, o, ldx, w, exec});
+                        LS_CUDA_TRY(cudaGraphLaunch(exec, s));
+                        done = true;
+                    }
+                    if (graph) cudaGraphDestroy(graph);
+                }
+                if (!done) { cudaGetLastError(); use_graph_cols = 0; }
+            }
+        }
+        if (!done && (rc = solve_launch_cols(w, r, ldr, o, ldx, s))) return rc;
+        launches += per;
+    }
+    return LS_OK;
+}
+
 // ls_msp_factor (l = 1) and ls_msp_factor3d.  Refusals come as early and as cheaply as possible: arguments (no device
 // needed), then the memory the dissection needs against the free device memory (before anything is allocated), then
 // the entries as they are routed (pattern, duplicates).
@@ -799,6 +1030,7 @@ static int msp_factor_entry(const char* fn, ls_handle* out, int64_t n, int64_t m
     if (rc) { delete M; return rc; }
     M->n = N; M->gn = n; M->gm = m; M->gl = l;
     M->solver = solver; M->fuse = fuse; M->tune = tune;
+    if (const char* e = getenv("LS_MSP_BATCH_COLS")) { const int v = atoi(e); if (v == 2 || v == 4 || v == 8) M->cols_max = v; }
     {
         int v = 0;
         if (cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, M->device) == cudaSuccess && (size_t)v > M->smem_max)
@@ -861,6 +1093,57 @@ int ls_msp_solve(ls_handle h, const ls_cdouble* rhs, ls_cdouble* x, int memloc) 
     return LS_OK;
 }
 
+// Refusals before any CUDA call: arguments, then the device memory the work arrays of this column count still need.
+int ls_msp_solve_batch(ls_handle h, const ls_cdouble* rhs, int64_t ldr, ls_cdouble* x, int64_t ldx, int nrhs, int memloc) {
+    LS_REQUIRE(nrhs >= 1, LS_ERR_INVALID, "ls_msp_solve_batch: nrhs = %d, at least one right-hand side needed", nrhs);
+    LS_REQUIRE(h && rhs && x, LS_ERR_INVALID, "ls_msp_solve_batch: null argument");
+    Msp* M = reinterpret_cast<Msp*>(h);
+    LS_REQUIRE(M->kind == KIND_MSP, LS_ERR_INVALID, "ls_msp_solve_batch: not an Msp factorisation handle");
+    LS_REQUIRE(memloc == LS_MEM_HOST || memloc == LS_MEM_DEVICE, LS_ERR_INVALID, "ls_msp_solve_batch: unknown memloc %d", memloc);
+    const int64_t N = M->n;
+    LS_REQUIRE(ldr >= N && ldx >= N, LS_ERR_INVALID, "ls_msp_solve_batch: leading dimensions ldr = %ld, ldx = %ld must be >= N = %ld",
+               (long)ldr, (long)ldx, (long)N);
+    {
+        // x may alias rhs only column for column (same start, same leading dimension)
+        const char* r0 = reinterpret_cast<const char*>(rhs);
+        const char* x0 = reinterpret_cast<const char*>(x);
+        const char* r1 = r0 + ((size_t)ldr * (nrhs - 1) + N) * sizeof(cd);
+        const char* x1 = x0 + ((size_t)ldx * (nrhs - 1) + N) * sizeof(cd);
+        const bool overlap = r0 < x1 && x0 < r1;
+        LS_REQUIRE(!overlap || (r0 == x0 && ldr == ldx), LS_ERR_INVALID,
+                   "ls_msp_solve_batch: x overlaps rhs other than in place (x == rhs needs ldx == ldr; ldr = %ld, ldx = %ld)",
+                   (long)ldr, (long)ldx);
+    }
+    const bool host = memloc == LS_MEM_HOST;
+    LS_CUDA_TRY(cudaSetDevice(M->device));
+    const size_t need = M->batch_bytes(nrhs, host, false);
+    if (need > 0) {
+        size_t free_b = 0, total_b = 0;
+        LS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        LS_REQUIRE(need <= free_b, LS_ERR_NOMEM,
+                   "ls_msp_solve_batch: work arrays for %d right-hand sides need %zu bytes of device memory; %zu of %zu bytes are free",
+                   nrhs, need, free_b, total_b);
+    }
+    int rc = M->batch_reserve(nrhs, host, false);
+    if (rc) return rc;
+    if (!host)
+        return M->solve_batch_dev(reinterpret_cast<const cd*>(rhs), (long)ldr, reinterpret_cast<cd*>(x), (long)ldx, nrhs, M->stream);
+    // host pointers: chunks of cols_max columns through the staging buffer, solved in place there
+    const cd* hr = reinterpret_cast<const cd*>(rhs);
+    cd* hx = reinterpret_cast<cd*>(x);
+    const size_t vb = (size_t)N * sizeof(cd);
+    for (int j0 = 0; j0 < nrhs; j0 += M->cols_max) {
+        const int w = std::min(nrhs - j0, M->cols_max);
+        LS_CUDA_TRY(cudaMemcpy2DAsync(M->d_bstage, vb, hr + (size_t)j0 * ldr, (size_t)ldr * sizeof(cd), vb, (size_t)w,
+                                      cudaMemcpyHostToDevice, M->stream));
+        if ((rc = M->solve_batch_dev(M->d_bstage, (long)N, M->d_bstage, (long)N, w, M->stream))) return rc;
+        LS_CUDA_TRY(cudaMemcpy2DAsync(hx + (size_t)j0 * ldx, (size_t)ldx * sizeof(cd), M->d_bstage, vb, vb, (size_t)w,
+                                      cudaMemcpyDeviceToHost, M->stream));
+        LS_CUDA_TRY(cudaStreamSynchronize(M->stream));
+    }
+    return LS_OK;
+}
+
 int ls_msp_info(ls_handle h, int64_t* factor_bytes, int* depth, double* factor_seconds) {
     LS_REQUIRE(h, LS_ERR_INVALID, "ls_msp_info: null handle");
     Msp* M = reinterpret_cast<Msp*>(h);
@@ -889,6 +1172,11 @@ int ls_msp_plan(ls_handle h, char* buf, int64_t cap) {
             const char* nm[3] = {"sinv", "fbs", "y"};
             for (int w = 0; w < 3; ++w) {
                 snprintf(line, sizeof line, " %s L%d U%d X%d", nm[w], 1 << ch[w]->lanes_log2, 1 << ch[w]->unr_log2, ch[w]->xs);
+                out += line;
+                // the multi-column kernel of ls_msp_solve_batch (same LANES): UNR and XS for 2, 4 and 8 columns
+                const lsmsp::Choice c2 = M->cols_choice((int)d, w, 2), c4 = M->cols_choice((int)d, w, 4), c8 = M->cols_choice((int)d, w, 8);
+                snprintf(line, sizeof line, " cols U%dX%d/U%dX%d/U%dX%d", 1 << c2.unr_log2, c2.xs, 1 << c4.unr_log2, c4.xs,
+                         1 << c8.unr_log2, c8.xs);
                 out += line;
             }
         }

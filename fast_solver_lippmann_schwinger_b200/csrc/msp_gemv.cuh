@@ -217,6 +217,198 @@ __global__ void __launch_bounds__(256, 2) k_msp_gemv2(const Gemv2 a, const Geo g
 }
 #endif
 
+// ---- multi-column variant: NRHS right-hand sides per factor read ---------------------------------------------------
+// The same sweep for NRHS vectors at once (msp.cu, ls_msp_solve_batch): every matrix element loaded from HBM feeds NRHS
+// complex FMAs.  Column j of each vector the sweep addresses lies at (column-0 address) + j * (its column stride); the
+// index arrays (xidx, sidx, pmap, oidx) are shared by all columns.  Per column, lane l adds columns l, l + LANES, ... in
+// the order of k_msp_gemv2 and the xor tree is the same, so for a given LANES every column of the result has the bits of
+// the single-vector kernel, whatever UNR, XS and NRHS are.
+struct Cols { long f, x, xg, tchild, y0, out; };
+
+template <int NRHS>
+LSMSP_HD void add_children_cols(const Gemv2& a, const Cols& cs, unsigned t, int p, cd (&v)[NRHS]) {
+    if (a.pmap == nullptr) return;
+    const int k0 = ldg_(&a.pmap[((long)t * 2 + 0) * a.Fp + p]);
+    const int k1 = ldg_(&a.pmap[((long)t * 2 + 1) * a.Fp + p]);
+    if (k0 >= 0)
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) { const cd w = a.tchild[(2L * t) * a.Bpc + k0 + j * cs.tchild]; v[j].x += w.x; v[j].y += w.y; }
+    if (k1 >= 0)
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) { const cd w = a.tchild[(2L * t + 1) * a.Bpc + k1 + j * cs.tchild]; v[j].x += w.x; v[j].y += w.y; }
+}
+
+// X(t, c) of every column; the index is chased once for all of them
+template <int NRHS>
+LSMSP_HD void fetch_x_cols(const Gemv2& a, const Cols& cs, unsigned t, int c, cd (&v)[NRHS]) {
+    if (a.xmode == 0) {
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) v[j] = a.x[(long)t * a.xstride + c + j * cs.x];
+        return;
+    }
+    if (a.xmode == 1) {
+        const int gi = ldg_(&a.xidx[(long)t * a.cols_p + c]);
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) v[j] = gi >= 0 ? a.xg[gi + j * cs.xg] : czero();
+        return;
+    }
+    const int gi = ldg_(&a.sidx[(long)t * a.cols_p + c]);
+#pragma unroll
+    for (int j = 0; j < NRHS; ++j) v[j] = gi >= 0 ? a.f[gi + j * cs.f] : czero();
+    add_children_cols<NRHS>(a, cs, t, c, v);
+}
+
+// X(t, c) of column j alone (the groups that fetch X themselves: one column live at a time)
+LSMSP_HD cd fetch_x_col(const Gemv2& a, const Cols& cs, unsigned t, int c, int j) {
+    if (a.xmode == 0) return a.x[(long)t * a.xstride + c + j * cs.x];
+    if (a.xmode == 1) {
+        const int gi = ldg_(&a.xidx[(long)t * a.cols_p + c]);
+        return gi >= 0 ? a.xg[gi + j * cs.xg] : czero();
+    }
+    cd v = czero();
+    const int gi = ldg_(&a.sidx[(long)t * a.cols_p + c]);
+    if (gi >= 0) v = a.f[gi + j * cs.f];
+    if (a.pmap != nullptr) {
+        const int k0 = ldg_(&a.pmap[((long)t * 2 + 0) * a.Fp + c]);
+        const int k1 = ldg_(&a.pmap[((long)t * 2 + 1) * a.Fp + c]);
+        if (k0 >= 0) { const cd w = a.tchild[(2L * t) * a.Bpc + k0 + j * cs.tchild]; v.x += w.x; v.y += w.y; }
+        if (k1 >= 0) { const cd w = a.tchild[(2L * t + 1) * a.Bpc + k1 + j * cs.tchild]; v.x += w.x; v.y += w.y; }
+    }
+    return v;
+}
+
+template <int NRHS>
+LSMSP_HD void fetch_y0_cols(const Gemv2& a, const Cols& cs, unsigned t, int r, cd (&v)[NRHS]) {
+#pragma unroll
+    for (int j = 0; j < NRHS; ++j) v[j] = a.ymode == 1 ? a.y0[(long)t * a.y0stride + r + j * cs.y0] : czero();
+    if (a.ymode == 2) add_children_cols<NRHS>(a, cs, t, a.cols_p + r, v);
+}
+
+// phase 1 (XS): column j of the CTA's X -> xs[j * npc * cols_p + tn * cols_p + c] (a block per column: the lanes of a
+// group read consecutive c, as in k_msp_gemv2)
+template <int NRHS>
+LSMSP_HD void stage_x_cols(const Gemv2& a, const Cols& cs, const Geo& g, unsigned bid, unsigned tid, cd* xs) {
+    unsigned tfirst, cnt;
+    if (g.cpn == 1) {
+        tfirst = bid * g.npc;
+        cnt = (unsigned)a.nodes - tfirst < g.npc ? (unsigned)a.nodes - tfirst : g.npc;
+    } else {
+        tfirst = bid / g.cpn;
+        cnt = 1;
+    }
+    const unsigned total = cnt * (unsigned)a.cols_p;
+    const long cstride = (long)g.npc * a.cols_p;
+    for (unsigned i = tid; i < total; i += 256u) {
+        const unsigned tn = i / (unsigned)a.cols_p;
+        const int c = (int)(i - tn * (unsigned)a.cols_p);
+        const unsigned t = tfirst + tn;
+        cd v[NRHS];
+        if (c < ldg_(&a.ncols[t])) fetch_x_cols<NRHS>(a, cs, t, c, v);
+        else
+#pragma unroll
+            for (int j = 0; j < NRHS; ++j) v[j] = czero();
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) xs[j * cstride + i] = v[j];
+    }
+}
+
+// phase 2: per-lane partial sums of the group's UNR rows for every column.  The UC * UNR matrix loads of a trip are issued
+// as one batch (as in accumulate); X is read one column at a time next to its use, so the registers held across the trip
+// are the matrix elements and the NRHS x UNR sums
+template <int LANES, int UNR, bool XS, int NRHS>
+LSMSP_HD void accumulate_cols(const Gemv2& a, const Cols& cs, const Geo& g, const ThreadMap& m, const cd* xs,
+                              double (&sr)[NRHS][UNR], double (&si)[NRHS][UNR]) {
+#pragma unroll
+    for (int j = 0; j < NRHS; ++j)
+#pragma unroll
+        for (int u = 0; u < UNR; ++u) { sr[j][u] = 0.0; si[j][u] = 0.0; }
+    if (!m.work) return;
+    const cd* base = a.M + ldg_(&a.moff[m.t]) + (long)m.r0 * m.nc;
+    const int nrow = (m.nr - m.r0) < UNR ? (m.nr - m.r0) : UNR;
+    const long cstride = (long)g.npc * a.cols_p;
+    const cd* xsn = XS ? xs + (long)m.tn * a.cols_p : nullptr;
+    constexpr int UC = (8 / UNR) > 0 ? (8 / UNR) : 1;
+    for (int c0 = m.lane; c0 < m.nc; c0 += LANES * UC) {
+        cd e[UC][UNR];
+#pragma unroll
+        for (int k = 0; k < UC; ++k) {
+            const int c = c0 + k * LANES;
+            const int cc = c < m.nc ? c : m.nc - 1;
+#pragma unroll
+            for (int u = 0; u < UNR; ++u) e[k][u] = ldg_(&base[(long)(u < nrow ? u : nrow - 1) * m.nc + cc]);
+        }
+#pragma unroll
+        for (int k = 0; k < UC; ++k) {
+            const int c = c0 + k * LANES;
+            const int cc = c < m.nc ? c : m.nc - 1;
+#pragma unroll
+            for (int u = 0; u < UNR; ++u) if (u >= nrow) e[k][u] = czero();
+#pragma unroll
+            for (int j = 0; j < NRHS; ++j) {
+                cd v = XS ? xsn[j * cstride + cc] : fetch_x_col(a, cs, m.t, cc, j);
+                if (c >= m.nc) v = czero();
+#pragma unroll
+                for (int u = 0; u < UNR; ++u) {
+                    sr[j][u] = fma(e[k][u].x, v.x, sr[j][u]);
+                    sr[j][u] = fma(-e[k][u].y, v.y, sr[j][u]);
+                    si[j][u] = fma(e[k][u].x, v.y, si[j][u]);
+                    si[j][u] = fma(e[k][u].y, v.x, si[j][u]);
+                }
+            }
+        }
+    }
+}
+
+// phase 4: lane l stores rows l, l + LANES, ... of every column
+template <int LANES, int UNR, int NRHS>
+LSMSP_HD void store_rows_cols(const Gemv2& a, const Cols& cs, const ThreadMap& m, const double (&sr)[NRHS][UNR],
+                              const double (&si)[NRHS][UNR]) {
+    if (!m.work) return;
+#pragma unroll
+    for (int u = 0; u < UNR; ++u) {
+        if ((u % LANES) != m.lane || m.r0 + u >= m.nr) continue;
+        const int r = m.r0 + u;
+        cd y[NRHS];
+        if (a.ymode != 0) fetch_y0_cols<NRHS>(a, cs, m.t, r, y);
+        const int gi = a.oidx ? a.oidx[(long)m.t * a.rows_p + r] : 0;
+#pragma unroll
+        for (int j = 0; j < NRHS; ++j) {
+            cd val;
+            val.x = a.sign * sr[j][u]; val.y = a.sign * si[j][u];
+            if (a.ymode != 0) { val.x += y[j].x; val.y += y[j].y; }
+            if (a.oidx) {
+                if (gi >= 0) a.og[gi + j * cs.out] = val;
+            } else {
+                a.out[(long)m.t * a.ostride + r + j * cs.out] = val;
+            }
+        }
+    }
+}
+
+#ifdef __CUDACC__
+template <int LANES, int UNR, bool XS, int NRHS>
+__global__ void __launch_bounds__(256, 2) k_msp_gemv2_cols(const Gemv2 a, const Cols cs, const Geo g) {
+    extern __shared__ double2 lsmsp_xs[];
+    if (XS) {
+        stage_x_cols<NRHS>(a, cs, g, blockIdx.x, threadIdx.x, lsmsp_xs);
+        __syncthreads();
+    }
+    const ThreadMap m = map_thread<LANES, UNR>(a, g, blockIdx.x, threadIdx.x);
+    double sr[NRHS][UNR], si[NRHS][UNR];
+    accumulate_cols<LANES, UNR, XS, NRHS>(a, cs, g, m, lsmsp_xs, sr, si);
+#pragma unroll
+    for (int j = 0; j < NRHS; ++j)
+#pragma unroll
+        for (int u = 0; u < UNR; ++u)
+#pragma unroll
+            for (int o = LANES / 2; o > 0; o >>= 1) {
+                sr[j][u] += __shfl_xor_sync(0xffffffffu, sr[j][u], o, LANES);
+                si[j][u] += __shfl_xor_sync(0xffffffffu, si[j][u], o, LANES);
+            }
+    store_rows_cols<LANES, UNR, NRHS>(a, cs, m, sr, si);
+}
+#endif
+
 // ---- launch geometry (host) -------------------------------------------------------------------------------------
 struct Choice { int lanes_log2, unr_log2, xs; };       // LANES = 1 << lanes_log2 (1..32), UNR = 1 << unr_log2 (1..8)
 
@@ -249,6 +441,23 @@ inline Choice default_choice(int cols_p, int xmode) {
     ch.lanes_log2 = lg;
     ch.unr_log2 = 2;
     ch.xs = xmode != 0 ? 1 : 0;
+    return ch;
+}
+
+// The multi-column kernel keeps NRHS x UNR complex sums per lane next to the 8 matrix elements in flight: UNR * NRHS <= 8
+// keeps them within the 128 registers of __launch_bounds__(256, 2) (ptxas reports no spills).
+constexpr int COLS_MAX = 8;                              // widest compiled NRHS; wider batches go in chunks
+LSMSP_HD int cols_unr_cap_log2(int nrhs) { return nrhs >= 8 ? 0 : nrhs >= 4 ? 1 : nrhs >= 2 ? 2 : 3; }
+
+// Geometry of the multi-column sweep: the LANES of the single-vector plan (the bits depend on it), UNR capped as above,
+// X staged whenever the single plan stages it or X is index-chased (one fetch then serves NRHS columns), provided the
+// staging buffer of NRHS columns fits in `limit` bytes
+inline Choice cols_choice(const Choice& single, int nrhs, int rows_p, int cols_p, int nodes, int xmode, size_t limit) {
+    Choice ch = single;
+    const int cap = cols_unr_cap_log2(nrhs);
+    if (ch.unr_log2 > cap) ch.unr_log2 = cap;
+    ch.xs = (single.xs || xmode != 0) ? 1 : 0;
+    if (ch.xs && launch_geo(rows_p, cols_p, nodes, ch).smem * (size_t)nrhs > limit) ch.xs = 0;
     return ch;
 }
 

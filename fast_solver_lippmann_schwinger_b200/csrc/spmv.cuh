@@ -41,6 +41,13 @@ struct MspBase : HandleBase {
     int launches_per_solve = 0;
     // out <- Msp^-1 rhs on device pointers (out may alias rhs), enqueued on stream s
     virtual int solve_dev(const cd* rhs, cd* out, cudaStream_t s) = 0;
+    // the same for nrhs column-major columns (leading dimensions ldr / ldx; out may alias rhs when ldx == ldr).
+    // batch_bytes: device memory a batch of nrhs columns still has to allocate (work arrays kept per chunk width, with
+    // `subsets` also those of every smaller column count, with `host` the staging of host-pointer calls); batch_reserve
+    // allocates it.  solve_batch_dev needs batch_reserve first.
+    virtual size_t batch_bytes(int nrhs, bool host, bool subsets) const = 0;
+    virtual int batch_reserve(int nrhs, bool host, bool subsets) = 0;
+    virtual int solve_batch_dev(const cd* rhs, long ldr, cd* out, long ldx, int nrhs, cudaStream_t s) = 0;
 };
 
 }  // namespace ls

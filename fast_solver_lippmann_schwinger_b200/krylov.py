@@ -131,6 +131,17 @@ class GPUMspFactorization(_Handle):
         return buf.value.decode()
 
     def solve(self, b, out=None):
+        """``MspInv \\ b``.  A host array of shape (N, K) is K right-hand sides solved together (ls_msp_solve_batch: each
+        stored factor block is read once per chunk of up to 4 columns); each column equals the solve of that column alone."""
+        if isinstance(b, np.ndarray) and b.ndim == 2:
+            if b.shape[0] != self.N or b.shape[1] < 1:
+                raise ValueError("DimensionMismatch: b is %s, Msp has %d unknowns" % (b.shape, self.N))
+            B = np.asfortranarray(b, dtype=np.complex128)
+            X = np.empty(B.shape, dtype=np.complex128, order="F") if out is None else out
+            if not (isinstance(X, np.ndarray) and X.shape == B.shape and X.dtype == np.complex128 and X.flags.f_contiguous):
+                raise ValueError("DimensionMismatch: out must be a Fortran-ordered complex128 array of shape %s" % (B.shape,))
+            check(lib().ls_msp_solve_batch(self.handle, ptr(B), self.N, ptr(X), self.N, B.shape[1], _lib.MEM_HOST))
+            return X
         if isinstance(b, DeviceBuffer):
             out = b if out is None else out
             check(lib().ls_msp_solve(self.handle, ptr(b), ptr(out), _lib.MEM_DEVICE))
@@ -254,6 +265,8 @@ def gmres_(x, A, b, Pl=None, abstol=0.0, reltol=None, restart=None, maxiter=None
     x is updated in place (numpy array or DeviceBuffer).  Returns x, or (x, history) with log=True.
     """
     N = A.size(1)
+    if isinstance(b, np.ndarray) and b.ndim == 2:
+        return _gmres_batch(x, A, b, Pl, abstol, reltol, restart, maxiter, log, initially_zero, workspace, orth_meth)
     reltol = float(np.sqrt(np.finfo(np.float64).eps)) if reltol is None else float(reltol)
     restart = min(20, N) if restart is None else int(restart)
     maxiter = getattr(A, "N_global", N) if maxiter is None else max(int(maxiter), 0)
@@ -289,3 +302,45 @@ def gmres_(x, A, b, Pl=None, abstol=0.0, reltol=None, restart=None, maxiter=None
     check(lib().ls_krylov_last_precond_host_seconds(ws.handle, C.byref(sec)))
     h.msp_host_seconds = float(sec.value)      # D2H + host Msp solve + H2D inside the loop (0 with solverType="GPU")
     return x, h
+
+
+def _gmres_batch(x, A, b, Pl, abstol, reltol, restart, maxiter, log, initially_zero, workspace, orth_meth):
+    """gmres_ with an N x K right-hand side: K independent GMRES runs in lockstep (ls_gmres_msp_batch) sharing A and the
+    device preconditioner; x (N x K) is updated in place and log=True returns one ConvergenceHistory per column."""
+    N = A.size(1)
+    if Pl is None or getattr(Pl, "MspGPU", None) is None:
+        raise _lib.LSUnsupported(_lib.LS_ERR_UNSUPPORTED, "gmres!: several right-hand sides need Pl with solverType='GPU'")
+    if orth_meth != "ModifiedGramSchmidt":
+        raise _lib.LSUnsupported(_lib.LS_ERR_UNSUPPORTED, "gmres!: several right-hand sides run ModifiedGramSchmidt")
+    if b.shape[0] != N or b.shape[1] < 1:
+        raise ValueError("DimensionMismatch: b is %s, the operator has %d unknowns" % (b.shape, N))
+    if not (isinstance(x, np.ndarray) and x.dtype == np.complex128 and x.shape == b.shape):
+        raise ValueError("DimensionMismatch: x must be a complex128 array of shape %s" % (b.shape,))
+    K = b.shape[1]
+    reltol = float(np.sqrt(np.finfo(np.float64).eps)) if reltol is None else float(reltol)
+    restart = min(20, N) if restart is None else int(restart)
+    maxiter = N if maxiter is None else max(int(maxiter), 0)
+    ws = workspace if workspace is not None else KrylovWorkspace(N)
+    check(lib().ls_krylov_set_orth(ws.handle, 0))
+    B = np.asfortranarray(b, dtype=np.complex128)
+    X = np.asfortranarray(x)
+    cap = maxiter if maxiter < 1_000_000 else 1_000_000
+    hist = np.zeros((max(cap, 1), K), dtype=np.float64, order="F")
+    niter = np.zeros(K, dtype=np.int64)
+    conv = np.zeros(K, dtype=np.int32)
+    mv = np.zeros(K, dtype=np.int64)
+    as_h = Pl.As.handle if Pl.As is not None else None
+    check(lib().ls_gmres_msp_batch(ws.handle, A.handle, as_h, Pl.MspGPU.handle, K, ptr(B), N, ptr(X), N, restart, maxiter,
+                                   reltol, float(abstol), 1 if initially_zero else 0, ptr(hist), max(cap, 1), ptr(niter),
+                                   ptr(conv), ptr(mv), _lib.MEM_HOST))
+    if X is not x:
+        x[...] = X
+    if not log:
+        return x
+    hs = []
+    for q in range(K):
+        n = min(int(niter[q]), cap)
+        h = ConvergenceHistory(hist[:n, q].copy(), int(niter[q]), bool(conv[q]), int(mv[q]), restart)
+        h.msp_host_seconds = 0.0
+        hs.append(h)
+    return x, hs

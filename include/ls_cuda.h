@@ -218,9 +218,20 @@ int ls_msp_factor3d(ls_handle* out, int64_t n, int64_t m, int64_t l, const int64
                     const ls_cdouble* nzval);
 /* x <- Msp^-1 rhs (x may alias rhs); host or device pointers per memloc */
 int ls_msp_solve(ls_handle msp, const ls_cdouble* rhs, ls_cdouble* x, int memloc);
+/* X <- Msp^-1 RHS for nrhs right-hand sides at once (several incident fields with one preconditioner): rhs and x are
+ * column-major N x nrhs arrays with leading dimensions ldr, ldx >= N; x may alias rhs when ldx == ldr (in place).
+ * Each stored factor block is read once per chunk of columns and applied to all of them (multi-column sweeps,
+ * csrc/msp_gemv.cuh): chunks of 4, 2 and 1 (LS_MSP_BATCH_COLS=8 / =2 at handle creation: chunks of up to 8 / 2).  Every column is bit-identical to ls_msp_solve of
+ * that column.  Work arrays for each chunk width are allocated on first use and kept by the handle; when the device
+ * has too little free memory for them -> LS_ERR_NOMEM before anything is allocated.  nrhs < 1, ld < N, a null pointer
+ * or an overlap of x and rhs other than in place -> LS_ERR_INVALID before any CUDA call.  Host or device pointers per
+ * memloc; with device pointers each chunk is replayed as a CUDA graph per (pointers, leading dimensions, width).      */
+int ls_msp_solve_batch(ls_handle msp, const ls_cdouble* rhs, int64_t ldr, ls_cdouble* x, int64_t ldx, int nrhs, int memloc);
 int ls_msp_info(ls_handle msp, int64_t* factor_bytes, int* depth, double* factor_seconds);
 /* one line per dissection depth: node count, padded block sizes and the kernel geometry (lanes per row group, rows per
- * group, X staged in shared memory) chosen for its three sweeps; first line: solver version, fusion, tuning time.
+ * group, X staged in shared memory) chosen for its three sweeps, each followed by "cols UuXx/UuXx/UuXx": rows per group
+ * and staging of the multi-column kernel of ls_msp_solve_batch for 2, 4 and 8 columns (same lanes); first line: solver
+ * version, fusion, tuning time.
  * Writes at most `cap` bytes including the terminator into `buf` (diagnostics for bench / profiles).               */
 int ls_msp_plan(ls_handle msp, char* buf, int64_t cap);
 /* ls_gmres with ldiv!(Pl, v) = Msp^-1 (As v) entirely on the device (`msp` from ls_msp_factor / ls_msp_factor3d, `As`
@@ -229,6 +240,19 @@ int ls_gmres_msp(ls_handle krylov, ls_handle op, ls_handle As, ls_handle msp,
                  const ls_cdouble* b, ls_cdouble* x, int restart, int64_t maxiter, double reltol,
                  double abstol, int initially_zero, double* resnorm_hist, int64_t hist_cap,
                  int64_t* niter, int* converged, int64_t* mv_products, int memloc);
+/* nrhs independent ls_gmres_msp runs side by side with one op, As and msp (several incident fields): b and x are
+ * column-major N x nrhs arrays (leading dimensions ldb, ldx >= N), resnorm_hist is hist_cap x nrhs (column q: system q's
+ * history), niter / converged / mv_products hold nrhs entries (each pointer nullable).  Each system keeps its own Krylov
+ * basis, Hessenberg matrix, restarts and tolerance and gets the bits ls_gmres_msp gives it alone; per lockstep iteration
+ * the applies, SpMVs and Gram-Schmidt steps run system by system and the Msp^-1 of all active systems is one
+ * ls_msp_solve_batch.  A system that converged or reached maxiter drops out; its x is formed as ls_gmres_msp forms it.
+ * Memory for nrhs bases of restart + 1 vectors (and the batched solve's work arrays) is checked against the free device
+ * memory before anything is allocated -> LS_ERR_NOMEM; nrhs < 1, ld < N, null pointers -> LS_ERR_INVALID before any
+ * CUDA call; a sharded operator -> LS_ERR_UNSUPPORTED.                                                               */
+int ls_gmres_msp_batch(ls_handle krylov, ls_handle op, ls_handle As, ls_handle msp, int nrhs,
+                       const ls_cdouble* b, int64_t ldb, ls_cdouble* x, int64_t ldx, int restart, int64_t maxiter,
+                       double reltol, double abstol, int initially_zero, double* resnorm_hist, int64_t hist_cap,
+                       int64_t* niter, int* converged, int64_t* mv_products, int memloc);
 /* wall time the last ls_gmres spent in D2H + msp_solve callback + H2D (the "Msp-solve" column of SURVEY.md H1) */
 int ls_krylov_last_precond_host_seconds(ls_handle krylov, double* seconds);
 

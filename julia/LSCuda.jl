@@ -238,6 +238,13 @@ function \(F::GPUMspFactorization, b::Vector{ComplexF64})
     check(ccall((:ls_msp_solve, libls), Cint, (Ptr{Cvoid}, Ptr{ComplexF64}, Ptr{ComplexF64}, Cint), F.h.ptr, b, x, LS_MEM_HOST))
     return x
 end
+"`F \\ B` for an N x K matrix: the K right-hand sides in one ls_msp_solve_batch (each factor block read once per chunk of columns)."
+function \(F::GPUMspFactorization, B::Matrix{ComplexF64})
+    X = similar(B)
+    check(ccall((:ls_msp_solve_batch, libls), Cint, (Ptr{Cvoid}, Ptr{ComplexF64}, Int64, Ptr{ComplexF64}, Int64, Cint, Cint),
+                F.h.ptr, B, size(B, 1), X, size(X, 1), size(B, 2), LS_MEM_HOST))
+    return X
+end
 function msp_info(F::GPUMspFactorization)
     fb = Ref{Int64}(0); dep = Ref{Cint}(0); sec = Ref{Float64}(0.0)
     check(ccall((:ls_msp_info, libls), Cint, (Ptr{Cvoid}, Ref{Int64}, Ref{Cint}, Ref{Float64}), F.h.ptr, fb, dep, sec))
@@ -262,6 +269,12 @@ GPUSparsifyingPreconditioner(Msp, As; solverType::String="UMFPACK", grid=nothing
 \(M::GPUSparsifyingPreconditioner, b::Array{ComplexF64,1}) = M.MspInv \ (M.As * b)                     # :132-145
 function ldiv!(M::GPUSparsifyingPreconditioner, b::AbstractArray{ComplexF64,1})                        # :147-166
     b[:] = M.MspInv \ (M.As * Vector(b))
+end
+# several right-hand sides: with solverType = "GPU" the Msp^-1 of all columns is one batched solve
+function ldiv!(M::GPUSparsifyingPreconditioner, B::Matrix{ComplexF64})
+    AB = reduce(hcat, [M.As * B[:, j] for j in 1:size(B, 2)])
+    B[:, :] = M.MspInv isa GPUMspFactorization ? M.MspInv \ AB : reduce(hcat, [M.MspInv \ AB[:, j] for j in 1:size(B, 2)])
+    return B
 end
 
 # ------------------------------------------------------- device-resident GMRES (whole loop on GPU)
@@ -305,6 +318,33 @@ function gmres_gpu!(x::Vector{ComplexF64}, A, b::Vector{ComplexF64}; Pl=nothing,
         K.ptr, A.h.ptr, as, cb isa Ptr ? cb : Base.unsafe_convert(Ptr{Cvoid}, cb), C_NULL, b, x, restart, maxiter,
         reltol, abstol, initially_zero, hist, maxiter, niter, conv, mv, LS_MEM_HOST))
     return log ? (x, (resnorm=hist[1:niter[]], iters=niter[], isconverged=conv[] != 0, mvps=mv[])) : x
+end
+
+"""
+    gmres_gpu!(X::Matrix, A, B::Matrix; Pl, abstol, reltol, restart, maxiter, log, initially_zero)
+
+K independent gmres! runs for the columns of B (several incident fields) in lockstep on the device
+(ls_gmres_msp_batch): Pl must be built with solverType = "GPU"; each system gets the history and x that
+gmres_gpu! gives it alone, and the Msp^-1 of all active systems is one batched solve per iteration.
+With log = true the second result is a vector of K histories.
+"""
+function gmres_gpu!(X::Matrix{ComplexF64}, A, B::Matrix{ComplexF64}; Pl, abstol=0.0, reltol=sqrt(eps(Float64)),
+                    restart=min(20, size(B, 1)), maxiter=size(B, 1), log=false, initially_zero=false)
+    N, K = size(B)
+    size(X) == (N, K) || throw(DimensionMismatch("X is $(size(X)), B is $(size(B))"))
+    Pl.MspInv isa GPUMspFactorization || throw(ArgumentError("several right-hand sides need Pl with solverType = \"GPU\""))
+    kh = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:ls_krylov_create, libls), Cint, (Ref{Ptr{Cvoid}}, Int64), kh, N))
+    W = Handle(kh[])
+    cap = min(maxiter, 1_000_000)                 # history rows kept, as in the Python mirror
+    hist = zeros(Float64, cap, K); niter = zeros(Int64, K); conv = zeros(Cint, K); mv = zeros(Int64, K)
+    check(ccall((:ls_gmres_msp_batch, libls), Cint,
+        (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Cint, Ptr{ComplexF64}, Int64, Ptr{ComplexF64}, Int64, Cint, Int64,
+         Float64, Float64, Cint, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Cint}, Ptr{Int64}, Cint),
+        W.ptr, A.h.ptr, Pl.As.h.ptr, Pl.MspInv.h.ptr, K, B, N, X, N, restart, maxiter,
+        reltol, abstol, initially_zero, hist, cap, niter, conv, mv, LS_MEM_HOST))
+    log || return X
+    return X, [(resnorm=hist[1:min(niter[q], cap), q], iters=niter[q], isconverged=conv[q] != 0, mvps=mv[q]) for q in 1:K]
 end
 
 export GPUFastM, op2d_info, GPUFastM3D, GPUFastM3DSharded, op3d_lines, nccl_unique_id, GPUSparsifyingPreconditioner, GPUSparseMatrixCSC, GPUMspFactorization, msp_info, fastconvolution, FFTconvolution,
