@@ -13,6 +13,7 @@
 //   mode B kernels: eight adjacent lines are interleaved across lanes (lane%8 = line) so that
 //                   strided lines (es large, ls == 1) are read/written as 128-byte segments.
 #pragma once
+#include <cuda.h>   // CUtensorMap (the type only: the maps are encoded through the runtime's driver entry point)
 #include "fft_engine.cuh"
 
 namespace lsk {
@@ -118,6 +119,7 @@ __device__ __forceinline__ long line_in(const LineAddr& a, long L) { return (L %
 __device__ __forceinline__ long line_out(const LineAddr& a, long L) { return (L % a.ldim0) * a.out_ls0 + (L / a.ldim0) * a.out_ls1; }
 
 // per-CTA shared memory: [exchange: LPC*N][(mid only) x copy: LPC*N][(mid, mode B only) spectrum: LPC*N][tw1][mbarrier]
+// (k_mid_swap: [exchange][lines: LPC*N][tw1][mbarrier], sized in launch_mid_swap)
 template <int N, bool MODE_B> struct Smem {
     static constexpr int LPC = MODE_B ? GeoB<N>::LPC : GeoA<N>::LPC;
     static constexpr int TW1N = EngTab<N>::TW1N;
@@ -292,30 +294,51 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
 // holds the input line x while r = 0 is transformed, then x and the r = 0 result trade places (each thread swaps
 // its own 16 elements, no barrier), and the r = 2 result is combined with the held one on the way out.  The spectrum
 // values are requested before the last butterfly stage and held in registers across it.
-template <int N, int MINB>
+// The lines move by tensor copies, not through the load/store pipe: their points are one x-slot (16 bytes) wide in
+// A and CW-interleaved in C, so an LSU access of a line used 16 bytes of every 128-byte (A) or 64-byte (C) line.
+// tmA: 2-D map of A as FLOAT64 {2 pn, lm}; line L is the boxes {2, BOX} at (2L, j0).  tmC: 3-D map of C
+// {2 CW, lm, pn/CW}; line L is the boxes {2, BOX, 1} at (2 (L % CW), j0, L / CW), CW = 2^CWS.  BOX = min(N, 256);
+// each line of the CTA has its own N / BOX boxes.  Thread 0 issues the loads into the buffer first thing (the table
+// set-up runs under them) and, after the combine has been written back into the same buffer, the stores.
+// With one resident CTA per SM (MINB = 1: N = 4096) the stores go through the load/store pipe instead: the CTA has to
+// wait until the tensor stores have read its shared memory before it exits, and no second CTA on the SM covers that
+// wait.  Measured on B200 (1000 W) at 4096^2 (apply, profiles/r4_p2_tma.log): TMA loads + LSU stores 1.498 ms, TMA both
+// ways 1.640 ms, LSU both ways 1.568 ms; at 2048^2 TMA both ways is the fastest (0.3025 / 0.309 / 0.336 ms).
+template <int N, int MINB, int CWS>
 __global__ void __launch_bounds__(GeoA<N>::THREADS, MINB)
-k_mid_swap(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict__ TAB, const LineAddr la, long line0) {
+k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmC, cd* C,
+           const cd* __restrict__ G, const cd* __restrict__ TAB) {
     typedef Map<N, false> M;
-    constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC, TH = GeoA<N>::THREADS;
+    constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
+    constexpr int BOX = N < 256 ? N : 256, NBOX = N / BOX;
+    constexpr bool TMA_STORE = MINB > 1;
     extern __shared__ __align__(128) cd sm[];
     M mp;
     cd* ex = sm;
-    cd* hold = sm + LPC * N + threadIdx.x;          // element a of this thread at hold[a*TH]
+    cd* lines = sm + LPC * N;                       // line l of the CTA, point j at lines[l*N + j]
+    cd* hold = lines + mp.line * N + mp.t;          // element a of this thread at hold[a*T]
     cd* tw1 = sm + 2 * LPC * N;
+    unsigned long long* bar = reinterpret_cast<unsigned long long*>(tw1 + EngTab<N>::TW1N);
+    const int L0 = blockIdx.x * LPC;
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        fence_proxy_async();
+        mbar_expect_tx(bar, (unsigned)(LPC * N * sizeof(cd)));
+#pragma unroll
+        for (int l = 0; l < LPC; ++l)
+#pragma unroll
+            for (int b = 0; b < NBOX; ++b) tma_load_2d(lines + l * N + b * BOX, &tmA, 2 * (L0 + l), b * BOX, bar);
+    }
     load_tw1<N>(tw1, TAB);
-    const long L = line0 + (long)blockIdx.x * LPC + mp.line;
+    const long L = L0 + mp.line;
     const int t = mp.t;
     const TwState<N> tw = make_tw<N>(t, TAB, tw1);
     const cd* gline = G + L * 2L * N;               // chunk rr of line L at gline + rr*N
+    __syncthreads();   // tw1 and the mbarrier initialisation visible
+    mbar_wait(bar, 0);
     cd v[E];
-    {
-        const cd* p = in + line_in(la, L) + (long)t * la.in_es;
 #pragma unroll
-        for (int a = 0; a < E; ++a) v[a] = p[(long)(a * T) * la.in_es];
-#pragma unroll
-        for (int a = 0; a < E; ++a) hold[a * TH] = v[a];
-    }
-    __syncthreads();   // tw1 visible
+    for (int a = 0; a < E; ++a) v[a] = hold[a * T];
 #pragma unroll 1
     for (int rr = 0; rr < 2; ++rr) {
         const int r = 2 * rr;
@@ -332,16 +355,34 @@ k_mid_swap(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict
             // x and the r = 0 result trade places
 #pragma unroll
             for (int a = 0; a < E; ++a) {
-                const cd xa = hold[a * TH];
-                hold[a * TH] = v[a];
+                const cd xa = hold[a * T];
+                hold[a * T] = v[a];
                 v[a] = xa;
             }
         }
     }
-    cd* o = out + line_out(la, L) + (long)t * la.out_es;
-    o[0] = cadd(hold[0], v[0]);
+    if constexpr (!TMA_STORE) {
+        // point j of line L at C[(L / CW)*(CW*N) + CW*j + L % CW] (< 2^25 elements: int offsets)
+        const int l = (int)L;
+        cd* o = C + (((l >> CWS) * N) << CWS) + (l & ((1 << CWS) - 1)) + (t << CWS);
+        o[0] = cadd(hold[0], v[0]);
 #pragma unroll
-    for (int a = 1; a < E; ++a) o[(long)(a * T) * la.out_es] = cfmac(v[a], c64(2 * a * (16 / E)), hold[a * TH]);
+        for (int a = 1; a < E; ++a) o[(a * T) << CWS] = cfmac(v[a], c64(2 * a * (16 / E)), hold[a * T]);
+        return;
+    }
+    hold[0] = cadd(hold[0], v[0]);
+#pragma unroll
+    for (int a = 1; a < E; ++a) hold[a * T] = cfmac(v[a], c64(2 * a * (16 / E)), hold[a * T]);
+    fence_proxy_async();   // these shared-memory writes before the tensor stores read them
+    __syncthreads();
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int l = 0; l < LPC; ++l)
+#pragma unroll
+            for (int b = 0; b < NBOX; ++b)
+                tma_store_3d(&tmC, 2 * ((L0 + l) & ((1 << CWS) - 1)), b * BOX, (L0 + l) >> CWS, lines + l * N + b * BOX);
+        bulk_store_drain();   // the CTA's shared memory must outlive the stores' reads of it
+    }
 }
 
 // cp.async helpers (inverse pass staging)
@@ -470,17 +511,19 @@ inline cudaError_t launch_mid(cudaStream_t s, long nlines, const cd* in, cd* out
 }
 
 // CTAs per SM asked of ptxas: 3 up to N = 256, 2 from 512 to 2048, 1 at 4096 (256-thread CTAs).  Measured on B200
-// (profiles/r2_e_notes.md): at N >= 1024 three CTAs are slower than two (168-register cap -> spills, and 3 x 66 KB of
-// shared memory leaves 30 KB of L1 for the strided line loads: 2048^2 0.297 vs 0.211 ms); at small N several lines
-// share a CTA and three CTAs win.
-template <int N>
-inline cudaError_t launch_mid_swap(cudaStream_t s, long nlines, const cd* in, cd* out, const cd* G, const cd* TAB,
-                                   const LineAddr& la) {
+// (profiles/r2_e_notes.md) before the lines moved by tensor copies: at N >= 1024 three CTAs were slower than two
+// (168-register cap -> spills, and 3 x 66 KB of shared memory left 30 KB of L1 for the then strided LSU line loads:
+// 2048^2 0.297 vs 0.211 ms); at small N several lines share a CTA and three CTAs win.  At the 168-register cap of three
+// CTAs the 256- and 128-point kernels still spill (ptxas: 76 and 4 bytes; 116 and 84 before the tensor copies); the
+// others do not spill (2048: 254 registers).
+template <int N, int CWS>
+inline cudaError_t launch_mid_swap(cudaStream_t s, long nlines, const CUtensorMap& tmA, const CUtensorMap& tmC, cd* C,
+                                   const cd* G, const cd* TAB) {
     constexpr int MINB = GeoA<N>::THREADS > 128 ? 1 : (N <= 256 ? 3 : 2);
-    constexpr int smem = (2 * GeoA<N>::LPC * N + EngTab<N>::TW1N) * (int)sizeof(cd);
+    constexpr int smem = (2 * GeoA<N>::LPC * N + EngTab<N>::TW1N) * (int)sizeof(cd) + 8;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_mid_swap<N, MINB>, smem, optin); if (e != cudaSuccess) return e; }
-    k_mid_swap<N, MINB><<<(unsigned)(nlines / GeoA<N>::LPC), GeoA<N>::THREADS, smem, s>>>(in, out, G, TAB, la, 0);
+    { cudaError_t e = smem_optin(k_mid_swap<N, MINB, CWS>, smem, optin); if (e != cudaSuccess) return e; }
+    k_mid_swap<N, MINB, CWS><<<(unsigned)(nlines / GeoA<N>::LPC), GeoA<N>::THREADS, smem, s>>>(tmA, tmC, C, G, TAB);
     return cudaPeekAtLastError();
 }
 

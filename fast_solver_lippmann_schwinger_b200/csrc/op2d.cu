@@ -23,6 +23,8 @@
 #include "op2d_base.cuh"
 #include "line_kernels.cuh"
 #include "gv_spectrum2d.cuh"
+#include <cudaTypedefs.h>
+#include <algorithm>
 
 using namespace ls;
 using namespace lsk;
@@ -44,6 +46,7 @@ struct Op2D : Op2DBase {
     cd* d_C = nullptr;        // P2 output: slot sx of column j at C[(sx/CW)*(CW*m) + CW*j + sx%CW]
     bool embed = false;       // LS_FLAG_EMBED: lines of ln x lm points carry the n x m grid (ln = n, lm = m otherwise)
     long ln = 0, lm = 0;
+    CUtensorMap tmA, tmC;     // 2x padding: P2's line loads from A and stores into C (encode_line_maps)
     int apply_dev(const cd* b, cd* y, int mode) override;
     void info(int* route, int64_t* n_line, int64_t* m_line, int* padding) const override {
         *route = embed ? 2 : 0; *n_line = ln; *m_line = lm; *padding = nr;
@@ -130,7 +133,7 @@ int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
         LineAddr la{CW, 1, CW, pn, 1, CW * m, CW};
         la.nr = op->nr;
         op->phase_begin(1);
-#define P2S(N) launch_mid_swap<N>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
+#define P2S(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm)
 #define P2F(N) launch_mid<N, false>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
         if (op->nr == 2) { LS_DISPATCH_E(m, P2S); } else { LS_DISPATCH_E(m, P2F); }
         op->phase_end(); op->launches++;
@@ -173,10 +176,8 @@ int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
         LS_CUDA_TRY(e);
     }
     {
-        LineAddr la{CW, 1, CW, pn, 1, CW * lm, CW};
-        la.nr = 2;
         op->phase_begin(1);
-#define E2(N) launch_mid_swap<N>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
+#define E2(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm)
         LS_DISPATCH_E(lm, E2);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -202,6 +203,45 @@ int Op2D::apply_dev(const cd* b, cd* y, int mode) {
 }
 
 namespace {
+
+// The 2x-padded P2 (k_mid_swap) moves its lines by tensor copies.  As FLOAT64 arrays with re, im innermost, line sx of A
+// is the box {2, BOX} at (2 sx, j0) of the 2-D view {2 pn, lm}, and line sx of C the box {2, BOX, 1} at
+// (2 (sx % CW), j0, sx / CW) of the 3-D view {2 CW, lm, pn / CW}, i.e. C[(sx/CW)*(CW*lm) + CW*j + sx%CW].
+// BOX = min(lm, 256), the largest box side.  cuTensorMapEncodeTiled is reached through the runtime's driver entry point,
+// so the library does not link against libcuda.
+int encode_line_maps(Op2D* op) {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+    LS_CUDA_TRY(cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &q));
+    LS_REQUIRE(q == cudaDriverEntryPointSuccess && fn, LS_ERR_CUDA, "the driver has no cuTensorMapEncodeTiled");
+    const auto encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
+    const cuuint64_t pn = (cuuint64_t)op->pn, lm = (cuuint64_t)op->lm;
+    const cuuint32_t box = (cuuint32_t)std::min<long>(op->lm, 256), unit[3] = {1, 1, 1};
+    const cuuint64_t dimA[2] = {2 * pn, lm}, strideA[1] = {pn * sizeof(cd)};
+    const cuuint32_t boxA[2] = {2, box};
+    const cuuint64_t dimC[3] = {2 * CW, lm, pn / CW}, strideC[2] = {CW * sizeof(cd), CW * lm * sizeof(cd)};
+    const cuuint32_t boxC[3] = {2, box, 1};
+    CUresult r = encode(&op->tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, op->d_A, dimA, strideA, boxA, unit,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const char* which = "A";
+    if (r == CUDA_SUCCESS) {
+        which = "C";
+        r = encode(&op->tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, op->d_C, dimC, strideC, boxC, unit,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    }
+    if (r != CUDA_SUCCESS) {
+        const char* msg = nullptr;
+        void* es = nullptr;
+        if (cudaGetDriverEntryPointByVersion("cuGetErrorString", &es, 6000, cudaEnableDefault, &q) == cudaSuccess && es)
+            reinterpret_cast<PFN_cuGetErrorString_v6000>(es)(r, &msg);
+        set_error("cuTensorMapEncodeTiled (P2 line map of %s, pn=%ld, lm=%ld) failed: %s (CUresult %d)", which,
+                  (long)pn, (long)lm, msg ? msg : "no message", (int)r);
+        return LS_ERR_CUDA;
+    }
+    return LS_OK;
+}
 
 // G2 = fft2(g2) / (2n 2m) in the slot order of the nr = 2 kernels (n, m: the line lengths, powers of two).
 // g2[jx2 + 2n*jy2]: the spatial kernel with its lags wrapped onto the 2n x 2m grid (negative lags at the end).
@@ -311,6 +351,7 @@ int create_embedded(ls_handle* out, long n, long m, long ne, long me, const doub
     op->pn = 2 * ln; op->pm = 2 * lm;
     TRY(op->dmalloc((void**)&op->d_A, (size_t)op->pn * lm * sizeof(cd)));
     TRY(op->dmalloc((void**)&op->d_C, (size_t)op->pn * lm * sizeof(cd)));
+    TRY(encode_line_maps(op));
     {   // columns [m, lm) of A are read by P2 and never written by P1
         cudaError_t e = cudaMemsetAsync(op->d_A, 0, (size_t)op->pn * lm * sizeof(cd), op->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(op->stream);
@@ -433,6 +474,7 @@ static int op2d_create_impl(ls_handle* out, int64_t n, int64_t m, int64_t ne, in
     op->pn = op->nr * n; op->pm = op->nr * m;
     TRY(op->dmalloc((void**)&op->d_A, (size_t)op->pn * m * sizeof(cd)));
     TRY(op->dmalloc((void**)&op->d_C, (size_t)op->pn * m * sizeof(cd)));
+    if (op->nr == 2) TRY(encode_line_maps(op));
     TRY(op->dmalloc((void**)&op->d_b, N * sizeof(cd)));
     TRY(op->dmalloc((void**)&op->d_y, N * sizeof(cd)));
 #undef TRY
