@@ -40,12 +40,14 @@ def main():
                          "any n <= 4096, e.g. h = 1/1000 (--n 1001), which the Bluestein general path refuses")
     ap.add_argument("--nrhs", type=int, default=1,
                     help="solve for K incident plane waves exp(ik(x cos t + y sin t)), t = 0, pi/K, ..., (K-1) pi/K, in one "
-                         "lockstep GMRES (ls_gmres_msp_batch); needs the device Msp (--msp gpu), implies --precond conv")
+                         "lockstep GMRES: with the device Msp (--msp gpu, implies --precond conv) ls_gmres_msp_batch; with "
+                         "--msp host Pl = I (ls_gmres_batch: the host Msp solve has no batched form)")
     args = ap.parse_args()
     if args.nrhs > 1:
-        if args.msp != "gpu":
-            ap.error("--nrhs > 1 needs --msp gpu")
-        args.precond = args.precond or "conv"
+        if args.msp == "gpu":
+            args.precond = args.precond or "conv"
+        else:
+            args.precond = None
     n = args.n
     if n % 2 == 1:                       # example.jl: x = -a/2:h:a/2, k = 1/h
         h = 1.0 / (n - 1)

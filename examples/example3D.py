@@ -39,9 +39,11 @@ def main():
                          "any n <= 512")
     ap.add_argument("--nrhs", type=int, default=1,
                     help="solve for K incident plane waves exp(ik(x cos t + y sin t)), t = 0, pi/K, ..., (K-1) pi/K, in one "
-                         "lockstep GMRES (ls_gmres_msp_batch); implies --precond --msp gpu")
+                         "lockstep GMRES (ls_gmres_msp_batch); implies --precond --msp gpu unless --no-precond")
+    ap.add_argument("--no-precond", action="store_true",
+                    help="with --nrhs: Pl = I (ls_gmres_batch), at k = 1/h faster than the preconditioner (DESIGN.md 3.5)")
     args = ap.parse_args()
-    if args.nrhs > 1:
+    if args.nrhs > 1 and not args.no_precond:
         args.precond, args.msp = True, "gpu"
     n = args.n
     h = 1.0 / n

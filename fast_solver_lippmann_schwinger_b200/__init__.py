@@ -5,7 +5,7 @@ Only what the path needs lives here: ``csrc/`` (CUDA kernels + the C ABI of incl
 ``sparsifier`` (the preconditioner's stencil matrices sampled through operator applies).
 """
 from ._lib import (DeviceBuffer, LSCudaError, LSUnsupported, PinnedArray, declared_symbols, lib)  # noqa: F401
-from .operators import FastM, FastM3D, FFTconvolution, fastconvolution, mul_  # noqa: F401
+from .operators import FastM, FastM3D, FFTconvolution, apply_batch, batch_cols, fastconvolution, mul_  # noqa: F401
 from .krylov import (ConvergenceHistory, GPUMspFactorization, GPUSparseMatrixCSC, KrylovWorkspace,  # noqa: F401
                      SparsifyingPreconditioner, cscmv_, gmres_)
 from . import sparsifier  # noqa: F401,E402

@@ -93,6 +93,8 @@ def lib():
         "ls_nccl_unique_id": (ci, [vp]),
         "ls_op3d_create_dist": (ci, [C.POINTER(vp), i64, i64, i64, vp, dbl, dbl, dbl, ci, ci, vp, ci]),
         "ls_op_size": (ci, [vp, C.POINTER(i64)]),
+        "ls_op_apply_batch": (ci, [vp, vp, i64, vp, i64, ci, ci, ci]),
+        "ls_op_batch_cols": (ci, [vp, C.POINTER(ci)]),
         "ls_spm_create": (ci, [C.POINTER(vp), i64, i64, vp, vp, vp]),
         "ls_spm_create_dist": (ci, [C.POINTER(vp), vp, i64, i64, vp, vp, vp]),
         "ls_spm_mv": (ci, [vp, CDouble, vp, CDouble, vp, ci]),
@@ -116,6 +118,7 @@ def lib():
                               C.POINTER(i64), C.POINTER(ci), C.POINTER(i64), ci]),
         "ls_gmres_msp_batch": (ci, [vp, vp, vp, vp, ci, vp, i64, vp, i64, ci, i64, dbl, dbl, ci, vp, i64,
                                     vp, vp, vp, ci]),
+        "ls_gmres_batch": (ci, [vp, vp, ci, vp, i64, vp, i64, ci, i64, dbl, dbl, ci, vp, i64, vp, vp, vp, ci]),
         "ls_krylov_last_precond_host_seconds": (ci, [vp, C.POINTER(dbl)]),
         "ls_sample_rows": (ci, [vp, vp, vp, ci, vp, i64]),
         "ls_gram": (ci, [vp, vp, i64, ci, vp]),

@@ -590,15 +590,15 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned pari
 }
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// tensor copies of one box through a tensor map (a __grid_constant__ kernel parameter): a 2-D load into shared memory
-// that completes on `bar`, and a 3-D store from shared memory in this thread's bulk group
-__device__ __forceinline__ void tma_load_2d(void* dst_smem, const void* map, int c0, int c1, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(smem_u32(dst_smem)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
+// tensor copies of one box through a tensor map (a __grid_constant__ kernel parameter): a 3-D load into shared memory
+// that completes on `bar`, and a 4-D store from shared memory in this thread's bulk group
+__device__ __forceinline__ void tma_load_3d(void* dst_smem, const void* map, int c0, int c1, int c2, unsigned long long* bar) {
+    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+                 ::"r"(smem_u32(dst_smem)), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ void tma_store_3d(const void* map, int c0, int c1, int c2, const void* src_smem) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];"
-                 ::"l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(src_smem)) : "memory");
+__device__ __forceinline__ void tma_store_4d(const void* map, int c0, int c1, int c2, int c3, const void* src_smem) {
+    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%1, %2, %3, %4}], [%5];"
+                 ::"l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(smem_u32(src_smem)) : "memory");
 }
 // commit this thread's bulk stores and wait until their shared-memory sources have been read
 __device__ __forceinline__ void bulk_store_drain() {

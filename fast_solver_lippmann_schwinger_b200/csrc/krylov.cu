@@ -16,6 +16,7 @@
 //   Hessenberg column per GMRES iteration.
 #include "ls_common.cuh"
 #include "spmv.cuh"
+#include <algorithm>
 #include <chrono>
 #include <cstring>
 
@@ -788,24 +789,26 @@ static int gmres_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, ls_sol
     return LS_OK;
 }
 
-// ls_gmres_msp_batch: nrhs independent GMRES(restart) runs of gmres_driver side by side with one operator, As and Msp.
-// Every system keeps its own basis, Hessenberg matrix, restarts, tolerance and history, and goes through exactly the
-// steps gmres_driver takes for it (same kernels, same inputs), so its history, counts and x have the bits of a run on its
-// own.  In each lockstep iteration the applies, SpMVs and Gram-Schmidt steps run system by system; the Msp^-1 of all
-// active systems is one batched solve (ls_msp_solve_batch: each factor block is read once per chunk of columns).  All
-// active systems share the iteration count and the position k in the restart cycle; a system that converges or
-// reaches maxiter drops out of the later solves.
+// ls_gmres_msp_batch / ls_gmres_batch: nrhs independent GMRES(restart) runs of gmres_driver side by side with one
+// operator and, with msp, one As and Msp (msp == nullptr: Pl = Identity, no As).  Every system keeps its own basis,
+// Hessenberg matrix, restarts, tolerance and history, and goes through exactly the steps gmres_driver takes for it (same
+// kernels, same inputs), so its history, counts and x have the bits of a run on its own.  In each lockstep iteration the
+// operator applies of all active systems go through the multi-column apply (chunks of batch_cols columns at the
+// systems' basis columns), the SpMVs and Gram-Schmidt steps run system by system, and the Msp^-1 of all active systems
+// is one batched solve (ls_msp_solve_batch: each factor block is read once per chunk of columns).  All active systems
+// share the iteration count and the position k in the restart cycle; a system that converges or reaches maxiter drops
+// out of the later applies and solves.
 static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, int nrhs, const ls_cdouble* b, int64_t ldb,
                               ls_cdouble* x, int64_t ldx, int restart, int64_t maxiter, double reltol, double abstol,
                               int initially_zero, double* resnorm_hist, int64_t hist_cap, int64_t* niter, int* converged,
                               int64_t* mv_products, int memloc) {
-    const char* fn = "ls_gmres_msp_batch";
+    const char* fn = msp ? "ls_gmres_msp_batch" : "ls_gmres_batch";
     LS_REQUIRE(op->op_size() == K->n, LS_ERR_INVALID, "%s: operator size %ld != workspace size %ld", fn, (long)op->op_size(), (long)K->n);
-    LS_REQUIRE(op->nccl_comm() == nullptr, LS_ERR_UNSUPPORTED, "%s: the device Msp factorisation is single-GPU", fn);
+    LS_REQUIRE(op->nccl_comm() == nullptr, LS_ERR_UNSUPPORTED, "%s: several right-hand sides are served on one GPU", fn);
     if (As) LS_REQUIRE(As->kind == KIND_SPM && As->nrows == K->n && As->x_len() == K->n && As->halo == 0, LS_ERR_INVALID,
                        "%s: As must be an N x N sparse-matrix handle", fn);
-    LS_REQUIRE(msp->kind == KIND_MSP && msp->n == K->n, LS_ERR_INVALID, "%s: the Msp factorisation has %ld unknowns, the operator %ld",
-               fn, (long)msp->n, (long)K->n);
+    if (msp) LS_REQUIRE(msp->kind == KIND_MSP && msp->n == K->n, LS_ERR_INVALID, "%s: the Msp factorisation has %ld unknowns, the operator %ld",
+                        fn, (long)msp->n, (long)K->n);
     const long n = K->n;
     if (restart <= 0) restart = 20;
     LS_REQUIRE(restart <= 64, LS_ERR_UNSUPPORTED, "%s: restart > 64 is not supported", fn);
@@ -815,10 +818,12 @@ static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, 
     const bool host = memloc == LS_MEM_HOST;
 
     // memory: nrhs bases of restart + 1 columns, nrhs columns for the batched solve, host staging of b and x, the
-    // batched solve's work arrays - checked against the free device memory before anything is allocated
-    const size_t needV = vb * (size_t)(restart + 1) * nrhs, needP = vb * nrhs, needBX = host ? 2 * vb * nrhs : 0;
+    // batched solve's and the multi-column apply's work arrays - checked against the free device memory before anything
+    // is allocated
+    const int wcols = std::min(nrhs, op->batch_cols());
+    const size_t needV = vb * (size_t)(restart + 1) * nrhs, needP = msp ? vb * nrhs : 0, needBX = host ? 2 * vb * nrhs : 0;
     size_t need = (K->Vb_bytes < needV ? needV : 0) + (K->Pb_bytes < needP ? needP : 0) + (K->bxb_bytes < needBX ? needBX : 0) +
-                  (K->d_ax ? 0 : 3 * vb) + msp->batch_bytes(nrhs, false, true);
+                  (K->d_ax ? 0 : 3 * vb) + (msp ? msp->batch_bytes(nrhs, false, true) : 0) + op->batch_bytes(wcols);
     if (need > 0) {
         size_t free_b = 0, total_b = 0;
         LS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
@@ -828,14 +833,15 @@ static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, 
     }
     int rc;
     if ((rc = K->ensure(&K->d_Vb, K->Vb_bytes, needV))) return rc;
-    if ((rc = K->ensure(&K->d_Pb, K->Pb_bytes, needP))) return rc;
+    if (msp && (rc = K->ensure(&K->d_Pb, K->Pb_bytes, needP))) return rc;
     if (host && (rc = K->ensure(&K->d_bxb, K->bxb_bytes, needBX))) return rc;
     if (!K->d_ax) {
         if ((rc = K->dmalloc((void**)&K->d_ax, vb))) return rc;
         if ((rc = K->dmalloc((void**)&K->d_b, vb))) return rc;
         if ((rc = K->dmalloc((void**)&K->d_x, vb))) return rc;
     }
-    if ((rc = msp->batch_reserve(nrhs, false, true))) return rc;
+    if (msp && (rc = msp->batch_reserve(nrhs, false, true))) return rc;
+    if ((rc = op->batch_reserve(wcols))) return rc;
 
     struct Sys {
         cd* V; const cd* db; cd* dx;
@@ -869,7 +875,7 @@ static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, 
     // ldiv!(Pl, v) for the listed vectors: As v into the solve's columns, one batched Msp^-1 in place, back into v
     auto precond = [&](const std::vector<cd*>& vs) -> int {
         const int na = (int)vs.size();
-        if (na == 0) return LS_OK;
+        if (na == 0 || !msp) return LS_OK;
         for (int i = 0; i < na; ++i) {
             cd* col = K->d_Pb + (size_t)i * n;
             if (As) {
@@ -929,13 +935,14 @@ static int gmres_batch_driver(Krylov* K, HandleBase* op, SpM* As, MspBase* msp, 
         for (int q = 0; q < nrhs; ++q) if (sys[q].active) act.push_back(q);
         if (act.empty()) break;
         // expand!: V_{k+1} = Pl^-1 (A V_k) for every active system
+        std::vector<const cd*> vk;
         std::vector<cd*> ws;
         for (int q : act) {
             Sys& S = sys[q];
-            cd* w = S.V + (long)S.k * n;
-            if ((rc = op->apply_dev(S.V + (long)(S.k - 1) * n, w, LS_APPLY_FASTCONVOLUTION))) return rc;
-            ws.push_back(w);
+            vk.push_back(S.V + (long)(S.k - 1) * n);
+            ws.push_back(S.V + (long)S.k * n);
         }
+        if ((rc = op->apply_list_dev(vk.data(), ws.data(), (int)act.size(), LS_APPLY_FASTCONVOLUTION))) return rc;
         if ((rc = precond(ws))) return rc;
         std::vector<int> restarting;
         for (size_t i = 0; i < act.size(); ++i) {
@@ -1026,6 +1033,26 @@ int ls_gmres_msp_batch(ls_handle kh, ls_handle op_h, ls_handle as_h, ls_handle m
     return gmres_batch_driver(K, reinterpret_cast<HandleBase*>(op_h), reinterpret_cast<SpM*>(as_h), reinterpret_cast<MspBase*>(msp_h),
                               nrhs, b, ldb, x, ldx, restart, maxiter, reltol, abstol, initially_zero, resnorm_hist, hist_cap, niter,
                               converged, mv_products, memloc);
+}
+
+// Argument refusals come before any CUDA call.
+int ls_gmres_batch(ls_handle kh, ls_handle op_h, int nrhs, const ls_cdouble* b, int64_t ldb, ls_cdouble* x, int64_t ldx, int restart,
+                   int64_t maxiter, double reltol, double abstol, int initially_zero, double* resnorm_hist, int64_t hist_cap,
+                   int64_t* niter, int* converged, int64_t* mv_products, int memloc) {
+    LS_REQUIRE(nrhs >= 1, LS_ERR_INVALID, "ls_gmres_batch: nrhs = %d, at least one system needed", nrhs);
+    LS_REQUIRE(kh && op_h && b && x, LS_ERR_INVALID, "ls_gmres_batch: null argument");
+    LS_REQUIRE(!resnorm_hist || hist_cap >= 0, LS_ERR_INVALID, "ls_gmres_batch: hist_cap = %ld", (long)hist_cap);
+    Krylov* K = reinterpret_cast<Krylov*>(kh);
+    LS_REQUIRE(K->kind == KIND_VEC, LS_ERR_INVALID, "ls_gmres_batch: not a Krylov workspace handle");
+    LS_REQUIRE(ldb >= K->n && ldx >= K->n, LS_ERR_INVALID, "ls_gmres_batch: leading dimensions ldb = %ld, ldx = %ld must be >= N = %ld",
+               (long)ldb, (long)ldx, (long)K->n);
+    LS_REQUIRE(memloc == LS_MEM_HOST || memloc == LS_MEM_DEVICE, LS_ERR_INVALID, "ls_gmres_batch: unknown memloc %d", memloc);
+    HandleBase* op = reinterpret_cast<HandleBase*>(op_h);
+    LS_REQUIRE(op->kind == KIND_OP2D || op->kind == KIND_OP3D, LS_ERR_INVALID, "ls_gmres_batch: not an operator handle");
+    LS_REQUIRE(op->dist_size() == 1, LS_ERR_UNSUPPORTED, "ls_gmres_batch: several right-hand sides are served on one GPU");
+    LS_CUDA_TRY(cudaSetDevice(K->device));
+    return gmres_batch_driver(K, op, nullptr, nullptr, nrhs, b, ldb, x, ldx, restart, maxiter, reltol, abstol, initially_zero,
+                              resnorm_hist, hist_cap, niter, converged, mv_products, memloc);
 }
 
 // ---- sparsifier sampling on the device (SURVEY.md 8(f) row 2) --------------------------------------------------------

@@ -115,6 +115,17 @@ __device__ __forceinline__ long slot_off(const LineAddr& a, long s, long es) {
          + ((s & ((1L << a.split2_shift) - 1)) >> a.split_shift) * a.split_stride
          + (s >> a.split2_shift) * a.split2_stride;
 }
+// Column pointers of k_fwd_pruned and k_inv_pruned: column c reads its lines at in[c] (and b at b[c]) and writes them
+// at out[c], with the one LineAddr of the launch.  The COLS instantiations serve a launch over several columns
+// (ls_op_apply_batch), column c = blockIdx.y; the others read column 0 at fixed parameter offsets.  A pointer loaded by
+// block index has to live in registers, which costs the single apply spills at the 168-register cap (ptxas: 2-D P1 at
+// 2048 points 140 -> 164 bytes), so the single apply keeps the fixed-offset instantiation.
+constexpr int MAX_COLS = 8;
+struct ColPtrs {
+    const cd* in[MAX_COLS];
+    const cd* b[MAX_COLS];
+    cd* out[MAX_COLS];
+};
 __device__ __forceinline__ long line_in(const LineAddr& a, long L) { return (L % a.ldim0) * a.in_ls0 + (L / a.ldim0) * a.in_ls1; }
 __device__ __forceinline__ long line_out(const LineAddr& a, long L) { return (L % a.ldim0) * a.out_ls0 + (L / a.ldim0) * a.out_ls1; }
 
@@ -131,11 +142,12 @@ template <int N, bool MODE_B> struct Smem {
 // in  : line L point j at in[L*in_ls + j*in_es], optionally scaled by the real nu (same addressing)
 // out : line L slot  s at out[L*out_ls + s*out_es], s = r*N + slot
 // MASK: points >= la.mask_pts and lines >= la.mask_lines are zeros (not read); their slots are written
-template <int N, bool MODE_B, bool MASK = false>
+template <int N, bool MODE_B, bool MASK = false, bool COLS = false>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MinB<N, MODE_B>::value)
-k_fwd_pruned(const cd* __restrict__ in, const double* __restrict__ nu, cd* __restrict__ out,
-             const cd* __restrict__ TAB, const LineAddr la, long line0) {
+k_fwd_pruned(const ColPtrs cp, const double* __restrict__ nu, const cd* __restrict__ TAB, const LineAddr la, long line0) {
     typedef Map<N, MODE_B> M;
+    const cd* __restrict__ in = cp.in[COLS ? blockIdx.y : 0];
+    cd* __restrict__ out = cp.out[COLS ? blockIdx.y : 0];
     constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
     extern __shared__ __align__(128) cd sm[];
     M mp;
@@ -197,10 +209,14 @@ k_fwd_pruned(const cd* __restrict__ in, const double* __restrict__ nu, cd* __res
 //       mode B: per (unit, r) one contiguous chunk, fetched by TMA bulk copy into shared memory
 //               while the previous block's inverse transform runs.
 // out : line L point j at out[L*out_ls + j*out_es]  (may alias in when strides agree)
+// Several columns (ncol > 1, mode B: the 3-D z pass): column c's lines start at in + c*cs / out + c*cs.  CTA x = g*ncol + c
+// serves the line group g of column c: the ncol CTAs that read the same spectrum chunk are dispatched together, and all
+// but the first find it in L2.  Mode A (the 2-D middle pass with LS_FLAG_PAD4) runs one column: the column arithmetic
+// costs it spills (ptxas: 24 - 52 bytes at 1024 - 4096 points).
 template <int N, bool MODE_B, int MINB = 1>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MINB)
 k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restrict__ TAB,
-            const LineAddr la, long line0) {
+            const LineAddr la, long line0, int ncol, long cs) {
     typedef Map<N, MODE_B> M;
     constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
     constexpr int LBK = MODE_B ? GeoB<N>::LB : 1;     // lines interleaved in a spectrum chunk
@@ -213,7 +229,14 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
     cd* gb = sm + 2 * LPC * N;                  // spectrum chunk(s) of the current r (mode B only)
     cd* tw1 = sm + (MODE_B ? 3 : 2) * LPC * N;
     unsigned long long* bar = reinterpret_cast<unsigned long long*>(tw1 + Smem<N, MODE_B>::TW1N);
-    const long Lcta = line0 + (long)blockIdx.x * LPC;
+    long grp = blockIdx.x;
+    if constexpr (MODE_B) {
+        const int col = (int)(blockIdx.x % (unsigned)ncol);
+        in += col * cs;
+        out += col * cs;
+        grp = blockIdx.x / (unsigned)ncol;
+    }
+    const long Lcta = line0 + grp * LPC;
     const long L = Lcta + mp.line;
     const int t = mp.t;
     const int nr = la.nr, rstep = 4 / la.nr;
@@ -296,8 +319,10 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
 // values are requested before the last butterfly stage and held in registers across it.
 // The lines move by tensor copies, not through the load/store pipe: their points are one x-slot (16 bytes) wide in
 // A and CW-interleaved in C, so an LSU access of a line used 16 bytes of every 128-byte (A) or 64-byte (C) line.
-// tmA: 2-D map of A as FLOAT64 {2 pn, lm}; line L is the boxes {2, BOX} at (2L, j0).  tmC: 3-D map of C
-// {2 CW, lm, pn/CW}; line L is the boxes {2, BOX, 1} at (2 (L % CW), j0, L / CW), CW = 2^CWS.  BOX = min(N, 256);
+// tmA: 3-D map of A as FLOAT64 {2 pn, lm, cols}; line L of column c is the boxes {2, BOX, 1} at (2L, j0, c).  tmC: 4-D
+// map of C {2 CW, lm, pn/CW, cols}; line L of column c is the boxes {2, BOX, 1, 1} at (2 (L % CW), j0, L / CW, c),
+// CW = 2^CWS.  Column c's C starts at C + c*ccs.  The grid is {columns, pn / LPC}: the CTAs of one line group, which
+// read the same spectrum lines, are dispatched together, and all but the first find those lines in L2.  BOX = min(N, 256);
 // each line of the CTA has its own N / BOX boxes.  Thread 0 issues the loads into the buffer first thing (the table
 // set-up runs under them) and, after the combine has been written back into the same buffer, the stores.
 // With one resident CTA per SM (MINB = 1: N = 4096) the stores go through the load/store pipe instead: the CTA has to
@@ -306,7 +331,7 @@ k_mid_fused(const cd* in, cd* out, const cd* __restrict__ G, const cd* __restric
 // ways 1.640 ms, LSU both ways 1.568 ms; at 2048^2 TMA both ways is the fastest (0.3025 / 0.309 / 0.336 ms).
 template <int N, int MINB, int CWS>
 __global__ void __launch_bounds__(GeoA<N>::THREADS, MINB)
-k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmC, cd* C,
+k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmC, cd* C, long ccs,
            const cd* __restrict__ G, const cd* __restrict__ TAB) {
     typedef Map<N, false> M;
     constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
@@ -319,7 +344,7 @@ k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
     cd* hold = lines + mp.line * N + mp.t;          // element a of this thread at hold[a*T]
     cd* tw1 = sm + 2 * LPC * N;
     unsigned long long* bar = reinterpret_cast<unsigned long long*>(tw1 + EngTab<N>::TW1N);
-    const int L0 = blockIdx.x * LPC;
+    const int L0 = blockIdx.y * LPC;        // column blockIdx.x (read where used: nothing holds it across the transforms)
     if (threadIdx.x == 0) {
         mbar_init(bar, 1);
         fence_proxy_async();
@@ -327,7 +352,7 @@ k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
 #pragma unroll
         for (int l = 0; l < LPC; ++l)
 #pragma unroll
-            for (int b = 0; b < NBOX; ++b) tma_load_2d(lines + l * N + b * BOX, &tmA, 2 * (L0 + l), b * BOX, bar);
+            for (int b = 0; b < NBOX; ++b) tma_load_3d(lines + l * N + b * BOX, &tmA, 2 * (L0 + l), b * BOX, blockIdx.x, bar);
     }
     load_tw1<N>(tw1, TAB);
     const long L = L0 + mp.line;
@@ -364,7 +389,7 @@ k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
     if constexpr (!TMA_STORE) {
         // point j of line L at C[(L / CW)*(CW*N) + CW*j + L % CW] (< 2^25 elements: int offsets)
         const int l = (int)L;
-        cd* o = C + (((l >> CWS) * N) << CWS) + (l & ((1 << CWS) - 1)) + (t << CWS);
+        cd* o = C + blockIdx.x * ccs + (((l >> CWS) * N) << CWS) + (l & ((1 << CWS) - 1)) + (t << CWS);
         o[0] = cadd(hold[0], v[0]);
 #pragma unroll
         for (int a = 1; a < E; ++a) o[(a * T) << CWS] = cfmac(v[a], c64(2 * a * (16 / E)), hold[a * T]);
@@ -380,7 +405,7 @@ k_mid_swap(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
         for (int l = 0; l < LPC; ++l)
 #pragma unroll
             for (int b = 0; b < NBOX; ++b)
-                tma_store_3d(&tmC, 2 * ((L0 + l) & ((1 << CWS) - 1)), b * BOX, (L0 + l) >> CWS, lines + l * N + b * BOX);
+                tma_store_4d(&tmC, 2 * ((L0 + l) & ((1 << CWS) - 1)), b * BOX, (L0 + l) >> CWS, blockIdx.x, lines + l * N + b * BOX);
         bulk_store_drain();   // the CTA's shared memory must outlive the stores' reads of it
     }
 }
@@ -400,11 +425,13 @@ template <int K> __device__ __forceinline__ void cp_async_wait() { asm volatile(
 // the kernel's three exposed DRAM latencies off the critical path.  The applies run staged; the set-up passes of the
 // compact spectrum do not.
 // MASK: only points < la.mask_pts of lines < la.mask_lines are written (and only their b values staged)
-template <int N, bool MODE_B, bool STAGED = false, bool MASK = false>
+template <int N, bool MODE_B, bool STAGED = false, bool MASK = false, bool COLS = false>
 __global__ void __launch_bounds__(MODE_B ? GeoB<N>::THREADS : GeoA<N>::THREADS, MinBInv<N, MODE_B>::value)
-k_inv_pruned(const cd* __restrict__ in, const cd* bsrc, cd* out, const cd* __restrict__ TAB, double scale,
-             const LineAddr la, long line0) {
+k_inv_pruned(const ColPtrs cp, const cd* __restrict__ TAB, double scale, const LineAddr la, long line0) {
     typedef Map<N, MODE_B> M;
+    const cd* __restrict__ in = cp.in[COLS ? blockIdx.y : 0];
+    const cd* bsrc = cp.b[COLS ? blockIdx.y : 0];
+    cd* out = cp.out[COLS ? blockIdx.y : 0];
     constexpr int E = Cfg<N>::E, T = N / E, LPC = M::G::LPC;
     extern __shared__ __align__(128) cd sm[];
     M mp;
@@ -486,27 +513,46 @@ template <class K> inline cudaError_t smem_optin(K kernel, int smem, unsigned lo
 
 // MASK launchers cover ceil(nlines / LPC) CTAs: nlines need not be a multiple of the lines per CTA (the lines past
 // nlines in the last CTA are masked by la.mask_lines and must still be addressable for the unmasked side)
+// the pointer list of one column
+inline ColPtrs one_col(const cd* in, const cd* b, cd* out) {
+    ColPtrs cp = {};
+    cp.in[0] = in; cp.b[0] = b; cp.out[0] = out;
+    return cp;
+}
+
 template <int N, bool B, bool MASK = false>
-inline cudaError_t launch_fwd(cudaStream_t s, long nlines, const cd* in, const double* nu, cd* out, const cd* TAB,
-                              const LineAddr& la) {
+inline cudaError_t launch_fwd_cols(cudaStream_t s, long nlines, const ColPtrs& cp, int ncol, const double* nu, const cd* TAB,
+                                   const LineAddr& la) {
     constexpr int smem = Smem<N, B>::fwd_bytes;
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_fwd_pruned<N, B, MASK>, smem, optin); if (e != cudaSuccess) return e; }
     const long grid = MASK ? (nlines + LPC - 1) / LPC : nlines / LPC;
-    k_fwd_pruned<N, B, MASK><<<(unsigned)grid, TH, smem, s>>>(in, nu, out, TAB, la, 0);
+    if (ncol == 1) {
+        { cudaError_t e = smem_optin(k_fwd_pruned<N, B, MASK>, smem, optin); if (e != cudaSuccess) return e; }
+        k_fwd_pruned<N, B, MASK><<<(unsigned)grid, TH, smem, s>>>(cp, nu, TAB, la, 0);
+    } else {
+        static unsigned long long optin_cols = 0;
+        { cudaError_t e = smem_optin(k_fwd_pruned<N, B, MASK, true>, smem, optin_cols); if (e != cudaSuccess) return e; }
+        k_fwd_pruned<N, B, MASK, true><<<dim3((unsigned)grid, (unsigned)ncol), TH, smem, s>>>(cp, nu, TAB, la, 0);
+    }
     return cudaPeekAtLastError();
+}
+template <int N, bool B, bool MASK = false>
+inline cudaError_t launch_fwd(cudaStream_t s, long nlines, const cd* in, const double* nu, cd* out, const cd* TAB,
+                              const LineAddr& la) {
+    return launch_fwd_cols<N, B, MASK>(s, nlines, one_col(in, nullptr, out), 1, nu, TAB, la);
 }
 
 template <int N, bool B>
 inline cudaError_t launch_mid(cudaStream_t s, long nlines, const cd* in, cd* out, const cd* G, const cd* TAB,
-                              const LineAddr& la) {
+                              const LineAddr& la, int ncol = 1, long cs = 0) {
     constexpr int smem = Smem<N, B>::mid_bytes;
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
     constexpr int MB = (B && GeoB<N>::LB == 4) ? 2 : 1;      // 4-line geometry: two CTAs per SM (128 registers)
+    if (!B && ncol != 1) return cudaErrorInvalidValue;         // mode A runs one column (k_mid_fused)
     { cudaError_t e = smem_optin(k_mid_fused<N, B, MB>, smem, optin); if (e != cudaSuccess) return e; }
-    k_mid_fused<N, B, MB><<<(unsigned)(nlines / LPC), TH, smem, s>>>(in, out, G, TAB, la, 0);
+    k_mid_fused<N, B, MB><<<(unsigned)(nlines / LPC * ncol), TH, smem, s>>>(in, out, G, TAB, la, 0, ncol, cs);
     return cudaPeekAtLastError();
 }
 
@@ -518,25 +564,36 @@ inline cudaError_t launch_mid(cudaStream_t s, long nlines, const cd* in, cd* out
 // others do not spill (2048: 254 registers).
 template <int N, int CWS>
 inline cudaError_t launch_mid_swap(cudaStream_t s, long nlines, const CUtensorMap& tmA, const CUtensorMap& tmC, cd* C,
-                                   const cd* G, const cd* TAB) {
+                                   const cd* G, const cd* TAB, int ncol = 1, long ccs = 0) {
     constexpr int MINB = GeoA<N>::THREADS > 128 ? 1 : (N <= 256 ? 3 : 2);
     constexpr int smem = (2 * GeoA<N>::LPC * N + EngTab<N>::TW1N) * (int)sizeof(cd) + 8;
     static unsigned long long optin = 0;
     { cudaError_t e = smem_optin(k_mid_swap<N, MINB, CWS>, smem, optin); if (e != cudaSuccess) return e; }
-    k_mid_swap<N, MINB, CWS><<<(unsigned)(nlines / GeoA<N>::LPC), GeoA<N>::THREADS, smem, s>>>(tmA, tmC, C, G, TAB);
+    k_mid_swap<N, MINB, CWS><<<dim3((unsigned)ncol, (unsigned)(nlines / GeoA<N>::LPC)), GeoA<N>::THREADS, smem, s>>>(tmA, tmC, C, ccs, G, TAB);
     return cudaPeekAtLastError();
 }
 
 template <int N, bool B, bool STAGED = false, bool MASK = false>
-inline cudaError_t launch_inv(cudaStream_t s, long nlines, const cd* in, const cd* bsrc, cd* out, const cd* TAB,
-                              double scale, const LineAddr& la) {
+inline cudaError_t launch_inv_cols(cudaStream_t s, long nlines, const ColPtrs& cp, int ncol, const cd* TAB, double scale,
+                                   const LineAddr& la) {
     constexpr int smem = Smem<N, B>::fwd_bytes + (STAGED ? Smem<N, B>::LPC * N * (int)sizeof(cd) : 0);
     constexpr int LPC = Smem<N, B>::LPC, TH = B ? GeoB<N>::THREADS : GeoA<N>::THREADS;
     static unsigned long long optin = 0;
-    { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED, MASK>, smem, optin); if (e != cudaSuccess) return e; }
     const long grid = MASK ? (nlines + LPC - 1) / LPC : nlines / LPC;
-    k_inv_pruned<N, B, STAGED, MASK><<<(unsigned)grid, TH, smem, s>>>(in, bsrc, out, TAB, scale, la, 0);
+    if (ncol == 1) {
+        { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED, MASK>, smem, optin); if (e != cudaSuccess) return e; }
+        k_inv_pruned<N, B, STAGED, MASK><<<(unsigned)grid, TH, smem, s>>>(cp, TAB, scale, la, 0);
+    } else {
+        static unsigned long long optin_cols = 0;
+        { cudaError_t e = smem_optin(k_inv_pruned<N, B, STAGED, MASK, true>, smem, optin_cols); if (e != cudaSuccess) return e; }
+        k_inv_pruned<N, B, STAGED, MASK, true><<<dim3((unsigned)grid, (unsigned)ncol), TH, smem, s>>>(cp, TAB, scale, la, 0);
+    }
     return cudaPeekAtLastError();
+}
+template <int N, bool B, bool STAGED = false, bool MASK = false>
+inline cudaError_t launch_inv(cudaStream_t s, long nlines, const cd* in, const cd* bsrc, cd* out, const cd* TAB,
+                              double scale, const LineAddr& la) {
+    return launch_inv_cols<N, B, STAGED, MASK>(s, nlines, one_col(in, bsrc, out), 1, TAB, scale, la);
 }
 
 }  // namespace lsk

@@ -56,6 +56,31 @@ struct HandleBase {
         return LS_ERR_INVALID;
     }
 
+    // Several columns per apply (ls_op_apply_batch, ls_gmres_batch).  batch_cols: the chunk width of one multi-column
+    // apply (1: the handle serves a batch column by column through apply_dev); batch_bytes: device bytes still to
+    // allocate before a chunk of ncol columns can run; batch_reserve: allocates them; apply_cols_dev: ncol <= the
+    // reserved width columns b[c] -> y[c], each with the bits of apply_dev of that column.
+    virtual int batch_cols() const { return 1; }
+    virtual size_t batch_bytes(int ncol) const { (void)ncol; return 0; }
+    virtual int batch_reserve(int ncol) { (void)ncol; return LS_OK; }
+    virtual int apply_cols_dev(const cd* const* b, cd* const* y, int ncol, int mode) {
+        for (int c = 0; c < ncol; ++c) {
+            int rc = apply_dev(b[c], y[c], mode);
+            if (rc) return rc;
+        }
+        return LS_OK;
+    }
+    // count columns in chunks of batch_cols(); the chunk width must be reserved
+    int apply_list_dev(const cd* const* b, cd* const* y, int count, int mode) {
+        const int w = batch_cols();
+        for (int j = 0; j < count; j += w) {
+            int rc = apply_cols_dev(b + j, y + j, count - j < w ? count - j : w, mode);
+            if (rc) return rc;
+        }
+        return LS_OK;
+    }
+    cd* d_bstage = nullptr; size_t bstage_bytes = 0;   // ls_op_apply_batch with host pointers: one chunk of b and y
+
     // sharded operators expose their communicator so that Krylov reductions can all-reduce on it
     virtual ncclComm_t nccl_comm() const { return nullptr; }
     virtual int dist_rank() const { return 0; }

@@ -36,6 +36,11 @@ namespace {
 constexpr int CW_SHIFT = 2;
 constexpr long CW = 1L << CW_SHIFT;
 
+// columns per multi-column apply (ls_op_apply_batch) of the 2x-padded routes.  Measured on B200 (1000 W,
+// profiles/r5_apply_batch.log, ms per column at K = 1 / 4): 201^2 embedded 0.033 / 0.0093, 2048^2 0.317 / 0.288,
+// 4096^2 1.498 / 1.449; 8 columns (two chunks) are no faster per column than 4.
+constexpr int BATCH_COLS = 4;
+
 struct Op2D : Op2DBase {
     int nr = 4;               // padding factor actually used by the applies (4: literal, 2: compact)
     long pn = 0, pm = 0;      // padded sizes nr*n, nr*m
@@ -47,7 +52,12 @@ struct Op2D : Op2DBase {
     bool embed = false;       // LS_FLAG_EMBED: lines of ln x lm points carry the n x m grid (ln = n, lm = m otherwise)
     long ln = 0, lm = 0;
     CUtensorMap tmA, tmC;     // 2x padding: P2's line loads from A and stores into C (encode_line_maps)
+    int cols = 1;             // columns of A and C (ls_op_apply_batch widens them on first use), pn*lm elements apart
     int apply_dev(const cd* b, cd* y, int mode) override;
+    int batch_cols() const override { return nr == 2 ? BATCH_COLS : 1; }
+    size_t batch_bytes(int ncol) const override { return ncol > cols ? 2 * (size_t)ncol * pn * lm * sizeof(cd) : 0; }
+    int batch_reserve(int ncol) override;
+    int apply_cols_dev(const cd* const* b, cd* const* y, int ncol, int mode) override;
     void info(int* route, int64_t* n_line, int64_t* m_line, int* padding) const override {
         *route = embed ? 2 : 0; *n_line = ln; *m_line = lm; *padding = nr;
     }
@@ -111,18 +121,31 @@ __global__ void k_fill_g2d_centred(cd* __restrict__ gout, long ne, long me, Gv2d
         default: e = cudaErrorInvalidValue;                                        \
     }
 
-int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
+// The pointer lists of the three passes for columns b[c] -> y[c], c < ncol: P1 b -> A, P3 C (and b) -> y.  Column c of A
+// and C starts c*pn*lm elements in.
+void pass_cols(const Op2D* op, const cd* const* b, cd* const* y, int ncol, bool full, ColPtrs& p1, ColPtrs& p3) {
+    p1 = ColPtrs{}; p3 = ColPtrs{};
+    const long cs = op->pn * op->lm;
+    for (int c = 0; c < ncol; ++c) {
+        p1.in[c] = b[c]; p1.out[c] = op->d_A + c * cs;
+        p3.in[c] = op->d_C + c * cs; p3.b[c] = full ? b[c] : nullptr; p3.out[c] = y[c];
+    }
+}
+
+int apply_device(Op2D* op, const cd* const* b, cd* const* y, int ncol, int mode) {
     cudaError_t e = cudaSuccess;
     cudaStream_t s = op->stream;
     const long n = op->n, m = op->m, pn = op->pn;
     const bool full = (mode == LS_APPLY_FASTCONVOLUTION);
     const double* nu = full ? op->d_nu : nullptr;   // Q2: GV FFTconvolution has no nu
+    ColPtrs p1, p3;
+    pass_cols(op, b, y, ncol, full, p1, p3);
     // P1: columns (x, contiguous): point i of column j at b[i + n*j] -> slot sx at A[sx + pn*j]
     {
         LineAddr la{1L << 40, n, 0, 1, pn, 0, 1};
         la.nr = op->nr;
         op->phase_begin(0);
-#define P1(N) launch_fwd<N, false>(s, m, b, nu, op->d_A, op->d_TABn, la)
+#define P1(N) launch_fwd_cols<N, false>(s, m, p1, ncol, nu, op->d_TABn, la)
         LS_DISPATCH_E(n, P1);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -133,7 +156,7 @@ int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
         LineAddr la{CW, 1, CW, pn, 1, CW * m, CW};
         la.nr = op->nr;
         op->phase_begin(1);
-#define P2S(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm)
+#define P2S(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm, ncol, pn * m)
 #define P2F(N) launch_mid<N, false>(s, pn, op->d_A, op->d_C, op->d_G, op->d_TABm, la)
         if (op->nr == 2) { LS_DISPATCH_E(m, P2S); } else { LS_DISPATCH_E(m, P2F); }
         op->phase_end(); op->launches++;
@@ -147,7 +170,7 @@ int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
         la.split_shift = CW_SHIFT; la.split_stride = CW * m;
         la.nr = op->nr;
         op->phase_begin(2);
-#define P3(N) launch_inv<N, false, true>(s, m, op->d_C, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
+#define P3(N) launch_inv_cols<N, false, true>(s, m, p3, ncol, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
         LS_DISPATCH_E(n, P3);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -159,25 +182,27 @@ int apply_device(Op2D* op, const cd* b, cd* y, int mode) {
 // (column stride n) with points >= n and lines >= m as zeros and covers ceil(m / LPC) CTAs; columns [m, lm) of A that
 // P2 reads stay zero from create time.  P3 writes points < n of lines < m only.  Greengard_Vico FFTconvolution has no
 // nu (Q2); the trapezoidal rule applies it in both modes (FastConvolution.jl:122 vs :141).
-int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
+int apply_embedded(Op2D* op, const cd* const* b, cd* const* y, int ncol, int mode) {
     cudaError_t e = cudaSuccess;
     cudaStream_t s = op->stream;
     const long n = op->n, m = op->m, ln = op->ln, lm = op->lm, pn = op->pn;
     const bool full = (mode == LS_APPLY_FASTCONVOLUTION);
     const double* nu = (full || op->quadrule == LS_QUAD_TRAPEZOIDAL) ? op->d_nu : nullptr;
+    ColPtrs p1, p3;
+    pass_cols(op, b, y, ncol, full, p1, p3);
     {
         LineAddr la{1L << 40, n, 0, 1, pn, 0, 1};
         la.nr = 2;
         la.mask_pts = (int16_t)n; la.mask_lines = (int)m;
         op->phase_begin(0);
-#define E1(N) launch_fwd<N, false, true>(s, m, b, nu, op->d_A, op->d_TABn, la)
+#define E1(N) launch_fwd_cols<N, false, true>(s, m, p1, ncol, nu, op->d_TABn, la)
         LS_DISPATCH_E(ln, E1);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
     }
     {
         op->phase_begin(1);
-#define E2(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm)
+#define E2(N) launch_mid_swap<N, CW_SHIFT>(s, pn, op->tmA, op->tmC, op->d_C, op->d_G, op->d_TABm, ncol, pn * lm)
         LS_DISPATCH_E(lm, E2);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -188,7 +213,7 @@ int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
         la.nr = 2;
         la.mask_pts = (int16_t)n; la.mask_lines = (int)m;
         op->phase_begin(2);
-#define E3(N) launch_inv<N, false, true, true>(s, m, op->d_C, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
+#define E3(N) launch_inv_cols<N, false, true, true>(s, m, p3, ncol, op->d_TABn, full ? op->omega * op->omega : 1.0, la)
         LS_DISPATCH_E(ln, E3);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -199,14 +224,21 @@ int apply_embedded(Op2D* op, const cd* b, cd* y, int mode) {
 }  // namespace
 
 int Op2D::apply_dev(const cd* b, cd* y, int mode) {
-    return embed ? apply_embedded(this, b, y, mode) : apply_device(this, b, y, mode);
+    return embed ? apply_embedded(this, &b, &y, 1, mode) : apply_device(this, &b, &y, 1, mode);
+}
+
+int Op2D::apply_cols_dev(const cd* const* b, cd* const* y, int ncol, int mode) {
+    if (nr != 2) return HandleBase::apply_cols_dev(b, y, ncol, mode);     // LS_FLAG_PAD4: column by column
+    LS_REQUIRE(ncol >= 1 && ncol <= cols, LS_ERR_INVALID, "2-D batched apply: %d columns, %d reserved", ncol, cols);
+    return embed ? apply_embedded(this, b, y, ncol, mode) : apply_device(this, b, y, ncol, mode);
 }
 
 namespace {
 
-// The 2x-padded P2 (k_mid_swap) moves its lines by tensor copies.  As FLOAT64 arrays with re, im innermost, line sx of A
-// is the box {2, BOX} at (2 sx, j0) of the 2-D view {2 pn, lm}, and line sx of C the box {2, BOX, 1} at
-// (2 (sx % CW), j0, sx / CW) of the 3-D view {2 CW, lm, pn / CW}, i.e. C[(sx/CW)*(CW*lm) + CW*j + sx%CW].
+// The 2x-padded P2 (k_mid_swap) moves its lines by tensor copies.  As FLOAT64 arrays with re, im innermost, line sx of
+// column c of A is the box {2, BOX, 1} at (2 sx, j0, c) of the 3-D view {2 pn, lm, cols}, and line sx of column c of C
+// the box {2, BOX, 1, 1} at (2 (sx % CW), j0, sx / CW, c) of the 4-D view {2 CW, lm, pn / CW, cols}, i.e.
+// C[c*pn*lm + (sx/CW)*(CW*lm) + CW*j + sx%CW].
 // BOX = min(lm, 256), the largest box side.  cuTensorMapEncodeTiled is reached through the runtime's driver entry point,
 // so the library does not link against libcuda.
 int encode_line_maps(Op2D* op) {
@@ -216,18 +248,20 @@ int encode_line_maps(Op2D* op) {
     LS_REQUIRE(q == cudaDriverEntryPointSuccess && fn, LS_ERR_CUDA, "the driver has no cuTensorMapEncodeTiled");
     const auto encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
     const cuuint64_t pn = (cuuint64_t)op->pn, lm = (cuuint64_t)op->lm;
-    const cuuint32_t box = (cuuint32_t)std::min<long>(op->lm, 256), unit[3] = {1, 1, 1};
-    const cuuint64_t dimA[2] = {2 * pn, lm}, strideA[1] = {pn * sizeof(cd)};
-    const cuuint32_t boxA[2] = {2, box};
-    const cuuint64_t dimC[3] = {2 * CW, lm, pn / CW}, strideC[2] = {CW * sizeof(cd), CW * lm * sizeof(cd)};
-    const cuuint32_t boxC[3] = {2, box, 1};
-    CUresult r = encode(&op->tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, op->d_A, dimA, strideA, boxA, unit,
+    const cuuint64_t cols = (cuuint64_t)op->cols;
+    const cuuint32_t box = (cuuint32_t)std::min<long>(op->lm, 256), unit[4] = {1, 1, 1, 1};
+    const cuuint64_t dimA[3] = {2 * pn, lm, cols}, strideA[2] = {pn * sizeof(cd), pn * lm * sizeof(cd)};
+    const cuuint32_t boxA[3] = {2, box, 1};
+    const cuuint64_t dimC[4] = {2 * CW, lm, pn / CW, cols};
+    const cuuint64_t strideC[3] = {CW * sizeof(cd), CW * lm * sizeof(cd), pn * lm * sizeof(cd)};
+    const cuuint32_t boxC[4] = {2, box, 1, 1};
+    CUresult r = encode(&op->tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, op->d_A, dimA, strideA, boxA, unit,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     const char* which = "A";
     if (r == CUDA_SUCCESS) {
         which = "C";
-        r = encode(&op->tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, op->d_C, dimC, strideC, boxC, unit,
+        r = encode(&op->tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 4, op->d_C, dimC, strideC, boxC, unit,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
@@ -242,6 +276,26 @@ int encode_line_maps(Op2D* op) {
     }
     return LS_OK;
 }
+
+}  // namespace
+
+// A and C for ncol columns: new arrays, zeroed (the embedded route reads columns [m, lm) of A, which P1 never writes),
+// the old ones freed once the stream has drained, the line maps encoded again.  The caller checked the free memory.
+int Op2D::batch_reserve(int ncol) {
+    if (ncol <= cols) return LS_OK;
+    const size_t bytes = (size_t)ncol * pn * lm * sizeof(cd);
+    cd *a = nullptr, *c = nullptr;
+    int rc;
+    if ((rc = dmalloc((void**)&a, bytes))) return rc;
+    if ((rc = dmalloc((void**)&c, bytes))) { dfree(a); return rc; }
+    LS_CUDA_TRY(cudaMemsetAsync(a, 0, bytes, stream));
+    LS_CUDA_TRY(cudaStreamSynchronize(stream));
+    dfree(d_A); dfree(d_C);
+    d_A = a; d_C = c; cols = ncol;
+    return encode_line_maps(this);
+}
+
+namespace {
 
 // G2 = fft2(g2) / (2n 2m) in the slot order of the nr = 2 kernels (n, m: the line lengths, powers of two).
 // g2[jx2 + 2n*jy2]: the spatial kernel with its lags wrapped onto the 2n x 2m grid (negative lags at the end).

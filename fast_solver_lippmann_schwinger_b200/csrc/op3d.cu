@@ -38,6 +38,12 @@ using namespace lsk;
 
 namespace {
 
+// columns per multi-column apply (ls_op_apply_batch) of the single-GPU 2x-padded routes.  Measured on B200 (1000 W,
+// profiles/r5_apply_batch.log, ms per column at K = 1 / 4): 48^3 embedded 0.045 / 0.028, 64^3 0.048 / 0.032, 256^3
+// 2.03 / 1.94; at 512^3 20.1 / 19.9 lies inside the run-to-run spread (19.3 - 20.3) while the three extra columns
+// would hold 38 GB of work arrays, so grids with 512-point lines go column by column.
+constexpr int BATCH_COLS3 = 4;
+
 struct Op3D : HandleBase {
     long n = 0, m = 0, l = 0, ne = 0, me = 0, le = 0;
     // LS_FLAG_EMBED: lines of ln x lm x ll points carry the n x m x l grid (ln = n, lm = m, ll = l otherwise)
@@ -80,6 +86,14 @@ struct Op3D : HandleBase {
     std::vector<cudaEvent_t> evIn, evOut;
     int64_t op_size() const override { return n * m * lloc; }
     int apply_dev(const cd* b, cd* y, int mode) override;
+    // ls_op_apply_batch: A1 and A2 hold `cols` columns, a1cs / a2cs elements apart (single GPU, 2x padding)
+    int cols = 1;
+    long a1cs() const { return pn * m * lloc; }
+    long a2cs() const { return nelc * pm * ll; }
+    int batch_cols() const override { return (P == 1 && nr == 2 && ln < 512 && ll < 512) ? BATCH_COLS3 : 1; }
+    size_t batch_bytes(int ncol) const override { return ncol > cols ? (size_t)ncol * (a1cs() + a2cs()) * sizeof(cd) : 0; }
+    int batch_reserve(int ncol) override;
+    int apply_cols_dev(const cd* const* b, cd* const* y, int ncol, int mode) override;
     ncclComm_t nccl_comm() const override { return comm; }
     int dist_rank() const override { return rank; }
     int dist_size() const override { return P; }
@@ -263,7 +277,8 @@ int setup_ce_exchange(Op3D* op) {
     return LS_OK;
 }
 
-int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
+// b[c] -> y[c], c < ncol (ncol = 1 unless single GPU): column c of A1 / A2 starts c*a1cs / c*a2cs elements in
+int apply_device3(Op3D* op, const cd* const* b, cd* const* y, int ncol, int mode) {
     cudaError_t e = cudaSuccess;
     cudaStream_t s = op->stream, sc = op->cstream;
     const long n = op->n, m = op->m, l = op->l, me = op->pm, nel = op->nel, lloc = op->lloc, nelc = op->nelc;
@@ -276,6 +291,7 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
     int shc = 0, shr = 0;
     while ((1L << shc) < nelc) ++shc;
     while ((1L << shr) < nel) ++shr;
+    const long a1cs = op->a1cs(), a2cs = op->a2cs();
     // P1: x lines (j, p_loc): in b[n*line + i]; slot sx -> rank q = sx/nel, chunk c = (sx%nel)/nelc:
     //     A1[c*cstride + q*blk + nelc*line + sx%nelc]
     //     embed: m*lloc need not fill the last CTA; its surplus lines wrap (ldim0) onto lines 0.. and write the same bits
@@ -284,9 +300,11 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
         LineAddr la{1L << 40, n, 0, 1, nelc, 0, 1};
         la.split_shift = shc; la.split_stride = cstride; la.split2_shift = shr; la.split2_stride = blk; la.nr = nr;
         if (embed) { la.ldim0 = m * lloc; la.mask_pts = (int16_t)n; la.mask_lines = INT_MAX; }
+        ColPtrs cp{};
+        for (int c = 0; c < ncol; ++c) { cp.in[c] = b[c]; cp.out[c] = op->d_A1 + c * a1cs; }
         op->phase_begin(0);
-#define C1(N) (embed ? launch_fwd<N, false, true>(s, m * lloc, b, full ? op->d_nu : nullptr, op->d_A1, op->d_TABn, la) \
-                     : launch_fwd<N, false>(s, m * lloc, b, full ? op->d_nu : nullptr, op->d_A1, op->d_TABn, la))
+#define C1(N) (embed ? launch_fwd_cols<N, false, true>(s, m * lloc, cp, ncol, full ? op->d_nu : nullptr, op->d_TABn, la) \
+                     : launch_fwd_cols<N, false>(s, m * lloc, cp, ncol, full ? op->d_nu : nullptr, op->d_TABn, la))
         LS3_DISPATCH(ln, C1);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -315,8 +333,10 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             LineAddr la{nelc, 1, nelc * m, nelc, 1, nelc * me, nelc};
             la.nr = nr;
             if (embed) { la.mask_pts = (int16_t)m; la.mask_lines = (int)(nelc * l); }
-#define C2(N) (embed ? launch_fwd<N, true, true>(s, nelc * ll, a1t, nullptr, op->d_A2, op->d_TABm, la) \
-                     : launch_fwd<N, true>(s, nelc * l, a1t, nullptr, op->d_A2, op->d_TABm, la))
+            ColPtrs cp{};
+            for (int c = 0; c < ncol; ++c) { cp.in[c] = a1t + c * a1cs; cp.out[c] = op->d_A2 + c * a2cs; }
+#define C2(N) (embed ? launch_fwd_cols<N, true, true>(s, nelc * ll, cp, ncol, nullptr, op->d_TABm, la) \
+                     : launch_fwd_cols<N, true>(s, nelc * l, cp, ncol, nullptr, op->d_TABm, la))
             op->phase_begin(1);
             LS3_DISPATCH(lm, C2);
             op->phase_end(); op->launches++;
@@ -327,7 +347,7 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             LineAddr la{1L << 40, 1, 0, nelc * me, 1, 0, nelc * me};
             la.nr = nr;
             op->phase_begin(2);
-#define C3(N) launch_mid<N, true>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la)
+#define C3(N) launch_mid<N, true>(s, nelc * me, op->d_A2, op->d_A2, Gc, op->d_TABl, la, ncol, a2cs)
             LS3_DISPATCH(ll, C3);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
@@ -339,9 +359,11 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
             LineAddr la{nelc, 1, nelc * me, nelc, 1, nelc * m, nelc};
             la.nr = nr;
             if (embed) { la.mask_pts = (int16_t)m; la.mask_lines = (int)(nelc * l); }
+            ColPtrs cp{};
+            for (int c = 0; c < ncol; ++c) { cp.in[c] = op->d_A2 + c * a2cs; cp.out[c] = c1t + c * a1cs; }
             op->phase_begin(3);
-#define C4(N) (embed ? launch_inv<N, true, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la) \
-                     : launch_inv<N, true, true>(s, nelc * l, op->d_A2, nullptr, c1t, op->d_TABm, 1.0, la))
+#define C4(N) (embed ? launch_inv_cols<N, true, true, true>(s, nelc * l, cp, ncol, op->d_TABm, 1.0, la) \
+                     : launch_inv_cols<N, true, true>(s, nelc * l, cp, ncol, op->d_TABm, 1.0, la))
             LS3_DISPATCH(lm, C4);
             op->phase_end(); op->launches++;
             LS_CUDA_TRY(e);
@@ -366,9 +388,11 @@ int apply_device3(Op3D* op, const cd* b, cd* y, int mode) {
         LineAddr la{1L << 40, nelc, 0, 1, n, 0, 1};
         la.split_shift = shc; la.split_stride = cstride; la.split2_shift = shr; la.split2_stride = blk; la.nr = nr;
         if (embed) { la.ldim0 = m * lloc; la.mask_pts = (int16_t)n; la.mask_lines = (int)(m * lloc); }
+        ColPtrs cp{};
+        for (int c = 0; c < ncol; ++c) { cp.in[c] = op->d_A1 + c * a1cs; cp.b[c] = full ? b[c] : nullptr; cp.out[c] = y[c]; }
         op->phase_begin(4);
-#define C5(N) (embed ? launch_inv<N, false, true, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la) \
-                     : launch_inv<N, false, true>(s, m * lloc, op->d_A1, full ? b : nullptr, y, op->d_TABn, full ? op->omega * op->omega : 1.0, la))
+#define C5(N) (embed ? launch_inv_cols<N, false, true, true>(s, m * lloc, cp, ncol, op->d_TABn, full ? op->omega * op->omega : 1.0, la) \
+                     : launch_inv_cols<N, false, true>(s, m * lloc, cp, ncol, op->d_TABn, full ? op->omega * op->omega : 1.0, la))
         LS3_DISPATCH(ln, C5);
         op->phase_end(); op->launches++;
         LS_CUDA_TRY(e);
@@ -740,7 +764,28 @@ int create3d(ls_handle* out, int64_t n, int64_t m, int64_t l, int64_t ne, int64_
 
 }  // namespace
 
-int Op3D::apply_dev(const cd* b, cd* y, int mode) { return apply_device3(this, b, y, mode); }
+int Op3D::apply_dev(const cd* b, cd* y, int mode) { return apply_device3(this, &b, &y, 1, mode); }
+
+int Op3D::apply_cols_dev(const cd* const* b, cd* const* y, int ncol, int mode) {
+    if (P != 1 || nr != 2) return HandleBase::apply_cols_dev(b, y, ncol, mode);     // column by column
+    LS_REQUIRE(ncol >= 1 && ncol <= cols, LS_ERR_INVALID, "3-D batched apply: %d columns, %d reserved", ncol, cols);
+    return apply_device3(this, b, y, ncol, mode);
+}
+
+// A1 and A2 for ncol columns: new arrays, the old ones freed once the stream has drained.  Every pass writes what the
+// next one reads (the embedded P2 writes the zero planes P3 transforms), so the new arrays need no initialisation.
+// The caller checked the free memory.
+int Op3D::batch_reserve(int ncol) {
+    if (ncol <= cols) return LS_OK;
+    cd *a1 = nullptr, *a2 = nullptr;
+    int rc;
+    if ((rc = dmalloc((void**)&a1, (size_t)ncol * a1cs() * sizeof(cd)))) return rc;
+    if ((rc = dmalloc((void**)&a2, (size_t)ncol * a2cs() * sizeof(cd)))) { dfree(a1); return rc; }
+    LS_CUDA_TRY(cudaStreamSynchronize(stream));
+    dfree(d_A1); dfree(d_A2);
+    d_A1 = a1; d_A2 = a2; cols = ncol;
+    return LS_OK;
+}
 
 extern "C" {
 

@@ -305,11 +305,12 @@ def gmres_(x, A, b, Pl=None, abstol=0.0, reltol=None, restart=None, maxiter=None
 
 
 def _gmres_batch(x, A, b, Pl, abstol, reltol, restart, maxiter, log, initially_zero, workspace, orth_meth):
-    """gmres_ with an N x K right-hand side: K independent GMRES runs in lockstep (ls_gmres_msp_batch) sharing A and the
-    device preconditioner; x (N x K) is updated in place and log=True returns one ConvergenceHistory per column."""
+    """gmres_ with an N x K right-hand side: K independent GMRES runs in lockstep sharing A (ls_gmres_batch with
+    Pl=None, ls_gmres_msp_batch with the device preconditioner); x (N x K) is updated in place and log=True returns one
+    ConvergenceHistory per column."""
     N = A.size(1)
-    if Pl is None or getattr(Pl, "MspGPU", None) is None:
-        raise _lib.LSUnsupported(_lib.LS_ERR_UNSUPPORTED, "gmres!: several right-hand sides need Pl with solverType='GPU'")
+    if Pl is not None and getattr(Pl, "MspGPU", None) is None:
+        raise _lib.LSUnsupported(_lib.LS_ERR_UNSUPPORTED, "gmres!: several right-hand sides need Pl=None or Pl with solverType='GPU'")
     if orth_meth != "ModifiedGramSchmidt":
         raise _lib.LSUnsupported(_lib.LS_ERR_UNSUPPORTED, "gmres!: several right-hand sides run ModifiedGramSchmidt")
     if b.shape[0] != N or b.shape[1] < 1:
@@ -329,10 +330,15 @@ def _gmres_batch(x, A, b, Pl, abstol, reltol, restart, maxiter, log, initially_z
     niter = np.zeros(K, dtype=np.int64)
     conv = np.zeros(K, dtype=np.int32)
     mv = np.zeros(K, dtype=np.int64)
-    as_h = Pl.As.handle if Pl.As is not None else None
-    check(lib().ls_gmres_msp_batch(ws.handle, A.handle, as_h, Pl.MspGPU.handle, K, ptr(B), N, ptr(X), N, restart, maxiter,
-                                   reltol, float(abstol), 1 if initially_zero else 0, ptr(hist), max(cap, 1), ptr(niter),
-                                   ptr(conv), ptr(mv), _lib.MEM_HOST))
+    if Pl is None:
+        check(lib().ls_gmres_batch(ws.handle, A.handle, K, ptr(B), N, ptr(X), N, restart, maxiter, reltol, float(abstol),
+                                   1 if initially_zero else 0, ptr(hist), max(cap, 1), ptr(niter), ptr(conv), ptr(mv),
+                                   _lib.MEM_HOST))
+    else:
+        as_h = Pl.As.handle if Pl.As is not None else None
+        check(lib().ls_gmres_msp_batch(ws.handle, A.handle, as_h, Pl.MspGPU.handle, K, ptr(B), N, ptr(X), N, restart,
+                                       maxiter, reltol, float(abstol), 1 if initially_zero else 0, ptr(hist), max(cap, 1),
+                                       ptr(niter), ptr(conv), ptr(mv), _lib.MEM_HOST))
     if X is not x:
         x[...] = X
     if not log:

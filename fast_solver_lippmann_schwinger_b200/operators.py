@@ -86,6 +86,45 @@ def _as_c128(b, N, name="b"):
     return np.ascontiguousarray(b)
 
 
+def _apply_cols(M, B, out, mode):
+    """The columns of an (N, K) complex128 array through one ls_op_apply_batch (each column with the bits of the single
+    apply of it); out, when given, is an (N, K) complex128 array that receives them."""
+    if B.dtype != np.complex128:
+        raise TypeError("b must be complex128 (Julia: Array{Complex{Float64},2}), got %s" % B.dtype)
+    if B.shape[0] != M.N or B.shape[1] < 1:
+        raise ValueError("DimensionMismatch: b has shape %s, operator needs (%d, K)" % (B.shape, M.N))
+    K = B.shape[1]
+    Bf = np.asfortranarray(B)
+    if out is None:
+        out = np.empty((M.N, K), dtype=np.complex128, order="F")
+    elif not (isinstance(out, np.ndarray) and out.dtype == np.complex128 and out.shape == B.shape):
+        raise ValueError("DimensionMismatch: Y must be a complex128 array of shape %s" % (B.shape,))
+    Y = out if out.flags.f_contiguous else np.empty((M.N, K), dtype=np.complex128, order="F")
+    check(lib().ls_op_apply_batch(M.handle, ptr(Bf), M.N, ptr(Y), M.N, K, mode, _lib.MEM_HOST))
+    if Y is not out:
+        out[...] = Y
+    return out
+
+
+def apply_batch(M, b, y, nrhs, ldb=None, ldy=None, mode=_lib.APPLY_FASTCONVOLUTION):
+    """ls_op_apply_batch on device memory: b and y are DeviceBuffers holding nrhs columns of M's N unknowns, column j at
+    j*ldb (j*ldy) elements (default N); y may be b for an in-place apply."""
+    if not (isinstance(b, DeviceBuffer) and isinstance(y, DeviceBuffer)):
+        raise TypeError("b and y must be DeviceBuffers (numpy arrays go through M * B)")
+    N = M.N
+    ldb = N if ldb is None else int(ldb)
+    ldy = N if ldy is None else int(ldy)
+    check(lib().ls_op_apply_batch(M.handle, ptr(b), ldb, ptr(y), ldy, int(nrhs), mode, _lib.MEM_DEVICE))
+    return y
+
+
+def batch_cols(M):
+    """ls_op_batch_cols: the columns M applies per multi-column launch (1: column by column)."""
+    c = C.c_int()
+    check(lib().ls_op_batch_cols(M.handle, C.byref(c)))
+    return int(c.value)
+
+
 class FastM(_Handle):
     """``struct FastM`` (FastConvolution.jl:11-27) with the apply on the GPU.
 
@@ -154,6 +193,8 @@ class FastM(_Handle):
                 raise TypeError("b and out must both be DeviceBuffer or both numpy arrays")
             check(lib().ls_op2d_apply(self.handle, ptr(b), ptr(out), mode, _lib.MEM_DEVICE))
             return out
+        if isinstance(b, np.ndarray) and b.ndim == 2:
+            return _apply_cols(self, b, out, mode)
         b = _as_c128(b, self.N)
         if out is None:
             out = np.empty(self.N, dtype=np.complex128)
@@ -168,7 +209,7 @@ class FastM(_Handle):
 
     def mul_(self, Y, b):
         """``LinearAlgebra.mul!(Y, M, b)`` FastConvolution.jl:50-54 (Y[:] = M*b)."""
-        if isinstance(Y, DeviceBuffer):
+        if isinstance(Y, DeviceBuffer) or (isinstance(b, np.ndarray) and b.ndim == 2):
             return self._apply(b, Y, _lib.APPLY_FASTCONVOLUTION)
         if not (isinstance(Y, np.ndarray) and Y.dtype == np.complex128 and Y.shape == (self.N,)):
             raise ValueError("DimensionMismatch: Y must be a complex128 vector of length %d" % self.N)
@@ -240,6 +281,8 @@ class FastM3D(_Handle):
                 raise TypeError("b and out must both be DeviceBuffer or both numpy arrays")
             check(lib().ls_op3d_apply(self.handle, ptr(b), ptr(out), mode, _lib.MEM_DEVICE))
             return out
+        if isinstance(b, np.ndarray) and b.ndim == 2:
+            return _apply_cols(self, b, out, mode)
         b = _as_c128(b, self.N)
         if out is None:
             out = np.empty(self.N, dtype=np.complex128)
@@ -253,6 +296,8 @@ class FastM3D(_Handle):
     __matmul__ = __mul__
 
     def mul_(self, Y, b):
+        if isinstance(b, np.ndarray) and b.ndim == 2:
+            return self._apply(b, Y, _lib.APPLY_FASTCONVOLUTION)
         if isinstance(Y, DeviceBuffer) or (isinstance(Y, np.ndarray) and Y.flags.c_contiguous and Y.dtype == np.complex128
                                            and Y.shape == (self.N,)):
             return self._apply(b, Y, _lib.APPLY_FASTCONVOLUTION)

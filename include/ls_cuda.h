@@ -141,6 +141,22 @@ int ls_op3d_lines(ls_handle h, int* route, int64_t* n_line, int64_t* m_line, int
  * mode 1: FFTconvolution(M, b)                                      (FastConvolution3D.jl:39-63) */
 int ls_op3d_apply(ls_handle h, const ls_cdouble* b, ls_cdouble* y, int mode, int memloc);
 
+/* ---- several right-hand sides through one operator ------------------------------------------ *
+ * Y[:, j] = M*B[:, j] (mode 0) or FFTconvolution(M, B[:, j]) (mode 1) for j < nrhs: b and y are column-major N x nrhs
+ * arrays (leading dimensions ldb, ldy >= N); y may alias b only in place (y == b, ldy == ldb).  Any single-GPU 2-D or
+ * 3-D operator handle; every column gets the bits of ls_op2d_apply / ls_op3d_apply of it.  The 2x-padded power-of-two
+ * routes (route 0 and 2 of ls_op2d_info / ls_op3d_lines) run ls_op_batch_cols columns per launch of each pass, so that
+ * the pass that reads the Green's spectrum reads each part of it from HBM once per chunk of columns; every other handle
+ * applies the columns one by one.  The work arrays of the extra columns (64 N bytes per column in 2-D, 96 N in 3-D; with
+ * host pointers also 32 N of staging) are allocated on first use, kept by the handle and freed by ls_destroy; too
+ * little free device memory -> LS_ERR_NOMEM before anything is allocated.  nrhs < 1, ld < N, a null pointer, an overlap
+ * other than in place or a handle that is not an operator -> LS_ERR_INVALID, a sharded operator (ls_op3d_create_dist)
+ * -> LS_ERR_UNSUPPORTED, both before any CUDA call.                                                                    */
+int ls_op_apply_batch(ls_handle op, const ls_cdouble* b, int64_t ldb, ls_cdouble* y, int64_t ldy, int nrhs, int mode,
+                      int memloc);
+/* columns per multi-column apply of the handle (1: ls_op_apply_batch applies its columns one by one) */
+int ls_op_batch_cols(ls_handle op, int* cols);
+
 /* ---- sparsifying matrix As: SparseMatrixCSC{ComplexF64,Int64}, preconditioner.jl:27-30 ------ *
  * Arrays exactly as Julia holds them (A.colptr, A.rowval, A.nzval; 1-based).  Converted once
  * to CSR/int32 on the device.                                                              */
@@ -244,8 +260,8 @@ int ls_gmres_msp(ls_handle krylov, ls_handle op, ls_handle As, ls_handle msp,
  * column-major N x nrhs arrays (leading dimensions ldb, ldx >= N), resnorm_hist is hist_cap x nrhs (column q: system q's
  * history), niter / converged / mv_products hold nrhs entries (each pointer nullable).  Each system keeps its own Krylov
  * basis, Hessenberg matrix, restarts and tolerance and gets the bits ls_gmres_msp gives it alone; per lockstep iteration
- * the applies, SpMVs and Gram-Schmidt steps run system by system and the Msp^-1 of all active systems is one
- * ls_msp_solve_batch.  A system that converged or reached maxiter drops out; its x is formed as ls_gmres_msp forms it.
+ * the operator applies of all active systems are ls_op_apply_batch chunks, the SpMVs and Gram-Schmidt steps run system
+ * by system and the Msp^-1 of all active systems is one ls_msp_solve_batch.  A system that converged or reached maxiter drops out; its x is formed as ls_gmres_msp forms it.
  * Memory for nrhs bases of restart + 1 vectors (and the batched solve's work arrays) is checked against the free device
  * memory before anything is allocated -> LS_ERR_NOMEM; nrhs < 1, ld < N, null pointers -> LS_ERR_INVALID before any
  * CUDA call; a sharded operator -> LS_ERR_UNSUPPORTED.                                                               */
@@ -253,6 +269,13 @@ int ls_gmres_msp_batch(ls_handle krylov, ls_handle op, ls_handle As, ls_handle m
                        const ls_cdouble* b, int64_t ldb, ls_cdouble* x, int64_t ldx, int restart, int64_t maxiter,
                        double reltol, double abstol, int initially_zero, double* resnorm_hist, int64_t hist_cap,
                        int64_t* niter, int* converged, int64_t* mv_products, int memloc);
+/* nrhs independent ls_gmres runs with Pl = Identity side by side with one op (several incident fields without a
+ * preconditioner); arguments as ls_gmres_msp_batch without As and msp.  Each system gets the bits ls_gmres (no As, no
+ * callback) gives it alone; per lockstep iteration the operator applies of all active systems are ls_op_apply_batch
+ * chunks and the Gram-Schmidt steps run system by system.  Same memory check and refusals as ls_gmres_msp_batch.     */
+int ls_gmres_batch(ls_handle krylov, ls_handle op, int nrhs, const ls_cdouble* b, int64_t ldb, ls_cdouble* x, int64_t ldx,
+                   int restart, int64_t maxiter, double reltol, double abstol, int initially_zero, double* resnorm_hist,
+                   int64_t hist_cap, int64_t* niter, int* converged, int64_t* mv_products, int memloc);
 /* wall time the last ls_gmres spent in D2H + msp_solve callback + H2D (the "Msp-solve" column of SURVEY.md H1) */
 int ls_krylov_last_precond_host_seconds(ls_handle krylov, double* seconds);
 

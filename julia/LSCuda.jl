@@ -110,6 +110,17 @@ FFTconvolution(M::GPUFastM, b::Vector{ComplexF64}) = apply!(similar(b), M, b, 1)
 *(M::GPUFastM, b::AbstractVector{ComplexF64}) = fastconvolution(M, b)                                   # :43-48
 mul!(Y::AbstractVector{ComplexF64}, M::GPUFastM, b::AbstractVector{ComplexF64}) = apply!(Y, M, b, 0)    # :50-54
 
+# several right-hand sides: the N x K columns through one ls_op_apply_batch (each column with the bits of the single apply)
+function apply!(Y::Matrix{ComplexF64}, M, B::Matrix{ComplexF64}, mode::Integer)
+    size(Y) == size(B) && size(B, 1) == length(M.nu) || throw(DimensionMismatch("B is $(size(B)), Y is $(size(Y))"))
+    N, K = size(B)
+    check(ccall((:ls_op_apply_batch, libls), Cint, (Ptr{Cvoid}, Ptr{ComplexF64}, Int64, Ptr{ComplexF64}, Int64, Cint, Cint, Cint),
+                M.h.ptr, B, N, Y, N, K, mode, LS_MEM_HOST))
+    return Y
+end
+*(M::GPUFastM, B::Matrix{ComplexF64}) = apply!(similar(B), M, B, 0)
+mul!(Y::Matrix{ComplexF64}, M::GPUFastM, B::Matrix{ComplexF64}) = apply!(Y, M, B, 0)
+
 # -------------------------------------------------------------------------------- FastM3D (3-D)
 struct GPUFastM3D
     h::Handle
@@ -143,6 +154,8 @@ end
 *(M::GPUFastM3D, b::Array{ComplexF64,1}; verbose::Bool=false) = apply!(similar(b), M, b, 0)     # FastConvolution3D.jl:31-37
 FFTconvolution(M::GPUFastM3D, b::Array{ComplexF64,1}; verbose::Bool=false) = apply!(similar(b), M, b, 1)   # :39-63
 mul!(Y::AbstractVector{ComplexF64}, M::GPUFastM3D, b::AbstractVector{ComplexF64}) = apply!(Y, M, b, 0)
+*(M::GPUFastM3D, B::Matrix{ComplexF64}) = apply!(similar(B), M, B, 0)
+mul!(Y::Matrix{ComplexF64}, M::GPUFastM3D, B::Matrix{ComplexF64}) = apply!(Y, M, B, 0)
 
 # ---------------------------------------------------- FastM3D slab-decomposed over several GPUs
 # One Julia process per GPU (Distributed.jl / MPI.jl).  Rank 0 calls nccl_unique_id() and broadcasts the
@@ -323,26 +336,36 @@ end
 """
     gmres_gpu!(X::Matrix, A, B::Matrix; Pl, abstol, reltol, restart, maxiter, log, initially_zero)
 
-K independent gmres! runs for the columns of B (several incident fields) in lockstep on the device
-(ls_gmres_msp_batch): Pl must be built with solverType = "GPU"; each system gets the history and x that
-gmres_gpu! gives it alone, and the Msp^-1 of all active systems is one batched solve per iteration.
+K independent gmres! runs for the columns of B (several incident fields) in lockstep on the device: with Pl = I
+(ls_gmres_batch) or with Pl built with solverType = "GPU" (ls_gmres_msp_batch); each system gets the history and x that
+gmres_gpu! gives it alone, the operator applies of all active systems are multi-column applies and, with Pl, the
+Msp^-1 of all active systems is one batched solve per iteration.
 With log = true the second result is a vector of K histories.
 """
-function gmres_gpu!(X::Matrix{ComplexF64}, A, B::Matrix{ComplexF64}; Pl, abstol=0.0, reltol=sqrt(eps(Float64)),
+function gmres_gpu!(X::Matrix{ComplexF64}, A, B::Matrix{ComplexF64}; Pl=I, abstol=0.0, reltol=sqrt(eps(Float64)),
                     restart=min(20, size(B, 1)), maxiter=size(B, 1), log=false, initially_zero=false)
     N, K = size(B)
     size(X) == (N, K) || throw(DimensionMismatch("X is $(size(X)), B is $(size(B))"))
-    Pl.MspInv isa GPUMspFactorization || throw(ArgumentError("several right-hand sides need Pl with solverType = \"GPU\""))
+    Pl === I || Pl.MspInv isa GPUMspFactorization ||
+        throw(ArgumentError("several right-hand sides need Pl = I or Pl with solverType = \"GPU\""))
     kh = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:ls_krylov_create, libls), Cint, (Ref{Ptr{Cvoid}}, Int64), kh, N))
     W = Handle(kh[])
     cap = min(maxiter, 1_000_000)                 # history rows kept, as in the Python mirror
     hist = zeros(Float64, cap, K); niter = zeros(Int64, K); conv = zeros(Cint, K); mv = zeros(Int64, K)
+    if Pl === I
+        check(ccall((:ls_gmres_batch, libls), Cint,
+            (Ptr{Cvoid}, Ptr{Cvoid}, Cint, Ptr{ComplexF64}, Int64, Ptr{ComplexF64}, Int64, Cint, Int64,
+             Float64, Float64, Cint, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Cint}, Ptr{Int64}, Cint),
+            W.ptr, A.h.ptr, K, B, N, X, N, restart, maxiter, reltol, abstol, initially_zero, hist, cap, niter, conv, mv,
+            LS_MEM_HOST))
+    else
     check(ccall((:ls_gmres_msp_batch, libls), Cint,
         (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Cint, Ptr{ComplexF64}, Int64, Ptr{ComplexF64}, Int64, Cint, Int64,
          Float64, Float64, Cint, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Cint}, Ptr{Int64}, Cint),
         W.ptr, A.h.ptr, Pl.As.h.ptr, Pl.MspInv.h.ptr, K, B, N, X, N, restart, maxiter,
         reltol, abstol, initially_zero, hist, cap, niter, conv, mv, LS_MEM_HOST))
+    end
     log || return X
     return X, [(resnorm=hist[1:min(niter[q], cap), q], iters=niter[q], isconverged=conv[q] != 0, mvps=mv[q]) for q in 1:K]
 end
